@@ -1,5 +1,5 @@
 #!/usr/bin/env python
-"""Benchmark of the cosmogp GP hot path on B200 (contract: see the task statement).
+"""Benchmark of the cosmogp GP hot path on B200.
 
 Workload (BASELINE.json configs[1], "C2"): 10^5 synthetic light curves x 60 epochs with a
 shared mean function.  One STEP = one pass of the hot path over the batch:
@@ -8,7 +8,11 @@ shared mean function.  One STEP = one pass of the hot path over the batch:
   variance on a shared 100-point grid (:270-361; grid of the multi-object notebook cell 22).
 metric = objects put through LL+predict per second ("fits/s"), whole job.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--objects B]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--objects B] [--dump-outputs DIR]
+
+--dump-outputs DIR writes what the last timed step computed as DIR/<name>.npy (float64): ll (k,), mean and var (k, 100)
+of k = min(objects, 32768) objects, a fixed seeded sample, and their indices in objects.npy.  The inputs are seeded,
+so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -29,6 +33,7 @@ HYP = (0.5, 2.0)
 NUGGET = 0.0
 YERR = 0.2
 N_CHECK = 32            # objects per rank whose timed-step outputs are checked against the oracle
+DUMP_OBJECTS = 32768    # --dump-outputs: 202 doubles per object (index, ll, mean and var on the grid), 53 MB in all
 
 
 def flops_ll(n):            # SURVEY.md section 8(d): build + POTRF + forward solve + norms
@@ -60,6 +65,20 @@ def make_c2(n_obj, seed):
         y[s:e] = spline(xs) + rng.normal(0, 0.3, (e - s, 1)) + (low @ z)[:, :, 0]
     ye = np.full((n_obj, N_EPOCH), YERR)
     return x, y, ye, tmean, ymean
+
+
+def dump_outputs(path, ll, mean, var):
+    """Write one step's outputs (device tensors: ll (B,), mean and var (B * M_GRID,)) for all objects, or for a sample of
+    DUMP_OBJECTS of them drawn from a fixed seed, as path/<name>.npy in float64."""
+    import torch
+    b = ll.shape[0]
+    idx = np.arange(b) if b <= DUMP_OBJECTS else np.sort(np.random.default_rng(0).choice(b, DUMP_OBJECTS, replace=False))
+    sel = torch.from_numpy(idx).to(ll.device)
+    arrays = {"objects": idx.astype(np.float64), "ll": ll[sel].cpu().numpy(),
+              "mean": mean.view(b, M_GRID)[sel].cpu().numpy(), "var": var.view(b, M_GRID)[sel].cpu().numpy()}
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
 
 
 class ClockSampler(threading.Thread):
@@ -331,7 +350,9 @@ def run_c5(args, rank, world, local):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20,
+                    help="timed steps of the headline measurement (the ll_evaluation leg runs max(5, K) calls, the e2e leg "
+                         "max(3, min(K, 10)) steps)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours")
     ap.add_argument("--objects", type=int, default=100000, help="objects per GPU (weak scaling) or in total (strong)")
@@ -340,7 +361,13 @@ def main():
     ap.add_argument("--workload", default="c2", choices=["c2", "c5"])
     ap.add_argument("--cpu-objects", type=int, default=0, help="objects per CPU baseline pass")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last step's ll, mean and var (rank 0's objects) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.workload != "c2"):
+        ap.error("--dump-outputs writes the outputs of the C2 workload of the GPU implementation")
     args.warmup = max(args.warmup, 3) if args.impl != "reference" else args.warmup
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -425,6 +452,8 @@ def main():
            "var": out[2][:N_CHECK * M_GRID].cpu().numpy().reshape(N_CHECK, M_GRID)}
     rel = lambda a, b: float(np.max(np.abs(a - b) / np.abs(b)))
     parity = max(rel(chk["ll"], ll_o), rel(chk["mean"], mean_o), rel(chk["var"], var_o))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *out)
 
     # the likelihood evaluation alone, as the optimiser drives it: the compact LL kernel (its own factorisation, rows retired)
     # + the device reduction + 16 bytes back; kernel time by CUDA events, wall time of the whole call

@@ -69,27 +69,57 @@ def test_shard_ranges_cover_and_balance():
 
 
 def test_reference_arm_times_the_unmodified_reference():
-    """`bench.py --impl reference` (the CPU arm the driver runs): a JSON line with impl == "reference" whose cpu_baseline
-    says kind == "reference" when baseline/_ref (or /root/reference) is present -- i.e. the numbers come from the
-    reference's own code, not from the oracle port."""
-    import json, os, subprocess, sys
+    """`bench.py --impl reference` (the CPU arm): a JSON line with impl == "reference" whose cpu_baseline says
+    kind == "reference" exactly when the reference is installed (baseline/_ref, by baseline/fetch_ref.py) -- i.e. the
+    numbers then come from the reference's own code -- and kind == "port" (the oracle restatement) otherwise."""
+    import importlib.util, json, os, subprocess, sys
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     from oracle import ref_loader
-    if not ref_loader.available():
-        import pytest
-        pytest.skip("no reference tree (baseline/_ref is installed by baseline/fetch_ref.py)")
     out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "0",
                           "--cpu-objects", "32"], capture_output=True, text=True, timeout=300)
     assert out.returncode == 0, out.stderr[-2000:]
     line = json.loads(out.stdout.strip().splitlines()[-1])
-    assert line["impl"] == "reference" and line["cpu_baseline"]["kind"] == "reference" and line["value"] > 0
+    kind = "reference" if ref_loader.available() else "port"
+    assert line["impl"] == "reference" and line["cpu_baseline"]["kind"] == kind and line["value"] > 0
     assert line["metric"] == "gp_fits_per_sec" and line["unit"] == "objects/s" and line["gpu_launches"] == 0
     assert line["e2e"]["h2d_bytes_per_step"] == 0 and line["cpu_baseline"]["svd_method_true"]["value"] > 0
-    # the installed copy under baseline/_ref is byte-identical to the reference tree when both are present
-    ref_root, inst = "/root/reference/cosmogp", os.path.join(root, "baseline", "_ref", "cosmogp")
+    # the installed copy under baseline/_ref is byte-identical to the source tree it was installed from when both are present
+    spec = importlib.util.spec_from_file_location("fetch_ref", os.path.join(root, "baseline", "fetch_ref.py"))
+    fetch_ref = importlib.util.module_from_spec(spec); spec.loader.exec_module(fetch_ref)
+    ref_root, inst = os.path.join(fetch_ref.SOURCE, "cosmogp"), os.path.join(fetch_ref.TARGET, "cosmogp")
     if os.path.isdir(ref_root) and os.path.isdir(inst):
         for name in ("Gaussian_process.py", "kernel.py", "inv_matrix.py", "mean.py", "pull.py", "__init__.py"):
             assert open(os.path.join(ref_root, name), "rb").read() == open(os.path.join(inst, name), "rb").read(), name
+
+
+def test_bench_dump_outputs(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: float64 .npy files of the step's outputs, all objects or a seeded sample of them that
+    is the same from run to run, within 64 MB at the workload's size; bad arguments are refused before any work."""
+    import os, subprocess, sys
+    import torch
+    import bench
+    assert bench.DUMP_OBJECTS * (2 + 2 * bench.M_GRID) * 8 <= 64 * 2 ** 20
+    rng = np.random.default_rng(3)
+    b, m = 50, bench.M_GRID
+    ll, mean, var = (torch.from_numpy(rng.standard_normal(k)) for k in (b, b * m, b * m))
+    monkeypatch.setattr(bench, "DUMP_OBJECTS", 16)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), ll, mean, var)
+    got = {n: np.load(tmp_path / "a" / (n + ".npy")) for n in ("objects", "ll", "mean", "var")}
+    assert all(a.dtype == np.float64 for a in got.values())
+    assert all(np.array_equal(a, np.load(tmp_path / "b" / (n + ".npy"))) for n, a in got.items())
+    idx = got["objects"].astype(np.int64)
+    assert len(idx) == 16 and len(set(idx)) == 16 and (np.diff(idx) > 0).all()
+    assert np.array_equal(got["ll"], ll.numpy()[idx])
+    assert np.array_equal(got["mean"], mean.numpy().reshape(b, m)[idx]) and np.array_equal(got["var"], var.numpy().reshape(b, m)[idx])
+    monkeypatch.setattr(bench, "DUMP_OBJECTS", 64)
+    bench.dump_outputs(str(tmp_path / "c"), ll, mean, var)
+    assert np.array_equal(np.load(tmp_path / "c" / "objects.npy"), np.arange(b))
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    for bad in (["--steps", "0"], ["--workload", "c5", "--dump-outputs", str(tmp_path / "d")]):
+        r = subprocess.run([sys.executable, os.path.join(root, "bench.py")] + bad, capture_output=True, text=True, timeout=120)
+        assert r.returncode == 2 and "error" in r.stderr
+    assert not (tmp_path / "d").exists()
 
 
 def test_pack_csr_fast_path_equals_per_object_conversion():

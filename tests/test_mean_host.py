@@ -1,12 +1,27 @@
 """Host-side mean function (cosmogp/mean.py): the batched evaluation must reproduce the reference's
-per-object `return_mean` bit for bit (same scipy calls).  Compared against the live reference when
-/root/reference is present, else against the oracle restatement."""
+per-object `return_mean` bit for bit (same scipy calls).  Compared against the reference's outputs stored
+in tests/golden, and on fresh random cases against the live reference when it is installed, else against
+the oracle restatement."""
 import numpy as np
 import pytest
 
-from conftest import assert_close
+from conftest import assert_close, golden
 from cosmogp_b200 import mean as M
 from oracle import gp_oracle as O, ref_loader
+
+
+def test_batched_mean_matches_stored_reference():
+    """y0 as the reference computed it: the template spline plus one offset per object (ragged_1d), and the plain
+    average per object without a template (mean_options, substract_mean=True)."""
+    g = golden("ragged_1d")
+    y0, _ = M.batched_mean(g["x"], g["y"], g["off"], 1, g["mean_y"], g["mean_x"], np.array([None] * (len(g["off"]) - 1)))
+    assert np.array_equal(y0, g["y0"])
+    for i in range(len(g["off"]) - 1):
+        a, b = g["off"][i], g["off"][i + 1]
+        assert np.array_equal(M.return_mean(g["y"][a:b], g["x"][a:b], mean_y=g["mean_y"], mean_xaxis=g["mean_x"]), g["y0"][a:b])
+    m = golden("mean_options")
+    y0n, _ = M.batched_mean(m["x"], m["y"], m["off"], 1, None, None, np.array([None] * (len(m["off"]) - 1)))
+    assert np.array_equal(y0n, m["y0_sub"])
 
 
 def _objects(rng, b):

@@ -178,10 +178,20 @@ def test_notebook_known_answers():
     assert_close(O.log_likelihood(w["y"][0], w["x"][0], h[:2], h[2]), w["ll_at_fit_chol"], 1e-10)
 
 
-@pytest.mark.skipif(not __import__("oracle.ref_loader").ref_loader.available(), reason="reference tree absent")
 def test_oracle_vs_live_reference_random():
-    """Extra pin in the build container: fresh random cases through the real reference."""
+    """The kernel matrices and inverses of the oracle against the reference: the reference's own outputs stored in the
+    fixtures (60-point 1D object with per-point errors, 30-point 2D object with a nugget; the svd_method=True path is
+    pinned by test_oracle_svd_path_against_the_reference_default), and fresh random cases when the reference is installed."""
     from oracle import ref_loader
+    g = golden("ragged_1d")
+    x0, ye0 = split(g["x"], g["off"])[0], split(g["y_err"], g["off"])[0]
+    assert_close(O.rbf_1d(x0, g["hyp"], nugget=float(g["nugget"]), y_err=ye0), g["kmat0"], 1e-14)
+    assert_close(O.cholesky_inverse(g["kmat0"]), g["kinv0"], 1e-15, 1e-15)
+    b = golden("batch_2d")
+    x2, ye2 = split(b["x"], b["off"])[2], split(b["y_err"], b["off"])[2]
+    assert_close(O.rbf_2d(x2, b["hyp"], nugget=float(b["nugget"]), y_err=ye2), b["kmat2"], 1e-12, 1e-300)
+    if not ref_loader.available():
+        return
     ref = ref_loader.load()
     rng = np.random.default_rng(99)
     for n in (3, 17, 64):
