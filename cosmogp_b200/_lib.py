@@ -81,6 +81,8 @@ SIGNATURES = {
     "cgp_large_solve_dev": (_int, [_ptr, _i64, _i64, _i64, _ptr, _ptr, _ptr, _ptr, _ptr]),
     "cgp_large_predict_dev": (_int, [_ptr, _i64, _i64, _i64, _int, _ptr, _ptr, _ptr, _dbl, _u32,
                                      _ptr, _i64, _ptr, _ptr, _ptr, _ptr, _i64, _ptr]),
+    "cgp_large_loo_dev": (_int, [_ptr, _i64, _i64, _i64, _int, _ptr, _ptr, _ptr] + _HYP + [_int, _ptr, _ptr, _i64]
+                          + [_ptr] * 4 + [_ptr]),
     "cgp_trsm_rows_dev": (_int, [_ptr, _i64, _i64, _ptr, _i64, _i64, _ptr]),
     "cgp_gemm_nt_dev": (_int, [_ptr, _i64, _ptr, _i64, _ptr, _i64, _i64, _i64, _i64, _dbl, _dbl, _int, _ptr]),
 }

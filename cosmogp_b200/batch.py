@@ -426,25 +426,33 @@ class DeviceBatch:
             return [flat[coff_h[i] :coff_h[i + 1]].reshape(sizes[i - i0], sizes[i - i0]) for i in range(i0, i1)], info
         return flat.reshape(k, m, m), info
 
-    def loo_dev(self, hyp, nugget, mean=None, mode=_lib.CGP_LOO_PLAIN, floor=0.0, flags=0):
+    def loo_dev(self, hyp, nugget, mean=None, mode=_lib.CGP_LOO_PLAIN, floor=0.0, flags=0, ranges=None):
         """Closed-form leave-one-out; `mean` (flat, host) replaces the batch's y0 when given.
+        ranges: (first, end) object ranges to compute, one launch each (default: every object in one launch); the
+        outputs span every point either way, and those of objects outside the ranges are left unwritten.
         -> pred, pred_var, pull, resid (flat DEVICE tensors), info (device)."""
         m = self._up(np.asarray(mean, dtype=np.float64)) if mean is not None else self.y0
         outs = [torch.empty(max(self.n_pts, 1), dtype=torch.float64, device=self.device) for _ in range(4)]
         oh = self._objhyp(hyp, nugget)
-        with torch.cuda.device(self.device):
-            if oh is not None:
-                rc = _lib.lib().cgp_loo_objhyp_dev(self.n_obj, self._p(self.off), self.max_n, self.dim, self._p(self.x),
-                                                   self._p(self.y), self._p(m), self._p(self.y_err), self._p(oh[0]),
-                                                   self._p(oh[1]), oh[2], float(floor), int(flags), int(mode),
-                                                   *[self._p(o) for o in outs], self._p(self._info), self._stream())
-            else:
-                h = self._hyp(hyp)
-                rc = _lib.lib().cgp_loo_batched_dev(self.n_obj, self._p(self.off), self.max_n, self.dim, self._p(self.x),
-                                                    self._p(self.y), self._p(m), self._p(self.y_err), _lib.hptr(h),
-                                                    float(nugget), float(floor), int(flags), int(mode),
-                                                    *[self._p(o) for o in outs], self._p(self._info), self._stream())
-        _lib.check(rc, "cgp_loo_objhyp_dev" if oh is not None else "cgp_loo_batched_dev")
+        h = None if oh is not None else self._hyp(hyp)
+        nh = 2 if self.dim == 1 else 4
+        for a, b in ([(0, self.n_obj)] if ranges is None else ranges):
+            # object range [a, b): the CSR offsets stay absolute, so the kernel reads and writes the full arrays
+            off, info = self._p(self.off) + 8 * a, self._p(self._info) + 4 * a
+            with torch.cuda.device(self.device):
+                if oh is not None:
+                    rc = _lib.lib().cgp_loo_objhyp_dev(b - a, off, self.max_n, self.dim, self._p(self.x),
+                                                       self._p(self.y), self._p(m), self._p(self.y_err),
+                                                       self._p(oh[0]) + 8 * nh * a,
+                                                       None if oh[1] is None else self._p(oh[1]) + 8 * a, oh[2],
+                                                       float(floor), int(flags), int(mode),
+                                                       *[self._p(o) for o in outs], info, self._stream())
+                else:
+                    rc = _lib.lib().cgp_loo_batched_dev(b - a, off, self.max_n, self.dim, self._p(self.x),
+                                                        self._p(self.y), self._p(m), self._p(self.y_err), _lib.hptr(h),
+                                                        float(nugget), float(floor), int(flags), int(mode),
+                                                        *[self._p(o) for o in outs], info, self._stream())
+            _lib.check(rc, "cgp_loo_objhyp_dev" if oh is not None else "cgp_loo_batched_dev")
         return [o[:self.n_pts] for o in outs] + [self._info[:self.n_obj]]
 
     def loo(self, hyp, nugget, mean=None, mode=_lib.CGP_LOO_PLAIN, floor=0.0, flags=0):

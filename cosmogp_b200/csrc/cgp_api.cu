@@ -751,4 +751,22 @@ int cgp_large_predict_dev(const double* a, int64_t n, int64_t n_pad, int64_t ld,
   return 0;
 }
 
+int cgp_large_loo_dev(const double* a, int64_t n, int64_t n_pad, int64_t ld, int dim,
+                      const double* y, const double* m, const double* y_err,
+                      const double* hyp, double nugget, double floor, unsigned flags, int mode,
+                      const int* info, double* vwork, int64_t chunk_rows,
+                      double* pred, double* pred_var, double* pull, double* resid, void* stream) {
+  if (!a || !y || !info || !vwork) return fail(CGP_ERR_ARG, "cgp_large_loo_dev: NULL argument");
+  if (n <= 0 || n_pad < n || n_pad % 128 || ld < n_pad || ld % 2)
+    return fail(CGP_ERR_ARG, "cgp_large_loo_dev: need 0 < n <= n_pad, n_pad a multiple of 128, ld >= n_pad and even");
+  if (chunk_rows <= 0 || chunk_rows % 128) return fail(CGP_ERR_ARG, "cgp_large_loo_dev: chunk_rows must be a positive multiple of 128");
+  if (mode != CGP_LOO_PLAIN && mode != CGP_LOO_RECENTER) return fail(CGP_ERR_ARG, "cgp_large_loo_dev: bad mode %d", mode);
+  Cov c; int rc = make_cov(dim, hyp, nugget, floor, flags, &c);
+  if (rc) return rc;
+  keep_pool_memory();
+  int e = large_loo(a, n, n_pad, ld, c, y, m, y_err, mode == CGP_LOO_RECENTER, info, vwork, chunk_rows,
+                    pred, pred_var, pull, resid, (cudaStream_t)stream);
+  return e ? cuda_fail(e, "cgp_large_loo_dev") : 0;
+}
+
 }  // extern "C"

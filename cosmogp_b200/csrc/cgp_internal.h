@@ -124,6 +124,12 @@ int large_cov_gram(int dim, const Cov& cov, const double* grid, const int64_t* g
                    const double* v, int ldv, const int* info, double* out, const int64_t* coff, cudaStream_t st);
 int large_dot_sq(const double* v, int64_t n, double* out, cudaStream_t st);
 int large_residual(const double* y, const double* y0, int64_t n, int64_t n_pad, double* r, cudaStream_t st);
+int large_sum(const double* v, int64_t n, double* out, cudaStream_t st);
+// negd[m] = -diag(K^-1)_m from the blocked factor, chunk_rows (% 128 == 0) rows at a time in v (chunk_rows x n_pad)
+int large_diag_inv(const double* a, int64_t n_pad, int64_t ld, double* v, int64_t chunk_rows, double* negd, cudaStream_t st);
+int large_loo(const double* a, int64_t n, int64_t n_pad, int64_t ld, const Cov& cov, const double* y, const double* m,
+              const double* yerr, int recenter, const int* info, double* vwork, int64_t chunk_rows,
+              double* pred, double* pvar, double* pull, double* resid, cudaStream_t st);
 
 // Launchers (cgp_small.cu).  max_n = largest object in the batch.  Return cudaError_t as int.
 int launch_small(Task task, int dim, int max_n, const SmallArgs& a, cudaStream_t stream);

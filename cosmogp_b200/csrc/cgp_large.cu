@@ -431,6 +431,48 @@ __global__ void residual_kernel(const double* y, const double* y0, int64_t n, in
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i < n_pad) r[i] = i < n ? y[i] - (y0 ? y0[i] : 0.0) : 0.0;
 }
+__global__ void ones_kernel(int64_t n, int64_t n_pad, double* v) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n_pad) v[i] = i < n ? 1.0 : 0.0;
+}
+// v[r][c] = (r == c) for r < rows, c < cols (cols even): the identity rows the diag(K^-1) solve starts from.
+__global__ void __launch_bounds__(256) identity_rows_kernel(double* v, int64_t ldv, int64_t rows, int64_t cols) {
+  const int64_t half = cols / 2, total = rows * half;
+  for (int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; t < total; t += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t r = t / half, c = (t - r * half) * 2;
+    *reinterpret_cast<double2*>(v + r * ldv + c) = make_double2(c == r ? 1.0 : 0.0, c + 1 == r ? 1.0 : 0.0);
+  }
+}
+// Closed-form leave-one-out of one object, the formulas of the shared-memory path (cgp_small.cu TASK_LOO):
+// d = diag(K^-1) arrives negated (row_norm_var_kernel with amp* = 0), alpha = K^-1 r; u = K^-1 1 and rsum = sum r
+// for the recentred mode only (u == nullptr otherwise).  NaN everywhere when the factorisation failed.
+__global__ void __launch_bounds__(256) loo_epilogue_kernel(const Cov cov, int64_t n, const double* __restrict__ y,
+                                                           const double* __restrict__ m, const double* __restrict__ yerr,
+                                                           const double* __restrict__ alpha, const double* __restrict__ negd,
+                                                           const double* __restrict__ u, const double* __restrict__ rsum,
+                                                           const int* __restrict__ info, double* pred, double* pvar,
+                                                           double* pull, double* resid) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const double rho = cov.amp_cross / cov.amp_auto;
+  const double amp_star = cov.amp_auto + cov.nugget2;
+  const double d = -negd[i];
+  const double yv = y[i], mi = m ? m[i] : 0.0, r = yv - mi;
+  const double ye = yerr ? yerr[i] : 0.0;
+  double pr = mi + rho * (r - alpha[i] / d);
+  if (u) {
+    const double delta = (rsum[0] - r) / (double)(n - 1);
+    pr += delta - delta * rho * (1.0 - u[i] / d);
+  }
+  double pv = fabs(amp_star - rho * rho * (cov.amp_auto + (ye * ye + cov.noise_const) - 1.0 / d));
+  double res = pr - yv;
+  double pl = res / sqrt(ye * ye + pv + cov.nugget2);
+  if (*info) { pr = nan(""); pv = pr; res = pr; pl = pr; }
+  if (pred) pred[i] = pr;
+  if (pvar) pvar[i] = pv;
+  if (resid) resid[i] = res;
+  if (pull) pull[i] = pl;
+}
 
 }  // namespace
 
@@ -812,6 +854,76 @@ int large_sum(const double* v, int64_t n, double* out, cudaStream_t st) {
 int large_residual(const double* y, const double* y0, int64_t n, int64_t n_pad, double* r, cudaStream_t st) {
   residual_kernel<<<(unsigned)((n_pad + 255) / 256), 256, 0, st>>>(y, y0, n, n_pad, r); count_launch();
   return (int)cudaGetLastError();
+}
+
+// negd[m] = -(K^-1)_mm = -|L^-1 e_m|^2 for m < n_pad, without forming K^-1.  Identity rows e_m, m in [r0, r0 + c),
+// are solved in chunks of c = chunk_rows rows staged in v (c x n_pad, leading dimension n_pad): row i of the chunk
+// becomes (L^-1 e_{r0+i})^T, which is zero left of column r0 + i, so the chunk only spans columns [r0, n_pad) and
+// block column k only involves the chunk's row blocks <= k.  Right-looking over pairs of block columns, as in
+// large_potrf: finish block columns k, k+1 (T_kk^T, one 128-wide update, T_{k+1}^T), then
+// V[:, k+2:] -= V[:, k:k+2] L[k+2:, k:k+2]^T with K = 256.  N^3/3 FLOPs in all, every one in gemm_nt.
+int large_diag_inv(const double* a, int64_t n_pad, int64_t ld, double* v, int64_t chunk_rows, double* negd, cudaStream_t st) {
+  const int nblk = (int)(n_pad / 128);
+  int e = 0;
+  auto gemm = [&](const double* A, const double* B, int64_t ldb, double* C, int64_t m, int64_t n, int k, double alpha,
+                  double beta) {
+    GemmArgs g;
+    g.a = A; g.lda = n_pad; g.b = B; g.ldb = ldb; g.c = C; g.ldc = n_pad;
+    g.m = (int)m; g.n = (int)n; g.k = k; g.alpha = alpha; g.beta = beta; g.lower_only = 0;
+    return launch_gemm_nt(g, st);
+  };
+  for (int64_t r0 = 0; r0 < n_pad && !e; r0 += chunk_rows) {
+    const int64_t c = n_pad - r0 < chunk_rows ? n_pad - r0 : chunk_rows;
+    const int kb0 = (int)(r0 / 128);
+    const int64_t w = n_pad - r0;
+    double* vc = v + r0;                               // column r0 of the chunk's rows
+    auto rows = [&](int k) { const int64_t r = (int64_t)(k - kb0 + 1) * 128; return r < c ? r : c; };
+    int64_t blocks = (c * (w / 2) + 255) / 256;
+    identity_rows_kernel<<<(unsigned)(blocks < 148 * 16 ? blocks : 148 * 16), 256, 0, st>>>(vc, n_pad, c, w);
+    count_launch();
+    for (int k = kb0; k < nblk && !e; k += 2) {
+      const int64_t j0 = (int64_t)(k - kb0) * 128;     // block column k inside the chunk
+      const double* lk = a + (int64_t)k * 128 * ld + (int64_t)k * 128;
+      if ((e = gemm(vc + j0, lk, ld, vc + j0, rows(k), 128, 128, 1.0, 0.0))) break;                 // V_k T_kk^T
+      if (k + 1 == nblk) break;
+      if ((e = gemm(vc + j0, lk + 128 * ld, ld, vc + j0 + 128, rows(k), 128, 128, -1.0, 1.0))) break;  // -= V_k L_{k+1,k}^T
+      if ((e = gemm(vc + j0 + 128, lk + 128 * ld + 128, ld, vc + j0 + 128, rows(k + 1), 128, 128, 1.0, 0.0))) break;
+      if (k + 2 < nblk)
+        e = gemm(vc + j0, lk + 256 * ld, ld, vc + j0 + 256, rows(k + 1), n_pad - (int64_t)(k + 2) * 128, 256, -1.0, 1.0);
+    }
+    if (!e) e = large_row_var(vc, n_pad, w, c, 0.0, negd + r0, st);
+  }
+  return e ? e : (int)cudaGetLastError();
+}
+
+// Leave-one-out pulls of one factored object (see cgp_large_loo_dev).  Stream-ordered scratch: alpha, -diag(K^-1),
+// K^-1 1 (n_pad each) and sum r.
+int large_loo(const double* a, int64_t n, int64_t n_pad, int64_t ld, const Cov& cov, const double* y, const double* m,
+              const double* yerr, int recenter, const int* info, double* vwork, int64_t chunk_rows,
+              double* pred, double* pvar, double* pull, double* resid, cudaStream_t st) {
+  double* ws = nullptr;
+  cudaError_t ce = cudaMallocAsync((void**)&ws, (3 * n_pad + 2) * sizeof(double), st);
+  if (ce != cudaSuccess) return (int)ce;
+  double* alpha = ws;
+  double* negd = ws + n_pad;
+  double* u = recenter ? ws + 2 * n_pad : nullptr;
+  double* rsum = ws + 3 * n_pad;
+  int e = large_residual(y, m, n, n_pad, alpha, st);
+  if (!e && recenter) e = large_sum(alpha, n, rsum, st);
+  if (!e) e = large_potrs(a, n_pad, ld, alpha, nullptr, 1, st);
+  if (!e && recenter) {
+    ones_kernel<<<(unsigned)((n_pad + 255) / 256), 256, 0, st>>>(n, n_pad, u); count_launch();
+    e = large_potrs(a, n_pad, ld, u, nullptr, 1, st);
+  }
+  if (!e) e = large_diag_inv(a, n_pad, ld, vwork, chunk_rows, negd, st);
+  if (!e) {
+    loo_epilogue_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(cov, n, y, m, yerr, alpha, negd, u, rsum, info,
+                                                                     pred, pvar, pull, resid);
+    count_launch();
+    e = (int)cudaGetLastError();
+  }
+  cudaFreeAsync(ws, st);
+  return e;
 }
 
 }  // namespace cgp

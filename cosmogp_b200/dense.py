@@ -3,6 +3,7 @@
 `LargeObject` is the N > 224 counterpart of DeviceBatch: the covariance is built in HBM
 (never on the host), factorised by the blocked FP64 tensor-core Cholesky and reused for the
 likelihood, alpha = K^-1 r, and predictions on arbitrarily long grids (BASELINE configs 3, 4).
+`LargeLoo` gives the leave-one-out pulls of such objects for build_pull.
 The free functions implement the reference's `kernel(...)` and `chol(matrix)` seams
 (cosmogp/Gaussian_process.py:6-9, 136-154) for single matrices of any size.
 """
@@ -133,6 +134,40 @@ class LargeObject:
         _lib.check(L.cgp_gemm_nt_dev(_p(u), self.n_pad, _p(u), self.n_pad, _p(kinv), self.n_pad, self.n_pad, self.n_pad,
                                      self.n_pad, 1.0, 0.0, 0, st), "cgp_gemm_nt_dev")
         return kinv[:self.n, :self.n].cpu().numpy()
+
+
+class LargeLoo:
+    """Closed-form leave-one-out pulls of objects too large for the shared-memory path, one object per launch
+    sequence: covariance build -> blocked Cholesky -> cgp_large_loo_dev, written straight into slices of device
+    outputs.  The factor buffer and the diag(K^-1) workspace are allocated once, for the largest object (max_n
+    points), and reused; nothing here synchronises.
+    chunk_rows: identity rows per pass of the diag(K^-1) solve (default: all rows while the workspace stays under
+    4 GB, i.e. up to about 23 000 points)."""
+
+    def __init__(self, max_n, dim, flags=0, chunk_rows=None):
+        self.dev = _dev()
+        self.dim, self.flags = int(dim), int(flags)
+        n_pad = pad128(max_n)
+        if chunk_rows is None:
+            chunk_rows = max(128, (4 << 30) // (8 * n_pad))
+        self.chunk = min(n_pad, int(chunk_rows) // 128 * 128 or 128)
+        self.a = torch.empty(n_pad * n_pad, dtype=torch.float64, device=self.dev)
+        self.vwork = torch.empty(self.chunk * n_pad, dtype=torch.float64, device=self.dev)
+
+    def run(self, x, y, m, y_err, hyp, nugget, mode, info, outs):
+        """x, y (and m, y_err, either may be None): device tensors of one object; info: one-element int32 device
+        tensor, receives the factorisation's status; outs: device tensors (pred, pred_var, pull, resid) of N doubles."""
+        L = _lib.lib()
+        n = int(y.numel())
+        n_pad = pad128(n)
+        h = _hyp(hyp, self.dim)
+        st = _stream(self.dev)
+        _lib.check(L.cgp_cov_matrix_dev(self.dim, _p(x), n, None, 0, _p(y_err), _lib.hptr(h), float(nugget), 0.0,
+                                        self.flags, _p(self.a), n_pad, n_pad, n_pad, st), "cgp_cov_matrix_dev")
+        _lib.check(L.cgp_potrf_dev(_p(self.a), n_pad, n_pad, None, _p(info), st), "cgp_potrf_dev")
+        _lib.check(L.cgp_large_loo_dev(_p(self.a), n, n_pad, n_pad, self.dim, _p(y), _p(m), _p(y_err), _lib.hptr(h),
+                                       float(nugget), 0.0, self.flags, int(mode), _p(info), _p(self.vwork), self.chunk,
+                                       *[_p(o) for o in outs], st), "cgp_large_loo_dev")
 
 
 def cholesky_inverse(matrix, return_logdet=False):

@@ -282,6 +282,19 @@ int cgp_large_predict_dev(const double* a, int64_t n, int64_t n_pad, int64_t ld,
                           const double* xnew, int64_t m, const double* new_y0, double* mean, double* var,
                           double* vwork, int64_t chunk_rows, void* stream);
 
+/* Leave-one-out pulls of one object factored by cgp_potrf_dev (build_pull.compute_pull, cosmogp/pull.py:43-102,
+ * for objects of any size), with the closed form and the mean modes of cgp_loo_batched_dev.  hyp / nugget / floor /
+ * flags must be those the factored covariance was built with; y, m (may be NULL), y_err (may be NULL) hold n values.
+ * diag(K^-1) comes from a blocked triangular solve on identity rows, N^3/3 FLOPs on the FP64 tensor pipe, in chunks
+ * of `chunk_rows` rows (multiple of 128) staged in vwork (chunk_rows x n_pad doubles).  info (device int) is the
+ * factorisation's: where it is nonzero the outputs are NaN (read on the device, no synchronisation).  Outputs
+ * (n doubles each, any may be NULL): pred, pred_var, pull, resid. */
+int cgp_large_loo_dev(const double* a, int64_t n, int64_t n_pad, int64_t ld, int dim,
+                      const double* y, const double* m, const double* y_err,
+                      const double* hyp, double nugget, double floor, unsigned flags, int mode,
+                      const int* info, double* vwork, int64_t chunk_rows,
+                      double* pred, double* pred_var, double* pull, double* resid, void* stream);
+
 /* v_m = L^-1 h_m for `rows` rows of V (rows x n_pad, rows % 128 == 0), in place. */
 int cgp_trsm_rows_dev(const double* a, int64_t n_pad, int64_t ld, double* v, int64_t ldv, int64_t rows, void* stream);
 
