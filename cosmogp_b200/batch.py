@@ -207,7 +207,10 @@ class DeviceBatch:
     def ll_objhyp(self, hyp_rows, idx, nugget_rows=None, nugget=0.0, floor=0.0, flags=0):
         """Log-likelihood of the objects `idx` (int array), object idx[k] using its own
         hyperparameters hyp_rows[k] (and nugget_rows[k]).  -> (ll (k,), info (k,)) host arrays.
-        Compact I/O: only the k active rows cross PCIe, through persistent pinned / device buffers."""
+        Compact I/O: only the k active rows cross PCIe, through persistent pinned / device buffers.
+        Objects of up to 224 points go through the shared-memory kernel (cgp_ll_objhyp_dev, with the largest small
+        size as max_n: the kernel a batch of the small objects alone gets), larger ones through the grouped blocked
+        factorisation (cgp_large_ll_objhyp_dev) in a workspace allocated once per batch.  One synchronisation."""
         k, nh = len(idx), (2 if self.dim == 1 else 4)
         if k == 0:
             return np.zeros(0), np.zeros(0, dtype=np.int32)
@@ -221,25 +224,53 @@ class DeviceBatch:
                             "ord_h": pin((b,), torch.int32), "ord_d": dev((b,), torch.int32),
                             "ll_h": pin((b,), torch.float64), "ll_d": dev((b,), torch.float64),
                             "info_h": pin((b,), torch.int32), "info_d": dev((b,), torch.int32)}
-        c["hyp_h"].numpy()[:k] = np.asarray(hyp_rows, dtype=np.float64).reshape(k, nh)
-        c["ord_h"].numpy()[:k] = idx
+            sizes = np.diff(self.off_host)
+            small = sizes <= _lib.CGP_SMALL_MAX_N
+            c["large"] = ~small
+            c["small_max_n"] = self.max_n if small.all() else (int(sizes[small].max()) if small.any() else 0)
+            if c["large"].any():
+                need = np.array([_lib.lib().cgp_large_ll_ws_doubles(int(n)) for n in sizes[c["large"]]], dtype=np.int64)
+                c["work"] = torch.empty(int(max(need.max(), min(need.sum(), (4 << 30) // 8))), dtype=torch.float64,
+                                        device=self.device)
+        idx = np.asarray(idx, dtype=np.int64)
+        big = c["large"][idx]
+        perm = np.concatenate([np.nonzero(~big)[0], np.nonzero(big)[0]]) if big.any() else None
+        ks = k - int(big.sum())
+        rows = np.asarray(hyp_rows, dtype=np.float64).reshape(k, nh)
+        c["hyp_h"].numpy()[:k] = rows if perm is None else rows[perm]
+        c["ord_h"].numpy()[:k] = idx if perm is None else idx[perm]
         c["hyp_d"][:k].copy_(c["hyp_h"][:k], non_blocking=True)
         c["ord_d"][:k].copy_(c["ord_h"][:k], non_blocking=True)
         nd = None
         if nugget_rows is not None:
-            c["nug_h"].numpy()[:k] = nugget_rows
+            nug = np.asarray(nugget_rows, dtype=np.float64)
+            c["nug_h"].numpy()[:k] = nug if perm is None else nug[perm]
             c["nug_d"][:k].copy_(c["nug_h"][:k], non_blocking=True)
             nd = c["nug_d"]
         with torch.cuda.device(self.device):
-            rc = _lib.lib().cgp_ll_objhyp_dev(self.n_obj, self._p(self.off), self.max_n, self.dim, self._p(self.x),
-                                              self._p(self.y), self._p(self.y0), self._p(self.y_err), self._p(c["hyp_d"]),
-                                              self._p(nd), float(nugget), float(floor), int(flags), self._p(c["ord_d"]), k,
-                                              self._p(c["ll_d"]), self._p(c["info_d"]), self._stream())
-        _lib.check(rc, "cgp_ll_objhyp_dev")
+            if ks:
+                rc = _lib.lib().cgp_ll_objhyp_dev(self.n_obj, self._p(self.off), c["small_max_n"], self.dim, self._p(self.x),
+                                                  self._p(self.y), self._p(self.y0), self._p(self.y_err), self._p(c["hyp_d"]),
+                                                  self._p(nd), float(nugget), float(floor), int(flags), self._p(c["ord_d"]), ks,
+                                                  self._p(c["ll_d"]), self._p(c["info_d"]), self._stream())
+                _lib.check(rc, "cgp_ll_objhyp_dev")
+            if ks < k:
+                order = c["ord_h"].numpy()[ks:k]                # host copy of the schedule
+                rc = _lib.lib().cgp_large_ll_objhyp_dev(self.n_obj, _lib.hptr(self.off_host), self.dim, self._p(self.x),
+                                                        self._p(self.y), self._p(self.y0), self._p(self.y_err),
+                                                        self._p(c["hyp_d"]) + 8 * nh * ks,
+                                                        None if nd is None else self._p(nd) + 8 * ks, float(nugget),
+                                                        float(floor), int(flags), order.ctypes.data, k - ks,
+                                                        self._p(c["ll_d"]) + 8 * ks, self._p(c["info_d"]) + 4 * ks,
+                                                        self._p(c["work"]), int(c["work"].numel()), self._stream())
+                _lib.check(rc, "cgp_large_ll_objhyp_dev")
         c["ll_h"][:k].copy_(c["ll_d"][:k], non_blocking=True)
         c["info_h"][:k].copy_(c["info_d"][:k], non_blocking=True)
         torch.cuda.current_stream(self.device).synchronize()
-        return c["ll_h"].numpy()[:k].copy(), c["info_h"].numpy()[:k].copy()
+        ll, info = c["ll_h"].numpy()[:k].copy(), c["info_h"].numpy()[:k].copy()
+        if perm is not None:
+            ll[perm], info[perm] = ll.copy(), info.copy()
+        return ll, info
 
     def fit_objects(self, start, nugget=0.0, floor=0.0, flags=0, xatol=1e-4, fatol=1e-4, maxiter=None, maxfun=None):
         """One Nelder-Mead fit per object, entirely on the device (cgp_fit_objects_dev).

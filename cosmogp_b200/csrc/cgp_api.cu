@@ -248,6 +248,38 @@ int cgp_ll_objhyp_dev(int64_t n_obj, const int64_t* off, int max_n, int dim,
   return run_small(TASK_LL, dim, max_n, a, (cudaStream_t)stream, "cgp_ll_objhyp_dev");
 }
 
+int64_t cgp_large_ll_ws_doubles(int64_t n) { return n < 0 ? 0 : large_ll_ws_doubles(n); }
+
+int cgp_large_ll_objhyp_dev(int64_t n_obj, const int64_t* off_host, int dim,
+                            const double* x, const double* y, const double* y0, const double* y_err,
+                            const double* hyp_obj, const double* nugget_obj, double nugget, double floor, unsigned flags,
+                            const int* order_host, int64_t n_active, double* ll_obj, int* info,
+                            double* work, int64_t work_doubles, void* stream) {
+  if (n_obj < 0 || n_active < 0) return fail(CGP_ERR_ARG, "cgp_large_ll_objhyp_dev: negative object count");
+  const int64_t k = order_host ? n_active : n_obj;
+  if (k == 0) return 0;
+  if (!off_host || !x || !y || !hyp_obj || !ll_obj || !info || !work)
+    return fail(CGP_ERR_ARG, "cgp_large_ll_objhyp_dev: NULL argument");
+  if (dim != 1 && dim != 2) return fail(CGP_ERR_ARG, "dim must be 1 or 2, got %d", dim);
+  if ((uintptr_t)work & 15) return fail(CGP_ERR_ARG, "cgp_large_ll_objhyp_dev: work must be 16-byte aligned");
+  int64_t need = 0;
+  for (int64_t j = 0; j < k; ++j) {
+    const int64_t b = order_host ? order_host[j] : j;
+    if (b < 0 || b >= n_obj) return fail(CGP_ERR_ARG, "cgp_large_ll_objhyp_dev: order[%lld] = %lld is not an object id", (long long)j, (long long)b);
+    const int64_t n = off_host[b + 1] - off_host[b];
+    if (n < 0 || n > 65535) return fail(CGP_ERR_SIZE, "cgp_large_ll_objhyp_dev: object %lld has %lld points (0..65535)", (long long)b, (long long)n);
+    const int64_t w = large_ll_ws_doubles(n);
+    if (w > need) need = w;
+  }
+  if (work_doubles < need)
+    return fail(CGP_ERR_SIZE, "cgp_large_ll_objhyp_dev: workspace of %lld doubles is below the %lld the largest active object needs",
+                (long long)work_doubles, (long long)need);
+  keep_pool_memory();
+  int e = large_ll_grouped(dim, off_host, x, y, y0, y_err, hyp_obj, nugget_obj, nugget, floor, flags, order_host, k, ll_obj, info,
+                           work, work_doubles, (cudaStream_t)stream);
+  return e ? cuda_fail(e, "cgp_large_ll_objhyp_dev") : 0;
+}
+
 int cgp_fit_objects_dev(int64_t n_obj, const int64_t* off, int max_n, int dim,
                         const double* x, const double* y, const double* y0, const double* y_err,
                         const double* start, int n_par, double nugget, double floor, unsigned flags,

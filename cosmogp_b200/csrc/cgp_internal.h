@@ -90,6 +90,8 @@ struct SmallArgs {
   // matrix source: when non-null the covariance of object b is READ from amat + aoff[b] (row-major,
   // leading dimension lda, lower triangle) instead of being generated from x (blocked large-object path)
   const double* amat; const int64_t* aoff; int64_t lda;
+  const int64_t* ld_obj;   // TASK_MATRICES, optional: object b's leading dimension of amat and of the matrix outputs
+                           // (replaces lda and mld), for groups of matrices of different sizes
   double* logdet;          // TASK_MATRICES: sum of log pivots per object (may be null)
   // TASK_PREDICT (N <= 64 kernel): when non-null, row (out0 + m) of vout (8 NB doubles per row) receives
   // v = L^-1 e(x*_m, .) of grid point m (unit amplitude) -- the factor of the bulk predictive-covariance writer
@@ -130,6 +132,12 @@ int large_diag_inv(const double* a, int64_t n_pad, int64_t ld, double* v, int64_
 int large_loo(const double* a, int64_t n, int64_t n_pad, int64_t ld, const Cov& cov, const double* y, const double* m,
               const double* yerr, int recenter, const int* info, double* vwork, int64_t chunk_rows,
               double* pred, double* pvar, double* pull, double* resid, cudaStream_t st);
+// grouped likelihood of large objects with per-object hyperparameters (see cgp_large_ll_objhyp_dev)
+int64_t large_ll_ws_doubles(int64_t n);
+int large_ll_grouped(int dim, const int64_t* off, const double* x, const double* y, const double* y0, const double* yerr,
+                     const double* hyp_obj, const double* nugget_obj, double nugget, double floor, unsigned flags,
+                     const int* order, int64_t n_active, double* ll, int* info, double* work, int64_t work_doubles,
+                     cudaStream_t st);
 
 // Launchers (cgp_small.cu).  max_n = largest object in the batch.  Return cudaError_t as int.
 int launch_small(Task task, int dim, int max_n, const SmallArgs& a, cudaStream_t stream);

@@ -15,6 +15,9 @@
 #include <math.h>
 #include <string.h>
 
+#include <algorithm>
+#include <vector>
+
 namespace cgp {
 namespace {
 
@@ -36,9 +39,10 @@ __device__ __forceinline__ void cp_async16(void* smem, const void* gmem) {
 __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;"); }
 template <int N> __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" :: "n"(N)); }
 
-__global__ void __launch_bounds__(GEMM_THREADS, 3)
-gemm_nt_kernel(const GemmArgs g) {
-  extern __shared__ __align__(16) double sm[];
+// One 64 x 128 tile (or one 64-row half of a lower-triangle 128 x 128 block) of C, `tile` in the launch order of
+// launch_gemm_nt.  Shared by the single-problem and the grouped kernels, so that a tile's arithmetic does not
+// depend on which launch computes it.
+__device__ __forceinline__ void gemm_nt_tile(double* sm, const GemmArgs& g, const int tile) {
   double* As = sm;                                 // [2][BM][PITCH]
   double* Bs = sm + 2 * BM * PITCH;                // [2][BN][PITCH]
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -47,15 +51,15 @@ gemm_nt_kernel(const GemmArgs g) {
 
   int bi, bj;                                      // bi: 64-row block, bj: 128-column block
   if (g.lower_only) {                              // linear index -> (I, bj) with I >= bj, two 64-row halves each
-    const int t = blockIdx.x >> 1;
+    const int t = tile >> 1;
     int I = (int)((sqrt(8.0 * t + 1.0) - 1.0) * 0.5);
     while ((I + 1) * (I + 2) / 2 <= t) ++I;
     while (I * (I + 1) / 2 > t) --I;
     bj = t - I * (I + 1) / 2;
-    bi = 2 * I + (blockIdx.x & 1);
+    bi = 2 * I + (tile & 1);
   } else {
     const int nbn = g.n / BN;
-    bi = blockIdx.x / nbn; bj = blockIdx.x - bi * nbn;
+    bi = tile / nbn; bj = tile - bi * nbn;
   }
   const double* ga = g.a + (int64_t)bi * BM * g.lda;
   const double* gb = g.b + (int64_t)bj * BN * g.ldb;
@@ -119,6 +123,33 @@ gemm_nt_kernel(const GemmArgs g) {
     }
 }
 
+__global__ void __launch_bounds__(GEMM_THREADS, 3)
+gemm_nt_kernel(const GemmArgs g) {
+  extern __shared__ __align__(16) double sm[];
+  gemm_nt_tile(sm, g, blockIdx.x);
+}
+
+// Many independent GEMMs in one launch: problem q owns tiles [tile_start[q], tile_start[q+1]) of the grid and
+// computes them exactly as gemm_nt_kernel would for that problem alone.
+__global__ void __launch_bounds__(GEMM_THREADS, 3)
+gemm_nt_grouped_kernel(const GemmArgs* __restrict__ probs, const int* __restrict__ tile_start, const int nprob) {
+  extern __shared__ __align__(16) double sm[];
+  __shared__ GemmArgs g;                           // read from shared memory where used: kernel-parameter-like register use
+  __shared__ int tile;
+  if (threadIdx.x == 0) {
+    const int t = blockIdx.x;
+    int lo = 0, hi = nprob - 1;                    // last problem with tile_start <= t
+    while (lo < hi) {
+      const int mid = (lo + hi + 1) >> 1;
+      if (tile_start[mid] <= t) lo = mid; else hi = mid - 1;
+    }
+    g = probs[lo];
+    tile = t - tile_start[lo];
+  }
+  __syncthreads();
+  gemm_nt_tile(sm, g, tile);
+}
+
 // ---------------------------------------------------------------------------------------
 // Covariance builder: out[r][c] = amp * exp(-q(row point r, col point c)/2) (+ noise on the
 // diagonal of an auto-covariance; identity padding beyond n / m).  One thread per 2 columns,
@@ -132,9 +163,7 @@ struct CovArgs {
 };
 
 template <int DIM>
-__global__ void cov_build_kernel(const CovArgs a) {
-  const int64_t c = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) * 2;
-  const int64_t r = blockIdx.y;
+__device__ __forceinline__ void cov_build_at(const CovArgs& a, const int64_t r, const int64_t c) {
   if (c >= a.cols_pad) return;
   double rx = 0.0, ry = 0.0;
   const bool rin = r < a.m;
@@ -163,6 +192,10 @@ __global__ void cov_build_kernel(const CovArgs a) {
   if (c + 1 < a.cols_pad) *reinterpret_cast<double2*>(p) = make_double2(v[0], v[1]);
   else p[0] = v[0];
 }
+template <int DIM>
+__global__ void cov_build_kernel(const CovArgs a) {
+  cov_build_at<DIM>(a, blockIdx.y, ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) * 2);
+}
 
 // ---------------------------------------------------------------------------------------
 // Triangular solves against the blocked factor (diagonal blocks hold T = L_kk^-1).
@@ -171,8 +204,8 @@ __global__ void cov_build_kernel(const CovArgs a) {
 // others apply it to their slice.  Input and output vectors are distinct, so there is no race on
 // the block being read.
 // forward step k: z_k = T_kk u_k -> zout;  u[row] -= L[row, k-block] z_k for rows below (in place).
-__global__ void __launch_bounds__(256) fwd_step_kernel(const double* a, int64_t ld, int64_t k0, int64_t n_pad,
-                                                       double* u, double* zout) {
+__device__ __forceinline__ void fwd_step_at(const double* a, int64_t ld, int64_t k0, int64_t n_pad, double* u, double* zout,
+                                            const int cta) {
   __shared__ double sw[128], sz[128];
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   if (tid < 128) sw[tid] = u[k0 + tid];
@@ -187,8 +220,8 @@ __global__ void __launch_bounds__(256) fwd_step_kernel(const double* a, int64_t 
     if (lane == 0) sz[r] = acc;
   }
   __syncthreads();
-  if (blockIdx.x == 0) { if (tid < 128) zout[k0 + tid] = sz[tid]; return; }
-  const int64_t row0 = k0 + 128 + (int64_t)(blockIdx.x - 1) * 64;
+  if (cta == 0) { if (tid < 128) zout[k0 + tid] = sz[tid]; return; }
+  const int64_t row0 = k0 + 128 + (int64_t)(cta - 1) * 64;
   for (int rr = warp * 8; rr < warp * 8 + 8; ++rr) {               // 64 rows per CTA
     const int64_t row = row0 + rr;
     if (row >= n_pad) break;
@@ -199,6 +232,10 @@ __global__ void __launch_bounds__(256) fwd_step_kernel(const double* a, int64_t 
     for (int o = 16; o; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
     if (lane == 0) u[row] -= acc;
   }
+}
+__global__ void __launch_bounds__(256) fwd_step_kernel(const double* a, int64_t ld, int64_t k0, int64_t n_pad,
+                                                       double* u, double* zout) {
+  fwd_step_at(a, ld, k0, n_pad, u, zout, blockIdx.x);
 }
 // backward step k: alpha_k = T_kk^T z_k -> aout;  z[col] -= L[k-block, col]^T alpha_k for cols left of k (in place).
 __global__ void __launch_bounds__(256) bwd_step_kernel(const double* a, int64_t ld, int64_t k0, double* z, double* aout) {
@@ -285,7 +322,7 @@ __global__ void __launch_bounds__(256) row_norm_var_kernel(const double* v, int6
   for (int o = 16; o; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
   if (lane == 0) var[r] = amp_star - acc;
 }
-__global__ void dot_sq_kernel(const double* v, int64_t n, double* out) {      // out[0] = |v|^2 (one CTA)
+__device__ __forceinline__ double block_dot_sq(const double* v, int64_t n) {   // |v|^2, valid in thread 0
   __shared__ double s[32];
   double acc = 0.0;
   for (int64_t i = threadIdx.x; i < n; i += blockDim.x) acc = fma(v[i], v[i], acc);
@@ -297,8 +334,12 @@ __global__ void dot_sq_kernel(const double* v, int64_t n, double* out) {      //
     acc = threadIdx.x < (blockDim.x >> 5) ? s[threadIdx.x] : 0.0;
 #pragma unroll
     for (int o = 16; o; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
-    if (threadIdx.x == 0) out[0] = acc;
   }
+  return acc;
+}
+__global__ void dot_sq_kernel(const double* v, int64_t n, double* out) {      // out[0] = |v|^2 (one CTA)
+  const double acc = block_dot_sq(v, n);
+  if (threadIdx.x == 0) out[0] = acc;
 }
 __global__ void sum_kernel(const double* v, int64_t n, double* out) {         // out[0] = sum v (one CTA, fixed order)
   __shared__ double s[32];
@@ -472,6 +513,82 @@ __global__ void __launch_bounds__(256) loo_epilogue_kernel(const Cov cov, int64_
   if (pvar) pvar[i] = pv;
   if (resid) resid[i] = res;
   if (pull) pull[i] = pl;
+}
+
+// ---------------------------------------------------------------------------------------
+// Grouped likelihood of many large objects, each with its own hyperparameters (large_ll_grouped).  Every kernel
+// below runs the body of its single-object counterpart on one object at a time, so an object's arithmetic does not
+// depend on the other objects of its launch.
+struct GroupObj {
+  const double* x; const double* y; const double* y0; const double* yerr;
+  double* a;                 // n_pad x n_pad covariance -> blocked factor (leading dimension n_pad)
+  double* u;                 // residual y - y0 (n_pad, zero padded), consumed by the forward sweep
+  double* z;                 // z = L^-1 (y - y0)
+  int64_t n, n_pad;
+  int64_t io;                // position in `order`: compact hyperparameters, nugget, ll and info
+  int64_t cta0;              // first CTA of the object in the covariance launch
+};
+struct GroupHyp {
+  const double* hyp_obj; const double* nugget_obj; double nugget, floor; unsigned flags;
+};
+
+template <int DIM>
+__device__ __forceinline__ Cov group_cov(const GroupHyp& h, int64_t io) {
+  return cov_from_hyp(DIM, h.hyp_obj + io * (DIM == 1 ? 2 : 4), h.nugget_obj ? h.nugget_obj[io] : h.nugget, h.floor, h.flags);
+}
+
+// Covariance of every object of a wave (the layout of cov_build_kernel) and its residual.  Object i owns
+// n_pad * ceil(n_pad / 256) CTAs from objs[i].cta0 on: one row, 256 columns each.
+template <int DIM>
+__global__ void __launch_bounds__(128) cov_build_grouped_kernel(const GroupObj* __restrict__ objs, const int n_obj,
+                                                                const GroupHyp h) {
+  const int64_t t = blockIdx.x;
+  int lo = 0, hi = n_obj - 1;
+  while (lo < hi) {
+    const int mid = (lo + hi + 1) >> 1;
+    if (objs[mid].cta0 <= t) lo = mid; else hi = mid - 1;
+  }
+  const GroupObj& o = objs[lo];
+  const int64_t per_row = (o.n_pad + 255) / 256;
+  const int64_t local = t - o.cta0, r = local / per_row, chunk = local - r * per_row;
+  CovArgs a;
+  a.dim = DIM; a.cov = group_cov<DIM>(h, o.io); a.autocov = 1;
+  a.xc = o.x; a.n = o.n; a.xr = o.x; a.m = o.n; a.yerr = o.yerr;
+  a.out = o.a; a.ld = o.n_pad; a.rows_pad = o.n_pad; a.cols_pad = o.n_pad;
+  cov_build_at<DIM>(a, r, (chunk * 128 + threadIdx.x) * 2);
+  if (chunk == 0 && threadIdx.x == 0) o.u[r] = r < o.n ? o.y[r] - (o.y0 ? o.y0[r] : 0.0) : 0.0;   // residual_kernel
+}
+
+// Forward sweep step k of the objects objs[0 .. gridDim.y): CTA x of object y runs fwd_step_kernel's CTA x.
+__global__ void __launch_bounds__(256) fwd_step_grouped_kernel(const GroupObj* __restrict__ objs, const int64_t k0) {
+  const GroupObj& o = objs[blockIdx.y];
+  if ((int64_t)blockIdx.x >= 1 + (o.n_pad - k0 - 128 + 63) / 64) return;
+  fwd_step_at(o.a, o.n_pad, k0, o.n_pad, o.u, o.z, blockIdx.x);
+}
+
+// One CTA per object: quad = |z|^2 (dot_sq_kernel), log det and info summed over the blocks in the order of
+// potrf_finish_kernel (block k of object i at ld_blocks[koff[k] + i]), and ll with the operation order of
+// dense.LargeObject.factor: -0.5 * ((quad + logdet) + n log 2 pi).  NaN where the factorisation failed.
+__global__ void __launch_bounds__(1024) ll_finish_grouped_kernel(const GroupObj* __restrict__ objs,
+                                                                 const double* __restrict__ ld_blocks,
+                                                                 const int* __restrict__ info_blocks,
+                                                                 const int64_t* __restrict__ koff,
+                                                                 double* __restrict__ ll, int* __restrict__ info) {
+  const int i = blockIdx.x;
+  const GroupObj& o = objs[i];
+  const double quad = block_dot_sq(o.z, o.n_pad);
+  if (threadIdx.x == 0) {
+    const int nblk = (int)(o.n_pad / 128);
+    double s = 0.0; int bad = 0;
+    for (int k = 0; k < nblk; ++k) {
+      s += ld_blocks[koff[k] + i];
+      const int ik = info_blocks[koff[k] + i];
+      if (!bad && ik) bad = k * 128 + ik;
+    }
+    const double log_2pi = 1.8378770664093453;                 // math.log(2 * math.pi)
+    ll[o.io] = bad ? nan("") : __dmul_rn(-0.5, __dadd_rn(__dadd_rn(quad, s), __dmul_rn((double)o.n, log_2pi)));
+    info[o.io] = bad;
+  }
 }
 
 }  // namespace
@@ -924,6 +1041,203 @@ int large_loo(const double* a, int64_t n, int64_t n_pad, int64_t ld, const Cov& 
   }
   cudaFreeAsync(ws, st);
   return e;
+}
+
+int64_t large_ll_ws_doubles(int64_t n) {
+  const int64_t np = n <= 0 ? 128 : (n + 127) / 128 * 128;
+  return np * np + 2 * np + 2 * (np / 128);          // covariance, residual, z, per-block log det and info
+}
+
+// Log-likelihoods of the objects order[0 .. n_active) (object ids; NULL: 0 .. n_active), object order[j] with the
+// hyperparameters of row j, by the blocked factorisation of large_potrf run for all objects of a wave at once.
+// Consecutive objects are packed into waves of at most work_doubles (each object's part: large_ll_ws_doubles); inside
+// a wave they are sorted by block count, so that the objects taking part in any step are a prefix of the wave.  Per
+// wave: one covariance launch; per pair of block columns two diagonal-block launches (launch_small in matrix-source
+// mode) and four grouped GEMM launches, with the shapes, tile split and alpha / beta large_potrf uses for each object
+// alone (the next pair's columns and the lower trailing update touch disjoint tiles, so they share one launch); one
+// forward-sweep launch per block; one epilogue.  The schedule (object descriptors, GEMM problems, block offsets)
+// crosses to the device in one copy into stream-ordered scratch.  The caller checks that every object fits.
+int large_ll_grouped(int dim, const int64_t* off, const double* x, const double* y, const double* y0, const double* yerr,
+                     const double* hyp_obj, const double* nugget_obj, double nugget, double floor, unsigned flags,
+                     const int* order, int64_t n_active, double* ll, int* info, double* work, int64_t work_doubles,
+                     cudaStream_t st) {
+  struct Item { int64_t j, b, n, n_pad; int nblk; };
+  std::vector<std::vector<Item>> waves;
+  {
+    std::vector<Item> cur; int64_t used = 0;
+    for (int64_t j = 0; j < n_active; ++j) {
+      Item it; it.j = j; it.b = order ? order[j] : j; it.n = off[it.b + 1] - off[it.b];
+      it.n_pad = it.n <= 0 ? 128 : (it.n + 127) / 128 * 128; it.nblk = (int)(it.n_pad / 128);
+      const int64_t need = large_ll_ws_doubles(it.n);
+      if (!cur.empty() && (used + need > work_doubles || cur.size() >= 65535)) { waves.push_back(cur); cur.clear(); used = 0; }
+      cur.push_back(it); used += need;
+    }
+    if (!cur.empty()) waves.push_back(cur);
+  }
+  std::vector<char> tab;
+  auto put = [&](const void* p, size_t bytes) {
+    const size_t o = (tab.size() + 15) & ~(size_t)15;
+    tab.resize(o + bytes);
+    memcpy(tab.data() + o, p, bytes);
+    return o;
+  };
+  struct Launch { int kind; int64_t grid, count, k0; size_t t0, t1, t2; double* ldb; int* infob; };
+  enum { L_COV, L_DIAG, L_GEMM, L_FWD, L_FIN };
+  std::vector<Launch> launches;
+  size_t w_max = 0;
+  for (auto& w : waves) w_max = std::max(w_max, w.size());
+  std::vector<int64_t> csr(w_max + 1);
+  for (size_t i = 0; i <= w_max; ++i) csr[i] = (int64_t)i * 128;
+  const size_t t_csr = put(csr.data(), csr.size() * sizeof(int64_t));
+
+  for (auto& w : waves) {
+    std::stable_sort(w.begin(), w.end(), [](const Item& p, const Item& q) { return p.nblk > q.nblk; });
+    const int W = (int)w.size(), nb_max = w[0].nblk;
+    std::vector<GroupObj> objs(W);
+    std::vector<int64_t> ld(W), koff(nb_max + 1, 0);
+    int64_t cur = 0, cta = 0;
+    for (int i = 0; i < W; ++i) {
+      const Item& it = w[i];
+      const int64_t o0 = off[it.b], np = it.n_pad;
+      GroupObj& g = objs[i];
+      g.x = x + dim * o0; g.y = y + o0; g.y0 = y0 ? y0 + o0 : nullptr; g.yerr = yerr ? yerr + o0 : nullptr;
+      g.a = work + cur; g.u = g.a + np * np; g.z = g.u + np;
+      g.n = it.n; g.n_pad = np; g.io = it.j; g.cta0 = cta;
+      cur += np * np + 2 * np; cta += np * ((np + 255) / 256);
+      ld[i] = np;
+    }
+    if (cta > 2147483647LL) return (int)cudaErrorInvalidValue;
+    auto count = [&](int k) { int c = 0; while (c < W && w[c].nblk > k) ++c; return c; };   // objects with block k
+    for (int k = 0; k < nb_max; ++k) koff[k + 1] = koff[k] + count(k);
+    double* ldb = work + cur;
+    int* infob = reinterpret_cast<int*>(work + cur + koff[nb_max]);
+    const size_t t_objs = put(objs.data(), W * sizeof(GroupObj));
+    const size_t t_ld = put(ld.data(), W * sizeof(int64_t));
+    const size_t t_koff = put(koff.data(), koff.size() * sizeof(int64_t));
+    launches.push_back({L_COV, cta, W, 0, t_objs, 0, 0, nullptr, nullptr});
+
+    auto diag = [&](int k) {
+      const int c = count(k);
+      std::vector<int64_t> aoff(c);
+      for (int i = 0; i < c; ++i) aoff[i] = (objs[i].a - work) + (int64_t)k * 128 * ld[i] + (int64_t)k * 128;
+      launches.push_back({L_DIAG, c, c, 0, put(aoff.data(), c * sizeof(int64_t)), t_ld, 0, ldb + koff[k], infob + koff[k]});
+    };
+    std::vector<GemmArgs> probs;
+    auto gemm = [&](double* A, double* B, double* C, int64_t ldx, int64_t m, int64_t n, int k, double alpha, double beta,
+                    int lower) {
+      GemmArgs g;
+      g.a = A; g.b = B; g.c = C; g.lda = ldx; g.ldb = ldx; g.ldc = ldx;
+      g.m = (int)m; g.n = (int)n; g.k = k; g.alpha = alpha; g.beta = beta; g.lower_only = lower;
+      probs.push_back(g);
+    };
+    auto flush = [&]() -> int {
+      if (probs.empty()) return 0;
+      std::vector<int> start(probs.size() + 1, 0);
+      for (size_t q = 0; q < probs.size(); ++q) {
+        const GemmArgs& g = probs[q];
+        const int64_t t128 = g.m / 128;
+        const int64_t tiles = g.lower_only ? t128 * (t128 + 1) : (int64_t)(g.m / BM) * (g.n / BN);
+        if (start[q] + tiles > 2147483647LL) return (int)cudaErrorInvalidValue;
+        start[q + 1] = start[q] + (int)tiles;
+      }
+      const size_t tp = put(probs.data(), probs.size() * sizeof(GemmArgs));
+      const size_t ts = put(start.data(), start.size() * sizeof(int));
+      launches.push_back({L_GEMM, start.back(), (int64_t)probs.size(), 0, tp, ts, 0, nullptr, nullptr});
+      probs.clear();
+      return 0;
+    };
+    int e = 0;
+    for (int p = 0; 2 * p < nb_max && !e; ++p) {
+      const int k = 2 * p;
+      const int64_t k0 = (int64_t)p * 256;
+      diag(k);
+      for (int i = 0; i < W && w[i].nblk > k + 1; ++i) {            // panel of block column k: L_ik = A_ik T_kk^T
+        const int64_t np = ld[i];
+        double* a = objs[i].a;
+        gemm(a + (k0 + 128) * np + k0, a + k0 * np + k0, a + (k0 + 128) * np + k0, np, np - k0 - 128, 128, 128, 1.0, 0.0, 0);
+      }
+      if ((e = flush())) break;
+      for (int i = 0; i < W && w[i].nblk > k + 1; ++i) {            // block column k+1 -= L[k+1:, k] L[k+1, k]^T
+        const int64_t np = ld[i];
+        double* a = objs[i].a;
+        double* panel = a + (k0 + 128) * np + k0;
+        gemm(panel, panel, a + (k0 + 128) * np + (k0 + 128), np, np - k0 - 128, 128, 128, -1.0, 1.0, 0);
+      }
+      if ((e = flush())) break;
+      if (nb_max <= k + 1) break;
+      diag(k + 1);
+      const int64_t k1 = k0 + 128;
+      for (int i = 0; i < W && w[i].nblk > k + 2; ++i) {            // panel of block column k+1
+        const int64_t np = ld[i];
+        double* a = objs[i].a;
+        gemm(a + (k1 + 128) * np + k1, a + k1 * np + k1, a + (k1 + 128) * np + k1, np, np - k1 - 128, 128, 128, 1.0, 0.0, 0);
+      }
+      if ((e = flush())) break;
+      for (int i = 0; i < W && w[i].nblk > k + 2; ++i) {            // the pair applied to what lies right of it, K = 256
+        const int64_t np = ld[i], rest = np - k0 - 256;
+        double* a = objs[i].a;
+        double* wp = a + (k0 + 256) * np + k0;
+        gemm(wp, wp, a + (k0 + 256) * np + (k0 + 256), np, rest, 128, 256, -1.0, 1.0, 0);
+        if (rest > 128) gemm(wp + 128 * np, wp + 128 * np, a + (k0 + 384) * np + (k0 + 384), np, rest - 128, 128, 256, -1.0, 1.0, 0);
+        if (rest > 256) gemm(wp + 256 * np, wp + 256 * np, a + (k0 + 512) * np + (k0 + 512), np, rest - 256, rest - 256, 256, -1.0, 1.0, 1);
+      }
+      e = flush();
+    }
+    if (e) return e;
+    for (int k = 0; k < nb_max; ++k)
+      launches.push_back({L_FWD, 1 + (ld[0] - (int64_t)k * 128 - 128 + 63) / 64, count(k), (int64_t)k * 128, t_objs, 0, 0,
+                          nullptr, nullptr});
+    launches.push_back({L_FIN, W, W, 0, t_objs, t_koff, 0, ldb, infob});
+  }
+
+  static bool init[16] = {false};
+  int dev = 0;
+  if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 16) return (int)cudaErrorInvalidDevice;
+  if (!init[dev]) {
+    cudaError_t ce = cudaFuncSetAttribute(gemm_nt_grouped_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GEMM_SMEM);
+    if (ce != cudaSuccess) return (int)ce;
+    init[dev] = true;
+  }
+  char* td = nullptr;
+  cudaError_t ce = cudaMallocAsync((void**)&td, tab.size(), st);
+  if (ce == cudaSuccess) ce = cudaMemcpyAsync(td, tab.data(), tab.size(), cudaMemcpyHostToDevice, st);
+  if (ce != cudaSuccess) { if (td) cudaFreeAsync(td, st); return (int)ce; }
+  GroupHyp h; h.hyp_obj = hyp_obj; h.nugget_obj = nugget_obj; h.nugget = nugget; h.floor = floor; h.flags = flags;
+  int e = 0;
+  for (const Launch& l : launches) {
+    const GroupObj* objs = reinterpret_cast<const GroupObj*>(td + l.t0);
+    switch (l.kind) {
+      case L_COV:
+        if (dim == 1) cov_build_grouped_kernel<1><<<(unsigned)l.grid, 128, 0, st>>>(objs, (int)l.count, h);
+        else cov_build_grouped_kernel<2><<<(unsigned)l.grid, 128, 0, st>>>(objs, (int)l.count, h);
+        break;
+      case L_DIAG: {
+        SmallArgs s; memset(&s, 0, sizeof s);
+        s.n_obj = l.count; s.off = reinterpret_cast<const int64_t*>(td + t_csr);
+        s.amat = work; s.aoff = reinterpret_cast<const int64_t*>(td + l.t0); s.ld_obj = reinterpret_cast<const int64_t*>(td + l.t1);
+        s.moff = s.aoff; s.linv = work;
+        s.logdet = l.ldb; s.info = l.infob;
+        s.cov.amp_auto = 1.0; s.cov.amp_cross = 1.0;
+        e = launch_small(TASK_MATRICES, 1, 128, s, st);  // counts its own launch
+        break;
+      }
+      case L_GEMM:
+        gemm_nt_grouped_kernel<<<(unsigned)l.grid, GEMM_THREADS, GEMM_SMEM, st>>>(
+            reinterpret_cast<const GemmArgs*>(td + l.t0), reinterpret_cast<const int*>(td + l.t1), (int)l.count);
+        break;
+      case L_FWD:
+        fwd_step_grouped_kernel<<<dim3((unsigned)l.grid, (unsigned)l.count), 256, 0, st>>>(objs, l.k0);
+        break;
+      case L_FIN:
+        ll_finish_grouped_kernel<<<(unsigned)l.grid, 1024, 0, st>>>(objs, l.ldb, l.infob,
+                                                                    reinterpret_cast<const int64_t*>(td + l.t1), ll, info);
+        break;
+    }
+    if (l.kind != L_DIAG) count_launch();
+    if (e) break;
+  }
+  cudaFreeAsync(td, st);
+  return e ? e : (int)cudaGetLastError();
 }
 
 }  // namespace cgp

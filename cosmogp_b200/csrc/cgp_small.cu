@@ -238,6 +238,7 @@ small_gp_kernel(const SmallArgs a, const int nbm, const int mode) {
     const int n = (int)(a.off[b + 1] - o0);
     const int nb = (n + 7) >> 3;
     const double* amat = a.amat ? a.amat + a.aoff[b] : nullptr;
+    const int64_t lda = (TASK == TASK_MATRICES && a.ld_obj) ? a.ld_obj[b] : a.lda;
     const int64_t io = a.compact_io ? oi : b;
     if (a.hyp_obj) cov = cov_from_hyp(DIM, a.hyp_obj + io * a.n_hyp, a.nugget_obj ? a.nugget_obj[io] : a.nugget_shared,
                                       a.floor_shared, a.flags);
@@ -325,7 +326,7 @@ small_gp_kernel(const SmallArgs a, const int nbm, const int mode) {
         else {
           double r0, r1;
           self_syrk(J, J, r0, r1);
-          k_tile_minus<DIM>(cov, px, noise, ld, n, J, J, L, r0, r1, dk0, dk1, amat, a.lda);
+          k_tile_minus<DIM>(cov, px, noise, ld, n, J, J, L, r0, r1, dk0, dk1, amat, lda);
         }
       }
       // tiles of block column J owned by this warp, two at a time; each tile accumulates its
@@ -367,8 +368,8 @@ small_gp_kernel(const SmallArgs a, const int nbm, const int mode) {
         }
         // both covariance tiles of a pair before either store: their four exp chains interleave in one straight line
         double k0, k1, m0 = 0.0, m1 = 0.0;
-        if (two) k_tile2_minus<DIM>(cov, px, noise, ld, n, I, I2, J, L, a0 + b0, a1 + b1, c0 + d0, c1 + d1, k0, k1, m0, m1, amat, a.lda);
-        else k_tile_minus<DIM>(cov, px, noise, ld, n, I, J, L, a0 + b0, a1 + b1, k0, k1, amat, a.lda);
+        if (two) k_tile2_minus<DIM>(cov, px, noise, ld, n, I, I2, J, L, a0 + b0, a1 + b1, c0 + d0, c1 + d1, k0, k1, m0, m1, amat, lda);
+        else k_tile_minus<DIM>(cov, px, noise, ld, n, I, J, L, a0 + b0, a1 + b1, k0, k1, amat, lda);
         if (I == J) {                                     // warp 0 (only without a dedicated diagonal warp)
           dk0 = k0; dk1 = k1;
         } else {
@@ -379,7 +380,7 @@ small_gp_kernel(const SmallArgs a, const int nbm, const int mode) {
       if (la && warp == WARPS - 1 && J + 1 < nb) {        // next diagonal tile, all but its last rank-8 term
         double r0, r1, k0, k1;
         self_syrk(J + 1, J, r0, r1);
-        k_tile_minus<DIM>(cov, px, noise, ld, n, J + 1, J + 1, L, r0, r1, k0, k1, amat, a.lda);
+        k_tile_minus<DIM>(cov, px, noise, ld, n, J + 1, J + 1, L, r0, r1, k0, k1, amat, lda);
         st_acc(tiles, slot(J + 1, J + 1), L, k0, k1);
       }
       double zw = 0.0;
@@ -608,7 +609,7 @@ small_gp_kernel(const SmallArgs a, const int nbm, const int mode) {
         if (a.logdet) a.logdet[b] = bad ? nan("") : log(lp_m) + (double)lp_e * 0.693147180559945309417232;
       }
       const int64_t mo = a.moff[b];
-      const int64_t mld = a.mld ? a.mld : n;
+      const int64_t mld = a.ld_obj ? lda : (a.mld ? a.mld : n);
       if (a.kmat && !amat) {
         for (int e = tid; e < n * n; e += NT) {
           const int i = e / n, j = e - i * n;

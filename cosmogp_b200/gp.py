@@ -2,7 +2,9 @@
 gaussian_process_nobject (cosmogp/Gaussian_process.py:78-393): same constructor
 arguments, methods, attributes and error behaviour; numpy in, numpy out.  The
 per-object Python loops of the reference (:207, :264, :304, :349) are replaced by
-single batched launches on a device-resident copy of the data.
+single batched launches on a device-resident copy of the data.  Objects above 224 points go through the blocked HBM
+factorisation: one at a time for shared hyperparameters (dense.LargeObject), all at once for the likelihood evaluations
+of per-object fits (cgp_large_ll_objhyp_dev).
 
 Differences (SURVEY.md section 9.1):
   * `svd_method`: every object is factorised by the device Cholesky kernels whatever the flag says (for a
@@ -329,6 +331,9 @@ class Gaussian_process:
         for all objects at once; every evaluation is one device launch.  optimizer='device': the
         simplices live on the device too (cgp_fit_objects_dev, no host round trips); 'host': the numpy
         statement of the same rules (cosmogp_b200.fit), kept as the cross-check -- both give identical results.
+        Objects above 224 points are fitted too: every evaluation factors all of them at once by the grouped blocked
+        factorisation (cgp_large_ll_objhyp_dev), driven by the numpy statement in both modes; with optimizer='device'
+        the objects of up to 224 points still run cgp_fit_objects_dev, on a batch of their own.
         Sets `hyperparameters_per_object` (N_sn, n_hyp), `nugget_per_object` (N_sn,) and
         `log_likelihood_per_object`; an object whose covariance is not positive definite at a trial
         point gets +inf there (the reference would abort with LinAlgError)."""
@@ -350,12 +355,106 @@ class Gaussian_process:
         assert optimizer in ('device', 'host')
         if optimizer == 'device' and not self._is_large:
             x, fval, its, calls = self.batch.fit_objects(x0, nugget=base_nugget, flags=self.flags)
+        elif optimizer == 'device':
+            # objects above 224 points: the small ones on the device optimiser over a batch of their own (their results
+            # are those of a batch of small objects alone), the large ones in lock step over the grouped likelihood
+            small = np.diff(self._off) <= _lib.CGP_SMALL_MAX_N
+            big = np.nonzero(~small)[0]
+            x, fval = np.empty_like(x0), np.empty(self.N_sn)
+            its, calls = np.empty(self.N_sn, dtype=np.int64), np.empty(self.N_sn, dtype=np.int64)
+            if small.any():
+                r = self._small_batch().fit_objects(x0[small], nugget=base_nugget, flags=self.flags)
+                x[small], fval[small], its[small], calls[small] = r
+            r = nelder_mead_lockstep(lambda X, idx: fun(X, big[idx]), x0[big])
+            x[big], fval[big], its[big], calls[big] = r
         else:
             x, fval, its, calls = nelder_mead_lockstep(fun, x0)
         self.hyperparameters_per_object = np.sqrt(x[:, :nh] ** 2)              # abs, like :249-250
         self.nugget_per_object = np.sqrt(x[:, nh] ** 2) if nugget else np.full(self.N_sn, base_nugget)
         self.log_likelihood_per_object = -fval
         self.fit_iterations, self.fit_evaluations = its, calls
+
+    def _small_batch(self):
+        """DeviceBatch of the objects of up to 224 points alone (uploaded once from host slices of the flat arrays):
+        per-object fits and predictions of a batch with larger objects give these objects exactly the results of a
+        batch without them."""
+        if getattr(self, "_small", None) is None:
+            sizes = np.diff(self._off)
+            keep = sizes <= _lib.CGP_SMALL_MAX_N
+            pts = np.repeat(keep, sizes)
+            off = np.zeros(int(keep.sum()) + 1, dtype=np.int64)
+            off[1:] = np.cumsum(sizes[keep])
+            cut = lambda a: None if a is None else np.ascontiguousarray(a[pts])
+            self._small = DeviceBatch(cut(self._x_flat), cut(self._y_flat), off, y0=cut(self._y0_flat),
+                                      y_err=cut(self._ye_flat), dim=self._dim)
+        return self._small
+
+    def _predict_per_object_large(self, new_binning, want_var, has_mean):
+        """get_prediction(per_object=True) on a batch with objects above 224 points: those objects one by one through
+        dense.LargeObject with their own fit, the others in one launch on _small_batch()."""
+        from .dense import LargeObject
+        hyp_b, nug_b = np.asarray(self.hyperparameters_per_object, dtype=float), np.asarray(self.nugget_per_object, dtype=float)
+        sizes = np.diff(self._off)
+        small = sizes <= _lib.CGP_SMALL_MAX_N
+        info = np.zeros(self.N_sn, dtype=np.int32)
+        own = new_binning is None
+        if own:
+            grid = self._x_flat
+            mean = np.empty(len(self._y_flat))
+            var = np.empty(len(self._y_flat)) if want_var else None
+            pts = np.repeat(small, sizes)
+        else:
+            grid = np.ascontiguousarray(new_binning, dtype=np.float64)
+            mean = np.empty((self.N_sn, len(grid)))
+            var = np.empty((self.N_sn, len(grid))) if want_var else None
+            tmpl = _mean.template_on_grid(grid, self._dim, self.Mean_Y, self.Time_mean) if has_mean else None
+        if small.any():
+            sb = self._small_batch()
+            if own:
+                m, v, inf = sb.predict(hyp_b[small], nug_b[small], grid[pts], goff=sb.off_host,
+                                       new_y0=self._y0_flat[pts] if has_mean else None, want_var=want_var, flags=self.flags)
+                mean[pts] = m
+                if want_var:
+                    var[pts] = v
+            else:
+                mt = (np.zeros(len(grid)) if tmpl is None else tmpl, self._diff_used[small]) if has_mean else None
+                m, v, inf = sb.predict(hyp_b[small], nug_b[small], grid, mean_template=mt, want_var=want_var, flags=self.flags)
+                mean[small] = m
+                if want_var:
+                    var[small] = v
+            info[small] = inf
+        for i in np.nonzero(~small)[0]:
+            o0, o1 = int(self._off[i]), int(self._off[i + 1])
+            obj = LargeObject(self._x_flat[o0:o1], self._y_flat[o0:o1], None if self._ye_flat is None else self._ye_flat[o0:o1],
+                              None if self._y0_flat is None else self._y0_flat[o0:o1], dim=self._dim, flags=self.flags)
+            try:
+                obj.factor(hyp_b[i], nug_b[i])
+            except np.linalg.LinAlgError:
+                info[i] = 1
+                continue
+            if own:
+                m, v = obj.predict(grid[o0:o1], new_y0=self._y0_flat[o0:o1] if has_mean else None, want_var=want_var)
+                mean[o0:o1] = m
+                if want_var:
+                    var[o0:o1] = v
+            else:
+                ny0 = ((tmpl if tmpl is not None else 0.0) + self._diff_used[i] * np.ones(len(grid))) if has_mean else None
+                mean[i], v = obj.predict(grid, new_y0=ny0, want_var=want_var)
+                if want_var:
+                    var[i] = v
+        self._raise_if_bad(info)
+        self.as_the_same_time = own
+        if own:
+            self.new_binning = self.Time
+            self.Prediction = RaggedView(mean, self._off)
+            self.prediction_variance = RaggedView(var, self._off) if want_var else None
+            self.warning_pf = self._y0_flat if has_mean else None
+        else:
+            self.new_binning = new_binning
+            rows = np.arange(self.N_sn + 1, dtype=np.int64) * len(grid)
+            self.Prediction = RaggedView(mean.reshape(-1), rows)
+            self.prediction_variance = RaggedView(var.reshape(-1), rows) if want_var else None
+            self.warning_pf = _LazyMeanOnGrid(np.zeros(len(grid)) if tmpl is None else tmpl, self._diff_used) if has_mean else None
 
     # ------------------------------------------------------------------ matrices
     def compute_kernel_matrix(self):
@@ -384,7 +483,9 @@ class Gaussian_process:
         new_binning None -> each object's own epochs.  COV: True (full matrices on
         access + diagonal), 'diag' (diagonal only) or False.  per_object=True predicts every
         object with its own fit (`hyperparameters_per_object`, `nugget_per_object`); COV must then
-        be 'diag' or False."""
+        be 'diag' or False.  With per_object=True, objects above 224 points are factored and predicted one by one
+        by dense.LargeObject, and the others in one launch on a batch of their own, so that their results are those
+        of a batch without the large objects; a covariance that is not positive definite raises LinAlgError."""
         hyp, nug = np.array(self.hyperparameters, dtype=float), float(self.nugget)
         if self._devices is not None:
             assert new_binning is not None and not per_object and COV in ('diag', False) and not self._is_large, \
@@ -397,8 +498,10 @@ class Gaussian_process:
         self.inv_kernel_matrix = _LazyMatrices(self.N_sn, lambda i: self._object_matrices(i, hyp, nug, bool(svd_method))[1])
         want_var = bool(COV)
 
+        if self._is_large and per_object:
+            self._predict_per_object_large(new_binning, want_var, has_mean)
+            return
         if self._is_large:
-            assert not per_object, "per-object hyperparameters are not wired for large objects"
             self.as_the_same_time = new_binning is None
             self.new_binning = self.Time if new_binning is None else new_binning
             self.Prediction, self.prediction_variance = [], ([] if want_var else None)
