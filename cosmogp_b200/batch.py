@@ -6,6 +6,8 @@ every likelihood evaluation of the optimiser, the prediction and the pulls are t
 single batched launches on it.  PyTorch only owns the buffers (pinned staging + device
 tensors) and the stream; all arithmetic is in libcosmogp_b200.so.
 """
+import functools
+
 import numpy as np
 import torch
 
@@ -41,6 +43,40 @@ def pack_csr(seq, dim=1):
     else:
         flat = np.zeros((0, 2) if dim == 2 else (0,), dtype=np.float64)
     return flat, off
+
+
+class SizeSplit:
+    """Which objects of a CSR batch (offsets `off`) the shared-memory kernels take: the "small" ones, of at most
+    CGP_SMALL_MAX_N points.  The others ("large") go through the blocked HBM factorisation.  Small objects run with the
+    largest small size as max_n, so that in a batch with large objects they get exactly the results of a batch without
+    them.  Host only: this is the one place that rule is written down.
+
+      sizes        points per object
+      small        bool mask over the objects
+      large        ids of the large objects, ascending
+      small_max_n  max_n of the small objects (0 when there are none)
+      runs         [(first, end)) ranges of consecutive small objects, maximal
+      points       bool mask over the points: those of small objects
+      small_off    CSR offsets of the small objects alone"""
+
+    def __init__(self, off):
+        self.sizes = np.diff(np.asarray(off, dtype=np.int64))
+        self.small = self.sizes <= _lib.CGP_SMALL_MAX_N
+        self.large = np.nonzero(~self.small)[0]
+        self.small_max_n = int(self.sizes[self.small].max(initial=0))
+        edges = np.concatenate([[-1], self.large, [len(self.sizes)]])
+        self.runs = [(int(a + 1), int(b)) for a, b in zip(edges[:-1], edges[1:]) if b > a + 1]
+
+    # per point: only built when a batch of the small objects alone is needed
+    @functools.cached_property
+    def points(self):
+        return np.repeat(self.small, self.sizes)
+
+    @functools.cached_property
+    def small_off(self):
+        off = np.zeros(int(self.small.sum()) + 1, dtype=np.int64)
+        off[1:] = np.cumsum(self.sizes[self.small])
+        return off
 
 
 class RaggedView(object):
@@ -224,12 +260,11 @@ class DeviceBatch:
                             "ord_h": pin((b,), torch.int32), "ord_d": dev((b,), torch.int32),
                             "ll_h": pin((b,), torch.float64), "ll_d": dev((b,), torch.float64),
                             "info_h": pin((b,), torch.int32), "info_d": dev((b,), torch.int32)}
-            sizes = np.diff(self.off_host)
-            small = sizes <= _lib.CGP_SMALL_MAX_N
-            c["large"] = ~small
-            c["small_max_n"] = self.max_n if small.all() else (int(sizes[small].max()) if small.any() else 0)
-            if c["large"].any():
-                need = np.array([_lib.lib().cgp_large_ll_ws_doubles(int(n)) for n in sizes[c["large"]]], dtype=np.int64)
+            split = SizeSplit(self.off_host)
+            c["large"] = ~split.small
+            c["small_max_n"] = split.small_max_n if len(split.large) else self.max_n
+            if len(split.large):
+                need = np.array([_lib.lib().cgp_large_ll_ws_doubles(int(n)) for n in split.sizes[split.large]], dtype=np.int64)
                 c["work"] = torch.empty(int(max(need.max(), min(need.sum(), (4 << 30) // 8))), dtype=torch.float64,
                                         device=self.device)
         idx = np.asarray(idx, dtype=np.int64)

@@ -198,12 +198,10 @@ def cholesky_inverse(matrix, return_logdet=False):
     return inv
 
 
-def object_matrices(sub, hyp, nugget, flags=0):
-    """kernel_matrix / inv_kernel_matrix of one object too large for the shared-memory path."""
-    obj = LargeObject(sub.x.cpu().numpy(), np.zeros(sub.n_pts), None if sub.y_err is None else sub.y_err.cpu().numpy(),
-                      dim=sub.dim, flags=flags)
-    k = covariance(sub.x.cpu().numpy(), hyp, sub.dim, nugget=nugget,
-                   y_err=None if sub.y_err is None else sub.y_err.cpu().numpy(), flags=flags)
+def object_matrices(x, y_err, hyp, nugget, dim, flags=0):
+    """kernel_matrix / inv_kernel_matrix of one object too large for the shared-memory path (host arrays in and out)."""
+    obj = LargeObject(x, np.zeros(len(x)), y_err, dim=dim, flags=flags)
+    k = covariance(x, hyp, dim, nugget=nugget, y_err=y_err, flags=flags)
     obj.factor(hyp, nugget)
     return k, obj.inverse()
 

@@ -2,9 +2,10 @@
 gaussian_process_nobject (cosmogp/Gaussian_process.py:78-393): same constructor
 arguments, methods, attributes and error behaviour; numpy in, numpy out.  The
 per-object Python loops of the reference (:207, :264, :304, :349) are replaced by
-single batched launches on a device-resident copy of the data.  Objects above 224 points go through the blocked HBM
-factorisation: one at a time for shared hyperparameters (dense.LargeObject), all at once for the likelihood evaluations
-of per-object fits (cgp_large_ll_objhyp_dev).
+single batched launches on a device-resident copy of the data.  Which objects are too large for those launches is
+decided in one place, batch.SizeSplit; they go through the blocked HBM factorisation: one at a time for shared
+hyperparameters (dense.LargeObject, every object of the batch then), all at once for the likelihood evaluations of
+per-object fits (cgp_large_ll_objhyp_dev), one at a time for per-object predictions.
 
 Differences (SURVEY.md section 9.1):
   * `svd_method`: every object is factorised by the device Cholesky kernels whatever the flag says (for a
@@ -29,7 +30,7 @@ from scipy.optimize import fmin
 
 from . import _lib
 from . import mean as _mean
-from .batch import DeviceBatch, RaggedView, pack_csr
+from .batch import DeviceBatch, RaggedView, SizeSplit, pack_csr
 from .kernel import init_rbf, rbf_kernel_1d, rbf_kernel_2d
 
 
@@ -106,6 +107,7 @@ class Gaussian_process:
         self._x_flat, self._off = pack_csr(Time, self._dim)
         self._y_flat, off_y = pack_csr(y, 1)
         assert np.array_equal(self._off, off_y), 'y and Time should have the same structure'
+        self._split = SizeSplit(self._off)
         if y_err is not None:
             self.y_err = y_err
             self._ye_flat, off_e = pack_csr(y_err, 1)
@@ -151,6 +153,7 @@ class Gaussian_process:
         sigma, L = init_rbf(Time, y)                     # the global initial guess (quirk Q6 uses the LAST object)
         obj.hyperparameters = np.array([sigma, L]) if obj._dim == 1 else np.array([sigma, L, L, 0.])
         obj._dist, obj.local_range, obj.N_total, obj._all_sizes = True, (a, b), len(y), sizes
+        obj._all_split = SizeSplit(np.concatenate([[0], np.cumsum(sizes, dtype=np.int64)]))
         return obj
 
     def gather(self, per_object_arrays, root=None):
@@ -187,28 +190,31 @@ class Gaussian_process:
         return self._batch
 
     @property
-    def _is_large(self):
-        """Objects beyond the shared-memory path (N > 224) go one by one through the HBM-resident
-        blocked factorisation (cosmogp_b200.dense.LargeObject).  Sharded objects decide from the sizes of ALL
-        objects, so that every rank takes the same branch (and the same collectives)."""
-        sizes = self._all_sizes if self._dist else np.diff(self._off)
-        return len(sizes) > 0 and int(np.max(sizes)) > _lib.CGP_SMALL_MAX_N
+    def _any_large(self):
+        """With shared hyperparameters, a batch with any large object (batch.SizeSplit) goes one object at a time
+        through the HBM-resident blocked factorisation (`_large_objects`).  Sharded objects decide from the sizes of
+        ALL objects, so that every rank takes the same branch (and the same collectives)."""
+        return len((self._all_split if self._dist else self._split).large) > 0
 
     @property
     def _device(self):
         import torch
         return torch.device("cuda", torch.cuda.current_device())
 
+    def _object_slices(self, i):
+        """host views x, y, y_err, y0 of object i (y_err and y0 are None when the batch has none)"""
+        o0, o1 = int(self._off[i]), int(self._off[i + 1])
+        return tuple(None if a is None else a[o0:o1] for a in (self._x_flat, self._y_flat, self._ye_flat, self._y0_flat))
+
+    def _large_object(self, i):
+        """dense.LargeObject of object i; its n_pad^2 factor lives as long as the object"""
+        from .dense import LargeObject
+        return LargeObject(*self._object_slices(i), dim=self._dim, flags=self.flags)
+
     def _large_objects(self):
+        """one LargeObject per object, kept: fits with shared hyperparameters evaluate them hundreds of times"""
         if getattr(self, "_large", None) is None:
-            from .dense import LargeObject
-            self._large = []
-            for i in range(self.N_sn):
-                o0, o1 = self._off[i], self._off[i + 1]
-                self._large.append(LargeObject(
-                    self._x_flat[o0:o1], self._y_flat[o0:o1],
-                    None if self._ye_flat is None else self._ye_flat[o0:o1],
-                    None if self._y0_flat is None else self._y0_flat[o0:o1], dim=self._dim, flags=self.flags))
+            self._large = [self._large_object(i) for i in range(self.N_sn)]
         return self._large
 
     @staticmethod
@@ -228,7 +234,7 @@ class Gaussian_process:
         else:
             Nugget = self.nugget
             hyperparameter = Hyperparameter
-        if self._is_large:
+        if self._any_large:
             per_object, info = np.zeros(self.N_sn), np.zeros(self.N_sn, dtype=np.int32)
             for i, o in enumerate(self._large_objects()):
                 try:
@@ -278,10 +284,8 @@ class Gaussian_process:
         Gaussian_process.py:59-73 and :332-361."""
         import warnings
         from .inv_matrix import svd_inverse
-        o0, o1 = int(self._off[i]), int(self._off[i + 1])
-        x, y = self._x_flat[o0:o1], self._y_flat[o0:o1]
-        ye = None if self._ye_flat is None else self._ye_flat[o0:o1]
-        r = y - (self._y0_flat[o0:o1] if self._y0_flat is not None else 0.0)
+        x, y, ye, y0 = self._object_slices(i)
+        r = y - (y0 if y0 is not None else 0.0)
         kw = {"flags": self.flags} if self._dim == 2 else {}
         hyp = np.asarray(hyperparameter, dtype=float)
         warnings.warn("covariance of object %d is not positive definite: pseudo-inverse by the host SVD reference "
@@ -353,20 +357,16 @@ class Gaussian_process:
             return f
 
         assert optimizer in ('device', 'host')
-        if optimizer == 'device' and not self._is_large:
-            x, fval, its, calls = self.batch.fit_objects(x0, nugget=base_nugget, flags=self.flags)
-        elif optimizer == 'device':
-            # objects above 224 points: the small ones on the device optimiser over a batch of their own (their results
-            # are those of a batch of small objects alone), the large ones in lock step over the grouped likelihood
-            small = np.diff(self._off) <= _lib.CGP_SMALL_MAX_N
-            big = np.nonzero(~small)[0]
+        if optimizer == 'device':
+            # small objects on the device optimiser, large ones in lock step over the grouped likelihood
+            small, big = self._split.small, self._split.large
             x, fval = np.empty_like(x0), np.empty(self.N_sn)
             its, calls = np.empty(self.N_sn, dtype=np.int64), np.empty(self.N_sn, dtype=np.int64)
-            if small.any():
-                r = self._small_batch().fit_objects(x0[small], nugget=base_nugget, flags=self.flags)
-                x[small], fval[small], its[small], calls[small] = r
-            r = nelder_mead_lockstep(lambda X, idx: fun(X, big[idx]), x0[big])
-            x[big], fval[big], its[big], calls[big] = r
+            sb = self._small_batch()
+            if sb is not None:
+                x[small], fval[small], its[small], calls[small] = sb.fit_objects(x0[small], nugget=base_nugget, flags=self.flags)
+            if len(big):
+                x[big], fval[big], its[big], calls[big] = nelder_mead_lockstep(lambda X, idx: fun(X, big[idx]), x0[big])
         else:
             x, fval, its, calls = nelder_mead_lockstep(fun, x0)
         self.hyperparameters_per_object = np.sqrt(x[:, :nh] ** 2)              # abs, like :249-250
@@ -375,86 +375,19 @@ class Gaussian_process:
         self.fit_iterations, self.fit_evaluations = its, calls
 
     def _small_batch(self):
-        """DeviceBatch of the objects of up to 224 points alone (uploaded once from host slices of the flat arrays):
-        per-object fits and predictions of a batch with larger objects give these objects exactly the results of a
-        batch without them."""
+        """The batch per-object fits and predictions run their small objects (batch.SizeSplit) on: `self.batch` when no
+        object is large, None when every object is, and otherwise a DeviceBatch of the small objects alone, uploaded
+        once from host slices, so that they get exactly the results of a batch without the large objects."""
+        split = self._split
+        if not len(split.large):
+            return self.batch
+        if not split.small.any():
+            return None
         if getattr(self, "_small", None) is None:
-            sizes = np.diff(self._off)
-            keep = sizes <= _lib.CGP_SMALL_MAX_N
-            pts = np.repeat(keep, sizes)
-            off = np.zeros(int(keep.sum()) + 1, dtype=np.int64)
-            off[1:] = np.cumsum(sizes[keep])
-            cut = lambda a: None if a is None else np.ascontiguousarray(a[pts])
-            self._small = DeviceBatch(cut(self._x_flat), cut(self._y_flat), off, y0=cut(self._y0_flat),
+            cut = lambda a: None if a is None else np.ascontiguousarray(a[split.points])
+            self._small = DeviceBatch(cut(self._x_flat), cut(self._y_flat), split.small_off, y0=cut(self._y0_flat),
                                       y_err=cut(self._ye_flat), dim=self._dim)
         return self._small
-
-    def _predict_per_object_large(self, new_binning, want_var, has_mean):
-        """get_prediction(per_object=True) on a batch with objects above 224 points: those objects one by one through
-        dense.LargeObject with their own fit, the others in one launch on _small_batch()."""
-        from .dense import LargeObject
-        hyp_b, nug_b = np.asarray(self.hyperparameters_per_object, dtype=float), np.asarray(self.nugget_per_object, dtype=float)
-        sizes = np.diff(self._off)
-        small = sizes <= _lib.CGP_SMALL_MAX_N
-        info = np.zeros(self.N_sn, dtype=np.int32)
-        own = new_binning is None
-        if own:
-            grid = self._x_flat
-            mean = np.empty(len(self._y_flat))
-            var = np.empty(len(self._y_flat)) if want_var else None
-            pts = np.repeat(small, sizes)
-        else:
-            grid = np.ascontiguousarray(new_binning, dtype=np.float64)
-            mean = np.empty((self.N_sn, len(grid)))
-            var = np.empty((self.N_sn, len(grid))) if want_var else None
-            tmpl = _mean.template_on_grid(grid, self._dim, self.Mean_Y, self.Time_mean) if has_mean else None
-        if small.any():
-            sb = self._small_batch()
-            if own:
-                m, v, inf = sb.predict(hyp_b[small], nug_b[small], grid[pts], goff=sb.off_host,
-                                       new_y0=self._y0_flat[pts] if has_mean else None, want_var=want_var, flags=self.flags)
-                mean[pts] = m
-                if want_var:
-                    var[pts] = v
-            else:
-                mt = (np.zeros(len(grid)) if tmpl is None else tmpl, self._diff_used[small]) if has_mean else None
-                m, v, inf = sb.predict(hyp_b[small], nug_b[small], grid, mean_template=mt, want_var=want_var, flags=self.flags)
-                mean[small] = m
-                if want_var:
-                    var[small] = v
-            info[small] = inf
-        for i in np.nonzero(~small)[0]:
-            o0, o1 = int(self._off[i]), int(self._off[i + 1])
-            obj = LargeObject(self._x_flat[o0:o1], self._y_flat[o0:o1], None if self._ye_flat is None else self._ye_flat[o0:o1],
-                              None if self._y0_flat is None else self._y0_flat[o0:o1], dim=self._dim, flags=self.flags)
-            try:
-                obj.factor(hyp_b[i], nug_b[i])
-            except np.linalg.LinAlgError:
-                info[i] = 1
-                continue
-            if own:
-                m, v = obj.predict(grid[o0:o1], new_y0=self._y0_flat[o0:o1] if has_mean else None, want_var=want_var)
-                mean[o0:o1] = m
-                if want_var:
-                    var[o0:o1] = v
-            else:
-                ny0 = ((tmpl if tmpl is not None else 0.0) + self._diff_used[i] * np.ones(len(grid))) if has_mean else None
-                mean[i], v = obj.predict(grid, new_y0=ny0, want_var=want_var)
-                if want_var:
-                    var[i] = v
-        self._raise_if_bad(info)
-        self.as_the_same_time = own
-        if own:
-            self.new_binning = self.Time
-            self.Prediction = RaggedView(mean, self._off)
-            self.prediction_variance = RaggedView(var, self._off) if want_var else None
-            self.warning_pf = self._y0_flat if has_mean else None
-        else:
-            self.new_binning = new_binning
-            rows = np.arange(self.N_sn + 1, dtype=np.int64) * len(grid)
-            self.Prediction = RaggedView(mean.reshape(-1), rows)
-            self.prediction_variance = RaggedView(var.reshape(-1), rows) if want_var else None
-            self.warning_pf = _LazyMeanOnGrid(np.zeros(len(grid)) if tmpl is None else tmpl, self._diff_used) if has_mean else None
 
     # ------------------------------------------------------------------ matrices
     def compute_kernel_matrix(self):
@@ -463,12 +396,11 @@ class Gaussian_process:
         self.kernel_matrix = _LazyMatrices(self.N_sn, lambda i: self._object_matrices(i, hyp, nug, True)[0])
 
     def _object_matrices(self, i, hyp, nug, svd=False):
-        o0, o1 = self._off[i], self._off[i + 1]
-        sub = DeviceBatch(self._x_flat[o0:o1], self._y_flat[o0:o1], np.array([0, o1 - o0], dtype=np.int64),
-                          y_err=None if self._ye_flat is None else self._ye_flat[o0:o1], dim=self._dim)
-        if sub.max_n > _lib.CGP_SMALL_MAX_N:
+        x, y, ye, _ = self._object_slices(i)
+        if not self._split.small[i]:
             from . import dense
-            return dense.object_matrices(sub, hyp, nug, self.flags)
+            return dense.object_matrices(x, ye, hyp, nug, self._dim, self.flags)
+        sub = DeviceBatch(x, y, np.array([0, len(y)], dtype=np.int64), y_err=ye, dim=self._dim)
         k, kinv, info = sub.matrices(hyp, nug, flags=self.flags)
         if info.any() and svd:                              # inv_kernel_matrix of the reference's default path (:319-320)
             from .inv_matrix import svd_inverse
@@ -483,100 +415,107 @@ class Gaussian_process:
         new_binning None -> each object's own epochs.  COV: True (full matrices on
         access + diagonal), 'diag' (diagonal only) or False.  per_object=True predicts every
         object with its own fit (`hyperparameters_per_object`, `nugget_per_object`); COV must then
-        be 'diag' or False.  With per_object=True, objects above 224 points are factored and predicted one by one
-        by dense.LargeObject, and the others in one launch on a batch of their own, so that their results are those
-        of a batch without the large objects; a covariance that is not positive definite raises LinAlgError."""
-        hyp, nug = np.array(self.hyperparameters, dtype=float), float(self.nugget)
+        be 'diag' or False.  Objects go down one of three routes, by batch.SizeSplit: the batched kernels; one
+        dense.LargeObject at a time (the large objects of a per-object prediction, or every object of a batch with a
+        large one under shared hyperparameters); and, under shared hyperparameters with svd_method=True, the host SVD
+        redo of the objects whose covariance is not positive definite.  Otherwise such an object raises LinAlgError."""
         if self._devices is not None:
-            assert new_binning is not None and not per_object and COV in ('diag', False) and not self._is_large, \
+            assert new_binning is not None and not per_object and COV in ('diag', False) and not self._any_large, \
                 "with devices=... predictions are on a shared grid with COV='diag' or False"
         if per_object:
             assert COV in ('diag', False), "per_object predictions provide the variance diagonal only"
-            hyp_b, nug_b = self.hyperparameters_per_object, self.nugget_per_object
         has_mean = self.substract_mean or self.Mean_Y is not None
-        self.compute_kernel_matrix()
-        self.inv_kernel_matrix = _LazyMatrices(self.N_sn, lambda i: self._object_matrices(i, hyp, nug, bool(svd_method))[1])
         want_var = bool(COV)
 
-        if self._is_large and per_object:
-            self._predict_per_object_large(new_binning, want_var, has_mean)
-            return
-        if self._is_large:
-            self.as_the_same_time = new_binning is None
-            self.new_binning = self.Time if new_binning is None else new_binning
-            self.Prediction, self.prediction_variance = [], ([] if want_var else None)
-            for i, obj in enumerate(self._large_objects()):
-                o0, o1 = self._off[i], self._off[i + 1]
-                try:
-                    obj.factor(hyp, nug)
-                    failed = False
-                except np.linalg.LinAlgError:
-                    if not svd_method:
-                        raise
-                    failed = True
-                if new_binning is None:
-                    grid, ny0 = self._x_flat[o0:o1], (self._y0_flat[o0:o1] if has_mean else None)
-                else:
-                    grid = np.ascontiguousarray(new_binning, dtype=np.float64)
-                    ny0 = None
-                    if has_mean:
-                        tmpl = _mean.template_on_grid(grid, self._dim, self.Mean_Y, self.Time_mean)
-                        ny0 = (tmpl if tmpl is not None else 0.0) + self._diff_used[i] * np.ones(len(grid))
-                if failed:
-                    _, m, v = self._svd_object(i, hyp, nug, grid, 0.0 if ny0 is None else ny0, want_var)
-                else:
-                    m, v = obj.predict(grid, new_y0=ny0, want_var=want_var)
-                self.Prediction.append(m)
-                if want_var:
-                    self.prediction_variance.append(v)
-            if COV is True:
-                self.get_covariance_matrix()
-            return
+        # hyperparameters: shared, or one row per object
+        hyp, nug = np.array(self.hyperparameters, dtype=float), float(self.nugget)
+        if per_object:
+            hyp_b, nug_b = np.asarray(self.hyperparameters_per_object, dtype=float), np.asarray(self.nugget_per_object, dtype=float)
+        self.compute_kernel_matrix()
+        self.inv_kernel_matrix = _LazyMatrices(self.N_sn, lambda i: self._object_matrices(i, hyp, nug, bool(svd_method))[1])
 
-        if new_binning is None:
-            self.as_the_same_time = True
-            self.new_binning = self.Time
-            grid, goff = self._x_flat, self._off
+        # the grid and the mean function on it; the outputs of object i are mean[rows[i]:rows[i + 1]]
+        own = new_binning is None
+        if own:
+            grid, rows = self._x_flat, self._off
             new_y0 = self._y0_flat if has_mean else None                   # :308-309
-            mean, var, info = self.batch.predict(hyp_b if per_object else hyp, nug_b if per_object else nug, grid,
-                                                 goff=goff, new_y0=new_y0, want_var=want_var, flags=self.flags)
-            if info.any() and svd_method and not per_object:
-                for i in np.nonzero(info)[0]:
-                    sl = slice(int(goff[i]), int(goff[i + 1]))
-                    _, mean[sl], v = self._svd_object(int(i), hyp, nug, grid[sl], new_y0[sl] if has_mean else 0.0, want_var)
-                    if want_var:
-                        var[sl] = v
-                info = np.zeros_like(info)
-            self._raise_if_bad(info)
-            self.Prediction = RaggedView(mean, goff)
-            self.prediction_variance = RaggedView(var, goff) if want_var else None
         else:
-            self.as_the_same_time = False
-            self.new_binning = new_binning
             grid = np.ascontiguousarray(new_binning, dtype=np.float64)
-            m = len(grid)
-            new_y0 = mean_template = None
+            rows = np.arange(self.N_sn + 1, dtype=np.int64) * len(grid)
+            new_y0 = None
             if has_mean:                                                    # :310-312 via mean.py:92-101
                 # mean on the grid = template(grid) + diff[sn]; without a template return_mean hands back
                 # y0 (= diff) for any new_x.  Only the M template values and the N_sn offsets are uploaded.
                 tmpl = _mean.template_on_grid(grid, self._dim, self.Mean_Y, self.Time_mean)
-                mean_template = (np.zeros(m) if tmpl is None else tmpl, self._diff_used)
-                new_y0 = _LazyMeanOnGrid(*mean_template)
-            kw = {"gather": self.gather_over_nvlink} if self._devices is not None else {}
-            mean, var, info = self.batch.predict(hyp_b if per_object else hyp, nug_b if per_object else nug, grid,
-                                                 mean_template=mean_template, want_var=want_var, flags=self.flags, **kw)
-            if info.any() and svd_method and not per_object:
-                for i in np.nonzero(info)[0]:
-                    ny0 = (mean_template[0] + mean_template[1][i]) if has_mean else 0.0
-                    _, mean[i], v = self._svd_object(int(i), hyp, nug, grid, ny0, want_var)
-                    if want_var:
-                        var[i] = v
-                info = np.zeros_like(info)
-            self._raise_if_bad(info)
-            # list-like row views built in O(1) (a real list of 10^5 row arrays costs ~15 ms)
-            rows = np.arange(self.N_sn + 1, dtype=np.int64) * m
-            self.Prediction = RaggedView(mean.reshape(-1), rows)
-            self.prediction_variance = RaggedView(var.reshape(-1), rows) if want_var else None
+                new_y0 = _LazyMeanOnGrid(np.zeros(len(grid)) if tmpl is None else tmpl, self._diff_used)
+
+        def on_grid(i):
+            """object i's grid and the mean function on it (None: zero)"""
+            if own:
+                s = slice(int(rows[i]), int(rows[i + 1]))
+                return grid[s], (None if new_y0 is None else new_y0[s])
+            return grid, (None if new_y0 is None else new_y0[i])
+
+        # routes: the batched kernels on `batched`, one LargeObject at a time for `one_by_one`
+        split = self._split
+        if per_object:
+            batched, one_by_one = self._small_batch(), split.large
+        elif self._any_large:
+            batched, one_by_one = None, range(self.N_sn)
+        else:
+            batched, one_by_one = self.batch, ()
+        whole = batched is not None and not len(one_by_one)      # the batched outputs are the outputs
+        if not whole:
+            mean, info = np.empty(int(rows[-1])), np.zeros(self.N_sn, dtype=np.int32)
+            var = np.empty(int(rows[-1])) if want_var else None
+        if batched is not None:
+            # the objects and points it holds: all of them, or the small ones of a mixed batch
+            objs, pts = (slice(None), slice(None)) if whole else (split.small, split.points)
+            if own:
+                kw = {"goff": batched.off_host, "new_y0": None if new_y0 is None else new_y0[pts]}
+            else:
+                kw = {"mean_template": None if new_y0 is None else (new_y0.template, new_y0.diff[objs])}
+            if self._devices is not None:
+                kw["gather"] = self.gather_over_nvlink
+            m, v, inf = batched.predict(hyp_b[objs] if per_object else hyp, nug_b[objs] if per_object else nug,
+                                        grid[pts] if own else grid, want_var=want_var, flags=self.flags, **kw)
+            if whole:
+                mean, var, info = m.reshape(-1), (v.reshape(-1) if want_var else None), inf
+            else:
+                at = pts if own else np.repeat(objs, len(grid))
+                mean[at] = m.reshape(-1)
+                if want_var:
+                    var[at] = v.reshape(-1)
+                info[objs] = inf
+        for i in one_by_one:
+            obj = self._large_object(i) if per_object else self._large_objects()[i]
+            try:
+                obj.factor(hyp_b[i] if per_object else hyp, nug_b[i] if per_object else nug)
+            except np.linalg.LinAlgError:
+                if not (per_object or svd_method):
+                    raise
+                info[i] = 1
+                continue
+            s = slice(int(rows[i]), int(rows[i + 1]))
+            g, ny0 = on_grid(i)
+            mean[s], v = obj.predict(g, new_y0=ny0, want_var=want_var)
+            if want_var:
+                var[s] = v
+        if info.any() and svd_method and not per_object:
+            for i in np.nonzero(info)[0]:
+                s = slice(int(rows[i]), int(rows[i + 1]))
+                g, ny0 = on_grid(i)
+                _, mean[s], v = self._svd_object(int(i), hyp, nug, g, 0.0 if ny0 is None else ny0, want_var)
+                if want_var:
+                    var[s] = v
+            info = np.zeros_like(info)
+        self._raise_if_bad(info)
+
+        self.as_the_same_time = own
+        self.new_binning = self.Time if own else new_binning
+        # list-like views built in O(1) (a real list of 10^5 row arrays costs ~15 ms)
+        self.Prediction = RaggedView(mean, rows)
+        self.prediction_variance = RaggedView(var, rows) if want_var else None
         self.warning_pf = new_y0
         if COV is True:
             self.get_covariance_matrix()

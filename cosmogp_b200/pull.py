@@ -2,14 +2,14 @@
 
 The reference refits the GP N times per object on N-1 points (pull.py:66-90, O(N^4));
 here one factorisation per object gives every leave-one-out prediction and variance in
-closed form from K^-1 (SURVEY.md section 8 row a8), all objects in one launch.  Objects above CGP_SMALL_MAX_N
-points are factorised in HBM one at a time (dense.LargeLoo) in the same call, with no size limit.
+closed form from K^-1 (SURVEY.md section 8 row a8), all objects in one launch.  The objects batch.SizeSplit calls
+large are factorised in HBM one at a time (dense.LargeLoo) in the same call, with no size limit.
 """
 import numpy as np
 
 from . import _lib
 from . import mean as _mean
-from .batch import DeviceBatch, RaggedView, pack_csr
+from .batch import DeviceBatch, RaggedView, SizeSplit, pack_csr
 
 
 class build_pull:
@@ -88,12 +88,22 @@ class build_pull:
             self._results.append({"batch": None, "off": off, "pull": pull, "residual": resid, "prediction": pred,
                                   "prediction_variance": pvar, "sums": mom, "n": len(pull)})
         else:
-            if np.diff(off).max(initial=0) <= _lib.CGP_SMALL_MAX_N:
-                batch = DeviceBatch(x_flat, y_flat, off, y0=template, y_err=ye_flat, dim=dim)
-                pred, pvar, pull, resid, info = batch.loo_dev(self.hyperparameters, self.nugget, mode=mode, flags=self.flags)
-                info = batch._down(info)
-            else:
-                batch, (pred, pvar, pull, resid), info = self._loo_by_size(x_flat, y_flat, off, template, ye_flat, dim, mode)
+            # one upload; the shared-memory kernel runs once per run of consecutive small objects, in place, with their
+            # own largest size as max_n; the large objects read and write their slices of the same arrays
+            split = SizeSplit(off)
+            batch = DeviceBatch(x_flat, y_flat, off, y0=template, y_err=ye_flat, dim=dim, max_n=split.small_max_n)
+            hyp, nug = self.hyperparameters, self.nugget
+            outs = batch.loo_dev(hyp, nug, mode=mode, flags=self.flags, ranges=split.runs)
+            if len(split.large):
+                from .dense import LargeLoo
+                loo = LargeLoo(int(split.sizes[split.large].max()), dim, flags=self.flags)
+                for i in split.large:
+                    p0, p1 = int(off[i]), int(off[i + 1])
+                    x, y, m, e = (None if t is None else t[p0:p1] for t in (batch.x, batch.y, batch.y0, batch.y_err))
+                    loo.run(x, y, m, e, np.asarray(hyp)[i] if np.ndim(hyp) == 2 else hyp,
+                            np.asarray(nug)[i] if np.ndim(nug) == 1 else nug, mode, outs[4][i:i + 1], [o[p0:p1] for o in outs[:4]])
+            pred, pvar, pull, resid = outs[:4]
+            info = batch._down(outs[4])            # every object's status, checked once after everything is launched
             bad = np.nonzero(info)[0]
             if len(bad):
                 raise np.linalg.LinAlgError("covariance of object %d is not positive definite" % int(bad[0]))
@@ -121,32 +131,6 @@ class build_pull:
                                           - (sum(p[0] for p in parts) / n_tot) ** 2))
         else:
             self.pull_average = self.pull_std = float("nan")
-
-    def _loo_by_size(self, x_flat, y_flat, off, template, ye_flat, dim, mode):
-        """Objects of up to CGP_SMALL_MAX_N points through the batched shared-memory kernel, one launch per run of
-        consecutive small objects, larger ones one at a time through dense.LargeLoo.  Everything reads the one
-        DeviceBatch of the whole call and writes straight into its outputs.  -> that DeviceBatch, the four outputs as
-        device tensors over all points in the original order, and the host info of every object (checked once, after
-        everything is launched)."""
-        sizes = np.diff(off)
-        is_large = sizes > _lib.CGP_SMALL_MAX_N
-        large = np.nonzero(is_large)[0]
-        # max_n of the small objects: the kernel (and so every bit of the small objects' outputs) is the one a batch
-        # of the small objects alone would get
-        batch = DeviceBatch(x_flat, y_flat, off, y0=template, y_err=ye_flat, dim=dim,
-                            max_n=int(sizes[~is_large].max(initial=0)))
-        edges = np.concatenate([[-1], large, [len(sizes)]])
-        runs = [(int(a + 1), int(b)) for a, b in zip(edges[:-1], edges[1:]) if b > a + 1]
-        hyp, nug = self.hyperparameters, self.nugget
-        outs = batch.loo_dev(hyp, nug, mode=mode, flags=self.flags, ranges=runs)
-        from .dense import LargeLoo
-        loo = LargeLoo(int(sizes[large].max()), dim, flags=self.flags)
-        for i in large:
-            p0, p1 = int(off[i]), int(off[i + 1])
-            x, y, m, e = (None if t is None else t[p0:p1] for t in (batch.x, batch.y, batch.y0, batch.y_err))
-            loo.run(x, y, m, e, np.asarray(hyp)[i] if np.ndim(hyp) == 2 else hyp,
-                    np.asarray(nug)[i] if np.ndim(nug) == 1 else nug, mode, outs[4][i:i + 1], [o[p0:p1] for o in outs[:4]])
-        return batch, outs[:4], batch._down(outs[4])
 
     # ---- results, brought to the host when read (10^6 x 40 pulls are 320 MB per array)
     def _flat(self, name):

@@ -163,3 +163,32 @@ def test_pack_csr_fast_path_equals_per_object_conversion():
     # equal-length objects handed over as one ndarray
     x = rng.standard_normal((5, 7)); f, o = pack_csr(x, 1)
     assert np.array_equal(f, x.ravel()) and np.array_equal(o, np.arange(6) * 7)
+
+
+def test_size_split():
+    """batch.SizeSplit, the one statement of which objects the shared-memory kernels take (at most 224 points): the mask,
+    the large ids, max_n of the small objects, their maximal runs, their points and their CSR offsets alone."""
+    from cosmogp_b200.batch import SizeSplit
+
+    def check(sizes, large, runs):
+        off = np.concatenate([[0], np.cumsum(sizes, dtype=np.int64)])
+        s = SizeSplit(off)
+        small = np.array([n <= 224 for n in sizes], dtype=bool)
+        assert np.array_equal(s.small, small) and s.small.dtype == bool
+        assert list(s.large) == large and s.runs == runs
+        assert s.small_max_n == max([n for n in sizes if n <= 224], default=0)
+        assert np.array_equal(s.points, np.repeat(small, np.asarray(sizes, dtype=np.int64)))
+        assert s.small_off.dtype == np.int64
+        assert list(s.small_off) == [0] + list(np.cumsum([n for n in sizes if n <= 224], dtype=np.int64))
+        # every small object exactly once, in order, and the runs hold nothing else
+        assert [i for a, b in runs for i in range(a, b)] == list(np.nonzero(small)[0])
+
+    check([], [], [])
+    check([5, 224, 60], [], [(0, 3)])                                       # all small: one run, max_n 224
+    check([225, 400, 1000], [0, 1, 2], [])                                  # all large: no run, max_n 0
+    check([300, 5, 7], [0], [(1, 3)])                                       # large first
+    check([5, 7, 300], [2], [(0, 2)])                                       # large last
+    check([5, 225, 226, 9, 224], [1, 2], [(0, 1), (3, 5)])                  # large ones adjacent; 224 small, 225 large
+    check([0, 225, 3, 400, 0], [1, 3], [(0, 1), (2, 3), (4, 5)])            # empty objects are small
+    check([224], [], [(0, 1)])
+    check([225], [0], [])
