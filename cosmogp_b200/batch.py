@@ -462,10 +462,12 @@ class DeviceBatch:
     def covariance(self, hyp, nugget, grid=None, objects=None, floor=0.0, flags=0):
         """covariance_matrix of the objects [i0, i1) (default: all) in ONE call (cgp_covariance_batched_dev):
         grid given (host array, shared by all objects) -> (k, M, M) host array; grid None -> every object on its own
-        epochs (new_binning=None) -> list of (N_b, N_b) host arrays.  Objects of <= 64 points."""
+        epochs (new_binning=None) -> list of (N_b, N_b) host arrays.  Objects of <= 64 points.
+        hyp (B, nh) with an optional (B,) nugget: object b with its own row, as in predict_dev (cgp_covariance_objhyp_dev)."""
         i0, i1 = (0, self.n_obj) if objects is None else (int(objects[0]), int(objects[1]))
         k = i1 - i0
-        h = self._hyp(hyp)
+        oh = self._objhyp(hyp, nugget)
+        h = None if oh is not None else self._hyp(hyp)
         own = grid is None
         if own:
             g, goff, m = self.x, self.off, 0
@@ -479,12 +481,19 @@ class DeviceBatch:
             m = int(g.shape[0]); tot = k * m * m
             goff_ptr = goff_host_ptr = coff_ptr = None
         out = torch.empty(max(tot, 1), dtype=torch.float64, device=self.device)
+        batch_args = (k, self.off.data_ptr() + 8 * i0, self.max_n, self.dim, self._p(self.x), self._p(self.y_err))
+        out_args = (self._p(g), goff_ptr, goff_host_ptr, m, self._p(out), coff_ptr, self._info.data_ptr() + 4 * i0,
+                    self._stream())
         with torch.cuda.device(self.device):
-            rc = _lib.lib().cgp_covariance_batched_dev(k, self.off.data_ptr() + 8 * i0, self.max_n, self.dim, self._p(self.x),
-                                                       self._p(self.y_err), _lib.hptr(h), float(nugget), float(floor), int(flags),
-                                                       self._p(g), goff_ptr, goff_host_ptr, m, self._p(out), coff_ptr,
-                                                       self._info.data_ptr() + 4 * i0, self._stream())
-        _lib.check(rc, "cgp_covariance_batched_dev")
+            if oh is not None:
+                nh = 2 if self.dim == 1 else 4
+                rc = _lib.lib().cgp_covariance_objhyp_dev(*batch_args, self._p(oh[0]) + 8 * nh * i0,
+                                                          None if oh[1] is None else self._p(oh[1]) + 8 * i0, oh[2],
+                                                          float(floor), int(flags), *out_args)
+            else:
+                rc = _lib.lib().cgp_covariance_batched_dev(*batch_args, _lib.hptr(h), float(nugget), float(floor), int(flags),
+                                                           *out_args)
+        _lib.check(rc, "cgp_covariance_objhyp_dev" if oh is not None else "cgp_covariance_batched_dev")
         flat = self._down(out[:tot], sync=False)
         info = self._down(self._info[i0:i1], sync=False)
         self._sync()

@@ -602,20 +602,28 @@ int cgp_loo_batched_host(int64_t n_obj, const int64_t* off, int dim,
 }
 
 // ------------------------------------------------------------------------------------ predictive covariance, in bulk
-int cgp_covariance_batched_dev(int64_t n_obj, const int64_t* off, int max_n, int dim,
-                               const double* x, const double* y_err,
-                               const double* hyp, double nugget, double floor, unsigned flags,
-                               const double* xnew, const int64_t* goff, const int64_t* goff_host, int64_t m_shared,
-                               double* cov, const int64_t* coff, int* info, void* stream) {
-  if (n_obj < 0 || (n_obj && (!off || !x || !xnew || !cov || !info))) return fail(CGP_ERR_ARG, "cgp_covariance_batched_dev: NULL argument");
-  if (goff && (!goff_host || !coff)) return fail(CGP_ERR_ARG, "cgp_covariance_batched_dev: per-object grids need goff_host and coff");
-  if (max_n <= 0 || max_n > 64) return fail(CGP_ERR_SIZE, "cgp_covariance_batched_dev: objects of 1..64 points (max_n = %d); larger ones go "
-                                            "through cgp_cov_matrix_dev / cgp_trsm_rows_dev / cgp_gemm_nt_dev", max_n);
+// hyp (shared) or hyp_obj / nugget_obj (per object, device arrays indexed by position in this call)
+static int covariance_impl(int64_t n_obj, const int64_t* off, int max_n, int dim,
+                           const double* x, const double* y_err, const double* hyp, const double* hyp_obj,
+                           const double* nugget_obj, double nugget, double floor, unsigned flags,
+                           const double* xnew, const int64_t* goff, const int64_t* goff_host, int64_t m_shared,
+                           double* cov, const int64_t* coff, int* info, void* stream) {
+  const char* name = hyp_obj ? "cgp_covariance_objhyp_dev" : "cgp_covariance_batched_dev";
+  char where[64];
+  if (n_obj < 0 || (n_obj && (!off || !x || !xnew || !cov || !info))) return fail(CGP_ERR_ARG, "%s: NULL argument", name);
+  if (goff && (!goff_host || !coff)) return fail(CGP_ERR_ARG, "%s: per-object grids need goff_host and coff", name);
+  if (max_n <= 0 || max_n > 64) return fail(CGP_ERR_SIZE, "%s: objects of 1..64 points (max_n = %d); larger ones go "
+                                            "through cgp_cov_matrix_dev / cgp_trsm_rows_dev / cgp_gemm_nt_dev", name, max_n);
   if (n_obj == 0) return 0;
   cudaStream_t st = (cudaStream_t)stream;
   SmallArgs a; memset(&a, 0, sizeof a);
-  int rc = make_cov(dim, hyp, nugget, floor, flags, &a.cov);
-  if (rc) return rc;
+  int rc = 0;
+  if (hyp_obj) {
+    if (dim != 1 && dim != 2) return fail(CGP_ERR_ARG, "dim must be 1 or 2, got %d", dim);
+    set_objhyp(a, dim, hyp_obj, nugget_obj, nugget, floor, flags);
+  } else if ((rc = make_cov(dim, hyp, nugget, floor, flags, &a.cov))) {
+    return rc;
+  }
   const int nb = (max_n + 7) / 8, ldv = 8 * nb;
   keep_pool_memory();
   // chunks of objects bound the workspace of V rows (512 MB) and the z dimension of the gram launch
@@ -631,12 +639,17 @@ int cgp_covariance_batched_dev(int64_t n_obj, const int64_t* off, int max_n, int
     double *vws = nullptr, *dummy = nullptr;
     cudaError_t ce = cudaMallocAsync((void**)&vws, (size_t)(rows ? rows : 1) * ldv * sizeof(double), st);
     if (ce == cudaSuccess) ce = cudaMallocAsync((void**)&dummy, (size_t)(rows ? rows : 1) * sizeof(double), st);
-    if (ce != cudaSuccess) { if (vws) cudaFreeAsync(vws, st); return cuda_fail((int)ce, "cgp_covariance_batched_dev (workspace)"); }
+    if (ce != cudaSuccess) {
+      if (vws) cudaFreeAsync(vws, st);
+      snprintf(where, sizeof where, "%s (workspace)", name);
+      return cuda_fail((int)ce, where);
+    }
     const int64_t row0 = goff ? goff_host[c0] : 0;          // per-object grids index rows absolutely: shift the bases
     SmallArgs f = a;
     f.n_obj = c1 - c0; f.off = off + c0; f.x = x; f.y = x; f.yerr = y_err; f.info = info + c0;
     f.xnew = xnew; f.goff = goff ? goff + c0 : nullptr; f.m_shared = m_shared;
     f.mean = dummy - row0; f.vout = vws - row0 * ldv;
+    if (hyp_obj) { f.hyp_obj = hyp_obj + c0 * f.n_hyp; if (nugget_obj) f.nugget_obj = nugget_obj + c0; }
     int split = 1;
     if (!goff && f.n_obj < 296) {
       const int64_t rbs = (m_shared + 7) / 8;
@@ -645,16 +658,36 @@ int cgp_covariance_batched_dev(int64_t n_obj, const int64_t* off, int max_n, int
       if (want > 1) split = (int)want;
     }
     f.split = split;
-    rc = run_small(TASK_PREDICT, dim, max_n, f, st, "cgp_covariance_batched_dev (factor)");
+    snprintf(where, sizeof where, "%s (factor)", name);
+    rc = run_small(TASK_PREDICT, dim, max_n, f, st, where);
     if (!rc) {
-      int e = large_cov_gram(dim, a.cov, xnew, goff ? goff + c0 : nullptr, goff ? m_max : m_shared, c1 - c0, vws - row0 * ldv, ldv,
-                             info + c0, goff ? cov : cov + c0 * m_shared * m_shared, goff ? coff + c0 : nullptr, st);
-      if (e) rc = cuda_fail(e, "cgp_covariance_batched_dev (gram)");
+      int e = large_cov_gram(dim, a.cov, f.hyp_obj, f.nugget_obj, nugget, flags, xnew, goff ? goff + c0 : nullptr,
+                             goff ? m_max : m_shared, c1 - c0, vws - row0 * ldv, ldv, info + c0,
+                             goff ? cov : cov + c0 * m_shared * m_shared, goff ? coff + c0 : nullptr, st);
+      if (e) { snprintf(where, sizeof where, "%s (gram)", name); rc = cuda_fail(e, where); }
     }
     cudaFreeAsync(vws, st); cudaFreeAsync(dummy, st);
     c0 = c1;
   }
   return rc;
+}
+
+int cgp_covariance_batched_dev(int64_t n_obj, const int64_t* off, int max_n, int dim,
+                               const double* x, const double* y_err,
+                               const double* hyp, double nugget, double floor, unsigned flags,
+                               const double* xnew, const int64_t* goff, const int64_t* goff_host, int64_t m_shared,
+                               double* cov, const int64_t* coff, int* info, void* stream) {
+  return covariance_impl(n_obj, off, max_n, dim, x, y_err, hyp, nullptr, nullptr, nugget, floor,
+                         flags, xnew, goff, goff_host, m_shared, cov, coff, info, stream);
+}
+
+int cgp_covariance_objhyp_dev(int64_t n_obj, const int64_t* off, int max_n, int dim, const double* x, const double* y_err,
+                              const double* hyp_obj, const double* nugget_obj, double nugget, double floor, unsigned flags,
+                              const double* xnew, const int64_t* goff, const int64_t* goff_host, int64_t m_shared,
+                              double* cov, const int64_t* coff, int* info, void* stream) {
+  if (!hyp_obj) return fail(CGP_ERR_ARG, "cgp_covariance_objhyp_dev: hyp_obj is NULL");
+  return covariance_impl(n_obj, off, max_n, dim, x, y_err, nullptr, hyp_obj, nugget_obj, nugget,
+                         floor, flags, xnew, goff, goff_host, m_shared, cov, coff, info, stream);
 }
 
 // ------------------------------------------------------------------------------------ matrices

@@ -121,8 +121,10 @@ int large_spline_mean(const double* t, const double* c, int nt, const double* x,
                       int64_t n_obj, const double* diff, double* out, cudaStream_t st);
 int large_moments(const double* v, int64_t n, double center, double* out2, cudaStream_t st);
 int large_ll_total(const double* ll, const int* info, int64_t n, double* out2, cudaStream_t st);
-// cov[b] = amp_auto K(g,g) + nugget^2 I - amp_cross^2 V_b V_b^T for objects b of a chunk (V rows from SmallArgs::vout, ldv doubles)
-int large_cov_gram(int dim, const Cov& cov, const double* grid, const int64_t* goff, int64_t m_shared, int64_t n_obj,
+// cov[b] = amp_auto K(g,g) + nugget^2 I - amp_cross^2 V_b V_b^T for objects b of a chunk (V rows from SmallArgs::vout, ldv doubles).
+// hyp_obj null: every object uses `cov`; otherwise object b uses hyp_obj[b * nh ..] and nugget_obj[b] (null -> nugget)
+int large_cov_gram(int dim, const Cov& cov, const double* hyp_obj, const double* nugget_obj, double nugget, unsigned flags,
+                   const double* grid, const int64_t* goff, int64_t m_shared, int64_t n_obj,
                    const double* v, int ldv, const int* info, double* out, const int64_t* coff, cudaStream_t st);
 int large_dot_sq(const double* v, int64_t n, double* out, cudaStream_t st);
 int large_residual(const double* y, const double* y0, int64_t n, int64_t n_pad, double* r, cudaStream_t st);

@@ -890,11 +890,12 @@ int large_ll_total(const double* ll, const int* info, int64_t n, double* out2, c
 // (cosmogp/Gaussian_process.py:356-361).  One CTA per 64 x 64 block: V_i^T and V_j^T staged in shared memory
 // (k-major, so that a thread's four rows are 32 contiguous bytes), 4 x 4 outputs per thread, K(g_i, g_j) generated
 // on the fly.  8 bytes written per ~64 FMAs + one exp: bound by the HBM write of the M x M matrices.
-template <int DIM>
+// OBJHYP: object b's CTAs build their own Cov from h (row b, as in the grouped likelihood) instead of reading `cov`.
+template <int DIM, bool OBJHYP>
 __global__ void __launch_bounds__(256) cov_gram_kernel(Cov cov, const double* __restrict__ grid, const int64_t* __restrict__ goff,
                                                        int64_t m_shared, const double* __restrict__ v, int ldv,
                                                        const int* __restrict__ info, double* __restrict__ out,
-                                                       const int64_t* __restrict__ coff) {
+                                                       const int64_t* __restrict__ coff, const GroupHyp h) {
   extern __shared__ __align__(16) double sm[];
   const int64_t b = blockIdx.z;
   const int64_t g0 = goff ? goff[b] : 0;
@@ -925,6 +926,7 @@ __global__ void __launch_bounds__(256) cov_gram_kernel(Cov cov, const double* __
 #pragma unroll
       for (int c = 0; c < 4; ++c) acc[r][c] = fma(av[r], bv[c], acc[r][c]);
   }
+  if constexpr (OBJHYP) cov = group_cov<DIM>(h, b);
   const bool bad = info && info[b] != 0;
   const double a2 = cov.amp_cross * cov.amp_cross;
   double* ob = out + (coff ? coff[b] : b * m_shared * m_shared);
@@ -945,23 +947,30 @@ __global__ void __launch_bounds__(256) cov_gram_kernel(Cov cov, const double* __
     }
   }
 }
-int large_cov_gram(int dim, const Cov& cov, const double* grid, const int64_t* goff, int64_t m_shared, int64_t n_obj,
+template <int DIM, bool OBJHYP>
+static cudaError_t launch_cov_gram(dim3 g, size_t smem, cudaStream_t st, const Cov& cov, const double* grid, const int64_t* goff,
+                                   int64_t m_shared, const double* v, int ldv, const int* info, double* out, const int64_t* coff,
+                                   const GroupHyp& h) {
+  cudaError_t e = cudaFuncSetAttribute(cov_gram_kernel<DIM, OBJHYP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (e != cudaSuccess) return e;
+  cov_gram_kernel<DIM, OBJHYP><<<g, 256, smem, st>>>(cov, grid, goff, goff ? 0 : m_shared, v, ldv, info, out, coff, h);
+  return cudaSuccess;
+}
+int large_cov_gram(int dim, const Cov& cov, const double* hyp_obj, const double* nugget_obj, double nugget, unsigned flags,
+                   const double* grid, const int64_t* goff, int64_t m_shared, int64_t n_obj,
                    const double* v, int ldv, const int* info, double* out, const int64_t* coff, cudaStream_t st) {
   if (n_obj <= 0 || m_shared <= 0) return 0;               // m_shared: the largest grid of the chunk (the grid's x / y extent)
   const size_t smem = (size_t)2 * 66 * ldv * sizeof(double);
   const unsigned nb = (unsigned)((m_shared + 63) / 64);
   if (n_obj > 65535) return (int)cudaErrorInvalidValue;
   const dim3 g(nb, nb, (unsigned)n_obj);
+  GroupHyp h; h.hyp_obj = hyp_obj; h.nugget_obj = nugget_obj; h.nugget = nugget; h.floor = 0.0; h.flags = flags;
   cudaError_t e;
-  if (dim == 1) {
-    e = cudaFuncSetAttribute(cov_gram_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return (int)e;
-    cov_gram_kernel<1><<<g, 256, smem, st>>>(cov, grid, goff, goff ? 0 : m_shared, v, ldv, info, out, coff);
-  } else {
-    e = cudaFuncSetAttribute(cov_gram_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return (int)e;
-    cov_gram_kernel<2><<<g, 256, smem, st>>>(cov, grid, goff, goff ? 0 : m_shared, v, ldv, info, out, coff);
-  }
+  if (dim == 1) e = hyp_obj ? launch_cov_gram<1, true>(g, smem, st, cov, grid, goff, m_shared, v, ldv, info, out, coff, h)
+                            : launch_cov_gram<1, false>(g, smem, st, cov, grid, goff, m_shared, v, ldv, info, out, coff, h);
+  else e = hyp_obj ? launch_cov_gram<2, true>(g, smem, st, cov, grid, goff, m_shared, v, ldv, info, out, coff, h)
+                   : launch_cov_gram<2, false>(g, smem, st, cov, grid, goff, m_shared, v, ldv, info, out, coff, h);
+  if (e != cudaSuccess) return (int)e;
   count_launch();
   return (int)cudaGetLastError();
 }

@@ -414,16 +414,19 @@ class Gaussian_process:
 
         new_binning None -> each object's own epochs.  COV: True (full matrices on
         access + diagonal), 'diag' (diagonal only) or False.  per_object=True predicts every
-        object with its own fit (`hyperparameters_per_object`, `nugget_per_object`); COV must then
-        be 'diag' or False.  Objects go down one of three routes, by batch.SizeSplit: the batched kernels; one
-        dense.LargeObject at a time (the large objects of a per-object prediction, or every object of a batch with a
-        large one under shared hyperparameters); and, under shared hyperparameters with svd_method=True, the host SVD
-        redo of the objects whose covariance is not positive definite.  Otherwise such an object raises LinAlgError."""
+        object with its own fit (`hyperparameters_per_object`, `nugget_per_object`); with COV=True
+        `covariance_matrix[i]` is then object i's predictive covariance under its fit as it stood at this call.
+        devices=... does not take per_object.  Objects go down one of three routes, by batch.SizeSplit: the batched
+        kernels; one dense.LargeObject at a time (the large objects of a per-object prediction, or every object of a
+        batch with a large one under shared hyperparameters); and, under shared hyperparameters with svd_method=True,
+        the host SVD redo of the objects whose covariance is not positive definite.  Otherwise such an object raises
+        LinAlgError."""
         if self._devices is not None:
             assert new_binning is not None and not per_object and COV in ('diag', False) and not self._any_large, \
-                "with devices=... predictions are on a shared grid with COV='diag' or False"
+                "with devices=... predictions use the shared hyperparameters (not per_object) on a shared grid, " \
+                "with COV='diag' or False"
         if per_object:
-            assert COV in ('diag', False), "per_object predictions provide the variance diagonal only"
+            assert COV in (True, 'diag', False), "per_object predictions take COV=True, 'diag' or False"
         has_mean = self.substract_mean or self.Mean_Y is not None
         want_var = bool(COV)
 
@@ -518,49 +521,77 @@ class Gaussian_process:
         self.prediction_variance = RaggedView(var, rows) if want_var else None
         self.warning_pf = new_y0
         if COV is True:
-            self.get_covariance_matrix()
+            if per_object:
+                self.covariance_matrix = self._covariance_matrices(np.array(hyp_b), np.array(nug_b))
+            else:
+                self.get_covariance_matrix()
 
     def get_covariance_matrix(self):
-        """covariance_matrix[sn] = K(grid,grid)+nugget^2 - H K^-1 H^T (:340-361).  Objects of <= 64 points: written in
-        bulk by cgp_covariance_batched_dev, a chunk of objects (<= 256 MB of matrices) per launch pair, when first
-        read; larger objects one by one through the blocked large-object path."""
+        """covariance_matrix[sn] = K(grid,grid)+nugget^2 - H K^-1 H^T (:340-361) under the shared hyperparameters.
+        Objects of <= 64 points: written in bulk by cgp_covariance_batched_dev, a chunk of objects (<= 256 MB of
+        matrices) per launch pair, when first read; larger objects one by one through the blocked large-object path."""
+        self.covariance_matrix = self._covariance_matrices(np.array(self.hyperparameters, dtype=float), float(self.nugget))
+
+    def _covariance_matrices(self, hyp, nug):
+        """covariance_matrix on the latest prediction's grid, built on access.  hyp (n_hyp,) and nug: shared, on
+        self.batch when every object has <= 64 points.  hyp (N_sn, n_hyp) and nug (N_sn,): object i with row i, the
+        small objects (batch.SizeSplit) on _small_batch() when each has <= 64 points (cgp_covariance_objhyp_dev).
+        Every other object goes one by one through the blocked large-object path."""
         from . import dense
-        hyp, nug = np.array(self.hyperparameters, dtype=float), float(self.nugget)
+        rows = np.ndim(hyp) == 2
         own = self.as_the_same_time
-        grid = None if own else np.ascontiguousarray(self.new_binning, dtype=np.float64)
+        grid = None if own else np.array(self.new_binning, dtype=np.float64)
 
         def make(i):
             o0, o1 = self._off[i], self._off[i + 1]
             g = self._x_flat[o0:o1] if own else grid
             return dense.predictive_covariance(
                 self._x_flat[o0:o1], None if self._ye_flat is None else self._ye_flat[o0:o1],
-                g, hyp, nug, self._dim, self.flags)
+                g, hyp[i] if rows else hyp, nug[i] if rows else nug, self._dim, self.flags)
 
-        sizes = np.diff(self._off)
-        if self._devices is not None or len(sizes) == 0 or int(sizes.max()) > 64:
-            self.covariance_matrix = _LazyMatrices(self.N_sn, make)
-            return
-        per = (sizes.astype(np.int64) ** 2 if own else np.full(self.N_sn, len(grid) ** 2, dtype=np.int64)) * 8
+        # the objects written in bulk (global ids, in the order of `batch`)
+        split = self._split
+        if rows:
+            ids = np.nonzero(split.small)[0]
+            if split.small_max_n > 64:
+                ids = ids[:0]
+        else:
+            ids = np.arange(self.N_sn)
+            if self._devices is not None or self.N_sn == 0 or int(split.sizes.max()) > 64:
+                ids = ids[:0]
+        if not len(ids):
+            return _LazyMatrices(self.N_sn, make)
+        pos = np.full(self.N_sn, -1, dtype=np.int64)         # object i is the batch's object pos[i]
+        pos[ids] = np.arange(len(ids))
+        bulk_hyp, bulk_nug = (hyp[ids], nug[ids]) if rows else (hyp, nug)
+        sizes = split.sizes[ids]
+        per = (sizes.astype(np.int64) ** 2 if own else np.full(len(ids), len(grid) ** 2, dtype=np.int64)) * 8
         bounds = [0]                                         # chunks of objects with <= 256 MB of matrices
         acc = 0
-        for i in range(self.N_sn):
-            if acc and acc + per[i] > (256 << 20):
-                bounds.append(i); acc = 0
-            acc += per[i]
-        bounds.append(self.N_sn)
+        for j in range(len(ids)):
+            if acc and acc + per[j] > (256 << 20):
+                bounds.append(j); acc = 0
+            acc += per[j]
+        bounds.append(len(ids))
         cache = {}
 
         def make_bulk(i):
-            c = int(np.searchsorted(bounds, i, side="right")) - 1
+            j = int(pos[i])
+            if j < 0:
+                return make(i)
+            c = int(np.searchsorted(bounds, j, side="right")) - 1
             if c not in cache:
                 cache.clear()                                # one chunk of host matrices alive at a time
-                mats, info = self.batch.covariance(hyp, nug, grid, objects=(bounds[c], bounds[c + 1]), flags=self.flags)
+                batch = self._small_batch() if rows else self.batch
+                mats, info = batch.covariance(bulk_hyp, bulk_nug, grid, objects=(bounds[c], bounds[c + 1]), flags=self.flags)
                 if info.any():
-                    self._raise_if_bad(np.concatenate([np.zeros(bounds[c], dtype=info.dtype), info]))
+                    full = np.zeros(self.N_sn, dtype=info.dtype)
+                    full[ids[bounds[c]:bounds[c + 1]]] = info
+                    self._raise_if_bad(full)
                 cache[c] = mats
-            return cache[c][i - bounds[c]]
+            return cache[c][j - bounds[c]]
 
-        self.covariance_matrix = _LazyMatrices(self.N_sn, make_bulk)
+        return _LazyMatrices(self.N_sn, make_bulk)
 
 
 class gaussian_process(Gaussian_process):

@@ -252,6 +252,14 @@ int cgp_covariance_batched_dev(int64_t n_obj, const int64_t* off, int max_n, int
                                const double* hyp, double nugget, double floor, unsigned flags,
                                const double* xnew, const int64_t* goff, const int64_t* goff_host, int64_t m_shared,
                                double* cov, const int64_t* coff, int* info, void* stream);
+/* cgp_covariance_batched_dev where object b uses its OWN hyperparameters hyp_obj[b*nh .. b*nh+nh) (nh = 2 or 4) and
+ * nugget_obj[b] (NULL -> the shared `nugget`), both device arrays indexed by position in this call: the
+ * covariance_matrix of each object of a per-object fit (get_prediction(per_object=True, COV=True)).  Same limits,
+ * layouts and NaN blocks. */
+int cgp_covariance_objhyp_dev(int64_t n_obj, const int64_t* off, int max_n, int dim, const double* x, const double* y_err,
+                              const double* hyp_obj, const double* nugget_obj, double nugget, double floor, unsigned flags,
+                              const double* xnew, const int64_t* goff, const int64_t* goff_host, int64_t m_shared,
+                              double* cov, const int64_t* coff, int* info, void* stream);
 
 /* ---- matrices for the attribute surface (kernel_matrix, inv_kernel_matrix:
  *      Gaussian_process.py:256-267, 319-325).  moff[n_obj+1]: CSR into the outputs in
