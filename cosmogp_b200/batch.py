@@ -57,7 +57,8 @@ class SizeSplit:
       small_max_n  max_n of the small objects (0 when there are none)
       runs         [(first, end)) ranges of consecutive small objects, maximal
       points       bool mask over the points: those of small objects
-      small_off    CSR offsets of the small objects alone"""
+      small_off    CSR offsets of the small objects alone
+      small_csr()  the same two for another CSR over the objects, e.g. one prediction grid per object"""
 
     def __init__(self, off):
         self.sizes = np.diff(np.asarray(off, dtype=np.int64))
@@ -74,9 +75,15 @@ class SizeSplit:
 
     @functools.cached_property
     def small_off(self):
-        off = np.zeros(int(self.small.sum()) + 1, dtype=np.int64)
-        off[1:] = np.cumsum(self.sizes[self.small])
-        return off
+        return self.small_csr(sizes=self.sizes)[1]
+
+    def small_csr(self, off=None, sizes=None):
+        """(bool mask over the entries of the small objects, offsets of the small objects alone) of a CSR over the
+        objects, given by its offsets or its sizes"""
+        sizes = np.diff(np.asarray(off, dtype=np.int64)) if sizes is None else sizes
+        sub = np.zeros(int(self.small.sum()) + 1, dtype=np.int64)
+        sub[1:] = np.cumsum(sizes[self.small])
+        return np.repeat(self.small, sizes), sub
 
 
 class RaggedView(object):
@@ -157,6 +164,11 @@ class DeviceBatch:
         t = torch.from_numpy(np.ascontiguousarray(a))
         self.h2d_bytes += t.numel() * t.element_size()
         return t.to(self.device, non_blocking=True)
+
+    def _up_grid(self, grid):
+        """a flat per-object grid; when every grid is empty one unread point stands in, since the entries take no NULL grid"""
+        g = np.asarray(grid, dtype=np.float64)
+        return self._up(g if len(g) else np.zeros((1,) + g.shape[1:]))
 
     def _stream(self):
         return torch.cuda.current_stream(self.device).cuda_stream
@@ -437,7 +449,7 @@ class DeviceBatch:
         offsets (B,)) for a shared template plus one offset per object (shared grid only): only M + B
         doubles are uploaded instead of B x M.
         -> mean, var (host; shape (B,M) for a shared grid, flat otherwise), info."""
-        g = self._up(np.asarray(grid, dtype=np.float64))
+        g = self._up_grid(grid) if goff is not None else self._up(np.asarray(grid, dtype=np.float64))
         go = self._up(np.asarray(goff, dtype=np.int64)) if goff is not None else None
         if mean_template is not None:
             assert goff is None and new_y0 is None
@@ -459,23 +471,29 @@ class DeviceBatch:
             var_h = var_h.reshape(self.n_obj, m) if want_var else None
         return mean_h, var_h, info_h
 
-    def covariance(self, hyp, nugget, grid=None, objects=None, floor=0.0, flags=0):
+    def covariance(self, hyp, nugget, grid=None, objects=None, floor=0.0, flags=0, goff=None):
         """covariance_matrix of the objects [i0, i1) (default: all) in ONE call (cgp_covariance_batched_dev):
         grid given (host array, shared by all objects) -> (k, M, M) host array; grid None -> every object on its own
-        epochs (new_binning=None) -> list of (N_b, N_b) host arrays.  Objects of <= 64 points.
+        epochs (new_binning=None) -> list of (N_b, N_b) host arrays; grid flat with goff (host int64 (B+1,)) -> one grid
+        per object, list of (M_b, M_b) host arrays.  Objects of <= 64 points.
         hyp (B, nh) with an optional (B,) nugget: object b with its own row, as in predict_dev (cgp_covariance_objhyp_dev)."""
         i0, i1 = (0, self.n_obj) if objects is None else (int(objects[0]), int(objects[1]))
         k = i1 - i0
         oh = self._objhyp(hyp, nugget)
         h = None if oh is not None else self._hyp(hyp)
-        own = grid is None
-        if own:
-            g, goff, m = self.x, self.off, 0
-            sizes = np.diff(self.off_host[i0:i1 + 1])
+        ragged = grid is None or goff is not None
+        if ragged:
+            if grid is None:
+                g, d_goff, goff_h = self.x, self.off, self.off_host
+            else:
+                goff_h = np.ascontiguousarray(goff, dtype=np.int64)
+                g, d_goff = self._up_grid(grid), self._up(goff_h)
+            m = 0
+            sizes = np.diff(goff_h[i0:i1 + 1])
             coff_h = np.zeros(self.n_obj + 1, dtype=np.int64)
             coff_h[i0 + 1:i1 + 1] = np.cumsum(sizes * sizes)
             coff, tot = self._up(coff_h), int(coff_h[i1])
-            goff_ptr, goff_host_ptr, coff_ptr = goff.data_ptr() + 8 * i0, self.off_host.ctypes.data + 8 * i0, coff.data_ptr() + 8 * i0
+            goff_ptr, goff_host_ptr, coff_ptr = d_goff.data_ptr() + 8 * i0, goff_h.ctypes.data + 8 * i0, coff.data_ptr() + 8 * i0
         else:
             g = self._up(np.asarray(grid, dtype=np.float64))
             m = int(g.shape[0]); tot = k * m * m
@@ -497,7 +515,7 @@ class DeviceBatch:
         flat = self._down(out[:tot], sync=False)
         info = self._down(self._info[i0:i1], sync=False)
         self._sync()
-        if own:
+        if ragged:
             return [flat[coff_h[i] :coff_h[i + 1]].reshape(sizes[i - i0], sizes[i - i0]) for i in range(i0, i1)], info
         return flat.reshape(k, m, m), info
 

@@ -347,10 +347,43 @@ static int predict_impl(int64_t n_obj, const int64_t* off, int max_n, int dim,
     if (want > 1) split = (int)want;
   }
   a.split = split;
+  // per-object grids, few objects: the same spreading with the number of work items set per object, by its share of
+  // the grid rows (CGP_GRID_PARTS=0: one item per object).  Every item refactorises its object and the 8-row blocks of
+  // the grid phase do not depend on which other blocks a warp takes, so the outputs equal those of one item per object.
+  static int grid_parts = -1;
+  if (grid_parts < 0) { const char* e = getenv("CGP_GRID_PARTS"); grid_parts = (e && !atoi(e)) ? 0 : 1; }
+  int64_t* part_off = nullptr;
+  if (goff && grid_parts && n_obj > 0 && n_obj < 296) {
+    std::vector<int64_t> g((size_t)n_obj + 1), parts((size_t)n_obj + 1, 0);
+    cudaError_t e = cudaMemcpyAsync(g.data(), goff, sizeof(int64_t) * (n_obj + 1), cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+    if (e != cudaSuccess) return cuda_fail((int)e, "read goff[]");
+    int64_t rbs_sum = 0;
+    for (int64_t b = 0; b < n_obj; ++b) rbs_sum += (g[b + 1] - g[b] + 7) / 8;
+    for (int64_t b = 0; b < n_obj; ++b) {
+      const int64_t rbs = (g[b + 1] - g[b] + 7) / 8, cap = (rbs + 3) / 4;
+      int64_t want = rbs_sum ? (int64_t)llround(592.0 * (double)rbs / (double)rbs_sum) : 1;
+      if (want > cap) want = cap;
+      parts[b + 1] = parts[b] + (want > 1 ? want : 1);   // an empty grid keeps one item: it writes the info
+    }
+    if (parts[n_obj] > n_obj) {
+      keep_pool_memory();
+      e = cudaMallocAsync((void**)&part_off, sizeof(int64_t) * (n_obj + 1), st);
+      if (e == cudaSuccess) e = cudaMemcpyAsync(part_off, parts.data(), sizeof(int64_t) * (n_obj + 1), cudaMemcpyHostToDevice, st);
+      if (e != cudaSuccess) {
+        if (part_off) cudaFreeAsync(part_off, st);
+        return cuda_fail((int)e, "cgp_predict_batched_dev (work table)");
+      }
+      a.part_off = part_off; a.n_parts = parts[n_obj];
+    }
+  }
   a.ll = ll_obj;                                          // the N <= 64 kernels emit it from the same factorisation
   if (ll_obj && max_n > 64) {                             // the generic kernel does not: one more launch
-    SmallArgs l = a; l.split = 1;
-    if ((rc = run_small(TASK_LL, dim, max_n, l, st, "cgp_step_batched_dev (likelihood)"))) return rc;
+    SmallArgs l = a; l.split = 1; l.part_off = nullptr;
+    if ((rc = run_small(TASK_LL, dim, max_n, l, st, "cgp_step_batched_dev (likelihood)"))) {
+      if (part_off) cudaFreeAsync(part_off, st);
+      return rc;
+    }
     a.ll = nullptr;
   }
   // Many small objects with variances: two kernels by default.  FACTOR (latency-bound factorisation, L^-1 and alpha
@@ -394,7 +427,9 @@ static int predict_impl(int64_t n_obj, const int64_t* off, int max_n, int dim,
     cudaFreeAsync(ws, st);
     return rc2;
   }
-  return run_small(TASK_PREDICT, dim, max_n, a, st, "cgp_predict_batched_dev");
+  rc = run_small(TASK_PREDICT, dim, max_n, a, st, "cgp_predict_batched_dev");
+  if (part_off) cudaFreeAsync(part_off, st);
+  return rc;
 }
 
 int cgp_predict_batched_dev(int64_t n_obj, const int64_t* off, int max_n, int dim,

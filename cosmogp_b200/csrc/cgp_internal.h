@@ -77,6 +77,9 @@ struct SmallArgs {
   double* mean;
   double* var;             // may be null
   int split;               // CTAs per object (each takes every split-th block of 8 grid points)
+  // optional, TASK_PREDICT on per-object grids: object oi has the work items [part_off[oi], part_off[oi+1]) (device,
+  // n_obj+1 entries, every object at least one item), which replace `split`; n_parts = part_off[n_obj] sizes the launch
+  const int64_t* part_off; int64_t n_parts;
   double* fws;             // TASK_FACTOR / TASK_PREDICT_F: factor workspace, fws_stride doubles per object
   int64_t fws_stride;
   // TASK_LOO
@@ -97,6 +100,24 @@ struct SmallArgs {
   // v = L^-1 e(x*_m, .) of grid point m (unit amplitude) -- the factor of the bulk predictive-covariance writer
   double* vout;
 };
+
+// Work item w of a grid-spreading task -> the position oi of its object; part / parts: which of the object's items it
+// is and how many the object has.  `split` items per object, or the table part_off (SmallArgs; binary search, as the
+// grouped GEMM finds its problem).  Each item takes every parts-th block of 8 grid points of its object.
+__device__ __forceinline__ int64_t work_item(const int64_t* part_off, int64_t n_obj, int split, int64_t w, int& part, int& parts) {
+  if (!part_off) {
+    const int64_t oi = w / split;
+    part = (int)(w - oi * split); parts = split;
+    return oi;
+  }
+  int64_t lo = 0, hi = n_obj - 1;
+  while (lo < hi) {
+    const int64_t mid = (lo + hi + 1) >> 1;
+    if (part_off[mid] <= w) lo = mid; else hi = mid - 1;
+  }
+  part = (int)(w - part_off[lo]); parts = (int)(part_off[lo + 1] - part_off[lo]);
+  return lo;
+}
 
 struct GemmArgs {          // C[m x n] = beta*C + alpha * A[m x k] * B[n x k]^T, all row-major
   const double* a; const double* b; double* c;

@@ -228,11 +228,12 @@ small_gp_kernel(const SmallArgs a, const int nbm, const int mode) {
   __shared__ int s_bad;
 
   const int split = (TASK == TASK_PREDICT) ? a.split : 1;
-  const int64_t n_work = (a.n_obj_dev ? (int64_t)*a.n_obj_dev : a.n_obj) * split;
+  const int64_t* const part_off = (TASK == TASK_PREDICT) ? a.part_off : nullptr;
+  const int64_t n_work = part_off ? a.n_parts : (a.n_obj_dev ? (int64_t)*a.n_obj_dev : a.n_obj) * split;
 
   for (int64_t w = blockIdx.x; w < n_work; w += gridDim.x) {
-    const int64_t oi = w / split;
-    const int part = (int)(w - oi * split);
+    int part, parts;
+    const int64_t oi = work_item(part_off, a.n_obj, split, w, part, parts);
     const int64_t b = a.order ? a.order[oi] : oi;
     const int64_t o0 = a.off[b];
     const int n = (int)(a.off[b + 1] - o0);
@@ -510,7 +511,7 @@ small_gp_kernel(const SmallArgs a, const int nbm, const int mode) {
       const int64_t out0 = a.goff ? g0 : b * a.m_shared;
       const int64_t n_rb = (m_pts + 7) >> 3;
       const double amp_star = cov.amp_auto + cov.nugget2;
-      for (int64_t rb = (int64_t)part * WARPS + warp; rb < n_rb; rb += (int64_t)split * WARPS) {
+      for (int64_t rb = (int64_t)part * WARPS + warp; rb < n_rb; rb += (int64_t)parts * WARPS) {
         const int64_t mi = 8 * rb + L.g;
         const bool live = mi < m_pts;
         double gx = 0.0, gy = 0.0;
@@ -731,7 +732,7 @@ small_gp_kernel(const SmallArgs a, const int nbm, const int mode) {
       const int64_t out0 = a.goff ? g0 : b * a.m_shared;
       const int64_t n_rb = (m_pts + 7) >> 3;
       const double amp_star = cov.amp_auto + cov.nugget2;
-      for (int64_t rb = (int64_t)part * WARPS + warp; rb < n_rb; rb += (int64_t)split * WARPS) {
+      for (int64_t rb = (int64_t)part * WARPS + warp; rb < n_rb; rb += (int64_t)parts * WARPS) {
         const int64_t mi = 8 * rb + L.g;
         const bool live = mi < m_pts;
         double gx = 0.0, gy = 0.0;
@@ -797,7 +798,7 @@ int launch_one(int nbm, const SmallArgs& a, cudaStream_t stream) {
   e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, WARPS * 32, smem);
   if (e != cudaSuccess) return (int)e;
   if (per_sm < 1) return (int)cudaErrorInvalidConfiguration;
-  const int64_t n_work = a.n_obj * (TASK == TASK_PREDICT ? a.split : 1);
+  const int64_t n_work = TASK != TASK_PREDICT ? a.n_obj : a.part_off ? a.n_parts : a.n_obj * a.split;
   int64_t grid = (int64_t)sm_count * per_sm;
   if (grid > n_work) grid = n_work;
   if (grid < 1) return 0;

@@ -217,7 +217,8 @@ gp64_kernel(const SmallArgs a, unsigned long long* __restrict__ ticket) {
   double* const ktab = tiles + NT * TILE + (WPC * (DIM + 1) + n_vec64(TASK)) * LD;      // behind the last vector
   if (KTAB) { exp_table_to_shared(ktab, lane); __syncwarp(); }
   const int split = (FUSED || PF) ? a.split : 1;
-  const int64_t n_work = (a.n_obj_dev ? (int64_t)*a.n_obj_dev : a.n_obj) * split;
+  const int64_t* const part_off = (FUSED || PF) ? a.part_off : nullptr;
+  const int64_t n_work = part_off ? a.n_parts : (a.n_obj_dev ? (int64_t)*a.n_obj_dev : a.n_obj) * split;
   // factor workspace of one object: NT tiles (T_J on the diagonal, -L[I][J] below) followed by z (LD doubles)
   __shared__ __align__(8) unsigned long long s_mbar;       // TMA completion barrier (TASK_PREDICT_F)
   __shared__ long long s_tk[2];                            // WPC > 1: the ticket drawn by thread 0, double buffered
@@ -240,7 +241,8 @@ gp64_kernel(const SmallArgs a, unsigned long long* __restrict__ ticket) {
   auto fetch = [&](int64_t w, Next& nx) {
     nx.n = -1;
     if (w >= n_work) return;
-    const int64_t oi = w / split;
+    int part, parts;
+    const int64_t oi = work_item(part_off, a.n_obj, split, w, part, parts);
     const int64_t b = a.order ? a.order[oi] : oi;
     nx.o0 = a.off[b];
     nx.n = (int)(a.off[b + 1] - nx.o0);
@@ -285,8 +287,8 @@ gp64_kernel(const SmallArgs a, unsigned long long* __restrict__ ticket) {
       t_next = (int64_t)atomicAdd(ticket, 1ULL) + 2 * (int64_t)gridDim.x;
       if (WPC > 1) s_tk[it & 1] = t_next;
     }
-    const int64_t oi = w / split;
-    const int part = (int)(w - oi * split);
+    int part, parts;
+    const int64_t oi = work_item(part_off, a.n_obj, split, w, part, parts);
     const int64_t b = a.order ? a.order[oi] : oi;
     const int64_t o0 = nx.o0;
     const int n = nx.n;
@@ -640,7 +642,7 @@ gp64_kernel(const SmallArgs a, unsigned long long* __restrict__ ticket) {
           pny0[u] = (lv && a.new_y0) ? (a.new_y0_diff ? a.new_y0[m] + a.new_y0_diff[b] : a.new_y0[out0 + m]) : 0.0;
         }
       };
-      const int64_t rb0 = (int64_t)(part * WPC + warp) * UB, rbs = (int64_t)split * WPC * UB;   // the warps of a CTA alternate over the passes
+      const int64_t rb0 = (int64_t)(part * WPC + warp) * UB, rbs = (int64_t)parts * WPC * UB;   // the warps of a CTA alternate over the passes
       grid_fetch(rb0);
       auto pass = [&](auto Uc, const int64_t rb, const int64_t rb_next) {
         constexpr int U = decltype(Uc)::value;
@@ -1010,7 +1012,8 @@ int launch64(const SmallArgs& a, cudaStream_t stream) {
     if (occ < 1) return (int)cudaErrorInvalidConfiguration;
     per_sm = occ;
   }
-  const int64_t n_work = a.n_obj * ((TASK == TASK_PREDICT || TASK == TASK_PREDICT_F || TASK == TASK_PREDICT_FU || TASK == TASK_PREDICT_U) ? a.split : 1);
+  constexpr bool GRID_TASK = TASK == TASK_PREDICT || TASK == TASK_PREDICT_F || TASK == TASK_PREDICT_FU || TASK == TASK_PREDICT_U;
+  const int64_t n_work = !GRID_TASK ? a.n_obj : a.part_off ? a.n_parts : a.n_obj * a.split;
   static int cap = -1;                                    // experiment knob: CGP_GP64_PER_SM=<blocks per SM>
   if (cap < 0) { const char* e = getenv("CGP_GP64_PER_SM"); cap = e ? atoi(e) : 0; }
   int64_t grid = (int64_t)sm_count * ((cap > 0 && cap < per_sm) ? cap : per_sm);

@@ -80,6 +80,14 @@ class _LazyMeanOnGrid:
         return out if dtype is None else out.astype(dtype)
 
 
+def is_per_object_grid(new_binning, dim):
+    """True when `new_binning` of get_prediction is one grid per object rather than one grid shared by all: a sequence
+    whose first element is itself a grid ((M_i,) in 1D, (M_i, 2) in 2D) -- a list, an object ndarray, or an equal-length
+    (B, M) / (B, M, 2) ndarray, the forms y and Time take.  None, a 1-D array or list of floats and an (M, 2) array
+    are shared grids."""
+    return new_binning is not None and len(new_binning) > 0 and np.ndim(new_binning[0]) == dim
+
+
 class Gaussian_process:
     "Gaussian process regressor (device-backed)."
 
@@ -130,6 +138,7 @@ class Gaussian_process:
             self.y0 = np.zeros(self.N_sn)
 
         self.as_the_same_time = True
+        self._grid_csr = (self._x_flat, self._off)       # the prediction grid as a CSR when it is one grid per object
         self._ll_per_object = None
         self._devices = devices
         self.gather_over_nvlink = False     # multi-GPU outputs: False = every GPU's own PCIe link, True = NCCL gather on GPU 0 first
@@ -166,6 +175,8 @@ class Gaussian_process:
         if not (self._dist and dist.is_initialized() and dist.get_world_size() > 1):
             return list(per_object_arrays)
         # equal-length outputs (shared grid); the width comes from the grid, not from the local objects (a rank may own none)
+        assert self.as_the_same_time or not is_per_object_grid(self.new_binning, self._dim), \
+            "gather() needs a prediction on a shared grid, not one grid per object"
         width = 0 if self.as_the_same_time else len(self.new_binning)
         assert width and all(p == width for p in per), "gather() needs a prediction on a shared grid"
         ranges = sharding.balanced_ranges(self._all_sizes, dist.get_world_size())
@@ -412,7 +423,9 @@ class Gaussian_process:
     def get_prediction(self, new_binning=None, COV=True, svd_method=True, per_object=False):
         """Interpolation (and its covariance) on a new grid (:270-361).
 
-        new_binning None -> each object's own epochs.  COV: True (full matrices on
+        new_binning None -> each object's own epochs; one grid per object (is_per_object_grid: a list of (M_i,) arrays in
+        1D, of (M_i, 2) arrays in 2D, or a (B, M) / (B, M, 2) ndarray) -> object i on its own grid, outputs as for
+        None; otherwise one grid shared by all objects.  COV: True (full matrices on
         access + diagonal), 'diag' (diagonal only) or False.  per_object=True predicts every
         object with its own fit (`hyperparameters_per_object`, `nugget_per_object`); with COV=True
         `covariance_matrix[i]` is then object i's predictive covariance under its fit as it stood at this call.
@@ -421,6 +434,10 @@ class Gaussian_process:
         batch with a large one under shared hyperparameters); and, under shared hyperparameters with svd_method=True,
         the host SVD redo of the objects whose covariance is not positive definite.  Otherwise such an object raises
         LinAlgError."""
+        own = new_binning is None
+        per_grid = own or is_per_object_grid(new_binning, self._dim)        # one grid per object: Time or the caller's
+        assert not (per_grid and not own and (self._devices is not None or self._dist)), \
+            "with devices=... or sharded(), predictions take a shared grid, not one grid per object"
         if self._devices is not None:
             assert new_binning is not None and not per_object and COV in ('diag', False) and not self._any_large, \
                 "with devices=... predictions use the shared hyperparameters (not per_object) on a shared grid, " \
@@ -437,11 +454,18 @@ class Gaussian_process:
         self.compute_kernel_matrix()
         self.inv_kernel_matrix = _LazyMatrices(self.N_sn, lambda i: self._object_matrices(i, hyp, nug, bool(svd_method))[1])
 
-        # the grid and the mean function on it; the outputs of object i are mean[rows[i]:rows[i + 1]]
-        own = new_binning is None
+        # the grid and the mean function on it; the outputs of object i are mean[rows[i]:rows[i + 1]].  One grid per
+        # object is the CSR (grid, rows), with the mean function flat on it; own epochs are the case grid = Time.
         if own:
             grid, rows = self._x_flat, self._off
             new_y0 = self._y0_flat if has_mean else None                   # :308-309
+        elif per_grid:
+            assert len(new_binning) == self.N_sn, "one grid per object: %d grids for %d objects" % (len(new_binning), self.N_sn)
+            grid, rows = pack_csr(new_binning, self._dim)
+            new_y0 = None
+            if has_mean:                                                    # template(grid_i) + diff[i], mean.py:92-101
+                tmpl = _mean.template_on_grid(grid, self._dim, self.Mean_Y, self.Time_mean) if len(grid) else None
+                new_y0 = (np.zeros(len(grid)) if tmpl is None else tmpl) + np.repeat(self._diff_used, np.diff(rows))
         else:
             grid = np.ascontiguousarray(new_binning, dtype=np.float64)
             rows = np.arange(self.N_sn + 1, dtype=np.int64) * len(grid)
@@ -454,7 +478,7 @@ class Gaussian_process:
 
         def on_grid(i):
             """object i's grid and the mean function on it (None: zero)"""
-            if own:
+            if per_grid:
                 s = slice(int(rows[i]), int(rows[i + 1]))
                 return grid[s], (None if new_y0 is None else new_y0[s])
             return grid, (None if new_y0 is None else new_y0[i])
@@ -473,19 +497,20 @@ class Gaussian_process:
             var = np.empty(int(rows[-1])) if want_var else None
         if batched is not None:
             # the objects and points it holds: all of them, or the small ones of a mixed batch
-            objs, pts = (slice(None), slice(None)) if whole else (split.small, split.points)
-            if own:
-                kw = {"goff": batched.off_host, "new_y0": None if new_y0 is None else new_y0[pts]}
+            objs = slice(None) if whole else split.small
+            if per_grid:                                     # the grid points of those objects, and their CSR
+                pts, goff = (slice(None), rows) if whole else split.small_csr(rows)
+                kw = {"goff": goff, "new_y0": None if new_y0 is None else new_y0[pts]}
             else:
                 kw = {"mean_template": None if new_y0 is None else (new_y0.template, new_y0.diff[objs])}
             if self._devices is not None:
                 kw["gather"] = self.gather_over_nvlink
             m, v, inf = batched.predict(hyp_b[objs] if per_object else hyp, nug_b[objs] if per_object else nug,
-                                        grid[pts] if own else grid, want_var=want_var, flags=self.flags, **kw)
+                                        grid[pts] if per_grid else grid, want_var=want_var, flags=self.flags, **kw)
             if whole:
                 mean, var, info = m.reshape(-1), (v.reshape(-1) if want_var else None), inf
             else:
-                at = pts if own else np.repeat(objs, len(grid))
+                at = pts if per_grid else np.repeat(objs, len(grid))
                 mean[at] = m.reshape(-1)
                 if want_var:
                     var[at] = v.reshape(-1)
@@ -501,6 +526,8 @@ class Gaussian_process:
                 continue
             s = slice(int(rows[i]), int(rows[i + 1]))
             g, ny0 = on_grid(i)
+            if not len(g):                                  # an empty grid: nothing to predict, the factor gave the info
+                continue
             mean[s], v = obj.predict(g, new_y0=ny0, want_var=want_var)
             if want_var:
                 var[s] = v
@@ -516,10 +543,11 @@ class Gaussian_process:
 
         self.as_the_same_time = own
         self.new_binning = self.Time if own else new_binning
+        self._grid_csr = (grid, rows) if per_grid else None
         # list-like views built in O(1) (a real list of 10^5 row arrays costs ~15 ms)
         self.Prediction = RaggedView(mean, rows)
         self.prediction_variance = RaggedView(var, rows) if want_var else None
-        self.warning_pf = new_y0
+        self.warning_pf = RaggedView(new_y0, rows) if per_grid and not own and new_y0 is not None else new_y0
         if COV is True:
             if per_object:
                 self.covariance_matrix = self._covariance_matrices(np.array(hyp_b), np.array(nug_b))
@@ -540,14 +568,22 @@ class Gaussian_process:
         from . import dense
         rows = np.ndim(hyp) == 2
         own = self.as_the_same_time
-        grid = None if own else np.array(self.new_binning, dtype=np.float64)
+        ragged = self._grid_csr is not None                  # one grid per object: own epochs or the caller's
+        if ragged:
+            grid, goff = self._grid_csr
+        else:
+            grid, goff = np.array(self.new_binning, dtype=np.float64), None
 
         def make(i):
             o0, o1 = self._off[i], self._off[i + 1]
-            g = self._x_flat[o0:o1] if own else grid
+            g = grid[goff[i]:goff[i + 1]] if ragged else grid
+            h, n = hyp[i] if rows else hyp, nug[i] if rows else nug
+            if not len(g):
+                return np.zeros((0, 0))
+            if o0 == o1:                                     # no data: the prior on the grid
+                return self.kernel(g, np.asarray(h, dtype=float), nugget=n, **({"flags": self.flags} if self._dim == 2 else {}))
             return dense.predictive_covariance(
-                self._x_flat[o0:o1], None if self._ye_flat is None else self._ye_flat[o0:o1],
-                g, hyp[i] if rows else hyp, nug[i] if rows else nug, self._dim, self.flags)
+                self._x_flat[o0:o1], None if self._ye_flat is None else self._ye_flat[o0:o1], g, h, n, self._dim, self.flags)
 
         # the objects written in bulk (global ids, in the order of `batch`)
         split = self._split
@@ -564,8 +600,7 @@ class Gaussian_process:
         pos = np.full(self.N_sn, -1, dtype=np.int64)         # object i is the batch's object pos[i]
         pos[ids] = np.arange(len(ids))
         bulk_hyp, bulk_nug = (hyp[ids], nug[ids]) if rows else (hyp, nug)
-        sizes = split.sizes[ids]
-        per = (sizes.astype(np.int64) ** 2 if own else np.full(len(ids), len(grid) ** 2, dtype=np.int64)) * 8
+        per = (np.diff(goff)[ids] ** 2 if ragged else np.full(len(ids), len(grid) ** 2, dtype=np.int64)) * 8
         bounds = [0]                                         # chunks of objects with <= 256 MB of matrices
         acc = 0
         for j in range(len(ids)):
@@ -583,7 +618,14 @@ class Gaussian_process:
             if c not in cache:
                 cache.clear()                                # one chunk of host matrices alive at a time
                 batch = self._small_batch() if rows else self.batch
-                mats, info = batch.covariance(bulk_hyp, bulk_nug, grid, objects=(bounds[c], bounds[c + 1]), flags=self.flags)
+                if own:
+                    g, kw = None, {}
+                elif ragged:                                 # the grids of the batch's objects, as one CSR
+                    pts, sub = (slice(None), goff) if len(ids) == self.N_sn else split.small_csr(goff)
+                    g, kw = grid[pts], {"goff": sub}
+                else:
+                    g, kw = grid, {}
+                mats, info = batch.covariance(bulk_hyp, bulk_nug, g, objects=(bounds[c], bounds[c + 1]), flags=self.flags, **kw)
                 if info.any():
                     full = np.zeros(self.N_sn, dtype=info.dtype)
                     full[ids[bounds[c]:bounds[c + 1]]] = info

@@ -185,7 +185,9 @@ int cgp_loo_objhyp_dev(int64_t n_obj, const int64_t* off, int max_n, int dim,
  *      (cosmogp/Gaussian_process.py:270-361).
  *      Grid: if goff == NULL the m_shared points of xnew are shared by all objects
  *      (new_binning given) and outputs are (n_obj, m_shared) row-major; otherwise
- *      goff[n_obj+1] is a CSR into xnew / new_y0 / mean / var (new_binning=None).
+ *      goff[n_obj+1] is a CSR into xnew / new_y0 / mean / var (per-object grids:
+ *      new_binning=None or one grid per object).  Below 296 objects the entry then reads
+ *      goff back (one synchronisation) to spread long grids over several CTAs.
  *      new_y0 (mean function on the grid, may be NULL) has the output layout.
  *      mean = H K^-1 (y - y0) + new_y0                      (:332-335)
  *      var  = diag(K(x*,x*) + nugget^2 - H K^-1 H^T)         (:356-361), may be NULL. */
