@@ -162,6 +162,13 @@ __host__ __device__ constexpr int n_vec64(int task) { return task == TASK_LOO ? 
 __host__ __device__ constexpr bool ktab64(int task, int nb) {
   return task == TASK_LOO || ((task == TASK_PREDICT || task == TASK_PREDICT_U || task == TASK_LL) && nb < 8);
 }
+__host__ __device__ constexpr bool uni64(int task) { return task == TASK_PREDICT_FU || task == TASK_PREDICT_U; }
+// uniform-grid kernels: per object point, the powers of the pass anchors E_a R^g (g < 8) and R^8 (see UNI in gp64_kernel)
+constexpr int UNI_ROWS = 9;
+// doubles per object point staged per warp: the coordinates and the noise, or the anchor powers of the uniform grid
+__host__ __device__ constexpr int px_rows64(int task, int dim) { return uni64(task) ? UNI_ROWS : dim + 1; }
+// the 2^(j/64) table of cgp_exp_tab: covariance tiles (ktab64) or the anchors of the uniform grid
+__host__ __device__ constexpr bool etab64(int task, int nb) { return ktab64(task, nb) || uni64(task); }
 // Warps per CTA that share one staged factor in the grid kernels (see WPC in gp64_kernel).  Measured at C2 with 2: 16 warps
 // per SM on 8 factors, but 7 passes split 4 + 3 between the two warps, two CTA barriers per object and 128-register
 // spills: grid kernel 2.13 -> 2.42 ms.  Kept at 1 (CGP64_GRID_WPC=2 at compile time selects the shared form; tested).
@@ -189,11 +196,12 @@ gp64_kernel(const SmallArgs a, unsigned long long* __restrict__ ticket) {
   constexpr int LD = 8 * NB;
   constexpr int NT = NB * (NB + 1) / 2;
   double* tiles = smem;
-  double* px = tiles + NT * TILE + warp * (DIM + 1) * LD;     // DIM * LD, one set per warp (the uniform-grid anchors live here)
+  constexpr int PXR = px_rows64(TASK, DIM);
+  double* px = tiles + NT * TILE + warp * PXR * LD;           // DIM * LD, one set per warp (the uniform-grid anchors live here)
   double* noise = px + DIM * LD;
-  double* vr = tiles + NT * TILE + WPC * (DIM + 1) * LD;      // r (becomes z); shared by the warps of the CTA
+  double* vr = tiles + NT * TILE + WPC * PXR * LD;            // r (becomes z); shared by the warps of the CTA
   constexpr bool PF = TASK == TASK_PREDICT_F || TASK == TASK_PREDICT_FU;      // predict from a stored factor
-  constexpr bool UNI = TASK == TASK_PREDICT_FU || TASK == TASK_PREDICT_U;      // ... on a uniformly spaced shared grid
+  constexpr bool UNI = uni64(TASK);                                            // ... on a uniformly spaced shared grid
   constexpr bool FUSED = TASK == TASK_PREDICT || TASK == TASK_PREDICT_U;       // factorise and predict in one pass (no workspace)
   constexpr bool PRED_LIKE = FUSED || TASK == TASK_FACTOR || PF;
   // Prediction needs no L^-1 (round 2): with the accumulator == operand layout the grid phase solves L v = h by block
@@ -214,8 +222,8 @@ gp64_kernel(const SmallArgs a, unsigned long long* __restrict__ ticket) {
   constexpr bool TAB = PF && !UNI && NB == 8 && WPC == 1;
   if (TAB) { exp_table_to_shared(noise, lane); __syncwarp(); }
   constexpr bool KTAB = ktab64(TASK, NB);
-  double* const ktab = tiles + NT * TILE + (WPC * (DIM + 1) + n_vec64(TASK)) * LD;      // behind the last vector
-  if (KTAB) { exp_table_to_shared(ktab, lane); __syncwarp(); }
+  double* const ktab = tiles + NT * TILE + (WPC * PXR + n_vec64(TASK)) * LD;      // behind the last vector
+  if (etab64(TASK, NB)) { exp_table_to_shared(ktab, lane); __syncwarp(); }
   const int split = (FUSED || PF) ? a.split : 1;
   const int64_t* const part_off = (FUSED || PF) ? a.part_off : nullptr;
   const int64_t n_work = part_off ? a.n_parts : (a.n_obj_dev ? (int64_t)*a.n_obj_dev : a.n_obj) * split;
@@ -237,7 +245,8 @@ gp64_kernel(const SmallArgs a, unsigned long long* __restrict__ ticket) {
   // already in flight into registers (HBM latency ~700 cycles would otherwise be exposed per
   // object) and the ticket for object i+2 is being drawn.
   constexpr int NR = (LD + 31) / 32;                     // staged values per lane
-  struct Next { int64_t o0; int n; double x[NR], y2[NR], r[NR], ye[NR]; };
+  // prediction: the factor kernel's status and the object's offset of the shared mean template come with the inputs
+  struct Next { int64_t o0; int n, bad; double ydiff, x[NR], y2[NR], r[NR], ye[NR]; };
   auto fetch = [&](int64_t w, Next& nx) {
     nx.n = -1;
     if (w >= n_work) return;
@@ -246,6 +255,8 @@ gp64_kernel(const SmallArgs a, unsigned long long* __restrict__ ticket) {
     const int64_t b = a.order ? a.order[oi] : oi;
     nx.o0 = a.off[b];
     nx.n = (int)(a.off[b + 1] - nx.o0);
+    nx.bad = PF ? a.info[b] : 0;
+    nx.ydiff = ((FUSED || PF) && a.new_y0 && a.new_y0_diff) ? a.new_y0_diff[b] : 0.0;
 #pragma unroll
     for (int k = 0; k < NR; ++k) {
       const int i = k * 32 + lane;
@@ -260,16 +271,17 @@ gp64_kernel(const SmallArgs a, unsigned long long* __restrict__ ticket) {
   // Uniform shared grid (UNI): g_j = g_first + j*delta.  Within a pass of 16 grid rows anchored at row j0,
   //   exp(h00 (g_j0 + k delta - x)^2) = E_a(x) * R(x)^k * C_k,  E_a = exp(h00 u^2), R = exp(2 h00 delta u), u = g_j0 - x,
   // C_k = exp(h00 k^2 delta^2): two exps per object point and pass instead of one per (grid row, object point).
-  // The caller guarantees l >= |delta|: whenever E_a underflows every product it scales is < 1e-110.
-  double uni_g0 = 0.0, uni_delta = 0.0, uni_c0 = 1.0, uni_c1 = 1.0, uni_c2 = 1.0, uni_2hd = 0.0;
+  // The caller guarantees l >= |delta|: whenever E_a underflows every product it scales is < 1e-110.  The substitution
+  // runs on H' = E_a R^k and C_k scales its results (k < 24: E_a R^k <= 1 / C_k <= e^264.5, C_k^2 >= e^-529).
+  double uni_g0 = 0.0, uni_delta = 0.0, uni_2hd = 0.0;
+  double* const uni_c = ktab + 64;                       // C_k, k < 24, behind the exp table (read at the stores only)
   if (UNI) {
     uni_g0 = a.xnew[0];
     uni_delta = (a.xnew[a.m_shared - 1] - uni_g0) / (double)(a.m_shared - 1);
-    const double k0 = (double)L.g * uni_delta, k1 = (double)(L.g + 8) * uni_delta;
-    uni_c0 = cgp_exp(cov.h00 * k0 * k0); uni_c1 = cgp_exp(cov.h00 * k1 * k1);
-    const double k2 = (double)(L.g + 16) * uni_delta;
-    uni_c2 = cgp_exp(cov.h00 * k2 * k2);
+    const double kd = (double)lane * uni_delta;
+    if (lane < 24) uni_c[lane] = cgp_exp(cov.h00 * kd * kd);
     uni_2hd = 2.0 * cov.h00 * uni_delta;
+    __syncwarp();
   }
   int64_t w = blockIdx.x, w_nxt = (int64_t)blockIdx.x + gridDim.x, t_next = 0;
   int it = 0;
@@ -314,10 +326,12 @@ gp64_kernel(const SmallArgs a, unsigned long long* __restrict__ ticket) {
     double xo[NR];                                       // UNI: this lane owns columns lane, lane+32
 #pragma unroll
     for (int k = 0; k < NR; ++k) xo[k] = UNI ? nx.x[k] : 0.0;
+    const double ydiff = nx.ydiff;
+    int bad = nx.bad;
     fetch(w_nxt, nx);
     __syncwarp();
     if (TASK == TASK_LOO) rsum = red_g(red_t(rsum));
-    double lp_m = 1.0; int lp_e = 0; int bad = 0;
+    double lp_m = 1.0; int lp_e = 0;
     const bool want_u = (TASK == TASK_LOO) && (a.loo_mode == 1);
     if (PF) {
       // factor tiles + z of this object: one TMA bulk copy each, global -> shared, completion on an mbarrier
@@ -332,7 +346,6 @@ gp64_kernel(const SmallArgs a, unsigned long long* __restrict__ ticket) {
         asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
                      :: "r"((unsigned)__cvta_generic_to_shared(va)), "l"(src + NT * TILE), "r"((unsigned)(LD * 8)), "r"(mb) : "memory");
       }
-      bad = a.info[b];
       unsigned done = 0;
       while (!done) {
         asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
@@ -639,7 +652,7 @@ gp64_kernel(const SmallArgs a, unsigned long long* __restrict__ ticket) {
             if (DIM == 1) pgx[u] = a.xnew[g0 + m];
             else { pgx[u] = a.xnew[2 * (g0 + m)]; pgy[u] = a.xnew[2 * (g0 + m) + 1]; }
           }
-          pny0[u] = (lv && a.new_y0) ? (a.new_y0_diff ? a.new_y0[m] + a.new_y0_diff[b] : a.new_y0[out0 + m]) : 0.0;
+          pny0[u] = (lv && a.new_y0) ? a.new_y0[a.new_y0_diff ? m : out0 + m] : 0.0;     // + ydiff at the store
         }
       };
       const int64_t rb0 = (int64_t)(part * WPC + warp) * UB, rbs = (int64_t)parts * WPC * UB;   // the warps of a CTA alternate over the passes
@@ -657,12 +670,15 @@ gp64_kernel(const SmallArgs a, unsigned long long* __restrict__ ticket) {
         // cross-covariance fragments (no amplitude), generated straight into the accumulators of the forward
         // substitution: lane (g,t) holds H[grid row g][columns 8P+2t, 8P+2t+1] = the start value of W_P
         double acc0[U][NB], acc1[U][NB];
+        // the anchors serve 16 grid rows: with one block per pass they are computed for every even block and the odd
+        // block that follows reuses them (rows g + 8); blocks that do not follow each other (split > 1) get their own
+        const bool second = UNI && (U == 1) && (rbs == 1) && (rb & 1);
         if constexpr (UNI) {
-          double2* anch = reinterpret_cast<double2*>(px);      // {E_a, R} per object point (px + noise: 2 LD doubles)
-          // the anchors serve 16 grid rows: with one block per pass they are computed for every even block and the odd
-          // block that follows reuses them (rows g + 8); blocks that do not follow each other (split > 1) get their own
-          const bool second = (U == 1) && (rbs == 1) && (rb & 1);
-          (void)second;
+          // the powers of the anchors, computed once per object point by the lane that owns it (the 8 lanes that share
+          // a column would otherwise each repeat them): E_a R^g in row g, g < 8, and R^8 in row 8.  With an even NB the
+          // odd rows are swizzled by 8 columns so that the 16-byte loads of a quarter warp (rows g, g + 1) hit distinct banks
+          double* pw = px;                                     // UNI_ROWS * LD doubles
+          constexpr int SWZ = (NB & 1) ? 0 : 8;
           if (!second) {
           __syncwarp();                                        // the previous pass has read its anchors
           const double gj0 = fma((double)(8 * rb), uni_delta, uni_g0);
@@ -670,34 +686,36 @@ gp64_kernel(const SmallArgs a, unsigned long long* __restrict__ ticket) {
           for (int k = 0; k < NR; ++k) {
             const int c = k * 32 + lane;
             const double uu = gj0 - xo[k];
-            double ea = cgp_exp(cov.h00 * uu * uu), rr = cgp_exp(uni_2hd * uu);
+            double ea = cgp_exp_tab(cov.h00 * uu * uu, ktab), rr = cgp_exp_tab(uni_2hd * uu, ktab);
             // padding columns and underflowed anchors contribute exactly 0 (R = 0 keeps 0 * R^k away from 0 * inf);
             // the consumers below then need no masks: rows past the end of the grid are never stored
             ea = (c < n && ea > 0.0) ? ea : 0.0;
             rr = (ea > 0.0) ? rr : 0.0;
-            if (c < LD) anch[c] = make_double2(ea, rr);
+            if (c < LD) {
+              const double r2 = rr * rr, r4 = r2 * r2;
+              // E_a first: every partial product E_a R^j = exp(h00 (u + j delta)^2) / C_j stays below e^24.5
+              const double e1 = ea * rr, e2 = ea * r2, e3 = e1 * r2;
+              const double e[8] = {ea, e1, e2, e3, ea * r4, e1 * r4, e2 * r4, e3 * r4};
+#pragma unroll
+              for (int g = 0; g < 8; ++g) pw[g * LD + (c ^ ((g & 1) * SWZ))] = e[g];
+              pw[(UNI_ROWS - 1) * LD + c] = r4 * r4;
+            }
           }
           __syncwarp();
           }
-          const bool b1 = L.g & 1, b2 = L.g & 2, b4 = L.g & 4;
 #pragma unroll
           for (int P = 0; P < NB; ++P) {
-            const int c0 = 8 * P + 2 * L.t, c1 = c0 + 1;   // this lane's two k-values of block P (see the layout note)
-            const double2 A0 = anch[c0], A1 = anch[c1];
-            // R^g by squaring (g is fixed per lane: predicated multiplies), R^(g+8) = R^g R^8
-            const double r02 = A0.y * A0.y, r04 = r02 * r02, r08 = r04 * r04;
-            const double r12 = A1.y * A1.y, r14 = r12 * r12, r18 = r14 * r14;
-            double p0 = b1 ? A0.y : 1.0, p1 = b1 ? A1.y : 1.0;
-            if (b2) { p0 *= r02; p1 *= r12; }
-            if (b4) { p0 *= r04; p1 *= r14; }
-            const double t0 = A0.x * p0, t1 = A1.x * p1;
+            const int c0 = 8 * P + 2 * L.t;                // this lane's two k-values of block P (see the layout note)
+            const double2 r8 = ld_vec2(pw + (UNI_ROWS - 1) * LD, c0);
+            const double2 er = ld_vec2(pw + L.g * LD, c0 ^ ((L.g & 1) * SWZ));
+            const double t0 = er.x, t1 = er.y;
+            // H' = E_a R^k (C_k is applied to the results, see the store): multiplied up in this order nothing overflows
             if constexpr (U >= 2) {
-              const double s0 = t0 * r08, s1 = t1 * r18;           // E R^(g+8): multiplied up in this order nothing overflows
-              acc0[0][P] = t0 * uni_c0; acc0[1][P] = s0 * uni_c1; acc1[0][P] = t1 * uni_c0; acc1[1][P] = s1 * uni_c1;
-              if constexpr (U == 3) { acc0[2][P] = (s0 * r08) * uni_c2; acc1[2][P] = (s1 * r18) * uni_c2; }
+              const double s0 = t0 * r8.x, s1 = t1 * r8.y;
+              acc0[0][P] = t0; acc0[1][P] = s0; acc1[0][P] = t1; acc1[1][P] = s1;
+              if constexpr (U == 3) { acc0[2][P] = s0 * r8.x; acc1[2][P] = s1 * r8.y; }
             } else {
-              const double cs = second ? uni_c1 : uni_c0;
-              acc0[0][P] = (second ? t0 * r08 : t0) * cs; acc1[0][P] = (second ? t1 * r18 : t1) * cs;
+              acc0[0][P] = second ? t0 * r8.x : t0; acc1[0][P] = second ? t1 * r8.y : t1;
             }
           }
         } else {
@@ -752,8 +770,10 @@ gp64_kernel(const SmallArgs a, unsigned long long* __restrict__ ticket) {
           const double pmt = red_t(pm[u] + pm2[u]);
           vv = red_t(vv + vv2);
           if (live[u] && L.t == 0) {
-            double mean = fma(cov.amp_cross, pmt, ny0[u]);
-            double var = fma(-cov.amp_cross * cov.amp_cross, vv, amp_star);
+            // UNI: v = C_k v' (k = g + 8u, or g + 8 for the second block of a pair): mean = amp C_k v'.z, var = amp* - (amp C_k)^2 |v'|^2
+            const double ac = UNI ? cov.amp_cross * uni_c[L.g + 8 * (second ? 1 : u)] : cov.amp_cross;
+            double mean = fma(ac, pmt, a.new_y0_diff ? ny0[u] + ydiff : ny0[u]);
+            double var = fma(-ac * ac, vv, amp_star);
             if (bad) { mean = nan(""); var = mean; }
             a.mean[out0 + mi[u]] = mean;
             if (a.var) a.var[out0 + mi[u]] = var;
@@ -996,8 +1016,8 @@ int launch64(const SmallArgs& a, cudaStream_t stream) {
   if ((TASK == TASK_LL && compact) || (TASK == TASK_FACTOR && fcompact)) return launch64_ll<DIM, NB>(a, stream);
   auto kern = gp64_kernel<DIM, TASK, NB>;
   constexpr int WPC = warps_per_cta(TASK);
-  const size_t smem = ((size_t)(NB * (NB + 1) / 2) * TILE + (size_t)(WPC * (DIM + 1) + n_vec64(TASK)) * 8 * NB
-                       + (ktab64(TASK, NB) ? 64 : 0)) * sizeof(double);
+  const size_t smem = ((size_t)(NB * (NB + 1) / 2) * TILE + (size_t)(WPC * px_rows64(TASK, DIM) + n_vec64(TASK)) * 8 * NB
+                       + (etab64(TASK, NB) ? 64 : 0) + (uni64(TASK) ? 24 : 0)) * sizeof(double);
   static int sm_counts[16] = {0}, per_sms[16] = {0};   // per device of this process
   int dev = 0;
   if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 16) return (int)cudaErrorInvalidDevice;
