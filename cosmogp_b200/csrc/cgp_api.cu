@@ -280,6 +280,57 @@ int cgp_large_ll_objhyp_dev(int64_t n_obj, const int64_t* off_host, int dim,
   return e ? cuda_fail(e, "cgp_large_ll_objhyp_dev") : 0;
 }
 
+int64_t cgp_large_cov_ws_doubles(int64_t n, int64_t m) { return n < 0 || m < 0 ? 0 : large_cov_ws_doubles(n, m); }
+
+int cgp_large_covariance_dev(int64_t n_obj, const int64_t* off_host, int dim, const double* x, const double* y_err,
+                             const double* hyp_rows_host, const double* nugget_rows_host, double nugget, double floor,
+                             unsigned flags, const double* xnew, const int64_t* goff_host, int64_t m_shared,
+                             const int* order_host, int64_t n_active, double* cov, const int64_t* coff_host, int* info,
+                             double* work, int64_t work_doubles, void* stream) {
+  const char* name = "cgp_large_covariance_dev";
+  if (n_obj < 0 || n_active < 0) return fail(CGP_ERR_ARG, "%s: negative object count", name);
+  const int64_t k = order_host ? n_active : n_obj;
+  if (k == 0) return 0;
+  if (!off_host || !x || !hyp_rows_host || !xnew || !cov || !coff_host || !info || !work)
+    return fail(CGP_ERR_ARG, "%s: NULL argument", name);
+  if (dim != 1 && dim != 2) return fail(CGP_ERR_ARG, "dim must be 1 or 2, got %d", dim);
+  if ((uintptr_t)work & 15) return fail(CGP_ERR_ARG, "%s: work must be 16-byte aligned", name);
+  // padded sizes stay within the 65535 rows cgp_cov_matrix_dev builds an auto-covariance for
+  const int64_t max_pts = 65535 / 128 * 128;
+  if (!goff_host && (m_shared < 0 || m_shared > max_pts))
+    return fail(CGP_ERR_SIZE, "%s: shared grid of %lld points (0..%lld)", name, (long long)m_shared, (long long)max_pts);
+  int64_t need = 0;
+  for (int64_t j = 0; j < k; ++j) {
+    const int64_t b = order_host ? order_host[j] : j;
+    if (b < 0 || b >= n_obj) return fail(CGP_ERR_ARG, "%s: order[%lld] = %lld is not an object id", name, (long long)j, (long long)b);
+    const int64_t n = off_host[b + 1] - off_host[b];
+    if (n < 0 || n > max_pts)
+      return fail(CGP_ERR_SIZE, "%s: object %lld has %lld points (0..%lld)", name, (long long)b, (long long)n, (long long)max_pts);
+    const int64_t m = goff_host ? goff_host[b + 1] - goff_host[b] : m_shared;
+    if (m < 0 || m > max_pts)
+      return fail(CGP_ERR_SIZE, "%s: grid of object %lld has %lld points (0..%lld)", name, (long long)b, (long long)m, (long long)max_pts);
+    if (coff_host[j + 1] - coff_host[j] != m * m)
+      return fail(CGP_ERR_ARG, "%s: coff[%lld + 1] - coff[%lld] is not the grid's %lld^2 entries", name, (long long)j, (long long)j, (long long)m);
+    const int64_t w = large_cov_ws_doubles(n, m);
+    if (w > need) need = w;
+  }
+  if (work_doubles < need)
+    return fail(CGP_ERR_SIZE, "%s: workspace of %lld doubles is below the %lld the largest active object needs", name,
+                (long long)work_doubles, (long long)need);
+  // Cov of every object on the host, as cgp_cov_matrix_dev builds them: the floor enters the data covariance only
+  const int nh = dim == 1 ? 2 : 4;
+  std::vector<Cov> covs((size_t)k), covs_g((size_t)k);
+  for (int64_t j = 0; j < k; ++j) {
+    const double nu = nugget_rows_host ? nugget_rows_host[j] : nugget;
+    covs[j] = cov_from_hyp(dim, hyp_rows_host + j * nh, nu, floor, flags);
+    covs_g[j] = cov_from_hyp(dim, hyp_rows_host + j * nh, nu, 0.0, flags);
+  }
+  keep_pool_memory();
+  int e = large_cov_grouped(dim, off_host, x, y_err, covs.data(), covs_g.data(), xnew, goff_host, m_shared, order_host, k, cov, coff_host,
+                            info, work, work_doubles, (cudaStream_t)stream);
+  return e ? cuda_fail(e, name) : 0;
+}
+
 int cgp_fit_objects_dev(int64_t n_obj, const int64_t* off, int max_n, int dim,
                         const double* x, const double* y, const double* y0, const double* y_err,
                         const double* start, int n_par, double nugget, double floor, unsigned flags,

@@ -591,6 +591,79 @@ __global__ void __launch_bounds__(1024) ll_finish_grouped_kernel(const GroupObj*
   }
 }
 
+// One object of a grouped predictive covariance (large_cov_grouped).  `cov` (with the floor, for A) and `cov_g` (without
+// it, for H and K**) come from the host, as cgp_cov_matrix_dev's do: the device's cov_from_hyp may contract the 2D
+// metric differently.
+struct CovObj {
+  Cov cov, cov_g;
+  const double* x; const double* yerr; const double* g;   // epochs, their errors (may be null), grid
+  double* a;                 // n_pad x n_pad covariance -> blocked factor
+  double* v;                 // m_pad x n_pad: H = K(g, x) -> V = rows of L^-1 H^T
+  double* c;                 // m_pad x m_pad: K(g, g) + nugget^2 I -> C
+  double* out;               // the object's m x m block of the packed output
+  int64_t n, n_pad, m, m_pad;
+  int64_t io;                // position in `order`: info
+  int64_t cta0;              // first CTA of the object in the build launch
+};
+
+// The three builds of dense.predictive_covariance (cgp_cov_matrix_dev's arguments) for every object of a wave:
+// A = K(x, x) + noise, H = K(g, x) and K** = K(g, g) + nugget^2 I.  Object i owns (n_pad + m_pad) * ceil(n_pad / 256)
+// + m_pad * ceil(m_pad / 256) CTAs from objs[i].cta0 on: one row of one matrix, 256 columns each.
+template <int DIM>
+__global__ void __launch_bounds__(128) cov3_build_grouped_kernel(const CovObj* __restrict__ objs, const int n_obj) {
+  const int64_t t = blockIdx.x;
+  int lo = 0, hi = n_obj - 1;
+  while (lo < hi) {
+    const int mid = (lo + hi + 1) >> 1;
+    if (objs[mid].cta0 <= t) lo = mid; else hi = mid - 1;
+  }
+  const CovObj& o = objs[lo];
+  const int64_t pn = (o.n_pad + 255) / 256, pm = (o.m_pad + 255) / 256;
+  int64_t local = t - o.cta0, per_row;
+  CovArgs a;
+  a.dim = DIM; a.cov = o.cov_g;
+  if (local < o.n_pad * pn) {                                     // A: auto-covariance of the epochs with y_err
+    per_row = pn;
+    a.cov = o.cov;
+    a.autocov = 1; a.xc = o.x; a.n = o.n; a.xr = o.x; a.m = o.n; a.yerr = o.yerr;
+    a.out = o.a; a.ld = o.n_pad; a.rows_pad = o.n_pad; a.cols_pad = o.n_pad;
+  } else if ((local -= o.n_pad * pn) < o.m_pad * pn) {           // H: grid rows against the epochs, zero padding
+    per_row = pn;
+    a.autocov = 0; a.xc = o.x; a.n = o.n; a.xr = o.g; a.m = o.m; a.yerr = nullptr;
+    a.out = o.v; a.ld = o.n_pad; a.rows_pad = o.m_pad; a.cols_pad = o.n_pad;
+  } else {                                                        // K**: auto-covariance of the grid, no y_err
+    local -= o.m_pad * pn;
+    per_row = pm;
+    a.autocov = 1; a.xc = o.g; a.n = o.m; a.xr = o.g; a.m = o.m; a.yerr = nullptr;
+    a.out = o.c; a.ld = o.m_pad; a.rows_pad = o.m_pad; a.cols_pad = o.m_pad;
+  }
+  const int64_t r = local / per_row, chunk = local - r * per_row;
+  cov_build_at<DIM>(a, r, (chunk * 128 + threadIdx.x) * 2);
+}
+
+// Object blockIdx.y of a wave: its info (the first failing pivot, summed over the blocks as potrf_finish_kernel does;
+// block k at infob[koff[k] + object]) and its leading m x m block of C packed to `out`, all NaN where info != 0.
+__global__ void __launch_bounds__(256) cov_pack_grouped_kernel(const CovObj* __restrict__ objs, const int* __restrict__ infob,
+                                                               const int64_t* __restrict__ koff, int* __restrict__ info) {
+  const int i = blockIdx.y;
+  const CovObj& o = objs[i];
+  __shared__ int bad_s;
+  if (threadIdx.x == 0) {
+    const int nblk = (int)(o.n_pad / 128);
+    int bad = 0;
+    for (int k = 0; k < nblk && !bad; ++k) { const int ik = infob[koff[k] + i]; if (ik) bad = k * 128 + ik; }
+    bad_s = bad;
+    if (blockIdx.x == 0) info[o.io] = bad;
+  }
+  __syncthreads();
+  const bool bad = bad_s != 0;
+  const int64_t m = o.m, mm = m * m;
+  for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < mm; e += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t r = e / m;
+    o.out[e] = bad ? nan("") : o.c[r * o.m_pad + (e - r * m)];
+  }
+}
+
 }  // namespace
 
 // =========================================================================================
@@ -1057,15 +1130,167 @@ int64_t large_ll_ws_doubles(int64_t n) {
   return np * np + 2 * np + 2 * (np / 128);          // covariance, residual, z, per-block log det and info
 }
 
+// ---------------------------------------------------------------------------------------
+// Schedules of the grouped large-object pipelines (large_ll_grouped, large_cov_grouped).  Every launch of every wave
+// is recorded on the host first; the arguments (object descriptors, GEMM problems, block offsets) are packed into one
+// byte table that crosses to the device in one copy into stream-ordered scratch.
+namespace {
+enum { L_DIAG, L_GEMM, L_COV, L_FWD, L_FIN, L_PACK };
+struct Launch { int kind; int64_t grid, count, k0; size_t t0, t1, t2; double* ldb; int* infob; };
+
+struct GroupSchedule {
+  std::vector<char> tab;
+  std::vector<Launch> launches;
+  std::vector<GemmArgs> probs;
+  size_t t_csr = 0;
+
+  size_t put(const void* p, size_t bytes) {
+    const size_t o = (tab.size() + 15) & ~(size_t)15;
+    tab.resize(o + bytes);
+    memcpy(tab.data() + o, p, bytes);
+    return o;
+  }
+  // the CSR {0, 128, 256, ..} the diagonal-block launches read, for waves of up to w_max objects
+  void block_csr(size_t w_max) {
+    std::vector<int64_t> csr(w_max + 1);
+    for (size_t i = 0; i <= w_max; ++i) csr[i] = (int64_t)i * 128;
+    t_csr = put(csr.data(), csr.size() * sizeof(int64_t));
+  }
+  void gemm(const double* A, int64_t lda, const double* B, int64_t ldb, double* C, int64_t ldc, int64_t m, int64_t n,
+            int64_t k, double alpha, double beta, int lower) {
+    GemmArgs g;
+    g.a = A; g.b = B; g.c = C; g.lda = lda; g.ldb = ldb; g.ldc = ldc;
+    g.m = (int)m; g.n = (int)n; g.k = (int)k; g.alpha = alpha; g.beta = beta; g.lower_only = lower;
+    probs.push_back(g);
+  }
+  // the GEMM problems recorded since the last flush as one grouped launch, tiles split as launch_gemm_nt splits them
+  int flush() {
+    if (probs.empty()) return 0;
+    std::vector<int> start(probs.size() + 1, 0);
+    for (size_t q = 0; q < probs.size(); ++q) {
+      const GemmArgs& g = probs[q];
+      const int64_t t128 = g.m / 128;
+      const int64_t tiles = g.lower_only ? t128 * (t128 + 1) : (int64_t)(g.m / BM) * (g.n / BN);
+      if (start[q] + tiles > 2147483647LL) return (int)cudaErrorInvalidValue;
+      start[q + 1] = start[q] + (int)tiles;
+    }
+    const size_t tp = put(probs.data(), probs.size() * sizeof(GemmArgs));
+    const size_t ts = put(start.data(), start.size() * sizeof(int));
+    launches.push_back({L_GEMM, start.back(), (int64_t)probs.size(), 0, tp, ts, 0, nullptr, nullptr});
+    probs.clear();
+    return 0;
+  }
+  // The blocked Cholesky of large_potrf for the matrices of one wave: object i's n_pad x n_pad matrix at a[i] (inside
+  // `work`, leading dimension ld[i] = n_pad, nblk[i] = n_pad / 128 blocks, sorted in decreasing order so that the objects
+  // taking part in any step are a prefix).  Per pair of block columns two diagonal-block launches (launch_small in
+  // matrix-source mode, ld table at t_ld) and four grouped GEMM launches, with the shapes, tile split and alpha / beta
+  // large_potrf uses for each object alone (the next pair's columns and the lower trailing update touch disjoint tiles,
+  // so they share one launch).  Block k of object i leaves its log det and info at ldb / infob[koff[k] + i].
+  int factor(double* work, const std::vector<double*>& a, const std::vector<int64_t>& ld, const std::vector<int>& nblk,
+             size_t t_ld, const std::vector<int64_t>& koff, double* ldb, int* infob) {
+    const int W = (int)a.size(), nb_max = nblk[0];
+    auto count = [&](int k) { int c = 0; while (c < W && nblk[c] > k) ++c; return c; };   // objects with block k
+    auto diag = [&](int k) {
+      const int c = count(k);
+      std::vector<int64_t> aoff(c);
+      for (int i = 0; i < c; ++i) aoff[i] = (a[i] - work) + (int64_t)k * 128 * ld[i] + (int64_t)k * 128;
+      launches.push_back({L_DIAG, c, c, 0, put(aoff.data(), c * sizeof(int64_t)), t_ld, 0, ldb + koff[k], infob + koff[k]});
+    };
+    int e = 0;
+    for (int p = 0; 2 * p < nb_max && !e; ++p) {
+      const int k = 2 * p;
+      const int64_t k0 = (int64_t)p * 256;
+      diag(k);
+      for (int i = 0; i < W && nblk[i] > k + 1; ++i) {            // panel of block column k: L_ik = A_ik T_kk^T
+        const int64_t np = ld[i];
+        double* ai = a[i];
+        gemm(ai + (k0 + 128) * np + k0, np, ai + k0 * np + k0, np, ai + (k0 + 128) * np + k0, np, np - k0 - 128, 128, 128,
+             1.0, 0.0, 0);
+      }
+      if ((e = flush())) break;
+      for (int i = 0; i < W && nblk[i] > k + 1; ++i) {            // block column k+1 -= L[k+1:, k] L[k+1, k]^T
+        const int64_t np = ld[i];
+        double* ai = a[i];
+        double* panel = ai + (k0 + 128) * np + k0;
+        gemm(panel, np, panel, np, ai + (k0 + 128) * np + (k0 + 128), np, np - k0 - 128, 128, 128, -1.0, 1.0, 0);
+      }
+      if ((e = flush())) break;
+      if (nb_max <= k + 1) break;
+      diag(k + 1);
+      const int64_t k1 = k0 + 128;
+      for (int i = 0; i < W && nblk[i] > k + 2; ++i) {            // panel of block column k+1
+        const int64_t np = ld[i];
+        double* ai = a[i];
+        gemm(ai + (k1 + 128) * np + k1, np, ai + k1 * np + k1, np, ai + (k1 + 128) * np + k1, np, np - k1 - 128, 128, 128,
+             1.0, 0.0, 0);
+      }
+      if ((e = flush())) break;
+      for (int i = 0; i < W && nblk[i] > k + 2; ++i) {            // the pair applied to what lies right of it, K = 256
+        const int64_t np = ld[i], rest = np - k0 - 256;
+        double* ai = a[i];
+        double* wp = ai + (k0 + 256) * np + k0;
+        gemm(wp, np, wp, np, ai + (k0 + 256) * np + (k0 + 256), np, rest, 128, 256, -1.0, 1.0, 0);
+        if (rest > 128)
+          gemm(wp + 128 * np, np, wp + 128 * np, np, ai + (k0 + 384) * np + (k0 + 384), np, rest - 128, 128, 256, -1.0, 1.0, 0);
+        if (rest > 256)
+          gemm(wp + 256 * np, np, wp + 256 * np, np, ai + (k0 + 512) * np + (k0 + 512), np, rest - 256, rest - 256, 256, -1.0,
+               1.0, 1);
+      }
+      e = flush();
+    }
+    return e;
+  }
+  // Copies the table to the device and runs the recorded launches in order: the diagonal blocks and the GEMMs here,
+  // every other kind through other(launch, device table).
+  template <class F>
+  int run(double* work, cudaStream_t st, F&& other) {
+    static bool init[16] = {false};
+    int dev = 0;
+    if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 16) return (int)cudaErrorInvalidDevice;
+    if (!init[dev]) {
+      cudaError_t ce = cudaFuncSetAttribute(gemm_nt_grouped_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GEMM_SMEM);
+      if (ce != cudaSuccess) return (int)ce;
+      init[dev] = true;
+    }
+    char* td = nullptr;
+    cudaError_t ce = cudaMallocAsync((void**)&td, tab.size(), st);
+    if (ce == cudaSuccess) ce = cudaMemcpyAsync(td, tab.data(), tab.size(), cudaMemcpyHostToDevice, st);
+    if (ce != cudaSuccess) { if (td) cudaFreeAsync(td, st); return (int)ce; }
+    int e = 0;
+    for (const Launch& l : launches) {
+      switch (l.kind) {
+        case L_DIAG: {
+          SmallArgs s; memset(&s, 0, sizeof s);
+          s.n_obj = l.count; s.off = reinterpret_cast<const int64_t*>(td + t_csr);
+          s.amat = work; s.aoff = reinterpret_cast<const int64_t*>(td + l.t0); s.ld_obj = reinterpret_cast<const int64_t*>(td + l.t1);
+          s.moff = s.aoff; s.linv = work;
+          s.logdet = l.ldb; s.info = l.infob;
+          s.cov.amp_auto = 1.0; s.cov.amp_cross = 1.0;
+          e = launch_small(TASK_MATRICES, 1, 128, s, st);  // counts its own launch
+          break;
+        }
+        case L_GEMM:
+          gemm_nt_grouped_kernel<<<(unsigned)l.grid, GEMM_THREADS, GEMM_SMEM, st>>>(
+              reinterpret_cast<const GemmArgs*>(td + l.t0), reinterpret_cast<const int*>(td + l.t1), (int)l.count);
+          break;
+        default:
+          other(l, td);
+      }
+      if (l.kind != L_DIAG) count_launch();
+      if (e) break;
+    }
+    cudaFreeAsync(td, st);
+    return e ? e : (int)cudaGetLastError();
+  }
+};
+}  // namespace
+
 // Log-likelihoods of the objects order[0 .. n_active) (object ids; NULL: 0 .. n_active), object order[j] with the
 // hyperparameters of row j, by the blocked factorisation of large_potrf run for all objects of a wave at once.
 // Consecutive objects are packed into waves of at most work_doubles (each object's part: large_ll_ws_doubles); inside
 // a wave they are sorted by block count, so that the objects taking part in any step are a prefix of the wave.  Per
-// wave: one covariance launch; per pair of block columns two diagonal-block launches (launch_small in matrix-source
-// mode) and four grouped GEMM launches, with the shapes, tile split and alpha / beta large_potrf uses for each object
-// alone (the next pair's columns and the lower trailing update touch disjoint tiles, so they share one launch); one
-// forward-sweep launch per block; one epilogue.  The schedule (object descriptors, GEMM problems, block offsets)
-// crosses to the device in one copy into stream-ordered scratch.  The caller checks that every object fits.
+// wave: one covariance launch; the factorisation (GroupSchedule::factor); one forward-sweep launch per block; one
+// epilogue.  The caller checks that every object fits.
 int large_ll_grouped(int dim, const int64_t* off, const double* x, const double* y, const double* y0, const double* yerr,
                      const double* hyp_obj, const double* nugget_obj, double nugget, double floor, unsigned flags,
                      const int* order, int64_t n_active, double* ll, int* info, double* work, int64_t work_doubles,
@@ -1083,27 +1308,18 @@ int large_ll_grouped(int dim, const int64_t* off, const double* x, const double*
     }
     if (!cur.empty()) waves.push_back(cur);
   }
-  std::vector<char> tab;
-  auto put = [&](const void* p, size_t bytes) {
-    const size_t o = (tab.size() + 15) & ~(size_t)15;
-    tab.resize(o + bytes);
-    memcpy(tab.data() + o, p, bytes);
-    return o;
-  };
-  struct Launch { int kind; int64_t grid, count, k0; size_t t0, t1, t2; double* ldb; int* infob; };
-  enum { L_COV, L_DIAG, L_GEMM, L_FWD, L_FIN };
-  std::vector<Launch> launches;
+  GroupSchedule s;
   size_t w_max = 0;
   for (auto& w : waves) w_max = std::max(w_max, w.size());
-  std::vector<int64_t> csr(w_max + 1);
-  for (size_t i = 0; i <= w_max; ++i) csr[i] = (int64_t)i * 128;
-  const size_t t_csr = put(csr.data(), csr.size() * sizeof(int64_t));
+  s.block_csr(w_max);
 
   for (auto& w : waves) {
     std::stable_sort(w.begin(), w.end(), [](const Item& p, const Item& q) { return p.nblk > q.nblk; });
     const int W = (int)w.size(), nb_max = w[0].nblk;
     std::vector<GroupObj> objs(W);
+    std::vector<double*> a(W);
     std::vector<int64_t> ld(W), koff(nb_max + 1, 0);
+    std::vector<int> nblk(W);
     int64_t cur = 0, cta = 0;
     for (int i = 0; i < W; ++i) {
       const Item& it = w[i];
@@ -1113,126 +1329,31 @@ int large_ll_grouped(int dim, const int64_t* off, const double* x, const double*
       g.a = work + cur; g.u = g.a + np * np; g.z = g.u + np;
       g.n = it.n; g.n_pad = np; g.io = it.j; g.cta0 = cta;
       cur += np * np + 2 * np; cta += np * ((np + 255) / 256);
-      ld[i] = np;
+      a[i] = g.a; ld[i] = np; nblk[i] = it.nblk;
     }
     if (cta > 2147483647LL) return (int)cudaErrorInvalidValue;
     auto count = [&](int k) { int c = 0; while (c < W && w[c].nblk > k) ++c; return c; };   // objects with block k
     for (int k = 0; k < nb_max; ++k) koff[k + 1] = koff[k] + count(k);
     double* ldb = work + cur;
     int* infob = reinterpret_cast<int*>(work + cur + koff[nb_max]);
-    const size_t t_objs = put(objs.data(), W * sizeof(GroupObj));
-    const size_t t_ld = put(ld.data(), W * sizeof(int64_t));
-    const size_t t_koff = put(koff.data(), koff.size() * sizeof(int64_t));
-    launches.push_back({L_COV, cta, W, 0, t_objs, 0, 0, nullptr, nullptr});
-
-    auto diag = [&](int k) {
-      const int c = count(k);
-      std::vector<int64_t> aoff(c);
-      for (int i = 0; i < c; ++i) aoff[i] = (objs[i].a - work) + (int64_t)k * 128 * ld[i] + (int64_t)k * 128;
-      launches.push_back({L_DIAG, c, c, 0, put(aoff.data(), c * sizeof(int64_t)), t_ld, 0, ldb + koff[k], infob + koff[k]});
-    };
-    std::vector<GemmArgs> probs;
-    auto gemm = [&](double* A, double* B, double* C, int64_t ldx, int64_t m, int64_t n, int k, double alpha, double beta,
-                    int lower) {
-      GemmArgs g;
-      g.a = A; g.b = B; g.c = C; g.lda = ldx; g.ldb = ldx; g.ldc = ldx;
-      g.m = (int)m; g.n = (int)n; g.k = k; g.alpha = alpha; g.beta = beta; g.lower_only = lower;
-      probs.push_back(g);
-    };
-    auto flush = [&]() -> int {
-      if (probs.empty()) return 0;
-      std::vector<int> start(probs.size() + 1, 0);
-      for (size_t q = 0; q < probs.size(); ++q) {
-        const GemmArgs& g = probs[q];
-        const int64_t t128 = g.m / 128;
-        const int64_t tiles = g.lower_only ? t128 * (t128 + 1) : (int64_t)(g.m / BM) * (g.n / BN);
-        if (start[q] + tiles > 2147483647LL) return (int)cudaErrorInvalidValue;
-        start[q + 1] = start[q] + (int)tiles;
-      }
-      const size_t tp = put(probs.data(), probs.size() * sizeof(GemmArgs));
-      const size_t ts = put(start.data(), start.size() * sizeof(int));
-      launches.push_back({L_GEMM, start.back(), (int64_t)probs.size(), 0, tp, ts, 0, nullptr, nullptr});
-      probs.clear();
-      return 0;
-    };
-    int e = 0;
-    for (int p = 0; 2 * p < nb_max && !e; ++p) {
-      const int k = 2 * p;
-      const int64_t k0 = (int64_t)p * 256;
-      diag(k);
-      for (int i = 0; i < W && w[i].nblk > k + 1; ++i) {            // panel of block column k: L_ik = A_ik T_kk^T
-        const int64_t np = ld[i];
-        double* a = objs[i].a;
-        gemm(a + (k0 + 128) * np + k0, a + k0 * np + k0, a + (k0 + 128) * np + k0, np, np - k0 - 128, 128, 128, 1.0, 0.0, 0);
-      }
-      if ((e = flush())) break;
-      for (int i = 0; i < W && w[i].nblk > k + 1; ++i) {            // block column k+1 -= L[k+1:, k] L[k+1, k]^T
-        const int64_t np = ld[i];
-        double* a = objs[i].a;
-        double* panel = a + (k0 + 128) * np + k0;
-        gemm(panel, panel, a + (k0 + 128) * np + (k0 + 128), np, np - k0 - 128, 128, 128, -1.0, 1.0, 0);
-      }
-      if ((e = flush())) break;
-      if (nb_max <= k + 1) break;
-      diag(k + 1);
-      const int64_t k1 = k0 + 128;
-      for (int i = 0; i < W && w[i].nblk > k + 2; ++i) {            // panel of block column k+1
-        const int64_t np = ld[i];
-        double* a = objs[i].a;
-        gemm(a + (k1 + 128) * np + k1, a + k1 * np + k1, a + (k1 + 128) * np + k1, np, np - k1 - 128, 128, 128, 1.0, 0.0, 0);
-      }
-      if ((e = flush())) break;
-      for (int i = 0; i < W && w[i].nblk > k + 2; ++i) {            // the pair applied to what lies right of it, K = 256
-        const int64_t np = ld[i], rest = np - k0 - 256;
-        double* a = objs[i].a;
-        double* wp = a + (k0 + 256) * np + k0;
-        gemm(wp, wp, a + (k0 + 256) * np + (k0 + 256), np, rest, 128, 256, -1.0, 1.0, 0);
-        if (rest > 128) gemm(wp + 128 * np, wp + 128 * np, a + (k0 + 384) * np + (k0 + 384), np, rest - 128, 128, 256, -1.0, 1.0, 0);
-        if (rest > 256) gemm(wp + 256 * np, wp + 256 * np, a + (k0 + 512) * np + (k0 + 512), np, rest - 256, rest - 256, 256, -1.0, 1.0, 1);
-      }
-      e = flush();
-    }
-    if (e) return e;
+    const size_t t_objs = s.put(objs.data(), W * sizeof(GroupObj));
+    const size_t t_ld = s.put(ld.data(), W * sizeof(int64_t));
+    const size_t t_koff = s.put(koff.data(), koff.size() * sizeof(int64_t));
+    s.launches.push_back({L_COV, cta, W, 0, t_objs, 0, 0, nullptr, nullptr});
+    if (int e = s.factor(work, a, ld, nblk, t_ld, koff, ldb, infob)) return e;
     for (int k = 0; k < nb_max; ++k)
-      launches.push_back({L_FWD, 1 + (ld[0] - (int64_t)k * 128 - 128 + 63) / 64, count(k), (int64_t)k * 128, t_objs, 0, 0,
-                          nullptr, nullptr});
-    launches.push_back({L_FIN, W, W, 0, t_objs, t_koff, 0, ldb, infob});
+      s.launches.push_back({L_FWD, 1 + (ld[0] - (int64_t)k * 128 - 128 + 63) / 64, count(k), (int64_t)k * 128, t_objs, 0, 0,
+                            nullptr, nullptr});
+    s.launches.push_back({L_FIN, W, W, 0, t_objs, t_koff, 0, ldb, infob});
   }
 
-  static bool init[16] = {false};
-  int dev = 0;
-  if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 16) return (int)cudaErrorInvalidDevice;
-  if (!init[dev]) {
-    cudaError_t ce = cudaFuncSetAttribute(gemm_nt_grouped_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GEMM_SMEM);
-    if (ce != cudaSuccess) return (int)ce;
-    init[dev] = true;
-  }
-  char* td = nullptr;
-  cudaError_t ce = cudaMallocAsync((void**)&td, tab.size(), st);
-  if (ce == cudaSuccess) ce = cudaMemcpyAsync(td, tab.data(), tab.size(), cudaMemcpyHostToDevice, st);
-  if (ce != cudaSuccess) { if (td) cudaFreeAsync(td, st); return (int)ce; }
   GroupHyp h; h.hyp_obj = hyp_obj; h.nugget_obj = nugget_obj; h.nugget = nugget; h.floor = floor; h.flags = flags;
-  int e = 0;
-  for (const Launch& l : launches) {
+  return s.run(work, st, [&](const Launch& l, const char* td) {
     const GroupObj* objs = reinterpret_cast<const GroupObj*>(td + l.t0);
     switch (l.kind) {
       case L_COV:
         if (dim == 1) cov_build_grouped_kernel<1><<<(unsigned)l.grid, 128, 0, st>>>(objs, (int)l.count, h);
         else cov_build_grouped_kernel<2><<<(unsigned)l.grid, 128, 0, st>>>(objs, (int)l.count, h);
-        break;
-      case L_DIAG: {
-        SmallArgs s; memset(&s, 0, sizeof s);
-        s.n_obj = l.count; s.off = reinterpret_cast<const int64_t*>(td + t_csr);
-        s.amat = work; s.aoff = reinterpret_cast<const int64_t*>(td + l.t0); s.ld_obj = reinterpret_cast<const int64_t*>(td + l.t1);
-        s.moff = s.aoff; s.linv = work;
-        s.logdet = l.ldb; s.info = l.infob;
-        s.cov.amp_auto = 1.0; s.cov.amp_cross = 1.0;
-        e = launch_small(TASK_MATRICES, 1, 128, s, st);  // counts its own launch
-        break;
-      }
-      case L_GEMM:
-        gemm_nt_grouped_kernel<<<(unsigned)l.grid, GEMM_THREADS, GEMM_SMEM, st>>>(
-            reinterpret_cast<const GemmArgs*>(td + l.t0), reinterpret_cast<const int*>(td + l.t1), (int)l.count);
         break;
       case L_FWD:
         fwd_step_grouped_kernel<<<dim3((unsigned)l.grid, (unsigned)l.count), 256, 0, st>>>(objs, l.k0);
@@ -1242,11 +1363,119 @@ int large_ll_grouped(int dim, const int64_t* off, const double* x, const double*
                                                                     reinterpret_cast<const int64_t*>(td + l.t1), ll, info);
         break;
     }
-    if (l.kind != L_DIAG) count_launch();
-    if (e) break;
+  });
+}
+
+int64_t large_cov_ws_doubles(int64_t n, int64_t m) {
+  const int64_t np = n <= 0 ? 128 : (n + 127) / 128 * 128, mp = m <= 0 ? 128 : (m + 127) / 128 * 128;
+  return np * np + mp * np + mp * mp;                // covariance / factor, H -> V, K** -> C
+}
+
+// Predictive covariance matrices of the objects order[0 .. n_active) (object ids; NULL: 0 .. n_active), object
+// order[j] with covs[j] for its own covariance and covs_g[j] for H and K**, on its grid (goff: xnew + dim * goff[b], m_b = goff[b+1] - goff[b]; NULL: the shared grid
+// xnew of m_shared points), by every step of dense.predictive_covariance run for all objects of a wave at once:
+// A = K(x, x) + noise, H and K** in one launch; the factorisation (GroupSchedule::factor); V = rows of L^-1 H^T as
+// large_trsm_rows computes it (one pair of grouped GEMM launches per block column); C = K** - V V^T (one grouped
+// GEMM launch); the packing of each leading m_b x m_b block to out + coff[j], NaN where info[j] != 0.  Waves and their
+// order as in large_ll_grouped, each object's part of the workspace large_cov_ws_doubles(n_b, m_b).  The block log
+// dets / infos live in stream-ordered scratch.  The caller checks that every object fits.
+int large_cov_grouped(int dim, const int64_t* off, const double* x, const double* yerr, const Cov* covs, const Cov* covs_g,
+                      const double* xnew, const int64_t* goff, int64_t m_shared, const int* order, int64_t n_active, double* out,
+                      const int64_t* coff, int* info, double* work, int64_t work_doubles, cudaStream_t st) {
+  struct Item { int64_t j, b, n, n_pad, m, m_pad; int nblk; };
+  std::vector<std::vector<Item>> waves;
+  {
+    std::vector<Item> cur; int64_t used = 0;
+    for (int64_t j = 0; j < n_active; ++j) {
+      Item it; it.j = j; it.b = order ? order[j] : j; it.n = off[it.b + 1] - off[it.b];
+      it.m = goff ? goff[it.b + 1] - goff[it.b] : m_shared;
+      it.n_pad = it.n <= 0 ? 128 : (it.n + 127) / 128 * 128; it.nblk = (int)(it.n_pad / 128);
+      it.m_pad = it.m <= 0 ? 128 : (it.m + 127) / 128 * 128;
+      const int64_t need = large_cov_ws_doubles(it.n, it.m);
+      if (!cur.empty() && (used + need > work_doubles || cur.size() >= 65535)) { waves.push_back(cur); cur.clear(); used = 0; }
+      cur.push_back(it); used += need;
+    }
+    if (!cur.empty()) waves.push_back(cur);
   }
-  cudaFreeAsync(td, st);
-  return e ? e : (int)cudaGetLastError();
+  GroupSchedule s;
+  size_t w_max = 0;
+  int64_t blocks = 0;
+  for (auto& w : waves) {
+    w_max = std::max(w_max, w.size());
+    int64_t b = 0;
+    for (const Item& it : w) b += it.nblk;
+    blocks = std::max(blocks, b);
+  }
+  s.block_csr(w_max);
+  double* blk = nullptr;                             // per-block log det and info of the wave being factored
+  cudaError_t ce = cudaMallocAsync((void**)&blk, (size_t)blocks * (sizeof(double) + sizeof(int)) + 16, st);
+  if (ce != cudaSuccess) return (int)ce;
+
+  int e = 0;
+  for (auto& w : waves) {
+    std::stable_sort(w.begin(), w.end(), [](const Item& p, const Item& q) { return p.nblk > q.nblk; });
+    const int W = (int)w.size(), nb_max = w[0].nblk;
+    std::vector<CovObj> objs(W);
+    std::vector<double*> a(W);
+    std::vector<int64_t> ld(W), koff(nb_max + 1, 0);
+    std::vector<int> nblk(W);
+    int64_t cur = 0, cta = 0, mm_max = 0;
+    for (int i = 0; i < W; ++i) {
+      const Item& it = w[i];
+      const int64_t np = it.n_pad, mp = it.m_pad;
+      CovObj& o = objs[i];
+      o.cov = covs[it.j]; o.cov_g = covs_g[it.j];
+      o.x = x + dim * off[it.b]; o.yerr = yerr ? yerr + off[it.b] : nullptr; o.g = goff ? xnew + dim * goff[it.b] : xnew;
+      o.a = work + cur; o.v = o.a + np * np; o.c = o.v + mp * np; o.out = out + coff[it.j];
+      o.n = it.n; o.n_pad = np; o.m = it.m; o.m_pad = mp; o.io = it.j; o.cta0 = cta;
+      cur += large_cov_ws_doubles(it.n, it.m);
+      cta += (np + mp) * ((np + 255) / 256) + mp * ((mp + 255) / 256);
+      mm_max = std::max(mm_max, it.m * it.m);
+      a[i] = o.a; ld[i] = np; nblk[i] = it.nblk;
+    }
+    if (cta > 2147483647LL) { e = (int)cudaErrorInvalidValue; break; }
+    for (int k = 0; k < nb_max; ++k) { int c = 0; while (c < W && nblk[c] > k) ++c; koff[k + 1] = koff[k] + c; }
+    double* ldb = blk;
+    int* infob = reinterpret_cast<int*>(blk + koff[nb_max]);
+    const size_t t_objs = s.put(objs.data(), W * sizeof(CovObj));
+    const size_t t_ld = s.put(ld.data(), W * sizeof(int64_t));
+    const size_t t_koff = s.put(koff.data(), koff.size() * sizeof(int64_t));
+    s.launches.push_back({L_COV, cta, W, 0, t_objs, 0, 0, nullptr, nullptr});
+    if ((e = s.factor(work, a, ld, nblk, t_ld, koff, ldb, infob))) break;
+    for (int k = 0; k < nb_max && !e; ++k) {       // large_trsm_rows: V[:,k] -= V[:,0:k] L[k,0:k]^T, then V[:,k] T_kk^T
+      const int64_t k0 = (int64_t)k * 128;
+      if (k > 0) {
+        for (int i = 0; i < W && nblk[i] > k; ++i)
+          s.gemm(objs[i].v, ld[i], a[i] + k0 * ld[i], ld[i], objs[i].v + k0, ld[i], objs[i].m_pad, 128, k0, -1.0, 1.0, 0);
+        if ((e = s.flush())) break;
+      }
+      for (int i = 0; i < W && nblk[i] > k; ++i)
+        s.gemm(objs[i].v + k0, ld[i], a[i] + k0 * ld[i] + k0, ld[i], objs[i].v + k0, ld[i], objs[i].m_pad, 128, 128, 1.0, 0.0, 0);
+      e = s.flush();
+    }
+    if (e) break;
+    for (int i = 0; i < W; ++i)                      // C = K** - V V^T, the whole m_pad x m_pad block
+      s.gemm(objs[i].v, ld[i], objs[i].v, ld[i], objs[i].c, objs[i].m_pad, objs[i].m_pad, objs[i].m_pad, ld[i], -1.0, 1.0, 0);
+    if ((e = s.flush())) break;
+    const int64_t gx = std::min<int64_t>(std::max<int64_t>((mm_max + 1023) / 1024, 1), 1024);
+    s.launches.push_back({L_PACK, gx, W, 0, t_objs, t_koff, 0, ldb, infob});
+  }
+  if (!e)
+    e = s.run(work, st, [&](const Launch& l, const char* td) {
+      const CovObj* objs = reinterpret_cast<const CovObj*>(td + l.t0);
+      switch (l.kind) {
+        case L_COV:
+          if (dim == 1) cov3_build_grouped_kernel<1><<<(unsigned)l.grid, 128, 0, st>>>(objs, (int)l.count);
+          else cov3_build_grouped_kernel<2><<<(unsigned)l.grid, 128, 0, st>>>(objs, (int)l.count);
+          break;
+        case L_PACK:
+          cov_pack_grouped_kernel<<<dim3((unsigned)l.grid, (unsigned)l.count), 256, 0, st>>>(
+              objs, l.infob, reinterpret_cast<const int64_t*>(td + l.t1), info);
+          break;
+      }
+    });
+  cudaFreeAsync(blk, st);
+  return e;
 }
 
 }  // namespace cgp

@@ -228,3 +228,80 @@ def predictive_covariance(x, y_err, grid, hyp, nugget, dim, flags=0):
     _lib.check(L.cgp_gemm_nt_dev(_p(v), obj.n_pad, _p(v), obj.n_pad, _p(c), m_pad, m_pad, m_pad, obj.n_pad,
                                  -1.0, 1.0, 0, st), "cgp_gemm_nt_dev")
     return c[:m, :m].cpu().numpy()
+
+
+def cov_ws_doubles(n, m):
+    """Device workspace (doubles) of objects of n points on grids of m in predictive_covariances, elementwise
+    (cgp_large_cov_ws_doubles): n_pad^2 + m_pad n_pad + m_pad^2 with both padded to a multiple of 128 (at least 128)."""
+    n_pad, m_pad = (np.maximum((np.asarray(v, dtype=np.int64) + 127) // 128, 1) * 128 for v in (n, m))
+    return n_pad * n_pad + m_pad * n_pad + m_pad * m_pad
+
+
+def plan_chunks(out_bytes, ws_bytes=None, out_budget=256 << 20, ws_budget=2 << 30):
+    """Bounds [0, .., K] of consecutive chunks of K items: a chunk closes before the item that would take its output
+    above out_budget or its workspace above ws_budget (a single item larger than either is a chunk of its own)."""
+    bounds, acc_o, acc_w = [0], 0, 0
+    ws = np.zeros(len(out_bytes), dtype=np.int64) if ws_bytes is None else ws_bytes
+    for j in range(len(out_bytes)):
+        if (acc_o or acc_w) and (acc_o + out_bytes[j] > out_budget or acc_w + ws[j] > ws_budget):
+            bounds.append(j)
+            acc_o = acc_w = 0
+        acc_o += int(out_bytes[j])
+        acc_w += int(ws[j])
+    bounds.append(len(out_bytes))
+    return bounds
+
+
+def _gather(flat, off, ids):
+    """The CSR segments `ids` of (flat, off) as a new CSR (flat rows, offsets)."""
+    lens = off[ids + 1] - off[ids]
+    new_off = np.zeros(len(ids) + 1, dtype=np.int64)
+    np.cumsum(lens, out=new_off[1:])
+    idx = np.repeat(off[ids] - new_off[:-1], lens) + np.arange(new_off[-1], dtype=np.int64)
+    return flat[idx], new_off
+
+
+def predictive_covariances(x, off, y_err, grid, goff, hyp, nugget, dim, flags=0, objects=None, work_doubles=None):
+    """predictive_covariance of many objects in one grouped call (cgp_large_covariance_dev), each matrix bit for bit
+    what predictive_covariance gives for that object alone.  x: the objects' points, flat ((P,) or (P, 2)) with CSR
+    offsets off; y_err: flat (P,) or None.  grid: one shared grid ((M,) or (M, 2), goff None) or one grid per object,
+    flat with CSR goff (grid = x, goff = off: the objects' own epochs).  objects: the object ids to compute (default
+    all).  hyp: (n_hyp,) shared, or one row per object of `objects`; nugget: scalar or one per object.  work_doubles:
+    device workspace (default: every object in one wave).  Returns (list of (m_b, m_b) host arrays, info per object);
+    a matrix is NaN where info != 0."""
+    dev = _dev()
+    L = _lib.lib()
+    off = np.asarray(off, dtype=np.int64)
+    ids = np.arange(len(off) - 1, dtype=np.int64) if objects is None else np.asarray(objects, dtype=np.int64)
+    k = len(ids)
+    nh = 2 if dim == 1 else 4
+    hyp = np.asarray(hyp, dtype=np.float64)
+    rows = np.ascontiguousarray(np.broadcast_to(hyp.reshape(-1, nh), (k, nh)) if hyp.ndim == 1 else hyp.reshape(k, nh))
+    nug_rows = None if np.ndim(nugget) == 0 else np.ascontiguousarray(nugget, dtype=np.float64).reshape(k)
+    if not k:
+        return [], np.zeros(0, dtype=np.int32)
+    xs, loff = _gather(np.asarray(x, dtype=np.float64), off, ids)        # only the requested objects go to the device
+    ye = None if y_err is None else _gather(np.asarray(y_err, dtype=np.float64), off, ids)[0]
+    if goff is None:
+        g, lgoff = np.asarray(grid, dtype=np.float64), None
+        m = np.full(k, len(g), dtype=np.int64)
+    else:
+        g, lgoff = _gather(np.asarray(grid, dtype=np.float64), np.asarray(goff, dtype=np.int64), ids)
+        m = np.diff(lgoff)
+    coff = np.zeros(k + 1, dtype=np.int64)
+    np.cumsum(m * m, out=coff[1:])
+    if work_doubles is None:
+        work_doubles = int(cov_ws_doubles(np.diff(loff), m).sum())
+    xd, yd = _t(xs if xs.size else np.zeros(2), dev), _t(ye, dev)      # placeholders keep empty inputs non-NULL
+    gd = _t(g.reshape(-1) if g.size else np.zeros(2), dev)
+    work = torch.empty(max(int(work_doubles), 2), dtype=torch.float64, device=dev)
+    out = torch.empty(max(int(coff[-1]), 1), dtype=torch.float64, device=dev)
+    info = torch.zeros(k, dtype=torch.int32, device=dev)
+    _lib.check(L.cgp_large_covariance_dev(k, _lib.hptr(loff), dim, _p(xd), _p(yd), _lib.hptr(rows), _lib.hptr(nug_rows),
+                                          float(0.0 if nug_rows is not None else nugget), 0.0, int(flags), _p(gd),
+                                          _lib.hptr(lgoff), int(m[0]) if lgoff is None else 0, None, k, _p(out),
+                                          _lib.hptr(coff), _p(info), _p(work), int(work_doubles), _stream(dev)),
+               "cgp_large_covariance_dev")
+    host = out.cpu().numpy()
+    mats = [host[coff[j]:coff[j + 1]].reshape(int(m[j]), int(m[j])) for j in range(k)]
+    return mats, info.cpu().numpy()

@@ -25,6 +25,8 @@ Differences (SURVEY.md section 9.1):
   * y, Time, y_err may also be 2-D ndarrays (equal-length objects), which avoids
     10^5 tiny numpy arrays.
 """
+import os
+
 import numpy as np
 from scipy.optimize import fmin
 
@@ -36,6 +38,9 @@ from .kernel import init_rbf, rbf_kernel_1d, rbf_kernel_2d
 
 _DEVICE = object()                       # marker: the per-object likelihoods of the latest evaluation are still on the device
 _NO_BAD = np.zeros(0, dtype=np.int32)
+# CGP_GROUPED_COV=0: covariance matrices of objects above 64 points one object at a time (dense.predictive_covariance),
+# for comparison with the grouped call (dense.predictive_covariances); read once
+_GROUPED_COV = os.environ.get("CGP_GROUPED_COV", "1") != "0"
 
 
 class _LazyMatrices(object):
@@ -557,14 +562,18 @@ class Gaussian_process:
     def get_covariance_matrix(self):
         """covariance_matrix[sn] = K(grid,grid)+nugget^2 - H K^-1 H^T (:340-361) under the shared hyperparameters.
         Objects of <= 64 points: written in bulk by cgp_covariance_batched_dev, a chunk of objects (<= 256 MB of
-        matrices) per launch pair, when first read; larger objects one by one through the blocked large-object path."""
+        matrices) per launch pair, when first read; larger objects a chunk at a time through the grouped blocked
+        large-object path (dense.predictive_covariances)."""
         self.covariance_matrix = self._covariance_matrices(np.array(self.hyperparameters, dtype=float), float(self.nugget))
 
     def _covariance_matrices(self, hyp, nug):
         """covariance_matrix on the latest prediction's grid, built on access.  hyp (n_hyp,) and nug: shared, on
         self.batch when every object has <= 64 points.  hyp (N_sn, n_hyp) and nug (N_sn,): object i with row i, the
         small objects (batch.SizeSplit) on _small_batch() when each has <= 64 points (cgp_covariance_objhyp_dev).
-        Every other object goes one by one through the blocked large-object path."""
+        Every other object with data and a non-empty grid goes through dense.predictive_covariances (the blocked
+        large-object path, grouped): a chunk of such objects (<= 256 MB of matrices, <= 2 GB of workspace) per call,
+        when one of them is first read; a non-positive-definite object raises LinAlgError when it is read.  Objects
+        without data (the prior) and empty grids are built here; one chunk of each kind is alive at a time."""
         from . import dense
         rows = np.ndim(hyp) == 2
         own = self.as_the_same_time
@@ -595,28 +604,30 @@ class Gaussian_process:
             ids = np.arange(self.N_sn)
             if self._devices is not None or self.N_sn == 0 or int(split.sizes.max()) > 64:
                 ids = ids[:0]
-        if not len(ids):
+        # the objects `make` would send to dense.predictive_covariance, grouped instead: data and a non-empty grid
+        m_obj = np.diff(goff) if ragged else np.full(self.N_sn, len(grid), dtype=np.int64)
+        grouped = np.ones(self.N_sn, dtype=bool)
+        grouped[ids] = False
+        grouped &= (split.sizes > 0) & (m_obj > 0) & _GROUPED_COV
+        gids = np.nonzero(grouped)[0]
+        if not len(ids) and not len(gids):
             return _LazyMatrices(self.N_sn, make)
-        pos = np.full(self.N_sn, -1, dtype=np.int64)         # object i is the batch's object pos[i]
+        pos = np.full(self.N_sn, -1, dtype=np.int64)         # object i is the bulk batch's object pos[i] ...
         pos[ids] = np.arange(len(ids))
+        gpos = np.full(self.N_sn, -1, dtype=np.int64)        # ... or the grouped call's object gpos[i]
+        gpos[gids] = np.arange(len(gids))
         bulk_hyp, bulk_nug = (hyp[ids], nug[ids]) if rows else (hyp, nug)
-        per = (np.diff(goff)[ids] ** 2 if ragged else np.full(len(ids), len(grid) ** 2, dtype=np.int64)) * 8
-        bounds = [0]                                         # chunks of objects with <= 256 MB of matrices
-        acc = 0
-        for j in range(len(ids)):
-            if acc and acc + per[j] > (256 << 20):
-                bounds.append(j); acc = 0
-            acc += per[j]
-        bounds.append(len(ids))
-        cache = {}
+        bounds = dense.plan_chunks(m_obj[ids] ** 2 * 8)      # chunks of objects with <= 256 MB of matrices
+        gout = m_obj[gids] ** 2 * 8                          # ... and <= 2 GB of workspace for the grouped objects
+        gbounds = dense.plan_chunks(gout, dense.cov_ws_doubles(split.sizes[gids], m_obj[gids]) * 8)
+        # one bulk chunk and one grouped chunk of host matrices alive at a time: reading a batch that interleaves the
+        # two kinds in index order builds each chunk once
+        bulk_cache, grouped_cache = {}, {}
 
-        def make_bulk(i):
-            j = int(pos[i])
-            if j < 0:
-                return make(i)
+        def make_bulk(j):
             c = int(np.searchsorted(bounds, j, side="right")) - 1
-            if c not in cache:
-                cache.clear()                                # one chunk of host matrices alive at a time
+            if c not in bulk_cache:
+                bulk_cache.clear()
                 batch = self._small_batch() if rows else self.batch
                 if own:
                     g, kw = None, {}
@@ -630,10 +641,31 @@ class Gaussian_process:
                     full = np.zeros(self.N_sn, dtype=info.dtype)
                     full[ids[bounds[c]:bounds[c + 1]]] = info
                     self._raise_if_bad(full)
-                cache[c] = mats
-            return cache[c][j - bounds[c]]
+                bulk_cache[c] = mats
+            return bulk_cache[c][j - bounds[c]]
 
-        return _LazyMatrices(self.N_sn, make_bulk)
+        def make_grouped(j):
+            c = int(np.searchsorted(gbounds, j, side="right")) - 1
+            if c not in grouped_cache:
+                grouped_cache.clear()
+                sel = gids[gbounds[c]:gbounds[c + 1]]
+                grouped_cache[c] = dense.predictive_covariances(
+                    self._x_flat, self._off, self._ye_flat, grid, goff if ragged else None, hyp[sel] if rows else hyp,
+                    nug[sel] if rows else nug, self._dim, self.flags, objects=sel)
+            mats, info = grouped_cache[c]
+            bad = int(info[j - gbounds[c]])
+            if bad:                                          # as LargeObject.factor: only this object raises
+                raise np.linalg.LinAlgError("%d-th leading minor of the covariance is not positive definite" % bad)
+            return mats[j - gbounds[c]]
+
+        def make_any(i):
+            if pos[i] >= 0:
+                return make_bulk(int(pos[i]))
+            if gpos[i] >= 0:
+                return make_grouped(int(gpos[i]))
+            return make(i)
+
+        return _LazyMatrices(self.N_sn, make_any)
 
 
 class gaussian_process(Gaussian_process):

@@ -262,6 +262,28 @@ int cgp_covariance_objhyp_dev(int64_t n_obj, const int64_t* off, int max_n, int 
                               const double* hyp_obj, const double* nugget_obj, double nugget, double floor, unsigned flags,
                               const double* xnew, const int64_t* goff, const int64_t* goff_host, int64_t m_shared,
                               double* cov, const int64_t* coff, int* info, void* stream);
+/* The covariance matrices of objects of any size (0..65408 points, grids of 0..65408: padded to 128, at most 65535
+ * rows), computed for all active objects of a wave at once by the blocked HBM path, each bit for bit as
+ * dense.predictive_covariance computes it alone: cov_j = K(g, g) + nugget_j^2 I - V V^T, V = rows of L^-1 H^T, where
+ * L L^T = K(x, x) + diag(y_err^2) + (floor^2 + nugget_j^2) I (floor = 0 is dense.predictive_covariance; the floor
+ * never enters K(g, g)).  off_host: the CSR offsets (HOST copy); x, y_err (may be NULL): device
+ * arrays of the batch.  The grid: one shared grid xnew of m_shared points (goff_host NULL), or object b's grid at
+ * xnew + dim * goff_host[b] with goff_host[b+1] - goff_host[b] points (HOST CSR; xnew = x, goff_host = off_host for the
+ * objects' own epochs).  order_host (HOST, may be NULL = objects 0 .. n_obj-1) lists the n_active object ids;
+ * hyp_rows_host (k x nh) and nugget_rows_host (k, may be NULL -> `nugget`) are HOST arrays indexed by position in the
+ * list (shared hyperparameters: one row repeated), as is coff_host (k+1, CSR of m_j^2: cov_j is the m_j x m_j
+ * row-major block at cov + coff_host[j]) and info (k, device).  A block is all NaN where info != 0 (the first failing
+ * pivot, as cgp_potrf_dev reports it).  work: caller-owned device workspace of work_doubles doubles (16-byte aligned);
+ * an object of n points on a grid of m needs cgp_large_cov_ws_doubles(n, m) of it; consecutive objects are packed into
+ * waves that fit.  An object's result does not depend on the other objects of the call, their order or the wave it
+ * lands in.  Does not synchronise.  Returns 0, or < 0 with nothing launched (-2 for a workspace below the largest
+ * active object's need). */
+int64_t cgp_large_cov_ws_doubles(int64_t n, int64_t m);
+int cgp_large_covariance_dev(int64_t n_obj, const int64_t* off_host, int dim, const double* x, const double* y_err,
+                             const double* hyp_rows_host, const double* nugget_rows_host, double nugget, double floor,
+                             unsigned flags, const double* xnew, const int64_t* goff_host, int64_t m_shared,
+                             const int* order_host, int64_t n_active, double* cov, const int64_t* coff_host, int* info,
+                             double* work, int64_t work_doubles, void* stream);
 
 /* ---- matrices for the attribute surface (kernel_matrix, inv_kernel_matrix:
  *      Gaussian_process.py:256-267, 319-325).  moff[n_obj+1]: CSR into the outputs in
