@@ -167,6 +167,13 @@ int64_t large_cov_ws_doubles(int64_t n, int64_t m);
 int large_cov_grouped(int dim, const int64_t* off, const double* x, const double* yerr, const Cov* covs, const Cov* covs_g,
                       const double* xnew, const int64_t* goff, int64_t m_shared, const int* order, int64_t n_active, double* out,
                       const int64_t* coff, int* info, double* work, int64_t work_doubles, cudaStream_t st);
+// grouped means and variance diagonals of large objects, covs[j] (data covariance, with the floor) and covs_g[j] (the
+// prediction, without it) built on the host (see cgp_large_predict_objhyp_dev)
+int64_t large_pred_ws_doubles(int64_t n, int64_t rows);
+int large_predict_grouped(int dim, const int64_t* off, const double* x, const double* y, const double* y0, const double* yerr,
+                          const Cov* covs, const Cov* covs_g, const double* xnew, const int64_t* goff, int64_t m_shared,
+                          const double* new_y0, const int* order, int64_t n_active, const int64_t* moff, double* mean,
+                          double* var, int* info, int64_t chunk_rows, double* work, int64_t work_doubles, cudaStream_t st);
 
 // Launchers (cgp_small.cu).  max_n = largest object in the batch.  Return cudaError_t as int.
 int launch_small(Task task, int dim, int max_n, const SmallArgs& a, cudaStream_t stream);

@@ -238,7 +238,7 @@ __global__ void __launch_bounds__(256) fwd_step_kernel(const double* a, int64_t 
   fwd_step_at(a, ld, k0, n_pad, u, zout, blockIdx.x);
 }
 // backward step k: alpha_k = T_kk^T z_k -> aout;  z[col] -= L[k-block, col]^T alpha_k for cols left of k (in place).
-__global__ void __launch_bounds__(256) bwd_step_kernel(const double* a, int64_t ld, int64_t k0, double* z, double* aout) {
+__device__ __forceinline__ void bwd_step_at(const double* a, int64_t ld, int64_t k0, double* z, double* aout, const int cta) {
   __shared__ double sw[128], sa[128], part[256];
   const int tid = threadIdx.x;
   if (tid < 128) sw[tid] = z[k0 + tid];
@@ -254,8 +254,8 @@ __global__ void __launch_bounds__(256) bwd_step_kernel(const double* a, int64_t 
   __syncthreads();
   if (tid < 128) sa[tid] = part[tid] + part[tid + 128];
   __syncthreads();
-  if (blockIdx.x == 0) { if (tid < 128) aout[k0 + tid] = sa[tid]; return; }
-  const int64_t col = (int64_t)(blockIdx.x - 1) * 128 + (tid & 127);
+  if (cta == 0) { if (tid < 128) aout[k0 + tid] = sa[tid]; return; }
+  const int64_t col = (int64_t)(cta - 1) * 128 + (tid & 127);
   const int h = tid >> 7;
   const double* p = a + (k0 + h * 64) * ld + col;
   double acc = 0.0;
@@ -265,16 +265,20 @@ __global__ void __launch_bounds__(256) bwd_step_kernel(const double* a, int64_t 
   __syncthreads();
   if (tid < 128) z[col] -= part[tid] + part[tid + 128];
 }
+__global__ void __launch_bounds__(256) bwd_step_kernel(const double* a, int64_t ld, int64_t k0, double* z, double* aout) {
+  bwd_step_at(a, ld, k0, z, aout, blockIdx.x);
+}
 
 // ---------------------------------------------------------------------------------------
 // Prediction epilogues.
-// mean[m] = amp_cross * sum_n exp(-q(m,n)/2) alpha_n + y0*[m]  -- cross-covariance never stored.
+// mean[m] = amp_cross * sum_n exp(-q(m,n)/2) alpha_n + y0*[m]  -- cross-covariance never stored.  CTA `cta` takes grid
+// rows [256 cta, 256 cta + 256); sh: 1024 staged columns of x (two rows of them in 2D) and alpha.
 template <int DIM>
-__global__ void __launch_bounds__(256) stream_mean_kernel(const Cov cov, const double* x, const double* alpha, int64_t n,
-                                                          const double* xnew, const double* new_y0, int64_t m, double* mean) {
-  extern __shared__ double sh[];
+__device__ __forceinline__ void stream_mean_at(double* sh, const Cov& cov, const double* x, const double* alpha, int64_t n,
+                                               const double* xnew, const double* new_y0, int64_t m, double* mean,
+                                               const int64_t cta) {
   double* sx = sh; double* sy = sh + 1024; double* sa = sh + (DIM == 2 ? 2048 : 1024);
-  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  const int64_t i = cta * blockDim.x + threadIdx.x;
   double gx = 0.0, gy = 0.0;
   if (i < m) { if (DIM == 1) gx = xnew[i]; else { gx = xnew[2 * i]; gy = xnew[2 * i + 1]; } }
   double acc = 0.0, acc2 = 0.0;
@@ -305,11 +309,17 @@ __global__ void __launch_bounds__(256) stream_mean_kernel(const Cov cov, const d
   }
   if (i < m) mean[i] = fma(cov.amp_cross, acc + acc2, new_y0 ? new_y0[i] : 0.0);
 }
-// var[m] = amp* - |v_m|^2 with v_m = row m of V (mc x n_pad): one warp per row.
-__global__ void __launch_bounds__(256) row_norm_var_kernel(const double* v, int64_t ld, int64_t n_pad, int64_t rows,
-                                                           double amp_star, double* var) {
+template <int DIM>
+__global__ void __launch_bounds__(256) stream_mean_kernel(const Cov cov, const double* x, const double* alpha, int64_t n,
+                                                          const double* xnew, const double* new_y0, int64_t m, double* mean) {
+  extern __shared__ double sh[];
+  stream_mean_at<DIM>(sh, cov, x, alpha, n, xnew, new_y0, m, mean, blockIdx.x);
+}
+// var[m] = amp* - |v_m|^2 with v_m = row m of V (mc x n_pad): one warp per row, rows [8 cta, 8 cta + 8).
+__device__ __forceinline__ void row_norm_var_at(const double* v, int64_t ld, int64_t n_pad, int64_t rows, double amp_star,
+                                                double* var, const int64_t cta) {
   const int lane = threadIdx.x & 31;
-  const int64_t r = (int64_t)blockIdx.x * 8 + (threadIdx.x >> 5);
+  const int64_t r = cta * 8 + (threadIdx.x >> 5);
   if (r >= rows) return;
   const double* p = v + r * ld;
   double acc = 0.0, acc2 = 0.0;
@@ -321,6 +331,10 @@ __global__ void __launch_bounds__(256) row_norm_var_kernel(const double* v, int6
 #pragma unroll
   for (int o = 16; o; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
   if (lane == 0) var[r] = amp_star - acc;
+}
+__global__ void __launch_bounds__(256) row_norm_var_kernel(const double* v, int64_t ld, int64_t n_pad, int64_t rows,
+                                                           double amp_star, double* var) {
+  row_norm_var_at(v, ld, n_pad, rows, amp_star, var, blockIdx.x);
 }
 __device__ __forceinline__ double block_dot_sq(const double* v, int64_t n) {   // |v|^2, valid in thread 0
   __shared__ double s[32];
@@ -560,8 +574,9 @@ __global__ void __launch_bounds__(128) cov_build_grouped_kernel(const GroupObj* 
 }
 
 // Forward sweep step k of the objects objs[0 .. gridDim.y): CTA x of object y runs fwd_step_kernel's CTA x.
-__global__ void __launch_bounds__(256) fwd_step_grouped_kernel(const GroupObj* __restrict__ objs, const int64_t k0) {
-  const GroupObj& o = objs[blockIdx.y];
+template <class Obj>
+__global__ void __launch_bounds__(256) fwd_step_grouped_kernel(const Obj* __restrict__ objs, const int64_t k0) {
+  const Obj& o = objs[blockIdx.y];
   if ((int64_t)blockIdx.x >= 1 + (o.n_pad - k0 - 128 + 63) / 64) return;
   fwd_step_at(o.a, o.n_pad, k0, o.n_pad, o.u, o.z, blockIdx.x);
 }
@@ -661,6 +676,121 @@ __global__ void __launch_bounds__(256) cov_pack_grouped_kernel(const CovObj* __r
   for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < mm; e += (int64_t)gridDim.x * blockDim.x) {
     const int64_t r = e / m;
     o.out[e] = bad ? nan("") : o.c[r * o.m_pad + (e - r * m)];
+  }
+}
+
+// The last object of objs[0 .. n_obj) whose first CTA (field f) is <= t: the object that owns CTA t of a grouped launch
+// (objects without CTAs share their successor's first CTA and are skipped).
+template <class O>
+__device__ __forceinline__ const O& owner(const O* __restrict__ objs, const int n_obj, const int64_t t, int64_t O::*f) {
+  int lo = 0, hi = n_obj - 1;
+  while (lo < hi) {
+    const int mid = (lo + hi + 1) >> 1;
+    if (objs[mid].*f <= t) lo = mid; else hi = mid - 1;
+  }
+  return objs[lo];
+}
+
+// One object of a grouped prediction (large_predict_grouped).  `cov` (with the floor, for A) and `cov_g` (without it, for
+// the mean, H and the variance) come from the host, as the make_cov calls of LargeObject.factor / cgp_large_predict_dev
+// build them.
+struct PredObj {
+  Cov cov, cov_g;
+  const double* x; const double* y; const double* y0; const double* yerr;
+  const double* g; const double* new_y0;   // grid (m points) and the mean function on it (may be null)
+  double* a;                 // n_pad x n_pad covariance -> blocked factor
+  double* u;                 // residual, consumed by the forward sweep
+  double* z;                 // L^-1 (y - y0), consumed by the backward sweep
+  double* alpha;             // K^-1 (y - y0)
+  double* mean; double* var; // the object's m outputs
+  int64_t n, n_pad, m;
+  int64_t io;                // position in `order`: info
+  int64_t cta_a, cta_mean;   // first CTA of the object in the build and in the mean launch
+};
+// One object's rows [r0, r0 + rows) of one variance pass.
+struct PassObj {
+  Cov cov_g;
+  const double* x; const double* g;       // epochs; grid row r0
+  double* v;                 // rows_pad x n_pad: H -> V
+  double* var;               // output row r0
+  int64_t n, n_pad, rows, rows_pad;
+  int64_t cta_h, cta_var;    // first CTA of the object in the H build and in the variance launch
+};
+
+// A = K(x, x) + noise and u = y - y0 of every object of a wave, as cov_build_grouped_kernel builds them.
+template <int DIM>
+__global__ void __launch_bounds__(128) pred_build_grouped_kernel(const PredObj* __restrict__ objs, const int n_obj) {
+  const int64_t t = blockIdx.x;
+  const PredObj& o = owner(objs, n_obj, t, &PredObj::cta_a);
+  const int64_t per_row = (o.n_pad + 255) / 256;
+  const int64_t local = t - o.cta_a, r = local / per_row, chunk = local - r * per_row;
+  if (chunk == 0 && threadIdx.x == 0) o.u[r] = r < o.n ? o.y[r] - (o.y0 ? o.y0[r] : 0.0) : 0.0;   // residual_kernel
+  CovArgs a;
+  a.dim = DIM; a.cov = o.cov; a.autocov = 1;
+  a.xc = o.x; a.n = o.n; a.xr = o.x; a.m = o.n; a.yerr = o.yerr;
+  a.out = o.a; a.ld = o.n_pad; a.rows_pad = o.n_pad; a.cols_pad = o.n_pad;
+  cov_build_at<DIM>(a, r, (chunk * 128 + threadIdx.x) * 2);
+}
+
+// Backward sweep launch s of the objects objs[0 .. gridDim.y): object y runs bwd_step_kernel's CTA x of its block
+// n_pad / 128 - 1 - s.
+__global__ void __launch_bounds__(256) bwd_step_grouped_kernel(const PredObj* __restrict__ objs, const int64_t s) {
+  const PredObj& o = objs[blockIdx.y];
+  const int64_t k = o.n_pad / 128 - 1 - s;
+  if ((int64_t)blockIdx.x > k) return;
+  bwd_step_at(o.a, o.n_pad, k * 128, o.z, o.alpha, blockIdx.x);
+}
+
+// stream_mean_kernel for every object of a wave: object i owns ceil(m / 256) CTAs from cta_mean on.
+template <int DIM>
+__global__ void __launch_bounds__(256) stream_mean_grouped_kernel(const PredObj* __restrict__ objs, const int n_obj) {
+  extern __shared__ double sh[];
+  const int64_t t = blockIdx.x;
+  const PredObj& o = owner(objs, n_obj, t, &PredObj::cta_mean);
+  stream_mean_at<DIM>(sh, o.cov_g, o.x, o.alpha, o.n, o.g, o.new_y0, o.m, o.mean, t - o.cta_mean);
+}
+
+// H = K(grid rows of the pass, x) of every object of a pass, zero padded as large_cov_build pads it: rows_pad *
+// ceil(n_pad / 256) CTAs per object.
+template <int DIM>
+__global__ void __launch_bounds__(128) pass_build_grouped_kernel(const PassObj* __restrict__ objs, const int n_obj) {
+  const int64_t t = blockIdx.x;
+  const PassObj& o = owner(objs, n_obj, t, &PassObj::cta_h);
+  const int64_t per_row = (o.n_pad + 255) / 256;
+  const int64_t local = t - o.cta_h, r = local / per_row, chunk = local - r * per_row;
+  CovArgs a;
+  a.dim = DIM; a.cov = o.cov_g; a.autocov = 0;
+  a.xc = o.x; a.n = o.n; a.xr = o.g; a.m = o.rows; a.yerr = nullptr;
+  a.out = o.v; a.ld = o.n_pad; a.rows_pad = o.rows_pad; a.cols_pad = o.n_pad;
+  cov_build_at<DIM>(a, r, (chunk * 128 + threadIdx.x) * 2);
+}
+
+// var = (amp_auto + nugget^2) - |v|^2 for the rows of a pass (row_norm_var_kernel): ceil(rows / 8) CTAs per object.
+__global__ void __launch_bounds__(256) row_var_grouped_kernel(const PassObj* __restrict__ objs, const int n_obj) {
+  const int64_t t = blockIdx.x;
+  const PassObj& o = owner(objs, n_obj, t, &PassObj::cta_var);
+  row_norm_var_at(o.v, o.n_pad, o.n_pad, o.rows, o.cov_g.amp_auto + o.cov_g.nugget2, o.var, t - o.cta_var);
+}
+
+// Object blockIdx.y of a wave: its info (as cov_pack_grouped_kernel finds it) and NaN over its mean and variance rows
+// where info != 0.
+__global__ void __launch_bounds__(256) pred_finish_grouped_kernel(const PredObj* __restrict__ objs, const int* __restrict__ infob,
+                                                                  const int64_t* __restrict__ koff, int* __restrict__ info) {
+  const int i = blockIdx.y;
+  const PredObj& o = objs[i];
+  __shared__ int bad_s;
+  if (threadIdx.x == 0) {
+    const int nblk = (int)(o.n_pad / 128);
+    int bad = 0;
+    for (int k = 0; k < nblk && !bad; ++k) { const int ik = infob[koff[k] + i]; if (ik) bad = k * 128 + ik; }
+    bad_s = bad;
+    if (blockIdx.x == 0) info[o.io] = bad;
+  }
+  __syncthreads();
+  if (!bad_s) return;
+  for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < o.m; e += (int64_t)gridDim.x * blockDim.x) {
+    o.mean[e] = nan("");
+    if (o.var) o.var[e] = nan("");
   }
 }
 
@@ -1135,7 +1265,7 @@ int64_t large_ll_ws_doubles(int64_t n) {
 // is recorded on the host first; the arguments (object descriptors, GEMM problems, block offsets) are packed into one
 // byte table that crosses to the device in one copy into stream-ordered scratch.
 namespace {
-enum { L_DIAG, L_GEMM, L_COV, L_FWD, L_FIN, L_PACK };
+enum { L_DIAG, L_GEMM, L_COV, L_FWD, L_FIN, L_PACK, L_BWD, L_MEAN, L_HB, L_VAR };
 struct Launch { int kind; int64_t grid, count, k0; size_t t0, t1, t2; double* ldb; int* infob; };
 
 struct GroupSchedule {
@@ -1356,7 +1486,7 @@ int large_ll_grouped(int dim, const int64_t* off, const double* x, const double*
         else cov_build_grouped_kernel<2><<<(unsigned)l.grid, 128, 0, st>>>(objs, (int)l.count, h);
         break;
       case L_FWD:
-        fwd_step_grouped_kernel<<<dim3((unsigned)l.grid, (unsigned)l.count), 256, 0, st>>>(objs, l.k0);
+        fwd_step_grouped_kernel<GroupObj><<<dim3((unsigned)l.grid, (unsigned)l.count), 256, 0, st>>>(objs, l.k0);
         break;
       case L_FIN:
         ll_finish_grouped_kernel<<<(unsigned)l.grid, 1024, 0, st>>>(objs, l.ldb, l.infob,
@@ -1470,6 +1600,168 @@ int large_cov_grouped(int dim, const int64_t* off, const double* x, const double
           break;
         case L_PACK:
           cov_pack_grouped_kernel<<<dim3((unsigned)l.grid, (unsigned)l.count), 256, 0, st>>>(
+              objs, l.infob, reinterpret_cast<const int64_t*>(td + l.t1), info);
+          break;
+      }
+    });
+  cudaFreeAsync(blk, st);
+  return e;
+}
+
+int64_t large_pred_ws_doubles(int64_t n, int64_t rows) {
+  const int64_t np = n <= 0 ? 128 : (n + 127) / 128 * 128, rp = rows <= 0 ? 0 : (rows + 127) / 128 * 128;
+  return np * np + 3 * np + rp * np;                 // covariance / factor, u, z, alpha, H -> V of one pass
+}
+
+// Means (and variance diagonals when var != null) of the objects order[0 .. n_active) on their grids (goff: xnew + dim *
+// goff[b], m_b = goff[b+1] - goff[b]; NULL: the shared grid xnew of m_shared points), object order[j] with covs[j] for A
+// and covs_g[j] for the rest, outputs at mean / var / new_y0 + moff[j], by every step of LargeObject.factor followed by
+// cgp_large_predict_dev run for all objects of a wave at once: A and u in one launch; the factorisation
+// (GroupSchedule::factor); one forward- and one backward-sweep launch per block; the streamed mean in one launch; then per
+// pass of at most chunk_rows grid rows (% 128 == 0) per object: H in one launch, V = rows of L^-1 H^T as large_trsm_rows
+// computes it, and the variance in one launch; last, info and NaN rows where info != 0.  A row's arithmetic does not
+// depend on the pass it falls in.  Waves and their order as in large_ll_grouped, each object's part of the workspace
+// large_pred_ws_doubles(n_b, var ? min(m_b, chunk_rows) : 0).  The caller checks that every object fits.
+int large_predict_grouped(int dim, const int64_t* off, const double* x, const double* y, const double* y0, const double* yerr,
+                          const Cov* covs, const Cov* covs_g, const double* xnew, const int64_t* goff, int64_t m_shared,
+                          const double* new_y0, const int* order, int64_t n_active, const int64_t* moff, double* mean,
+                          double* var, int* info, int64_t chunk_rows, double* work, int64_t work_doubles, cudaStream_t st) {
+  struct Item { int64_t j, b, n, n_pad, m, rows; int nblk; };
+  std::vector<std::vector<Item>> waves;
+  {
+    std::vector<Item> cur; int64_t used = 0;
+    for (int64_t j = 0; j < n_active; ++j) {
+      Item it; it.j = j; it.b = order ? order[j] : j; it.n = off[it.b + 1] - off[it.b];
+      it.m = goff ? goff[it.b + 1] - goff[it.b] : m_shared;
+      it.n_pad = it.n <= 0 ? 128 : (it.n + 127) / 128 * 128; it.nblk = (int)(it.n_pad / 128);
+      it.rows = var ? std::min(it.m, chunk_rows) : 0;
+      const int64_t need = large_pred_ws_doubles(it.n, it.rows);
+      if (!cur.empty() && (used + need > work_doubles || cur.size() >= 65535)) { waves.push_back(cur); cur.clear(); used = 0; }
+      cur.push_back(it); used += need;
+    }
+    if (!cur.empty()) waves.push_back(cur);
+  }
+  GroupSchedule s;
+  size_t w_max = 0;
+  int64_t blocks = 0;
+  for (auto& w : waves) {
+    w_max = std::max(w_max, w.size());
+    int64_t b = 0;
+    for (const Item& it : w) b += it.nblk;
+    blocks = std::max(blocks, b);
+  }
+  s.block_csr(w_max);
+  double* blk = nullptr;                             // per-block log det and info of the wave being factored
+  cudaError_t ce = cudaMallocAsync((void**)&blk, (size_t)blocks * (sizeof(double) + sizeof(int)) + 16, st);
+  if (ce != cudaSuccess) return (int)ce;
+
+  int e = 0;
+  for (auto& w : waves) {
+    std::stable_sort(w.begin(), w.end(), [](const Item& p, const Item& q) { return p.nblk > q.nblk; });
+    const int W = (int)w.size(), nb_max = w[0].nblk;
+    std::vector<PredObj> objs(W);
+    std::vector<double*> a(W), v(W);
+    std::vector<int64_t> ld(W), koff(nb_max + 1, 0);
+    std::vector<int> nblk(W);
+    int64_t cur = 0, cta = 0, cta_mean = 0, m_max = 0;
+    for (int i = 0; i < W; ++i) {
+      const Item& it = w[i];
+      const int64_t np = it.n_pad, o0 = off[it.b];
+      PredObj& o = objs[i];
+      o.cov = covs[it.j]; o.cov_g = covs_g[it.j];
+      o.x = x + dim * o0; o.y = y + o0; o.y0 = y0 ? y0 + o0 : nullptr; o.yerr = yerr ? yerr + o0 : nullptr;
+      o.g = goff ? xnew + dim * goff[it.b] : xnew; o.new_y0 = new_y0 ? new_y0 + moff[it.j] : nullptr;
+      o.a = work + cur; o.u = o.a + np * np; o.z = o.u + np; o.alpha = o.z + np; v[i] = o.alpha + np;
+      o.mean = mean + moff[it.j]; o.var = var ? var + moff[it.j] : nullptr;
+      o.n = it.n; o.n_pad = np; o.m = it.m; o.io = it.j; o.cta_a = cta; o.cta_mean = cta_mean;
+      cur += large_pred_ws_doubles(it.n, it.rows);
+      cta += np * ((np + 255) / 256); cta_mean += (it.m + 255) / 256;
+      m_max = std::max(m_max, it.m);
+      a[i] = o.a; ld[i] = np; nblk[i] = it.nblk;
+    }
+    if (cta > 2147483647LL || cta_mean > 2147483647LL) { e = (int)cudaErrorInvalidValue; break; }
+    auto count = [&](int k) { int c = 0; while (c < W && nblk[c] > k) ++c; return c; };   // objects with block k
+    for (int k = 0; k < nb_max; ++k) koff[k + 1] = koff[k] + count(k);
+    double* ldb = blk;
+    int* infob = reinterpret_cast<int*>(blk + koff[nb_max]);
+    const size_t t_objs = s.put(objs.data(), W * sizeof(PredObj));
+    const size_t t_ld = s.put(ld.data(), W * sizeof(int64_t));
+    const size_t t_koff = s.put(koff.data(), koff.size() * sizeof(int64_t));
+    s.launches.push_back({L_COV, cta, W, 0, t_objs, 0, 0, nullptr, nullptr});
+    if ((e = s.factor(work, a, ld, nblk, t_ld, koff, ldb, infob))) break;
+    for (int k = 0; k < nb_max; ++k)                 // large_potrs: z = L^-1 u
+      s.launches.push_back({L_FWD, 1 + (ld[0] - (int64_t)k * 128 - 128 + 63) / 64, count(k), (int64_t)k * 128, t_objs, 0, 0,
+                            nullptr, nullptr});
+    for (int q = 0; q < nb_max; ++q)                 // large_potrs_backward: alpha = L^-T z, block nblk - 1 - q of each
+      s.launches.push_back({L_BWD, nb_max - q, count(q), q, t_objs, 0, 0, nullptr, nullptr});
+    if (cta_mean) s.launches.push_back({L_MEAN, cta_mean, W, 0, t_objs, 0, 0, nullptr, nullptr});
+    for (int64_t r0 = 0; var && r0 < m_max && !e; r0 += chunk_rows) {   // variance passes
+      std::vector<PassObj> pass;
+      std::vector<int> who;                          // wave position of each object of the pass
+      int64_t cta_h = 0, cta_var = 0;
+      for (int i = 0; i < W; ++i) {
+        const PredObj& o = objs[i];
+        if (o.m <= r0) continue;
+        PassObj p;
+        p.cov_g = o.cov_g; p.x = o.x; p.g = o.g + dim * r0; p.v = v[i]; p.var = o.var + r0;
+        p.n = o.n; p.n_pad = o.n_pad; p.rows = std::min(chunk_rows, o.m - r0); p.rows_pad = (p.rows + 127) / 128 * 128;
+        p.cta_h = cta_h; p.cta_var = cta_var;
+        cta_h += p.rows_pad * ((p.n_pad + 255) / 256); cta_var += (p.rows + 7) / 8;
+        pass.push_back(p); who.push_back(i);
+      }
+      if (cta_h > 2147483647LL) { e = (int)cudaErrorInvalidValue; break; }
+      const int P = (int)pass.size();
+      const size_t t_pass = s.put(pass.data(), P * sizeof(PassObj));
+      s.launches.push_back({L_HB, cta_h, P, 0, t_pass, 0, 0, nullptr, nullptr});
+      for (int k = 0; k < nb_max && !e; ++k) {       // large_trsm_rows: V[:,k] -= V[:,0:k] L[k,0:k]^T, then V[:,k] T_kk^T
+        const int64_t k0 = (int64_t)k * 128;
+        if (k > 0) {
+          for (int q = 0; q < P; ++q) {
+            const int i = who[q];
+            if (nblk[i] > k) s.gemm(v[i], ld[i], a[i] + k0 * ld[i], ld[i], v[i] + k0, ld[i], pass[q].rows_pad, 128, k0, -1.0, 1.0, 0);
+          }
+          if ((e = s.flush())) break;
+        }
+        for (int q = 0; q < P; ++q) {
+          const int i = who[q];
+          if (nblk[i] > k) s.gemm(v[i] + k0, ld[i], a[i] + k0 * ld[i] + k0, ld[i], v[i] + k0, ld[i], pass[q].rows_pad, 128, 128, 1.0, 0.0, 0);
+        }
+        e = s.flush();
+      }
+      s.launches.push_back({L_VAR, cta_var, P, 0, t_pass, 0, 0, nullptr, nullptr});
+    }
+    if (e) break;
+    const int64_t gx = std::min<int64_t>(std::max<int64_t>((m_max + 1023) / 1024, 1), 1024);
+    s.launches.push_back({L_FIN, gx, W, 0, t_objs, t_koff, 0, ldb, infob});
+  }
+  if (!e)
+    e = s.run(work, st, [&](const Launch& l, const char* td) {
+      const PredObj* objs = reinterpret_cast<const PredObj*>(td + l.t0);
+      const PassObj* pass = reinterpret_cast<const PassObj*>(td + l.t0);
+      switch (l.kind) {
+        case L_COV:
+          if (dim == 1) pred_build_grouped_kernel<1><<<(unsigned)l.grid, 128, 0, st>>>(objs, (int)l.count);
+          else pred_build_grouped_kernel<2><<<(unsigned)l.grid, 128, 0, st>>>(objs, (int)l.count);
+          break;
+        case L_FWD:
+          fwd_step_grouped_kernel<PredObj><<<dim3((unsigned)l.grid, (unsigned)l.count), 256, 0, st>>>(objs, l.k0);
+          break;
+        case L_BWD:
+          bwd_step_grouped_kernel<<<dim3((unsigned)l.grid, (unsigned)l.count), 256, 0, st>>>(objs, l.k0);
+          break;
+        case L_MEAN:
+          if (dim == 1) stream_mean_grouped_kernel<1><<<(unsigned)l.grid, 256, 2 * 1024 * sizeof(double), st>>>(objs, (int)l.count);
+          else stream_mean_grouped_kernel<2><<<(unsigned)l.grid, 256, 3 * 1024 * sizeof(double), st>>>(objs, (int)l.count);
+          break;
+        case L_HB:
+          if (dim == 1) pass_build_grouped_kernel<1><<<(unsigned)l.grid, 128, 0, st>>>(pass, (int)l.count);
+          else pass_build_grouped_kernel<2><<<(unsigned)l.grid, 128, 0, st>>>(pass, (int)l.count);
+          break;
+        case L_VAR:
+          row_var_grouped_kernel<<<(unsigned)l.grid, 256, 0, st>>>(pass, (int)l.count);
+          break;
+        case L_FIN:
+          pred_finish_grouped_kernel<<<dim3((unsigned)l.grid, (unsigned)l.count), 256, 0, st>>>(
               objs, l.infob, reinterpret_cast<const int64_t*>(td + l.t1), info);
           break;
       }

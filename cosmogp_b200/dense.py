@@ -305,3 +305,84 @@ def predictive_covariances(x, off, y_err, grid, goff, hyp, nugget, dim, flags=0,
     host = out.cpu().numpy()
     mats = [host[coff[j]:coff[j + 1]].reshape(int(m[j]), int(m[j])) for j in range(k)]
     return mats, info.cpu().numpy()
+
+
+def pred_ws_doubles(n, rows):
+    """Device workspace (doubles) of objects of n points in predictions, `rows` grid rows per variance pass (0: means
+    only), elementwise (cgp_large_pred_ws_doubles): n_pad^2 + 3 n_pad + rows_pad n_pad."""
+    n_pad = np.maximum((np.asarray(n, dtype=np.int64) + 127) // 128, 1) * 128
+    rows_pad = (np.asarray(rows, dtype=np.int64) + 127) // 128 * 128
+    return n_pad * n_pad + 3 * n_pad + rows_pad * n_pad
+
+
+def predictions(x, off, y, y0, y_err, grid, goff, new_y0, hyp, nugget, dim, flags=0, objects=None, want_var=True,
+                chunk_rows=None):
+    """LargeObject(x_b, y_b, y_err_b, y0_b).factor(hyp, nugget) followed by .predict(grid_b, new_y0_b) for many objects,
+    in grouped calls (cgp_large_predict_objhyp_dev), each mean and variance bit for bit that loop's.  x, y, y0, y_err:
+    the objects' points, flat with CSR offsets off (y0, y_err may be None).  grid: one shared grid ((M,) or (M, 2), goff
+    None) or one grid per object, flat with CSR goff (grid = x, goff = off: the objects' own epochs).  objects: the object
+    ids to predict (default all).  new_y0: the mean function on the grids, flat in the output layout (the grids of
+    `objects` one after the other), or None.  hyp: (n_hyp,) shared, or one row per object of `objects`; nugget: scalar or
+    one per object.  chunk_rows: grid rows per variance pass and object (a multiple of 128; default: a pass of up to 2 GB
+    per object, as LargeObject.predict).  The objects go in chunks of <= 256 MB of outputs and <= 2 GB of workspace
+    (plan_chunks).  Returns (mean, variance or None, flat in the output layout; CSR of the output rows; info per
+    object); an object's rows are NaN where info != 0."""
+    dev = _dev()
+    L = _lib.lib()
+    off = np.asarray(off, dtype=np.int64)
+    ids = np.arange(len(off) - 1, dtype=np.int64) if objects is None else np.asarray(objects, dtype=np.int64)
+    k = len(ids)
+    nh = 2 if dim == 1 else 4
+    hyp = np.asarray(hyp, dtype=np.float64)
+    rows = np.ascontiguousarray(np.broadcast_to(hyp.reshape(-1, nh), (k, nh)) if hyp.ndim == 1 else hyp.reshape(k, nh))
+    nug_rows = np.ascontiguousarray(np.broadcast_to(np.asarray(nugget, dtype=np.float64), (k,)))
+    n = off[ids + 1] - off[ids]
+    m = np.diff(np.asarray(goff, dtype=np.int64))[ids] if goff is not None else np.full(k, len(grid), dtype=np.int64)
+    moff = np.zeros(k + 1, dtype=np.int64)
+    np.cumsum(m, out=moff[1:])
+    mean = np.empty(int(moff[-1]))
+    var = np.empty(int(moff[-1])) if want_var else None
+    info = np.zeros(k, dtype=np.int32)
+    if not k:
+        return mean, var, moff, info
+    if chunk_rows is None:
+        chunk_rows = max(128, (2 << 30) // (8 * pad128(int(n.max()))))
+    chunk_rows = int(chunk_rows) // 128 * 128 or 128
+    ws = pred_ws_doubles(n, np.minimum(m, chunk_rows) if want_var else 0)
+    bounds = plan_chunks(m * (16 if want_var else 8), ws * 8)
+    work = torch.empty(max(max(int(ws[b0:b1].sum()) for b0, b1 in zip(bounds[:-1], bounds[1:])), 2),
+                       dtype=torch.float64, device=dev)
+    st = _stream(dev)
+    new_y0 = None if new_y0 is None else np.asarray(new_y0, dtype=np.float64).reshape(-1)
+    for b0, b1 in zip(bounds[:-1], bounds[1:]):
+        sel = ids[b0:b1]
+        xs, loff = _gather(np.asarray(x, dtype=np.float64), off, sel)      # only the requested objects go to the device
+        ys = _gather(np.asarray(y, dtype=np.float64), off, sel)[0]
+        y0s = None if y0 is None else _gather(np.asarray(y0, dtype=np.float64), off, sel)[0]
+        yes = None if y_err is None else _gather(np.asarray(y_err, dtype=np.float64), off, sel)[0]
+        if goff is None:
+            g, lgoff = np.asarray(grid, dtype=np.float64), None
+        else:
+            g, lgoff = _gather(np.asarray(grid, dtype=np.float64), np.asarray(goff, dtype=np.int64), sel)
+        c0, c1 = int(moff[b0]), int(moff[b1])
+        lmoff = np.ascontiguousarray(moff[b0:b1 + 1] - c0)
+        # every device array bound to a name until the call has been enqueued
+        xd = _t(xs if xs.size else np.zeros(2), dev)                    # placeholders keep empty inputs non-NULL
+        yd = _t(ys if ys.size else np.zeros(2), dev)
+        y0d, yed = _t(y0s, dev), _t(yes, dev)
+        gd = _t(g.reshape(-1) if g.size else np.zeros(2), dev)
+        ny0 = None if new_y0 is None else _t(new_y0[c0:c1], dev)
+        md = torch.empty(max(c1 - c0, 1), dtype=torch.float64, device=dev)
+        vd = torch.empty(max(c1 - c0, 1), dtype=torch.float64, device=dev) if want_var else None
+        infod = torch.zeros(b1 - b0, dtype=torch.int32, device=dev)
+        hr, nr = np.ascontiguousarray(rows[b0:b1]), np.ascontiguousarray(nug_rows[b0:b1])
+        _lib.check(L.cgp_large_predict_objhyp_dev(
+            b1 - b0, _lib.hptr(loff), dim, _p(xd), _p(yd), _p(y0d), _p(yed), _lib.hptr(hr), _lib.hptr(nr), 0.0, 0.0,
+            int(flags), _p(gd), _lib.hptr(lgoff), int(len(g)) if lgoff is None else 0, _p(ny0), None, b1 - b0,
+            _lib.hptr(lmoff), _p(md), _p(vd), _p(infod), chunk_rows, _p(work), int(work.numel()), st),
+            "cgp_large_predict_objhyp_dev")
+        mean[c0:c1] = md[:c1 - c0].cpu().numpy()
+        if want_var:
+            var[c0:c1] = vd[:c1 - c0].cpu().numpy()
+        info[b0:b1] = infod.cpu().numpy()
+    return mean, var, moff, info

@@ -3,9 +3,10 @@ gaussian_process_nobject (cosmogp/Gaussian_process.py:78-393): same constructor
 arguments, methods, attributes and error behaviour; numpy in, numpy out.  The
 per-object Python loops of the reference (:207, :264, :304, :349) are replaced by
 single batched launches on a device-resident copy of the data.  Which objects are too large for those launches is
-decided in one place, batch.SizeSplit; they go through the blocked HBM factorisation: one at a time for shared
-hyperparameters (dense.LargeObject, every object of the batch then), all at once for the likelihood evaluations of
-per-object fits (cgp_large_ll_objhyp_dev), one at a time for per-object predictions.
+decided in one place, batch.SizeSplit; they go through the blocked HBM factorisation: one at a time for likelihoods
+under shared hyperparameters (dense.LargeObject, every object of the batch then), all at once for the likelihood
+evaluations of per-object fits (cgp_large_ll_objhyp_dev) and for predictions (dense.predictions: the large objects of a
+per-object prediction, or every object of a batch with a large one under shared hyperparameters).
 
 Differences (SURVEY.md section 9.1):
   * `svd_method`: every object is factorised by the device Cholesky kernels whatever the flag says (for a
@@ -207,8 +208,9 @@ class Gaussian_process:
 
     @property
     def _any_large(self):
-        """With shared hyperparameters, a batch with any large object (batch.SizeSplit) goes one object at a time
-        through the HBM-resident blocked factorisation (`_large_objects`).  Sharded objects decide from the sizes of
+        """With shared hyperparameters, a batch with any large object (batch.SizeSplit) goes through the HBM-resident
+        blocked factorisation: likelihoods one object at a time (`_large_objects`), predictions all objects in grouped
+        calls (dense.predictions).  Sharded objects decide from the sizes of
         ALL objects, so that every rank takes the same branch (and the same collectives)."""
         return len((self._all_split if self._dist else self._split).large) > 0
 
@@ -435,8 +437,8 @@ class Gaussian_process:
         object with its own fit (`hyperparameters_per_object`, `nugget_per_object`); with COV=True
         `covariance_matrix[i]` is then object i's predictive covariance under its fit as it stood at this call.
         devices=... does not take per_object.  Objects go down one of three routes, by batch.SizeSplit: the batched
-        kernels; one dense.LargeObject at a time (the large objects of a per-object prediction, or every object of a
-        batch with a large one under shared hyperparameters); and, under shared hyperparameters with svd_method=True,
+        kernels; the grouped blocked path, dense.predictions (the large objects of a per-object prediction, or every
+        object of a batch with a large one under shared hyperparameters); and, under shared hyperparameters with svd_method=True,
         the host SVD redo of the objects whose covariance is not positive definite.  Otherwise such an object raises
         LinAlgError."""
         own = new_binning is None
@@ -488,15 +490,15 @@ class Gaussian_process:
                 return grid[s], (None if new_y0 is None else new_y0[s])
             return grid, (None if new_y0 is None else new_y0[i])
 
-        # routes: the batched kernels on `batched`, one LargeObject at a time for `one_by_one`
+        # routes: the batched kernels on `batched`, the grouped blocked path (dense.predictions) for `blocked`
         split = self._split
         if per_object:
-            batched, one_by_one = self._small_batch(), split.large
+            batched, blocked = self._small_batch(), split.large
         elif self._any_large:
-            batched, one_by_one = None, range(self.N_sn)
+            batched, blocked = None, np.arange(self.N_sn, dtype=np.int64)
         else:
-            batched, one_by_one = self.batch, ()
-        whole = batched is not None and not len(one_by_one)      # the batched outputs are the outputs
+            batched, blocked = self.batch, ()
+        whole = batched is not None and not len(blocked)         # the batched outputs are the outputs
         if not whole:
             mean, info = np.empty(int(rows[-1])), np.zeros(self.N_sn, dtype=np.int32)
             var = np.empty(int(rows[-1])) if want_var else None
@@ -520,22 +522,26 @@ class Gaussian_process:
                 if want_var:
                     var[at] = v.reshape(-1)
                 info[objs] = inf
-        for i in one_by_one:
-            obj = self._large_object(i) if per_object else self._large_objects()[i]
-            try:
-                obj.factor(hyp_b[i] if per_object else hyp, nug_b[i] if per_object else nug)
-            except np.linalg.LinAlgError:
-                if not (per_object or svd_method):
-                    raise
-                info[i] = 1
-                continue
-            s = slice(int(rows[i]), int(rows[i + 1]))
-            g, ny0 = on_grid(i)
-            if not len(g):                                  # an empty grid: nothing to predict, the factor gave the info
-                continue
-            mean[s], v = obj.predict(g, new_y0=ny0, want_var=want_var)
+        if len(blocked):
+            from . import dense
+            if new_y0 is None:                               # the mean function in the outputs' layout of `blocked`
+                ny0 = None
+            elif per_grid:
+                ny0 = dense._gather(new_y0, rows, blocked)[0]
+            else:                                            # template + diff[i], the add of _LazyMeanOnGrid
+                ny0 = new_y0.template[None, :] + new_y0.diff[blocked][:, None]
+            m, v, _, inf = dense.predictions(self._x_flat, self._off, self._y_flat, self._y0_flat, self._ye_flat, grid,
+                                             rows if per_grid else None, ny0, hyp_b[blocked] if per_object else hyp,
+                                             nug_b[blocked] if per_object else nug, self._dim, self.flags,
+                                             objects=blocked, want_var=want_var)
+            bad = np.nonzero(inf)[0]
+            if len(bad) and not (per_object or svd_method):  # the error LargeObject.factor raises for the first one
+                raise np.linalg.LinAlgError("%d-th leading minor of the covariance is not positive definite" % int(inf[bad[0]]))
+            at = dense._gather(np.arange(int(rows[-1]), dtype=np.int64), rows, blocked)[0]
+            mean[at] = m
             if want_var:
-                var[s] = v
+                var[at] = v
+            info[blocked] = inf != 0
         if info.any() and svd_method and not per_object:
             for i in np.nonzero(info)[0]:
                 s = slice(int(rows[i]), int(rows[i + 1]))

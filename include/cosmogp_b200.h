@@ -284,6 +284,28 @@ int cgp_large_covariance_dev(int64_t n_obj, const int64_t* off_host, int dim, co
                              unsigned flags, const double* xnew, const int64_t* goff_host, int64_t m_shared,
                              const int* order_host, int64_t n_active, double* cov, const int64_t* coff_host, int* info,
                              double* work, int64_t work_doubles, void* stream);
+/* The means (and variance diagonals) of objects of any size (0..65408 points) on grids of any length, computed for all
+ * active objects of a wave at once by the blocked HBM path, each bit for bit what cgp_cov_matrix_dev + cgp_potrf_dev +
+ * cgp_large_solve_dev (dense.LargeObject.factor) followed by cgp_large_predict_dev compute for it alone:
+ * mean_j = amp_cross H K^-1 (y - y0) + new_y0 and var_j = (amp_auto + nugget_j^2) - |rows of L^-1 H^T|^2, where
+ * L L^T = K(x, x) + diag(y_err^2) + (floor^2 + nugget_j^2) I.  Objects, grids, order_host, hyp_rows_host and
+ * nugget_rows_host as in cgp_large_covariance_dev; y, y0 (may be NULL) and y_err (may be NULL): device arrays of the
+ * batch.  moff_host (HOST, k+1): CSR of m_j over the list; object order_host[j]'s outputs are mean / var + moff_host[j]
+ * (device; var NULL: means only) and it reads new_y0 + moff_host[j] (device, may be NULL: zero mean function).
+ * info (k, device): the first failing pivot; NaN rows where info != 0.  Variances are computed chunk_rows (a positive
+ * multiple of 128) grid rows per object at a time; a row's bits do not depend on chunk_rows.  work: caller-owned device
+ * workspace of work_doubles doubles (16-byte aligned); an object of n points on a grid of m needs
+ * cgp_large_pred_ws_doubles(n, var ? min(m, chunk_rows) : 0) of it; consecutive objects are packed into waves that fit.
+ * Does not synchronise.  Returns 0, or < 0 with nothing launched (-2 for a workspace below the largest active object's
+ * need). */
+int64_t cgp_large_pred_ws_doubles(int64_t n, int64_t rows);
+int cgp_large_predict_objhyp_dev(int64_t n_obj, const int64_t* off_host, int dim, const double* x, const double* y,
+                                 const double* y0, const double* y_err, const double* hyp_rows_host,
+                                 const double* nugget_rows_host, double nugget, double floor, unsigned flags,
+                                 const double* xnew, const int64_t* goff_host, int64_t m_shared, const double* new_y0,
+                                 const int* order_host, int64_t n_active, const int64_t* moff_host, double* mean,
+                                 double* var, int* info, int64_t chunk_rows, double* work, int64_t work_doubles,
+                                 void* stream);
 
 /* ---- matrices for the attribute surface (kernel_matrix, inv_kernel_matrix:
  *      Gaussian_process.py:256-267, 319-325).  moff[n_obj+1]: CSR into the outputs in
