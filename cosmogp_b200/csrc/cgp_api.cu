@@ -141,6 +141,42 @@ static int count_bad(const int* info, int64_t n) {
   return c > 2147483647 ? 2147483647 : (int)c;
 }
 
+// The active objects order[0 .. k) (object ids; NULL: 0 .. k) of a grouped large-object entry: each must be an object
+// id with 0 .. max_pts points and pass check(j, b, n, w), the entry's own checks, which set w to its workspace; the
+// workspace must hold the largest w.
+template <class F>
+static int check_active(const char* name, int64_t n_obj, const int64_t* off, const int* order, int64_t k, int64_t max_pts,
+                        int64_t work_doubles, F&& check) {
+  int64_t need = 0;
+  for (int64_t j = 0; j < k; ++j) {
+    const int64_t b = order ? order[j] : j;
+    if (b < 0 || b >= n_obj) return fail(CGP_ERR_ARG, "%s: order[%lld] = %lld is not an object id", name, (long long)j, (long long)b);
+    const int64_t n = off[b + 1] - off[b];
+    if (n < 0 || n > max_pts)
+      return fail(CGP_ERR_SIZE, "%s: object %lld has %lld points (0..%lld)", name, (long long)b, (long long)n, (long long)max_pts);
+    int64_t w = 0;
+    if (int rc = check(j, b, n, w)) return rc;
+    if (w > need) need = w;
+  }
+  if (work_doubles < need)
+    return fail(CGP_ERR_SIZE, "%s: workspace of %lld doubles is below the %lld the largest active object needs", name,
+                (long long)work_doubles, (long long)need);
+  return 0;
+}
+
+// Cov of the active objects on the host from their hyperparameter rows, as the per-object paths build them: covs[j]
+// with the floor (the data covariance only), covs_g[j] without it.  Nugget j: nugget_rows[j], or `nugget` when NULL.
+static void host_covs(int dim, const double* hyp_rows, const double* nugget_rows, double nugget, double floor, unsigned flags,
+                      int64_t k, std::vector<Cov>& covs, std::vector<Cov>& covs_g) {
+  const int nh = dim == 1 ? 2 : 4;
+  covs.resize((size_t)k); covs_g.resize((size_t)k);
+  for (int64_t j = 0; j < k; ++j) {
+    const double nu = nugget_rows ? nugget_rows[j] : nugget;
+    covs[j] = cov_from_hyp(dim, hyp_rows + j * nh, nu, floor, flags);
+    covs_g[j] = cov_from_hyp(dim, hyp_rows + j * nh, nu, 0.0, flags);
+  }
+}
+
 }  // namespace cgp
 
 using namespace cgp;
@@ -262,18 +298,9 @@ int cgp_large_ll_objhyp_dev(int64_t n_obj, const int64_t* off_host, int dim,
     return fail(CGP_ERR_ARG, "cgp_large_ll_objhyp_dev: NULL argument");
   if (dim != 1 && dim != 2) return fail(CGP_ERR_ARG, "dim must be 1 or 2, got %d", dim);
   if ((uintptr_t)work & 15) return fail(CGP_ERR_ARG, "cgp_large_ll_objhyp_dev: work must be 16-byte aligned");
-  int64_t need = 0;
-  for (int64_t j = 0; j < k; ++j) {
-    const int64_t b = order_host ? order_host[j] : j;
-    if (b < 0 || b >= n_obj) return fail(CGP_ERR_ARG, "cgp_large_ll_objhyp_dev: order[%lld] = %lld is not an object id", (long long)j, (long long)b);
-    const int64_t n = off_host[b + 1] - off_host[b];
-    if (n < 0 || n > 65535) return fail(CGP_ERR_SIZE, "cgp_large_ll_objhyp_dev: object %lld has %lld points (0..65535)", (long long)b, (long long)n);
-    const int64_t w = large_ll_ws_doubles(n);
-    if (w > need) need = w;
-  }
-  if (work_doubles < need)
-    return fail(CGP_ERR_SIZE, "cgp_large_ll_objhyp_dev: workspace of %lld doubles is below the %lld the largest active object needs",
-                (long long)work_doubles, (long long)need);
+  int rc = check_active("cgp_large_ll_objhyp_dev", n_obj, off_host, order_host, k, 65535, work_doubles,
+                        [](int64_t, int64_t, int64_t n, int64_t& w) { w = large_ll_ws_doubles(n); return 0; });
+  if (rc) return rc;
   keep_pool_memory();
   int e = large_ll_grouped(dim, off_host, x, y, y0, y_err, hyp_obj, nugget_obj, nugget, floor, flags, order_host, k, ll_obj, info,
                            work, work_doubles, (cudaStream_t)stream);
@@ -299,32 +326,18 @@ int cgp_large_covariance_dev(int64_t n_obj, const int64_t* off_host, int dim, co
   const int64_t max_pts = 65535 / 128 * 128;
   if (!goff_host && (m_shared < 0 || m_shared > max_pts))
     return fail(CGP_ERR_SIZE, "%s: shared grid of %lld points (0..%lld)", name, (long long)m_shared, (long long)max_pts);
-  int64_t need = 0;
-  for (int64_t j = 0; j < k; ++j) {
-    const int64_t b = order_host ? order_host[j] : j;
-    if (b < 0 || b >= n_obj) return fail(CGP_ERR_ARG, "%s: order[%lld] = %lld is not an object id", name, (long long)j, (long long)b);
-    const int64_t n = off_host[b + 1] - off_host[b];
-    if (n < 0 || n > max_pts)
-      return fail(CGP_ERR_SIZE, "%s: object %lld has %lld points (0..%lld)", name, (long long)b, (long long)n, (long long)max_pts);
+  int rc = check_active(name, n_obj, off_host, order_host, k, max_pts, work_doubles, [&](int64_t j, int64_t b, int64_t n, int64_t& w) {
     const int64_t m = goff_host ? goff_host[b + 1] - goff_host[b] : m_shared;
     if (m < 0 || m > max_pts)
       return fail(CGP_ERR_SIZE, "%s: grid of object %lld has %lld points (0..%lld)", name, (long long)b, (long long)m, (long long)max_pts);
     if (coff_host[j + 1] - coff_host[j] != m * m)
       return fail(CGP_ERR_ARG, "%s: coff[%lld + 1] - coff[%lld] is not the grid's %lld^2 entries", name, (long long)j, (long long)j, (long long)m);
-    const int64_t w = large_cov_ws_doubles(n, m);
-    if (w > need) need = w;
-  }
-  if (work_doubles < need)
-    return fail(CGP_ERR_SIZE, "%s: workspace of %lld doubles is below the %lld the largest active object needs", name,
-                (long long)work_doubles, (long long)need);
-  // Cov of every object on the host, as cgp_cov_matrix_dev builds them: the floor enters the data covariance only
-  const int nh = dim == 1 ? 2 : 4;
-  std::vector<Cov> covs((size_t)k), covs_g((size_t)k);
-  for (int64_t j = 0; j < k; ++j) {
-    const double nu = nugget_rows_host ? nugget_rows_host[j] : nugget;
-    covs[j] = cov_from_hyp(dim, hyp_rows_host + j * nh, nu, floor, flags);
-    covs_g[j] = cov_from_hyp(dim, hyp_rows_host + j * nh, nu, 0.0, flags);
-  }
+    w = large_cov_ws_doubles(n, m);
+    return 0;
+  });
+  if (rc) return rc;
+  std::vector<Cov> covs, covs_g;                     // as cgp_cov_matrix_dev builds them
+  host_covs(dim, hyp_rows_host, nugget_rows_host, nugget, floor, flags, k, covs, covs_g);
   keep_pool_memory();
   int e = large_cov_grouped(dim, off_host, x, y_err, covs.data(), covs_g.data(), xnew, goff_host, m_shared, order_host, k, cov, coff_host,
                             info, work, work_doubles, (cudaStream_t)stream);
@@ -352,31 +365,17 @@ int cgp_large_predict_objhyp_dev(int64_t n_obj, const int64_t* off_host, int dim
   if (!goff_host && m_shared < 0) return fail(CGP_ERR_ARG, "%s: negative grid size", name);
   // padded sizes stay within the 65535 rows cgp_cov_matrix_dev builds an auto-covariance for
   const int64_t max_pts = 65535 / 128 * 128;
-  int64_t need = 0;
-  for (int64_t j = 0; j < k; ++j) {
-    const int64_t b = order_host ? order_host[j] : j;
-    if (b < 0 || b >= n_obj) return fail(CGP_ERR_ARG, "%s: order[%lld] = %lld is not an object id", name, (long long)j, (long long)b);
-    const int64_t n = off_host[b + 1] - off_host[b];
-    if (n < 0 || n > max_pts)
-      return fail(CGP_ERR_SIZE, "%s: object %lld has %lld points (0..%lld)", name, (long long)b, (long long)n, (long long)max_pts);
+  int rc = check_active(name, n_obj, off_host, order_host, k, max_pts, work_doubles, [&](int64_t j, int64_t b, int64_t n, int64_t& w) {
     const int64_t m = goff_host ? goff_host[b + 1] - goff_host[b] : m_shared;
     if (m < 0) return fail(CGP_ERR_ARG, "%s: grid of object %lld has %lld points", name, (long long)b, (long long)m);
     if (moff_host[j + 1] - moff_host[j] != m)
       return fail(CGP_ERR_ARG, "%s: moff[%lld + 1] - moff[%lld] is not the grid's %lld points", name, (long long)j, (long long)j, (long long)m);
-    const int64_t w = large_pred_ws_doubles(n, var ? std::min(m, chunk_rows) : 0);
-    if (w > need) need = w;
-  }
-  if (work_doubles < need)
-    return fail(CGP_ERR_SIZE, "%s: workspace of %lld doubles is below the %lld the largest active object needs", name,
-                (long long)work_doubles, (long long)need);
-  // Cov of every object on the host, as LargeObject's make_cov calls build them: the floor enters the data covariance only
-  const int nh = dim == 1 ? 2 : 4;
-  std::vector<Cov> covs((size_t)k), covs_g((size_t)k);
-  for (int64_t j = 0; j < k; ++j) {
-    const double nu = nugget_rows_host ? nugget_rows_host[j] : nugget;
-    covs[j] = cov_from_hyp(dim, hyp_rows_host + j * nh, nu, floor, flags);
-    covs_g[j] = cov_from_hyp(dim, hyp_rows_host + j * nh, nu, 0.0, flags);
-  }
+    w = large_pred_ws_doubles(n, var ? std::min(m, chunk_rows) : 0);
+    return 0;
+  });
+  if (rc) return rc;
+  std::vector<Cov> covs, covs_g;                     // as LargeObject's make_cov calls build them
+  host_covs(dim, hyp_rows_host, nugget_rows_host, nugget, floor, flags, k, covs, covs_g);
   keep_pool_memory();
   int e = large_predict_grouped(dim, off_host, x, y, y0, y_err, covs.data(), covs_g.data(), xnew, goff_host, m_shared, new_y0,
                                 order_host, k, moff_host, mean, var, info, chunk_rows, work, work_doubles, (cudaStream_t)stream);

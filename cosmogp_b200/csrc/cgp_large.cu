@@ -546,6 +546,28 @@ struct GroupHyp {
   const double* hyp_obj; const double* nugget_obj; double nugget, floor; unsigned flags;
 };
 
+// The last object of objs[0 .. n_obj) whose first CTA (field f) is <= t: the object that owns CTA t of a grouped launch
+// (objects without CTAs share their successor's first CTA and are skipped).
+template <class O>
+__device__ __forceinline__ const O& owner(const O* __restrict__ objs, const int n_obj, const int64_t t, int64_t O::*f) {
+  int lo = 0, hi = n_obj - 1;
+  while (lo < hi) {
+    const int mid = (lo + hi + 1) >> 1;
+    if (objs[mid].*f <= t) lo = mid; else hi = mid - 1;
+  }
+  return objs[lo];
+}
+
+// The first failing pivot of object i of a wave, as potrf_finish_kernel reports it: k * 128 + info of its first block k
+// with info != 0 (block k at infob[koff[k] + i]), 0 when every block is positive definite.
+__device__ __forceinline__ int first_bad_pivot(const int* __restrict__ infob, const int64_t* __restrict__ koff, int i, int nblk) {
+  for (int k = 0; k < nblk; ++k) {
+    const int ik = infob[koff[k] + i];
+    if (ik) return k * 128 + ik;
+  }
+  return 0;
+}
+
 template <int DIM>
 __device__ __forceinline__ Cov group_cov(const GroupHyp& h, int64_t io) {
   return cov_from_hyp(DIM, h.hyp_obj + io * (DIM == 1 ? 2 : 4), h.nugget_obj ? h.nugget_obj[io] : h.nugget, h.floor, h.flags);
@@ -557,12 +579,7 @@ template <int DIM>
 __global__ void __launch_bounds__(128) cov_build_grouped_kernel(const GroupObj* __restrict__ objs, const int n_obj,
                                                                 const GroupHyp h) {
   const int64_t t = blockIdx.x;
-  int lo = 0, hi = n_obj - 1;
-  while (lo < hi) {
-    const int mid = (lo + hi + 1) >> 1;
-    if (objs[mid].cta0 <= t) lo = mid; else hi = mid - 1;
-  }
-  const GroupObj& o = objs[lo];
+  const GroupObj& o = owner(objs, n_obj, t, &GroupObj::cta0);
   const int64_t per_row = (o.n_pad + 255) / 256;
   const int64_t local = t - o.cta0, r = local / per_row, chunk = local - r * per_row;
   CovArgs a;
@@ -594,12 +611,9 @@ __global__ void __launch_bounds__(1024) ll_finish_grouped_kernel(const GroupObj*
   const double quad = block_dot_sq(o.z, o.n_pad);
   if (threadIdx.x == 0) {
     const int nblk = (int)(o.n_pad / 128);
-    double s = 0.0; int bad = 0;
-    for (int k = 0; k < nblk; ++k) {
-      s += ld_blocks[koff[k] + i];
-      const int ik = info_blocks[koff[k] + i];
-      if (!bad && ik) bad = k * 128 + ik;
-    }
+    double s = 0.0;
+    for (int k = 0; k < nblk; ++k) s += ld_blocks[koff[k] + i];
+    const int bad = first_bad_pivot(info_blocks, koff, i, nblk);
     const double log_2pi = 1.8378770664093453;                 // math.log(2 * math.pi)
     ll[o.io] = bad ? nan("") : __dmul_rn(-0.5, __dadd_rn(__dadd_rn(quad, s), __dmul_rn((double)o.n, log_2pi)));
     info[o.io] = bad;
@@ -627,12 +641,7 @@ struct CovObj {
 template <int DIM>
 __global__ void __launch_bounds__(128) cov3_build_grouped_kernel(const CovObj* __restrict__ objs, const int n_obj) {
   const int64_t t = blockIdx.x;
-  int lo = 0, hi = n_obj - 1;
-  while (lo < hi) {
-    const int mid = (lo + hi + 1) >> 1;
-    if (objs[mid].cta0 <= t) lo = mid; else hi = mid - 1;
-  }
-  const CovObj& o = objs[lo];
+  const CovObj& o = owner(objs, n_obj, t, &CovObj::cta0);
   const int64_t pn = (o.n_pad + 255) / 256, pm = (o.m_pad + 255) / 256;
   int64_t local = t - o.cta0, per_row;
   CovArgs a;
@@ -656,17 +665,15 @@ __global__ void __launch_bounds__(128) cov3_build_grouped_kernel(const CovObj* _
   cov_build_at<DIM>(a, r, (chunk * 128 + threadIdx.x) * 2);
 }
 
-// Object blockIdx.y of a wave: its info (the first failing pivot, summed over the blocks as potrf_finish_kernel does;
-// block k at infob[koff[k] + object]) and its leading m x m block of C packed to `out`, all NaN where info != 0.
+// Object blockIdx.y of a wave: its info (first_bad_pivot) and its leading m x m block of C packed to `out`, all NaN
+// where info != 0.
 __global__ void __launch_bounds__(256) cov_pack_grouped_kernel(const CovObj* __restrict__ objs, const int* __restrict__ infob,
                                                                const int64_t* __restrict__ koff, int* __restrict__ info) {
   const int i = blockIdx.y;
   const CovObj& o = objs[i];
   __shared__ int bad_s;
   if (threadIdx.x == 0) {
-    const int nblk = (int)(o.n_pad / 128);
-    int bad = 0;
-    for (int k = 0; k < nblk && !bad; ++k) { const int ik = infob[koff[k] + i]; if (ik) bad = k * 128 + ik; }
+    const int bad = first_bad_pivot(infob, koff, i, (int)(o.n_pad / 128));
     bad_s = bad;
     if (blockIdx.x == 0) info[o.io] = bad;
   }
@@ -677,18 +684,6 @@ __global__ void __launch_bounds__(256) cov_pack_grouped_kernel(const CovObj* __r
     const int64_t r = e / m;
     o.out[e] = bad ? nan("") : o.c[r * o.m_pad + (e - r * m)];
   }
-}
-
-// The last object of objs[0 .. n_obj) whose first CTA (field f) is <= t: the object that owns CTA t of a grouped launch
-// (objects without CTAs share their successor's first CTA and are skipped).
-template <class O>
-__device__ __forceinline__ const O& owner(const O* __restrict__ objs, const int n_obj, const int64_t t, int64_t O::*f) {
-  int lo = 0, hi = n_obj - 1;
-  while (lo < hi) {
-    const int mid = (lo + hi + 1) >> 1;
-    if (objs[mid].*f <= t) lo = mid; else hi = mid - 1;
-  }
-  return objs[lo];
 }
 
 // One object of a grouped prediction (large_predict_grouped).  `cov` (with the floor, for A) and `cov_g` (without it, for
@@ -772,17 +767,14 @@ __global__ void __launch_bounds__(256) row_var_grouped_kernel(const PassObj* __r
   row_norm_var_at(o.v, o.n_pad, o.n_pad, o.rows, o.cov_g.amp_auto + o.cov_g.nugget2, o.var, t - o.cta_var);
 }
 
-// Object blockIdx.y of a wave: its info (as cov_pack_grouped_kernel finds it) and NaN over its mean and variance rows
-// where info != 0.
+// Object blockIdx.y of a wave: its info (first_bad_pivot) and NaN over its mean and variance rows where info != 0.
 __global__ void __launch_bounds__(256) pred_finish_grouped_kernel(const PredObj* __restrict__ objs, const int* __restrict__ infob,
                                                                   const int64_t* __restrict__ koff, int* __restrict__ info) {
   const int i = blockIdx.y;
   const PredObj& o = objs[i];
   __shared__ int bad_s;
   if (threadIdx.x == 0) {
-    const int nblk = (int)(o.n_pad / 128);
-    int bad = 0;
-    for (int k = 0; k < nblk && !bad; ++k) { const int ik = infob[koff[k] + i]; if (ik) bad = k * 128 + ik; }
+    const int bad = first_bad_pivot(infob, koff, i, (int)(o.n_pad / 128));
     bad_s = bad;
     if (blockIdx.x == 0) info[o.io] = bad;
   }
@@ -1261,12 +1253,68 @@ int64_t large_ll_ws_doubles(int64_t n) {
 }
 
 // ---------------------------------------------------------------------------------------
-// Schedules of the grouped large-object pipelines (large_ll_grouped, large_cov_grouped).  Every launch of every wave
-// is recorded on the host first; the arguments (object descriptors, GEMM problems, block offsets) are packed into one
-// byte table that crosses to the device in one copy into stream-ordered scratch.
+// Schedules of the grouped large-object pipelines (large_ll_grouped, large_cov_grouped, large_predict_grouped).  Every
+// launch of every wave is recorded on the host first; the arguments (object descriptors, GEMM problems, block offsets)
+// are packed into one byte table that crosses to the device in one copy into stream-ordered scratch.
 namespace {
 enum { L_DIAG, L_GEMM, L_COV, L_FWD, L_FIN, L_PACK, L_BWD, L_MEAN, L_HB, L_VAR };
 struct Launch { int kind; int64_t grid, count, k0; size_t t0, t1, t2; double* ldb; int* infob; };
+
+// One object of a wave: position j in `order`, object id b, n points, n_pad = 128 nblk (at least one block).
+struct WaveItem { int64_t j, b, n, n_pad; int nblk; };
+using Waves = std::vector<std::vector<WaveItem>>;
+
+// The objects order[0 .. n_active) (object ids; NULL: 0 .. n_active) packed into consecutive waves: a wave closes
+// before the object whose part of the workspace, need(item), would take it above work_doubles, and at 65535 objects
+// (the y extent of the per-object launches).  Inside a wave the objects are sorted by decreasing block count (stable),
+// so that the objects taking part in any step of the factorisation are a prefix of the wave.
+template <class F>
+Waves plan_waves(const int* order, int64_t n_active, const int64_t* off, int64_t work_doubles, F&& need) {
+  Waves waves;
+  std::vector<WaveItem> cur; int64_t used = 0;
+  for (int64_t j = 0; j < n_active; ++j) {
+    WaveItem it; it.j = j; it.b = order ? order[j] : j; it.n = off[it.b + 1] - off[it.b];
+    it.n_pad = it.n <= 0 ? 128 : (it.n + 127) / 128 * 128; it.nblk = (int)(it.n_pad / 128);
+    const int64_t w = need(it);
+    if (!cur.empty() && (used + w > work_doubles || cur.size() >= 65535)) { waves.push_back(cur); cur.clear(); used = 0; }
+    cur.push_back(it); used += w;
+  }
+  if (!cur.empty()) waves.push_back(cur);
+  for (auto& w : waves)
+    std::stable_sort(w.begin(), w.end(), [](const WaveItem& p, const WaveItem& q) { return p.nblk > q.nblk; });
+  return waves;
+}
+
+// One sorted wave as the factorisation sees it: object i's n_pad x n_pad matrix at a[i], leading dimension ld[i] =
+// n_pad, nblk[i] = n_pad / 128 blocks.  Block k of object i leaves its log det and info at [koff[k] + i] of the wave's
+// block arrays.  t_ld, t_koff: ld and koff in the schedule's table.
+struct WaveTables {
+  std::vector<double*> a;
+  std::vector<int64_t> ld, koff;
+  std::vector<int> nblk;
+  size_t t_ld = 0, t_koff = 0;
+  int count(int k) const { int c = 0; while (c < (int)nblk.size() && nblk[c] > k) ++c; return c; }   // objects with block k
+};
+
+// Per-block log dets and infos of the wave being factored (large_cov_grouped, large_predict_grouped), in stream-ordered
+// scratch sized for the wave with the most blocks and freed when it goes out of scope.
+struct BlockScratch {
+  double* p = nullptr;
+  cudaStream_t st;
+  explicit BlockScratch(cudaStream_t s) : st(s) {}
+  ~BlockScratch() { if (p) cudaFreeAsync(p, st); }
+  int alloc(const Waves& waves) {
+    int64_t blocks = 0;
+    for (const auto& w : waves) {
+      int64_t b = 0;
+      for (const WaveItem& it : w) b += it.nblk;
+      blocks = std::max(blocks, b);
+    }
+    return (int)cudaMallocAsync((void**)&p, (size_t)blocks * (sizeof(double) + sizeof(int)) + 16, st);
+  }
+  double* ldb() const { return p; }
+  int* infob(const WaveTables& t) const { return reinterpret_cast<int*>(p + t.koff.back()); }
+};
 
 struct GroupSchedule {
   std::vector<char> tab;
@@ -1280,11 +1328,24 @@ struct GroupSchedule {
     memcpy(tab.data() + o, p, bytes);
     return o;
   }
-  // the CSR {0, 128, 256, ..} the diagonal-block launches read, for waves of up to w_max objects
-  void block_csr(size_t w_max) {
+  // the CSR {0, 128, 256, ..} the diagonal-block launches read, for the largest wave
+  void block_csr(const Waves& waves) {
+    size_t w_max = 0;
+    for (const auto& w : waves) w_max = std::max(w_max, w.size());
     std::vector<int64_t> csr(w_max + 1);
     for (size_t i = 0; i <= w_max; ++i) csr[i] = (int64_t)i * 128;
     t_csr = put(csr.data(), csr.size() * sizeof(int64_t));
+  }
+  // the tables of the sorted wave w whose matrices are at a[i]; ld and koff go into the table
+  WaveTables tables(const std::vector<WaveItem>& w, std::vector<double*> a) {
+    WaveTables t;
+    const int W = (int)w.size(), nb_max = w[0].nblk;
+    t.a = std::move(a); t.ld.resize(W); t.nblk.resize(W); t.koff.assign(nb_max + 1, 0);
+    for (int i = 0; i < W; ++i) { t.ld[i] = w[i].n_pad; t.nblk[i] = w[i].nblk; }
+    for (int k = 0; k < nb_max; ++k) t.koff[k + 1] = t.koff[k] + t.count(k);
+    t.t_ld = put(t.ld.data(), W * sizeof(int64_t));
+    t.t_koff = put(t.koff.data(), t.koff.size() * sizeof(int64_t));
+    return t;
   }
   void gemm(const double* A, int64_t lda, const double* B, int64_t ldb, double* C, int64_t ldc, int64_t m, int64_t n,
             int64_t k, double alpha, double beta, int lower) {
@@ -1310,21 +1371,21 @@ struct GroupSchedule {
     probs.clear();
     return 0;
   }
-  // The blocked Cholesky of large_potrf for the matrices of one wave: object i's n_pad x n_pad matrix at a[i] (inside
-  // `work`, leading dimension ld[i] = n_pad, nblk[i] = n_pad / 128 blocks, sorted in decreasing order so that the objects
-  // taking part in any step are a prefix).  Per pair of block columns two diagonal-block launches (launch_small in
-  // matrix-source mode, ld table at t_ld) and four grouped GEMM launches, with the shapes, tile split and alpha / beta
-  // large_potrf uses for each object alone (the next pair's columns and the lower trailing update touch disjoint tiles,
-  // so they share one launch).  Block k of object i leaves its log det and info at ldb / infob[koff[k] + i].
-  int factor(double* work, const std::vector<double*>& a, const std::vector<int64_t>& ld, const std::vector<int>& nblk,
-             size_t t_ld, const std::vector<int64_t>& koff, double* ldb, int* infob) {
+  // The blocked Cholesky of large_potrf for the matrices of one wave (the objects taking part in any step are a prefix).
+  // Per pair of block columns two diagonal-block launches (launch_small in matrix-source mode, ld table at t.t_ld) and
+  // four grouped GEMM launches, with the shapes, tile split and alpha / beta large_potrf uses for each object alone (the
+  // next pair's columns and the lower trailing update touch disjoint tiles, so they share one launch).  Block k of
+  // object i leaves its log det and info at ldb / infob[t.koff[k] + i].
+  int factor(double* work, const WaveTables& t, double* ldb, int* infob) {
+    const std::vector<double*>& a = t.a;
+    const std::vector<int64_t>& ld = t.ld;
+    const std::vector<int>& nblk = t.nblk;
     const int W = (int)a.size(), nb_max = nblk[0];
-    auto count = [&](int k) { int c = 0; while (c < W && nblk[c] > k) ++c; return c; };   // objects with block k
     auto diag = [&](int k) {
-      const int c = count(k);
+      const int c = t.count(k);
       std::vector<int64_t> aoff(c);
       for (int i = 0; i < c; ++i) aoff[i] = (a[i] - work) + (int64_t)k * 128 * ld[i] + (int64_t)k * 128;
-      launches.push_back({L_DIAG, c, c, 0, put(aoff.data(), c * sizeof(int64_t)), t_ld, 0, ldb + koff[k], infob + koff[k]});
+      launches.push_back({L_DIAG, c, c, 0, put(aoff.data(), c * sizeof(int64_t)), t.t_ld, 0, ldb + t.koff[k], infob + t.koff[k]});
     };
     int e = 0;
     for (int p = 0; 2 * p < nb_max && !e; ++p) {
@@ -1365,6 +1426,29 @@ struct GroupSchedule {
         if (rest > 256)
           gemm(wp + 256 * np, np, wp + 256 * np, np, ai + (k0 + 512) * np + (k0 + 512), np, rest - 256, rest - 256, 256, -1.0,
                1.0, 1);
+      }
+      e = flush();
+    }
+    return e;
+  }
+  // V = rows of L^-1 H^T for objects of a factored wave, as large_trsm_rows computes it: per block column k,
+  // V[:, k] -= V[:, 0:k] L[k, 0:k]^T (from k = 1 on), then V[:, k] T_kk^T, each one grouped launch over the entries
+  // whose object has block k.  Entry: the rows_pad x n_pad matrix V at v of wave object i.
+  struct RowSolve { double* v; int64_t rows_pad; int i; };
+  int trsm_rows(const WaveTables& t, const std::vector<RowSolve>& vs) {
+    int e = 0;
+    for (int k = 0; k < t.nblk[0] && !e; ++k) {
+      const int64_t k0 = (int64_t)k * 128;
+      if (k > 0) {
+        for (const RowSolve& r : vs) {
+          const int64_t ld = t.ld[r.i];
+          if (t.nblk[r.i] > k) gemm(r.v, ld, t.a[r.i] + k0 * ld, ld, r.v + k0, ld, r.rows_pad, 128, k0, -1.0, 1.0, 0);
+        }
+        if ((e = flush())) break;
+      }
+      for (const RowSolve& r : vs) {
+        const int64_t ld = t.ld[r.i];
+        if (t.nblk[r.i] > k) gemm(r.v + k0, ld, t.a[r.i] + k0 * ld + k0, ld, r.v + k0, ld, r.rows_pad, 128, 128, 1.0, 0.0, 0);
       }
       e = flush();
     }
@@ -1416,65 +1500,44 @@ struct GroupSchedule {
 }  // namespace
 
 // Log-likelihoods of the objects order[0 .. n_active) (object ids; NULL: 0 .. n_active), object order[j] with the
-// hyperparameters of row j, by the blocked factorisation of large_potrf run for all objects of a wave at once.
-// Consecutive objects are packed into waves of at most work_doubles (each object's part: large_ll_ws_doubles); inside
-// a wave they are sorted by block count, so that the objects taking part in any step are a prefix of the wave.  Per
-// wave: one covariance launch; the factorisation (GroupSchedule::factor); one forward-sweep launch per block; one
-// epilogue.  The caller checks that every object fits.
+// hyperparameters of row j, by the blocked factorisation of large_potrf run for all objects of a wave at once (waves:
+// plan_waves, each object's part of the workspace large_ll_ws_doubles).  Per wave: one covariance launch; the
+// factorisation (GroupSchedule::factor); one forward-sweep launch per block; one epilogue.  The caller checks that
+// every object fits.
 int large_ll_grouped(int dim, const int64_t* off, const double* x, const double* y, const double* y0, const double* yerr,
                      const double* hyp_obj, const double* nugget_obj, double nugget, double floor, unsigned flags,
                      const int* order, int64_t n_active, double* ll, int* info, double* work, int64_t work_doubles,
                      cudaStream_t st) {
-  struct Item { int64_t j, b, n, n_pad; int nblk; };
-  std::vector<std::vector<Item>> waves;
-  {
-    std::vector<Item> cur; int64_t used = 0;
-    for (int64_t j = 0; j < n_active; ++j) {
-      Item it; it.j = j; it.b = order ? order[j] : j; it.n = off[it.b + 1] - off[it.b];
-      it.n_pad = it.n <= 0 ? 128 : (it.n + 127) / 128 * 128; it.nblk = (int)(it.n_pad / 128);
-      const int64_t need = large_ll_ws_doubles(it.n);
-      if (!cur.empty() && (used + need > work_doubles || cur.size() >= 65535)) { waves.push_back(cur); cur.clear(); used = 0; }
-      cur.push_back(it); used += need;
-    }
-    if (!cur.empty()) waves.push_back(cur);
-  }
+  const Waves waves = plan_waves(order, n_active, off, work_doubles, [](const WaveItem& it) { return large_ll_ws_doubles(it.n); });
   GroupSchedule s;
-  size_t w_max = 0;
-  for (auto& w : waves) w_max = std::max(w_max, w.size());
-  s.block_csr(w_max);
+  s.block_csr(waves);
 
-  for (auto& w : waves) {
-    std::stable_sort(w.begin(), w.end(), [](const Item& p, const Item& q) { return p.nblk > q.nblk; });
-    const int W = (int)w.size(), nb_max = w[0].nblk;
+  for (const auto& w : waves) {
+    const int W = (int)w.size();
     std::vector<GroupObj> objs(W);
     std::vector<double*> a(W);
-    std::vector<int64_t> ld(W), koff(nb_max + 1, 0);
-    std::vector<int> nblk(W);
     int64_t cur = 0, cta = 0;
     for (int i = 0; i < W; ++i) {
-      const Item& it = w[i];
+      const WaveItem& it = w[i];
       const int64_t o0 = off[it.b], np = it.n_pad;
       GroupObj& g = objs[i];
       g.x = x + dim * o0; g.y = y + o0; g.y0 = y0 ? y0 + o0 : nullptr; g.yerr = yerr ? yerr + o0 : nullptr;
       g.a = work + cur; g.u = g.a + np * np; g.z = g.u + np;
       g.n = it.n; g.n_pad = np; g.io = it.j; g.cta0 = cta;
       cur += np * np + 2 * np; cta += np * ((np + 255) / 256);
-      a[i] = g.a; ld[i] = np; nblk[i] = it.nblk;
+      a[i] = g.a;
     }
     if (cta > 2147483647LL) return (int)cudaErrorInvalidValue;
-    auto count = [&](int k) { int c = 0; while (c < W && w[c].nblk > k) ++c; return c; };   // objects with block k
-    for (int k = 0; k < nb_max; ++k) koff[k + 1] = koff[k] + count(k);
-    double* ldb = work + cur;
-    int* infob = reinterpret_cast<int*>(work + cur + koff[nb_max]);
     const size_t t_objs = s.put(objs.data(), W * sizeof(GroupObj));
-    const size_t t_ld = s.put(ld.data(), W * sizeof(int64_t));
-    const size_t t_koff = s.put(koff.data(), koff.size() * sizeof(int64_t));
+    const WaveTables t = s.tables(w, std::move(a));
+    double* ldb = work + cur;                        // the block log dets and infos follow the objects
+    int* infob = reinterpret_cast<int*>(ldb + t.koff.back());
     s.launches.push_back({L_COV, cta, W, 0, t_objs, 0, 0, nullptr, nullptr});
-    if (int e = s.factor(work, a, ld, nblk, t_ld, koff, ldb, infob)) return e;
-    for (int k = 0; k < nb_max; ++k)
-      s.launches.push_back({L_FWD, 1 + (ld[0] - (int64_t)k * 128 - 128 + 63) / 64, count(k), (int64_t)k * 128, t_objs, 0, 0,
+    if (int e = s.factor(work, t, ldb, infob)) return e;
+    for (int k = 0; k < w[0].nblk; ++k)
+      s.launches.push_back({L_FWD, 1 + (t.ld[0] - (int64_t)k * 128 - 128 + 63) / 64, t.count(k), (int64_t)k * 128, t_objs, 0, 0,
                             nullptr, nullptr});
-    s.launches.push_back({L_FIN, W, W, 0, t_objs, t_koff, 0, ldb, infob});
+    s.launches.push_back({L_FIN, W, W, 0, t_objs, t.t_koff, 0, ldb, infob});
   }
 
   GroupHyp h; h.hyp_obj = hyp_obj; h.nugget_obj = nugget_obj; h.nugget = nugget; h.floor = floor; h.flags = flags;
@@ -1504,108 +1567,65 @@ int64_t large_cov_ws_doubles(int64_t n, int64_t m) {
 // Predictive covariance matrices of the objects order[0 .. n_active) (object ids; NULL: 0 .. n_active), object
 // order[j] with covs[j] for its own covariance and covs_g[j] for H and K**, on its grid (goff: xnew + dim * goff[b], m_b = goff[b+1] - goff[b]; NULL: the shared grid
 // xnew of m_shared points), by every step of dense.predictive_covariance run for all objects of a wave at once:
-// A = K(x, x) + noise, H and K** in one launch; the factorisation (GroupSchedule::factor); V = rows of L^-1 H^T as
-// large_trsm_rows computes it (one pair of grouped GEMM launches per block column); C = K** - V V^T (one grouped
-// GEMM launch); the packing of each leading m_b x m_b block to out + coff[j], NaN where info[j] != 0.  Waves and their
-// order as in large_ll_grouped, each object's part of the workspace large_cov_ws_doubles(n_b, m_b).  The block log
-// dets / infos live in stream-ordered scratch.  The caller checks that every object fits.
+// A = K(x, x) + noise, H and K** in one launch; the factorisation (GroupSchedule::factor); V = rows of L^-1 H^T
+// (GroupSchedule::trsm_rows); C = K** - V V^T (one grouped GEMM launch); the packing of each leading m_b x m_b block to
+// out + coff[j], NaN where info[j] != 0.  Waves: plan_waves, each object's part of the workspace
+// large_cov_ws_doubles(n_b, m_b).  The caller checks that every object fits.
 int large_cov_grouped(int dim, const int64_t* off, const double* x, const double* yerr, const Cov* covs, const Cov* covs_g,
                       const double* xnew, const int64_t* goff, int64_t m_shared, const int* order, int64_t n_active, double* out,
                       const int64_t* coff, int* info, double* work, int64_t work_doubles, cudaStream_t st) {
-  struct Item { int64_t j, b, n, n_pad, m, m_pad; int nblk; };
-  std::vector<std::vector<Item>> waves;
-  {
-    std::vector<Item> cur; int64_t used = 0;
-    for (int64_t j = 0; j < n_active; ++j) {
-      Item it; it.j = j; it.b = order ? order[j] : j; it.n = off[it.b + 1] - off[it.b];
-      it.m = goff ? goff[it.b + 1] - goff[it.b] : m_shared;
-      it.n_pad = it.n <= 0 ? 128 : (it.n + 127) / 128 * 128; it.nblk = (int)(it.n_pad / 128);
-      it.m_pad = it.m <= 0 ? 128 : (it.m + 127) / 128 * 128;
-      const int64_t need = large_cov_ws_doubles(it.n, it.m);
-      if (!cur.empty() && (used + need > work_doubles || cur.size() >= 65535)) { waves.push_back(cur); cur.clear(); used = 0; }
-      cur.push_back(it); used += need;
-    }
-    if (!cur.empty()) waves.push_back(cur);
-  }
+  auto grid_size = [&](int64_t b) { return goff ? goff[b + 1] - goff[b] : m_shared; };
+  const Waves waves = plan_waves(order, n_active, off, work_doubles,
+                                 [&](const WaveItem& it) { return large_cov_ws_doubles(it.n, grid_size(it.b)); });
   GroupSchedule s;
-  size_t w_max = 0;
-  int64_t blocks = 0;
-  for (auto& w : waves) {
-    w_max = std::max(w_max, w.size());
-    int64_t b = 0;
-    for (const Item& it : w) b += it.nblk;
-    blocks = std::max(blocks, b);
-  }
-  s.block_csr(w_max);
-  double* blk = nullptr;                             // per-block log det and info of the wave being factored
-  cudaError_t ce = cudaMallocAsync((void**)&blk, (size_t)blocks * (sizeof(double) + sizeof(int)) + 16, st);
-  if (ce != cudaSuccess) return (int)ce;
+  s.block_csr(waves);
+  BlockScratch blk(st);
+  if (int ce = blk.alloc(waves)) return ce;
 
-  int e = 0;
-  for (auto& w : waves) {
-    std::stable_sort(w.begin(), w.end(), [](const Item& p, const Item& q) { return p.nblk > q.nblk; });
-    const int W = (int)w.size(), nb_max = w[0].nblk;
+  for (const auto& w : waves) {
+    const int W = (int)w.size();
     std::vector<CovObj> objs(W);
     std::vector<double*> a(W);
-    std::vector<int64_t> ld(W), koff(nb_max + 1, 0);
-    std::vector<int> nblk(W);
+    std::vector<GroupSchedule::RowSolve> vs(W);
     int64_t cur = 0, cta = 0, mm_max = 0;
     for (int i = 0; i < W; ++i) {
-      const Item& it = w[i];
-      const int64_t np = it.n_pad, mp = it.m_pad;
+      const WaveItem& it = w[i];
+      const int64_t m = grid_size(it.b), np = it.n_pad, mp = m <= 0 ? 128 : (m + 127) / 128 * 128;
       CovObj& o = objs[i];
       o.cov = covs[it.j]; o.cov_g = covs_g[it.j];
       o.x = x + dim * off[it.b]; o.yerr = yerr ? yerr + off[it.b] : nullptr; o.g = goff ? xnew + dim * goff[it.b] : xnew;
       o.a = work + cur; o.v = o.a + np * np; o.c = o.v + mp * np; o.out = out + coff[it.j];
-      o.n = it.n; o.n_pad = np; o.m = it.m; o.m_pad = mp; o.io = it.j; o.cta0 = cta;
-      cur += large_cov_ws_doubles(it.n, it.m);
+      o.n = it.n; o.n_pad = np; o.m = m; o.m_pad = mp; o.io = it.j; o.cta0 = cta;
+      cur += large_cov_ws_doubles(it.n, m);
       cta += (np + mp) * ((np + 255) / 256) + mp * ((mp + 255) / 256);
-      mm_max = std::max(mm_max, it.m * it.m);
-      a[i] = o.a; ld[i] = np; nblk[i] = it.nblk;
+      mm_max = std::max(mm_max, m * m);
+      a[i] = o.a; vs[i] = {o.v, mp, i};
     }
-    if (cta > 2147483647LL) { e = (int)cudaErrorInvalidValue; break; }
-    for (int k = 0; k < nb_max; ++k) { int c = 0; while (c < W && nblk[c] > k) ++c; koff[k + 1] = koff[k] + c; }
-    double* ldb = blk;
-    int* infob = reinterpret_cast<int*>(blk + koff[nb_max]);
+    if (cta > 2147483647LL) return (int)cudaErrorInvalidValue;
     const size_t t_objs = s.put(objs.data(), W * sizeof(CovObj));
-    const size_t t_ld = s.put(ld.data(), W * sizeof(int64_t));
-    const size_t t_koff = s.put(koff.data(), koff.size() * sizeof(int64_t));
+    const WaveTables t = s.tables(w, std::move(a));
     s.launches.push_back({L_COV, cta, W, 0, t_objs, 0, 0, nullptr, nullptr});
-    if ((e = s.factor(work, a, ld, nblk, t_ld, koff, ldb, infob))) break;
-    for (int k = 0; k < nb_max && !e; ++k) {       // large_trsm_rows: V[:,k] -= V[:,0:k] L[k,0:k]^T, then V[:,k] T_kk^T
-      const int64_t k0 = (int64_t)k * 128;
-      if (k > 0) {
-        for (int i = 0; i < W && nblk[i] > k; ++i)
-          s.gemm(objs[i].v, ld[i], a[i] + k0 * ld[i], ld[i], objs[i].v + k0, ld[i], objs[i].m_pad, 128, k0, -1.0, 1.0, 0);
-        if ((e = s.flush())) break;
-      }
-      for (int i = 0; i < W && nblk[i] > k; ++i)
-        s.gemm(objs[i].v + k0, ld[i], a[i] + k0 * ld[i] + k0, ld[i], objs[i].v + k0, ld[i], objs[i].m_pad, 128, 128, 1.0, 0.0, 0);
-      e = s.flush();
-    }
-    if (e) break;
-    for (int i = 0; i < W; ++i)                      // C = K** - V V^T, the whole m_pad x m_pad block
-      s.gemm(objs[i].v, ld[i], objs[i].v, ld[i], objs[i].c, objs[i].m_pad, objs[i].m_pad, objs[i].m_pad, ld[i], -1.0, 1.0, 0);
-    if ((e = s.flush())) break;
+    if (int e = s.factor(work, t, blk.ldb(), blk.infob(t))) return e;
+    if (int e = s.trsm_rows(t, vs)) return e;
+    for (const CovObj& o : objs)                     // C = K** - V V^T, the whole m_pad x m_pad block
+      s.gemm(o.v, o.n_pad, o.v, o.n_pad, o.c, o.m_pad, o.m_pad, o.m_pad, o.n_pad, -1.0, 1.0, 0);
+    if (int e = s.flush()) return e;
     const int64_t gx = std::min<int64_t>(std::max<int64_t>((mm_max + 1023) / 1024, 1), 1024);
-    s.launches.push_back({L_PACK, gx, W, 0, t_objs, t_koff, 0, ldb, infob});
+    s.launches.push_back({L_PACK, gx, W, 0, t_objs, t.t_koff, 0, blk.ldb(), blk.infob(t)});
   }
-  if (!e)
-    e = s.run(work, st, [&](const Launch& l, const char* td) {
-      const CovObj* objs = reinterpret_cast<const CovObj*>(td + l.t0);
-      switch (l.kind) {
-        case L_COV:
-          if (dim == 1) cov3_build_grouped_kernel<1><<<(unsigned)l.grid, 128, 0, st>>>(objs, (int)l.count);
-          else cov3_build_grouped_kernel<2><<<(unsigned)l.grid, 128, 0, st>>>(objs, (int)l.count);
-          break;
-        case L_PACK:
-          cov_pack_grouped_kernel<<<dim3((unsigned)l.grid, (unsigned)l.count), 256, 0, st>>>(
-              objs, l.infob, reinterpret_cast<const int64_t*>(td + l.t1), info);
-          break;
-      }
-    });
-  cudaFreeAsync(blk, st);
-  return e;
+  return s.run(work, st, [&](const Launch& l, const char* td) {
+    const CovObj* objs = reinterpret_cast<const CovObj*>(td + l.t0);
+    switch (l.kind) {
+      case L_COV:
+        if (dim == 1) cov3_build_grouped_kernel<1><<<(unsigned)l.grid, 128, 0, st>>>(objs, (int)l.count);
+        else cov3_build_grouped_kernel<2><<<(unsigned)l.grid, 128, 0, st>>>(objs, (int)l.count);
+        break;
+      case L_PACK:
+        cov_pack_grouped_kernel<<<dim3((unsigned)l.grid, (unsigned)l.count), 256, 0, st>>>(
+            objs, l.infob, reinterpret_cast<const int64_t*>(td + l.t1), info);
+        break;
+    }
+  });
 }
 
 int64_t large_pred_ws_doubles(int64_t n, int64_t rows) {
@@ -1618,54 +1638,30 @@ int64_t large_pred_ws_doubles(int64_t n, int64_t rows) {
 // and covs_g[j] for the rest, outputs at mean / var / new_y0 + moff[j], by every step of LargeObject.factor followed by
 // cgp_large_predict_dev run for all objects of a wave at once: A and u in one launch; the factorisation
 // (GroupSchedule::factor); one forward- and one backward-sweep launch per block; the streamed mean in one launch; then per
-// pass of at most chunk_rows grid rows (% 128 == 0) per object: H in one launch, V = rows of L^-1 H^T as large_trsm_rows
-// computes it, and the variance in one launch; last, info and NaN rows where info != 0.  A row's arithmetic does not
-// depend on the pass it falls in.  Waves and their order as in large_ll_grouped, each object's part of the workspace
+// pass of at most chunk_rows grid rows (% 128 == 0) per object: H in one launch, V = rows of L^-1 H^T
+// (GroupSchedule::trsm_rows), and the variance in one launch; last, info and NaN rows where info != 0.  A row's
+// arithmetic does not depend on the pass it falls in.  Waves: plan_waves, each object's part of the workspace
 // large_pred_ws_doubles(n_b, var ? min(m_b, chunk_rows) : 0).  The caller checks that every object fits.
 int large_predict_grouped(int dim, const int64_t* off, const double* x, const double* y, const double* y0, const double* yerr,
                           const Cov* covs, const Cov* covs_g, const double* xnew, const int64_t* goff, int64_t m_shared,
                           const double* new_y0, const int* order, int64_t n_active, const int64_t* moff, double* mean,
                           double* var, int* info, int64_t chunk_rows, double* work, int64_t work_doubles, cudaStream_t st) {
-  struct Item { int64_t j, b, n, n_pad, m, rows; int nblk; };
-  std::vector<std::vector<Item>> waves;
-  {
-    std::vector<Item> cur; int64_t used = 0;
-    for (int64_t j = 0; j < n_active; ++j) {
-      Item it; it.j = j; it.b = order ? order[j] : j; it.n = off[it.b + 1] - off[it.b];
-      it.m = goff ? goff[it.b + 1] - goff[it.b] : m_shared;
-      it.n_pad = it.n <= 0 ? 128 : (it.n + 127) / 128 * 128; it.nblk = (int)(it.n_pad / 128);
-      it.rows = var ? std::min(it.m, chunk_rows) : 0;
-      const int64_t need = large_pred_ws_doubles(it.n, it.rows);
-      if (!cur.empty() && (used + need > work_doubles || cur.size() >= 65535)) { waves.push_back(cur); cur.clear(); used = 0; }
-      cur.push_back(it); used += need;
-    }
-    if (!cur.empty()) waves.push_back(cur);
-  }
+  auto grid_size = [&](int64_t b) { return goff ? goff[b + 1] - goff[b] : m_shared; };
+  auto pass_rows = [&](int64_t b) { return var ? std::min(grid_size(b), chunk_rows) : (int64_t)0; };
+  const Waves waves = plan_waves(order, n_active, off, work_doubles,
+                                 [&](const WaveItem& it) { return large_pred_ws_doubles(it.n, pass_rows(it.b)); });
   GroupSchedule s;
-  size_t w_max = 0;
-  int64_t blocks = 0;
-  for (auto& w : waves) {
-    w_max = std::max(w_max, w.size());
-    int64_t b = 0;
-    for (const Item& it : w) b += it.nblk;
-    blocks = std::max(blocks, b);
-  }
-  s.block_csr(w_max);
-  double* blk = nullptr;                             // per-block log det and info of the wave being factored
-  cudaError_t ce = cudaMallocAsync((void**)&blk, (size_t)blocks * (sizeof(double) + sizeof(int)) + 16, st);
-  if (ce != cudaSuccess) return (int)ce;
+  s.block_csr(waves);
+  BlockScratch blk(st);
+  if (int ce = blk.alloc(waves)) return ce;
 
-  int e = 0;
-  for (auto& w : waves) {
-    std::stable_sort(w.begin(), w.end(), [](const Item& p, const Item& q) { return p.nblk > q.nblk; });
+  for (const auto& w : waves) {
     const int W = (int)w.size(), nb_max = w[0].nblk;
     std::vector<PredObj> objs(W);
     std::vector<double*> a(W), v(W);
-    std::vector<int64_t> ld(W), koff(nb_max + 1, 0);
-    std::vector<int> nblk(W);
     int64_t cur = 0, cta = 0, cta_mean = 0, m_max = 0;
     for (int i = 0; i < W; ++i) {
-      const Item& it = w[i];
+      const WaveItem& it = w[i];
       const int64_t np = it.n_pad, o0 = off[it.b];
       PredObj& o = objs[i];
       o.cov = covs[it.j]; o.cov_g = covs_g[it.j];
@@ -1673,31 +1669,26 @@ int large_predict_grouped(int dim, const int64_t* off, const double* x, const do
       o.g = goff ? xnew + dim * goff[it.b] : xnew; o.new_y0 = new_y0 ? new_y0 + moff[it.j] : nullptr;
       o.a = work + cur; o.u = o.a + np * np; o.z = o.u + np; o.alpha = o.z + np; v[i] = o.alpha + np;
       o.mean = mean + moff[it.j]; o.var = var ? var + moff[it.j] : nullptr;
-      o.n = it.n; o.n_pad = np; o.m = it.m; o.io = it.j; o.cta_a = cta; o.cta_mean = cta_mean;
-      cur += large_pred_ws_doubles(it.n, it.rows);
-      cta += np * ((np + 255) / 256); cta_mean += (it.m + 255) / 256;
-      m_max = std::max(m_max, it.m);
-      a[i] = o.a; ld[i] = np; nblk[i] = it.nblk;
+      o.n = it.n; o.n_pad = np; o.m = grid_size(it.b); o.io = it.j; o.cta_a = cta; o.cta_mean = cta_mean;
+      cur += large_pred_ws_doubles(it.n, pass_rows(it.b));
+      cta += np * ((np + 255) / 256); cta_mean += (o.m + 255) / 256;
+      m_max = std::max(m_max, o.m);
+      a[i] = o.a;
     }
-    if (cta > 2147483647LL || cta_mean > 2147483647LL) { e = (int)cudaErrorInvalidValue; break; }
-    auto count = [&](int k) { int c = 0; while (c < W && nblk[c] > k) ++c; return c; };   // objects with block k
-    for (int k = 0; k < nb_max; ++k) koff[k + 1] = koff[k] + count(k);
-    double* ldb = blk;
-    int* infob = reinterpret_cast<int*>(blk + koff[nb_max]);
+    if (cta > 2147483647LL || cta_mean > 2147483647LL) return (int)cudaErrorInvalidValue;
     const size_t t_objs = s.put(objs.data(), W * sizeof(PredObj));
-    const size_t t_ld = s.put(ld.data(), W * sizeof(int64_t));
-    const size_t t_koff = s.put(koff.data(), koff.size() * sizeof(int64_t));
+    const WaveTables t = s.tables(w, std::move(a));
     s.launches.push_back({L_COV, cta, W, 0, t_objs, 0, 0, nullptr, nullptr});
-    if ((e = s.factor(work, a, ld, nblk, t_ld, koff, ldb, infob))) break;
+    if (int e = s.factor(work, t, blk.ldb(), blk.infob(t))) return e;
     for (int k = 0; k < nb_max; ++k)                 // large_potrs: z = L^-1 u
-      s.launches.push_back({L_FWD, 1 + (ld[0] - (int64_t)k * 128 - 128 + 63) / 64, count(k), (int64_t)k * 128, t_objs, 0, 0,
+      s.launches.push_back({L_FWD, 1 + (t.ld[0] - (int64_t)k * 128 - 128 + 63) / 64, t.count(k), (int64_t)k * 128, t_objs, 0, 0,
                             nullptr, nullptr});
     for (int q = 0; q < nb_max; ++q)                 // large_potrs_backward: alpha = L^-T z, block nblk - 1 - q of each
-      s.launches.push_back({L_BWD, nb_max - q, count(q), q, t_objs, 0, 0, nullptr, nullptr});
+      s.launches.push_back({L_BWD, nb_max - q, t.count(q), q, t_objs, 0, 0, nullptr, nullptr});
     if (cta_mean) s.launches.push_back({L_MEAN, cta_mean, W, 0, t_objs, 0, 0, nullptr, nullptr});
-    for (int64_t r0 = 0; var && r0 < m_max && !e; r0 += chunk_rows) {   // variance passes
+    for (int64_t r0 = 0; var && r0 < m_max; r0 += chunk_rows) {   // variance passes
       std::vector<PassObj> pass;
-      std::vector<int> who;                          // wave position of each object of the pass
+      std::vector<GroupSchedule::RowSolve> vs;
       int64_t cta_h = 0, cta_var = 0;
       for (int i = 0; i < W; ++i) {
         const PredObj& o = objs[i];
@@ -1707,67 +1698,49 @@ int large_predict_grouped(int dim, const int64_t* off, const double* x, const do
         p.n = o.n; p.n_pad = o.n_pad; p.rows = std::min(chunk_rows, o.m - r0); p.rows_pad = (p.rows + 127) / 128 * 128;
         p.cta_h = cta_h; p.cta_var = cta_var;
         cta_h += p.rows_pad * ((p.n_pad + 255) / 256); cta_var += (p.rows + 7) / 8;
-        pass.push_back(p); who.push_back(i);
+        pass.push_back(p); vs.push_back({v[i], p.rows_pad, i});
       }
-      if (cta_h > 2147483647LL) { e = (int)cudaErrorInvalidValue; break; }
+      if (cta_h > 2147483647LL) return (int)cudaErrorInvalidValue;
       const int P = (int)pass.size();
       const size_t t_pass = s.put(pass.data(), P * sizeof(PassObj));
       s.launches.push_back({L_HB, cta_h, P, 0, t_pass, 0, 0, nullptr, nullptr});
-      for (int k = 0; k < nb_max && !e; ++k) {       // large_trsm_rows: V[:,k] -= V[:,0:k] L[k,0:k]^T, then V[:,k] T_kk^T
-        const int64_t k0 = (int64_t)k * 128;
-        if (k > 0) {
-          for (int q = 0; q < P; ++q) {
-            const int i = who[q];
-            if (nblk[i] > k) s.gemm(v[i], ld[i], a[i] + k0 * ld[i], ld[i], v[i] + k0, ld[i], pass[q].rows_pad, 128, k0, -1.0, 1.0, 0);
-          }
-          if ((e = s.flush())) break;
-        }
-        for (int q = 0; q < P; ++q) {
-          const int i = who[q];
-          if (nblk[i] > k) s.gemm(v[i] + k0, ld[i], a[i] + k0 * ld[i] + k0, ld[i], v[i] + k0, ld[i], pass[q].rows_pad, 128, 128, 1.0, 0.0, 0);
-        }
-        e = s.flush();
-      }
+      if (int e = s.trsm_rows(t, vs)) return e;
       s.launches.push_back({L_VAR, cta_var, P, 0, t_pass, 0, 0, nullptr, nullptr});
     }
-    if (e) break;
     const int64_t gx = std::min<int64_t>(std::max<int64_t>((m_max + 1023) / 1024, 1), 1024);
-    s.launches.push_back({L_FIN, gx, W, 0, t_objs, t_koff, 0, ldb, infob});
+    s.launches.push_back({L_FIN, gx, W, 0, t_objs, t.t_koff, 0, blk.ldb(), blk.infob(t)});
   }
-  if (!e)
-    e = s.run(work, st, [&](const Launch& l, const char* td) {
-      const PredObj* objs = reinterpret_cast<const PredObj*>(td + l.t0);
-      const PassObj* pass = reinterpret_cast<const PassObj*>(td + l.t0);
-      switch (l.kind) {
-        case L_COV:
-          if (dim == 1) pred_build_grouped_kernel<1><<<(unsigned)l.grid, 128, 0, st>>>(objs, (int)l.count);
-          else pred_build_grouped_kernel<2><<<(unsigned)l.grid, 128, 0, st>>>(objs, (int)l.count);
-          break;
-        case L_FWD:
-          fwd_step_grouped_kernel<PredObj><<<dim3((unsigned)l.grid, (unsigned)l.count), 256, 0, st>>>(objs, l.k0);
-          break;
-        case L_BWD:
-          bwd_step_grouped_kernel<<<dim3((unsigned)l.grid, (unsigned)l.count), 256, 0, st>>>(objs, l.k0);
-          break;
-        case L_MEAN:
-          if (dim == 1) stream_mean_grouped_kernel<1><<<(unsigned)l.grid, 256, 2 * 1024 * sizeof(double), st>>>(objs, (int)l.count);
-          else stream_mean_grouped_kernel<2><<<(unsigned)l.grid, 256, 3 * 1024 * sizeof(double), st>>>(objs, (int)l.count);
-          break;
-        case L_HB:
-          if (dim == 1) pass_build_grouped_kernel<1><<<(unsigned)l.grid, 128, 0, st>>>(pass, (int)l.count);
-          else pass_build_grouped_kernel<2><<<(unsigned)l.grid, 128, 0, st>>>(pass, (int)l.count);
-          break;
-        case L_VAR:
-          row_var_grouped_kernel<<<(unsigned)l.grid, 256, 0, st>>>(pass, (int)l.count);
-          break;
-        case L_FIN:
-          pred_finish_grouped_kernel<<<dim3((unsigned)l.grid, (unsigned)l.count), 256, 0, st>>>(
-              objs, l.infob, reinterpret_cast<const int64_t*>(td + l.t1), info);
-          break;
-      }
-    });
-  cudaFreeAsync(blk, st);
-  return e;
+  return s.run(work, st, [&](const Launch& l, const char* td) {
+    const PredObj* objs = reinterpret_cast<const PredObj*>(td + l.t0);
+    const PassObj* pass = reinterpret_cast<const PassObj*>(td + l.t0);
+    switch (l.kind) {
+      case L_COV:
+        if (dim == 1) pred_build_grouped_kernel<1><<<(unsigned)l.grid, 128, 0, st>>>(objs, (int)l.count);
+        else pred_build_grouped_kernel<2><<<(unsigned)l.grid, 128, 0, st>>>(objs, (int)l.count);
+        break;
+      case L_FWD:
+        fwd_step_grouped_kernel<PredObj><<<dim3((unsigned)l.grid, (unsigned)l.count), 256, 0, st>>>(objs, l.k0);
+        break;
+      case L_BWD:
+        bwd_step_grouped_kernel<<<dim3((unsigned)l.grid, (unsigned)l.count), 256, 0, st>>>(objs, l.k0);
+        break;
+      case L_MEAN:
+        if (dim == 1) stream_mean_grouped_kernel<1><<<(unsigned)l.grid, 256, 2 * 1024 * sizeof(double), st>>>(objs, (int)l.count);
+        else stream_mean_grouped_kernel<2><<<(unsigned)l.grid, 256, 3 * 1024 * sizeof(double), st>>>(objs, (int)l.count);
+        break;
+      case L_HB:
+        if (dim == 1) pass_build_grouped_kernel<1><<<(unsigned)l.grid, 128, 0, st>>>(pass, (int)l.count);
+        else pass_build_grouped_kernel<2><<<(unsigned)l.grid, 128, 0, st>>>(pass, (int)l.count);
+        break;
+      case L_VAR:
+        row_var_grouped_kernel<<<(unsigned)l.grid, 256, 0, st>>>(pass, (int)l.count);
+        break;
+      case L_FIN:
+        pred_finish_grouped_kernel<<<dim3((unsigned)l.grid, (unsigned)l.count), 256, 0, st>>>(
+            objs, l.infob, reinterpret_cast<const int64_t*>(td + l.t1), info);
+        break;
+    }
+  });
 }
 
 }  // namespace cgp

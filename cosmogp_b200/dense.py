@@ -261,6 +261,34 @@ def _gather(flat, off, ids):
     return flat[idx], new_off
 
 
+def _request(off, objects, grid, goff, hyp, nugget, dim):
+    """The objects of a grouped call: (off as int64, their ids (objects, default all), their (k, n_hyp) hyperparameter
+    rows and k nugget rows (hyp, nugget: shared, or one per object of `objects`), their grid sizes)."""
+    off = np.asarray(off, dtype=np.int64)
+    ids = np.arange(len(off) - 1, dtype=np.int64) if objects is None else np.asarray(objects, dtype=np.int64)
+    k = len(ids)
+    nh = 2 if dim == 1 else 4
+    rows = np.ascontiguousarray(np.broadcast_to(np.asarray(hyp, dtype=np.float64).reshape(-1, nh), (k, nh)))
+    nug_rows = np.ascontiguousarray(np.broadcast_to(np.asarray(nugget, dtype=np.float64).reshape(-1), (k,)))
+    m = np.diff(np.asarray(goff, dtype=np.int64))[ids] if goff is not None else np.full(k, len(grid), dtype=np.int64)
+    return off, ids, rows, nug_rows, m
+
+
+def _upload(dev, sel, off, grid, goff, *points):
+    """The objects `sel` on the device, and only those: each per-point array of `points` (x first; None stays None)
+    gathered into one CSR, and the shared grid or their grids gathered into one CSR.  Returns (point CSR, grid CSR or
+    None for a shared grid, grid size for a shared grid or 0, device grid, device point arrays); placeholders keep
+    empty arrays non-NULL."""
+    def up(a):
+        return _t(a.reshape(-1) if a.size else np.zeros(2), dev)
+    csr = [None if a is None else _gather(np.asarray(a, dtype=np.float64), off, sel) for a in points]
+    if goff is None:
+        g, lgoff = np.asarray(grid, dtype=np.float64), None
+    else:
+        g, lgoff = _gather(np.asarray(grid, dtype=np.float64), np.asarray(goff, dtype=np.int64), sel)
+    return csr[0][1], lgoff, len(g) if lgoff is None else 0, up(g), [None if c is None else up(c[0]) for c in csr]
+
+
 def predictive_covariances(x, off, y_err, grid, goff, hyp, nugget, dim, flags=0, objects=None, work_doubles=None):
     """predictive_covariance of many objects in one grouped call (cgp_large_covariance_dev), each matrix bit for bit
     what predictive_covariance gives for that object alone.  x: the objects' points, flat ((P,) or (P, 2)) with CSR
@@ -271,35 +299,20 @@ def predictive_covariances(x, off, y_err, grid, goff, hyp, nugget, dim, flags=0,
     a matrix is NaN where info != 0."""
     dev = _dev()
     L = _lib.lib()
-    off = np.asarray(off, dtype=np.int64)
-    ids = np.arange(len(off) - 1, dtype=np.int64) if objects is None else np.asarray(objects, dtype=np.int64)
+    off, ids, rows, nug_rows, m = _request(off, objects, grid, goff, hyp, nugget, dim)
     k = len(ids)
-    nh = 2 if dim == 1 else 4
-    hyp = np.asarray(hyp, dtype=np.float64)
-    rows = np.ascontiguousarray(np.broadcast_to(hyp.reshape(-1, nh), (k, nh)) if hyp.ndim == 1 else hyp.reshape(k, nh))
-    nug_rows = None if np.ndim(nugget) == 0 else np.ascontiguousarray(nugget, dtype=np.float64).reshape(k)
     if not k:
         return [], np.zeros(0, dtype=np.int32)
-    xs, loff = _gather(np.asarray(x, dtype=np.float64), off, ids)        # only the requested objects go to the device
-    ye = None if y_err is None else _gather(np.asarray(y_err, dtype=np.float64), off, ids)[0]
-    if goff is None:
-        g, lgoff = np.asarray(grid, dtype=np.float64), None
-        m = np.full(k, len(g), dtype=np.int64)
-    else:
-        g, lgoff = _gather(np.asarray(grid, dtype=np.float64), np.asarray(goff, dtype=np.int64), ids)
-        m = np.diff(lgoff)
+    loff, lgoff, m_shared, gd, (xd, yd) = _upload(dev, ids, off, grid, goff, x, y_err)
     coff = np.zeros(k + 1, dtype=np.int64)
     np.cumsum(m * m, out=coff[1:])
     if work_doubles is None:
         work_doubles = int(cov_ws_doubles(np.diff(loff), m).sum())
-    xd, yd = _t(xs if xs.size else np.zeros(2), dev), _t(ye, dev)      # placeholders keep empty inputs non-NULL
-    gd = _t(g.reshape(-1) if g.size else np.zeros(2), dev)
     work = torch.empty(max(int(work_doubles), 2), dtype=torch.float64, device=dev)
     out = torch.empty(max(int(coff[-1]), 1), dtype=torch.float64, device=dev)
     info = torch.zeros(k, dtype=torch.int32, device=dev)
     _lib.check(L.cgp_large_covariance_dev(k, _lib.hptr(loff), dim, _p(xd), _p(yd), _lib.hptr(rows), _lib.hptr(nug_rows),
-                                          float(0.0 if nug_rows is not None else nugget), 0.0, int(flags), _p(gd),
-                                          _lib.hptr(lgoff), int(m[0]) if lgoff is None else 0, None, k, _p(out),
+                                          0.0, 0.0, int(flags), _p(gd), _lib.hptr(lgoff), m_shared, None, k, _p(out),
                                           _lib.hptr(coff), _p(info), _p(work), int(work_doubles), _stream(dev)),
                "cgp_large_covariance_dev")
     host = out.cpu().numpy()
@@ -329,15 +342,9 @@ def predictions(x, off, y, y0, y_err, grid, goff, new_y0, hyp, nugget, dim, flag
     object); an object's rows are NaN where info != 0."""
     dev = _dev()
     L = _lib.lib()
-    off = np.asarray(off, dtype=np.int64)
-    ids = np.arange(len(off) - 1, dtype=np.int64) if objects is None else np.asarray(objects, dtype=np.int64)
+    off, ids, rows, nug_rows, m = _request(off, objects, grid, goff, hyp, nugget, dim)
     k = len(ids)
-    nh = 2 if dim == 1 else 4
-    hyp = np.asarray(hyp, dtype=np.float64)
-    rows = np.ascontiguousarray(np.broadcast_to(hyp.reshape(-1, nh), (k, nh)) if hyp.ndim == 1 else hyp.reshape(k, nh))
-    nug_rows = np.ascontiguousarray(np.broadcast_to(np.asarray(nugget, dtype=np.float64), (k,)))
     n = off[ids + 1] - off[ids]
-    m = np.diff(np.asarray(goff, dtype=np.int64))[ids] if goff is not None else np.full(k, len(grid), dtype=np.int64)
     moff = np.zeros(k + 1, dtype=np.int64)
     np.cumsum(m, out=moff[1:])
     mean = np.empty(int(moff[-1]))
@@ -355,22 +362,10 @@ def predictions(x, off, y, y0, y_err, grid, goff, new_y0, hyp, nugget, dim, flag
     st = _stream(dev)
     new_y0 = None if new_y0 is None else np.asarray(new_y0, dtype=np.float64).reshape(-1)
     for b0, b1 in zip(bounds[:-1], bounds[1:]):
-        sel = ids[b0:b1]
-        xs, loff = _gather(np.asarray(x, dtype=np.float64), off, sel)      # only the requested objects go to the device
-        ys = _gather(np.asarray(y, dtype=np.float64), off, sel)[0]
-        y0s = None if y0 is None else _gather(np.asarray(y0, dtype=np.float64), off, sel)[0]
-        yes = None if y_err is None else _gather(np.asarray(y_err, dtype=np.float64), off, sel)[0]
-        if goff is None:
-            g, lgoff = np.asarray(grid, dtype=np.float64), None
-        else:
-            g, lgoff = _gather(np.asarray(grid, dtype=np.float64), np.asarray(goff, dtype=np.int64), sel)
+        # every device array bound to a name until the call has been enqueued
+        loff, lgoff, m_shared, gd, (xd, yd, y0d, yed) = _upload(dev, ids[b0:b1], off, grid, goff, x, y, y0, y_err)
         c0, c1 = int(moff[b0]), int(moff[b1])
         lmoff = np.ascontiguousarray(moff[b0:b1 + 1] - c0)
-        # every device array bound to a name until the call has been enqueued
-        xd = _t(xs if xs.size else np.zeros(2), dev)                    # placeholders keep empty inputs non-NULL
-        yd = _t(ys if ys.size else np.zeros(2), dev)
-        y0d, yed = _t(y0s, dev), _t(yes, dev)
-        gd = _t(g.reshape(-1) if g.size else np.zeros(2), dev)
         ny0 = None if new_y0 is None else _t(new_y0[c0:c1], dev)
         md = torch.empty(max(c1 - c0, 1), dtype=torch.float64, device=dev)
         vd = torch.empty(max(c1 - c0, 1), dtype=torch.float64, device=dev) if want_var else None
@@ -378,7 +373,7 @@ def predictions(x, off, y, y0, y_err, grid, goff, new_y0, hyp, nugget, dim, flag
         hr, nr = np.ascontiguousarray(rows[b0:b1]), np.ascontiguousarray(nug_rows[b0:b1])
         _lib.check(L.cgp_large_predict_objhyp_dev(
             b1 - b0, _lib.hptr(loff), dim, _p(xd), _p(yd), _p(y0d), _p(yed), _lib.hptr(hr), _lib.hptr(nr), 0.0, 0.0,
-            int(flags), _p(gd), _lib.hptr(lgoff), int(len(g)) if lgoff is None else 0, _p(ny0), None, b1 - b0,
+            int(flags), _p(gd), _lib.hptr(lgoff), m_shared, _p(ny0), None, b1 - b0,
             _lib.hptr(lmoff), _p(md), _p(vd), _p(infod), chunk_rows, _p(work), int(work.numel()), st),
             "cgp_large_predict_objhyp_dev")
         mean[c0:c1] = md[:c1 - c0].cpu().numpy()

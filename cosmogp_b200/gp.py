@@ -26,8 +26,6 @@ Differences (SURVEY.md section 9.1):
   * y, Time, y_err may also be 2-D ndarrays (equal-length objects), which avoids
     10^5 tiny numpy arrays.
 """
-import os
-
 import numpy as np
 from scipy.optimize import fmin
 
@@ -39,9 +37,6 @@ from .kernel import init_rbf, rbf_kernel_1d, rbf_kernel_2d
 
 _DEVICE = object()                       # marker: the per-object likelihoods of the latest evaluation are still on the device
 _NO_BAD = np.zeros(0, dtype=np.int32)
-# CGP_GROUPED_COV=0: covariance matrices of objects above 64 points one object at a time (dense.predictive_covariance),
-# for comparison with the grouped call (dense.predictive_covariances); read once
-_GROUPED_COV = os.environ.get("CGP_GROUPED_COV", "1") != "0"
 
 
 class _LazyMatrices(object):
@@ -589,16 +584,12 @@ class Gaussian_process:
         else:
             grid, goff = np.array(self.new_binning, dtype=np.float64), None
 
-        def make(i):
-            o0, o1 = self._off[i], self._off[i + 1]
+        def make(i):                                         # an empty grid, or no data: the prior on the grid
             g = grid[goff[i]:goff[i + 1]] if ragged else grid
             h, n = hyp[i] if rows else hyp, nug[i] if rows else nug
             if not len(g):
                 return np.zeros((0, 0))
-            if o0 == o1:                                     # no data: the prior on the grid
-                return self.kernel(g, np.asarray(h, dtype=float), nugget=n, **({"flags": self.flags} if self._dim == 2 else {}))
-            return dense.predictive_covariance(
-                self._x_flat[o0:o1], None if self._ye_flat is None else self._ye_flat[o0:o1], g, h, n, self._dim, self.flags)
+            return self.kernel(g, np.asarray(h, dtype=float), nugget=n, **({"flags": self.flags} if self._dim == 2 else {}))
 
         # the objects written in bulk (global ids, in the order of `batch`)
         split = self._split
@@ -610,11 +601,11 @@ class Gaussian_process:
             ids = np.arange(self.N_sn)
             if self._devices is not None or self.N_sn == 0 or int(split.sizes.max()) > 64:
                 ids = ids[:0]
-        # the objects `make` would send to dense.predictive_covariance, grouped instead: data and a non-empty grid
+        # the objects of the grouped calls: every other object with data and a non-empty grid
         m_obj = np.diff(goff) if ragged else np.full(self.N_sn, len(grid), dtype=np.int64)
         grouped = np.ones(self.N_sn, dtype=bool)
         grouped[ids] = False
-        grouped &= (split.sizes > 0) & (m_obj > 0) & _GROUPED_COV
+        grouped &= (split.sizes > 0) & (m_obj > 0)
         gids = np.nonzero(grouped)[0]
         if not len(ids) and not len(gids):
             return _LazyMatrices(self.N_sn, make)

@@ -5,15 +5,15 @@
   2d_1000_grid300    : 256 2D objects of 1 000 points on a shared 300-point grid
 Per shape: the device time of the entry over all objects (CUDA events, 2 GB workspace as the facade uses), its model
 FLOPs over the DMMA ceiling cgp_fp64_peak(1) measured in this run; the wall time of get_prediction(COV=True) and of
-reading every covariance_matrix[i] through the facade, against CGP_GROUPED_COV=0 (one dense.predictive_covariance per
-object), whose read loop is timed on 200 objects and extrapolated.  Writes profiles/bench_grouped_cov_r01.json.
+reading every covariance_matrix[i] through the facade, against a loop of dense.predictive_covariance, one object at a
+time, timed on 200 objects and extrapolated.  Writes profiles/bench_grouped_cov_r01.json.
    python tests/perf_grouped_cov.py [--out profiles/bench_grouped_cov_r01.json]"""
 import argparse, json, os, subprocess, sys, time, zlib
 import numpy as np, torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 import cosmogp_b200 as cg
-from cosmogp_b200 import _lib, dense, gp as gp_mod
+from cosmogp_b200 import _lib, dense
 
 ap = argparse.ArgumentParser()
 ap.add_argument("--out", default=os.path.join(ROOT, "profiles", "bench_grouped_cov_r01.json"))
@@ -130,18 +130,21 @@ def shape(name, dim, B, N, M, per_object, own):
         a, b = facade(B)
         pred.append(a); read.append(b)
     k = min(200, B)
-    gp_mod._GROUPED_COV = False
-    try:
-        facade(2)
-        la, lb = facade(k)
-    finally:
-        gp_mod._GROUPED_COV = True
+
+    def loop(k):
+        t0 = time.perf_counter()
+        for i in range(k):
+            dense.predictive_covariance(x[i], ye[i], x[i] if own else grid, hyp[i], nugs[i], dim)
+        return time.perf_counter() - t0
+
+    loop(2)
+    lb = loop(k)
     r["facade"] = {"get_prediction_s": pred, "read_all_matrices_s": read,
                    "grouped_total_s": float(min(p + q for p, q in zip(pred, read))),
                    "loop_read_timed_objects": k, "loop_read_timed_s": lb,
                    "loop_total_s_extrapolated": float(min(pred)) + lb * B / k,
-                   "note": "CGP_GROUPED_COV=0 read loop timed on %d objects and extrapolated to %d; get_prediction "
-                           "itself does not depend on the knob" % (k, B)}
+                   "note": "loop of dense.predictive_covariance timed on %d objects and extrapolated to %d, plus "
+                           "the grouped get_prediction time" % (k, B)}
     r["facade"]["speedup_total"] = r["facade"]["loop_total_s_extrapolated"] / r["facade"]["grouped_total_s"]
     out["shapes"][name] = r
     print(name, json.dumps(r), flush=True)
