@@ -71,6 +71,9 @@ SIGNATURES = {
     "cgp_large_pred_ws_doubles": (_i64, [_i64, _i64]),
     "cgp_large_predict_objhyp_dev": (_int, [_i64, _ptr, _int, _ptr, _ptr, _ptr, _ptr, _ptr, _ptr, _dbl, _dbl, _u32, _ptr,
                                             _ptr, _i64, _ptr, _ptr, _i64, _ptr, _ptr, _ptr, _ptr, _i64, _ptr, _i64, _ptr]),
+    "cgp_large_loo_ws_doubles": (_i64, [_i64, _i64]),
+    "cgp_large_loo_objhyp_dev": (_int, [_i64, _ptr, _int, _ptr, _ptr, _ptr, _ptr, _ptr, _ptr, _dbl, _dbl, _u32, _int, _ptr,
+                                        _i64, _ptr, _ptr, _ptr, _ptr, _ptr, _i64, _ptr, _i64, _ptr]),
     "cgp_matrices_batched_dev": (_int, _BATCH_DEV + [_ptr] * 2 + _HYP + [_ptr, _ptr, _ptr, _ptr, _ptr]),
     "cgp_set_nccl_library": (_int, [C.c_char_p]),
     "cgp_shard_ranges": (_int, [_i64, _ptr, _int, _ptr]),

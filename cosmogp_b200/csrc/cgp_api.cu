@@ -382,6 +382,40 @@ int cgp_large_predict_objhyp_dev(int64_t n_obj, const int64_t* off_host, int dim
   return e ? cuda_fail(e, name) : 0;
 }
 
+int64_t cgp_large_loo_ws_doubles(int64_t n, int64_t chunk_rows) {
+  return n < 0 || chunk_rows <= 0 ? 0 : large_loo_ws_doubles(n, chunk_rows);
+}
+
+int cgp_large_loo_objhyp_dev(int64_t n_obj, const int64_t* off_host, int dim, const double* x, const double* y,
+                             const double* m, const double* y_err, const double* hyp_rows_host,
+                             const double* nugget_rows_host, double nugget, double floor, unsigned flags, int mode,
+                             const int* order_host, int64_t n_active, int* info, double* pred, double* pred_var,
+                             double* pull, double* resid, int64_t chunk_rows, double* work, int64_t work_doubles,
+                             void* stream) {
+  const char* name = "cgp_large_loo_objhyp_dev";
+  if (n_obj < 0 || n_active < 0) return fail(CGP_ERR_ARG, "%s: negative object count", name);
+  if (mode != CGP_LOO_PLAIN && mode != CGP_LOO_RECENTER) return fail(CGP_ERR_ARG, "%s: bad mode %d", name, mode);
+  if (chunk_rows <= 0 || chunk_rows % 128) return fail(CGP_ERR_ARG, "%s: chunk_rows must be a positive multiple of 128", name);
+  const int64_t k = order_host ? n_active : n_obj;
+  if (k == 0) return 0;
+  if (!off_host || !x || !y || !hyp_rows_host || !info || !work) return fail(CGP_ERR_ARG, "%s: NULL argument", name);
+  if (dim != 1 && dim != 2) return fail(CGP_ERR_ARG, "dim must be 1 or 2, got %d", dim);
+  if ((uintptr_t)work & 15) return fail(CGP_ERR_ARG, "%s: work must be 16-byte aligned", name);
+  // padded sizes stay within the 65535 rows cgp_cov_matrix_dev builds an auto-covariance for
+  const int64_t max_pts = 65535 / 128 * 128;
+  int rc = check_active(name, n_obj, off_host, order_host, k, max_pts, work_doubles, [&](int64_t, int64_t, int64_t n, int64_t& w) {
+    w = large_loo_ws_doubles(n, chunk_rows);
+    return 0;
+  });
+  if (rc) return rc;
+  std::vector<Cov> covs, covs_g;                     // covs: as cgp_cov_matrix_dev and cgp_large_loo_dev build them
+  host_covs(dim, hyp_rows_host, nugget_rows_host, nugget, floor, flags, k, covs, covs_g);
+  keep_pool_memory();
+  int e = large_loo_grouped(dim, off_host, x, y, m, y_err, covs.data(), mode == CGP_LOO_RECENTER, order_host, k, info, pred,
+                            pred_var, pull, resid, chunk_rows, work, work_doubles, (cudaStream_t)stream);
+  return e ? cuda_fail(e, name) : 0;
+}
+
 int cgp_fit_objects_dev(int64_t n_obj, const int64_t* off, int max_n, int dim,
                         const double* x, const double* y, const double* y0, const double* y_err,
                         const double* start, int n_par, double nugget, double floor, unsigned flags,

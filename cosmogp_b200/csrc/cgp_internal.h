@@ -174,6 +174,11 @@ int large_predict_grouped(int dim, const int64_t* off, const double* x, const do
                           const Cov* covs, const Cov* covs_g, const double* xnew, const int64_t* goff, int64_t m_shared,
                           const double* new_y0, const int* order, int64_t n_active, const int64_t* moff, double* mean,
                           double* var, int* info, int64_t chunk_rows, double* work, int64_t work_doubles, cudaStream_t st);
+// grouped leave-one-out pulls of large objects, covs[j] built on the host (see cgp_large_loo_objhyp_dev)
+int64_t large_loo_ws_doubles(int64_t n, int64_t chunk_rows);
+int large_loo_grouped(int dim, const int64_t* off, const double* x, const double* y, const double* m, const double* yerr,
+                      const Cov* covs, int recenter, const int* order, int64_t n_active, int* info, double* pred, double* pvar,
+                      double* pull, double* resid, int64_t chunk_rows, double* work, int64_t work_doubles, cudaStream_t st);
 
 // Launchers (cgp_small.cu).  max_n = largest object in the batch.  Return cudaError_t as int.
 int launch_small(Task task, int dim, int max_n, const SmallArgs& a, cudaStream_t stream);

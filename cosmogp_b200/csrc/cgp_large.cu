@@ -355,7 +355,7 @@ __global__ void dot_sq_kernel(const double* v, int64_t n, double* out) {      //
   const double acc = block_dot_sq(v, n);
   if (threadIdx.x == 0) out[0] = acc;
 }
-__global__ void sum_kernel(const double* v, int64_t n, double* out) {         // out[0] = sum v (one CTA, fixed order)
+__device__ __forceinline__ double block_sum(const double* v, int64_t n) {     // sum v in a fixed order, valid in thread 0
   __shared__ double s[32];
   double acc = 0.0;
   for (int64_t i = threadIdx.x; i < n; i += blockDim.x) acc += v[i];
@@ -367,8 +367,12 @@ __global__ void sum_kernel(const double* v, int64_t n, double* out) {         //
     acc = threadIdx.x < (blockDim.x >> 5) ? s[threadIdx.x] : 0.0;
 #pragma unroll
     for (int o = 16; o; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
-    if (threadIdx.x == 0) out[0] = acc;
   }
+  return acc;
+}
+__global__ void sum_kernel(const double* v, int64_t n, double* out) {         // out[0] = sum v (one CTA)
+  const double acc = block_sum(v, n);
+  if (threadIdx.x == 0) out[0] = acc;
 }
 // Mean function at the epochs on the device: the cubic B-spline scipy's InterpolatedUnivariateSpline holds
 // (knots t[0..nt), coefficients c) evaluated as FITPACK does (splev.f: knot interval by search, clamped to the end
@@ -491,24 +495,25 @@ __global__ void ones_kernel(int64_t n, int64_t n_pad, double* v) {
   if (i < n_pad) v[i] = i < n ? 1.0 : 0.0;
 }
 // v[r][c] = (r == c) for r < rows, c < cols (cols even): the identity rows the diag(K^-1) solve starts from.
-__global__ void __launch_bounds__(256) identity_rows_kernel(double* v, int64_t ldv, int64_t rows, int64_t cols) {
+// Pairs t0, t0 + step, .. of the rows * cols / 2 pairs of entries.
+__device__ __forceinline__ void identity_rows_at(double* v, int64_t ldv, int64_t rows, int64_t cols, int64_t t0, int64_t step) {
   const int64_t half = cols / 2, total = rows * half;
-  for (int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; t < total; t += (int64_t)gridDim.x * blockDim.x) {
+  for (int64_t t = t0; t < total; t += step) {
     const int64_t r = t / half, c = (t - r * half) * 2;
     *reinterpret_cast<double2*>(v + r * ldv + c) = make_double2(c == r ? 1.0 : 0.0, c + 1 == r ? 1.0 : 0.0);
   }
 }
-// Closed-form leave-one-out of one object, the formulas of the shared-memory path (cgp_small.cu TASK_LOO):
-// d = diag(K^-1) arrives negated (row_norm_var_kernel with amp* = 0), alpha = K^-1 r; u = K^-1 1 and rsum = sum r
-// for the recentred mode only (u == nullptr otherwise).  NaN everywhere when the factorisation failed.
-__global__ void __launch_bounds__(256) loo_epilogue_kernel(const Cov cov, int64_t n, const double* __restrict__ y,
-                                                           const double* __restrict__ m, const double* __restrict__ yerr,
-                                                           const double* __restrict__ alpha, const double* __restrict__ negd,
-                                                           const double* __restrict__ u, const double* __restrict__ rsum,
-                                                           const int* __restrict__ info, double* pred, double* pvar,
-                                                           double* pull, double* resid) {
-  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n) return;
+__global__ void __launch_bounds__(256) identity_rows_kernel(double* v, int64_t ldv, int64_t rows, int64_t cols) {
+  identity_rows_at(v, ldv, rows, cols, (int64_t)blockIdx.x * blockDim.x + threadIdx.x, (int64_t)gridDim.x * blockDim.x);
+}
+// Closed-form leave-one-out at point i of one object, the formulas of the shared-memory path (cgp_small.cu TASK_LOO):
+// d = diag(K^-1) arrives negated (row_norm_var_at with amp* = 0), alpha = K^-1 r; u = K^-1 1 and rsum = sum r for the
+// recentred mode only (u == nullptr otherwise).  NaN everywhere when the factorisation failed (bad != 0).
+__device__ __forceinline__ void loo_epilogue_at(const Cov& cov, int64_t n, const double* __restrict__ y,
+                                                const double* __restrict__ m, const double* __restrict__ yerr,
+                                                const double* __restrict__ alpha, const double* __restrict__ negd,
+                                                const double* __restrict__ u, const double* __restrict__ rsum, const int bad,
+                                                double* pred, double* pvar, double* pull, double* resid, const int64_t i) {
   const double rho = cov.amp_cross / cov.amp_auto;
   const double amp_star = cov.amp_auto + cov.nugget2;
   const double d = -negd[i];
@@ -522,11 +527,21 @@ __global__ void __launch_bounds__(256) loo_epilogue_kernel(const Cov cov, int64_
   double pv = fabs(amp_star - rho * rho * (cov.amp_auto + (ye * ye + cov.noise_const) - 1.0 / d));
   double res = pr - yv;
   double pl = res / sqrt(ye * ye + pv + cov.nugget2);
-  if (*info) { pr = nan(""); pv = pr; res = pr; pl = pr; }
+  if (bad) { pr = nan(""); pv = pr; res = pr; pl = pr; }
   if (pred) pred[i] = pr;
   if (pvar) pvar[i] = pv;
   if (resid) resid[i] = res;
   if (pull) pull[i] = pl;
+}
+__global__ void __launch_bounds__(256) loo_epilogue_kernel(const Cov cov, int64_t n, const double* __restrict__ y,
+                                                           const double* __restrict__ m, const double* __restrict__ yerr,
+                                                           const double* __restrict__ alpha, const double* __restrict__ negd,
+                                                           const double* __restrict__ u, const double* __restrict__ rsum,
+                                                           const int* __restrict__ info, double* pred, double* pvar,
+                                                           double* pull, double* resid) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  loo_epilogue_at(cov, n, y, m, yerr, alpha, negd, u, rsum, *info, pred, pvar, pull, resid, i);
 }
 
 // ---------------------------------------------------------------------------------------
@@ -590,10 +605,11 @@ __global__ void __launch_bounds__(128) cov_build_grouped_kernel(const GroupObj* 
   if (chunk == 0 && threadIdx.x == 0) o.u[r] = r < o.n ? o.y[r] - (o.y0 ? o.y0[r] : 0.0) : 0.0;   // residual_kernel
 }
 
-// Forward sweep step k of the objects objs[0 .. gridDim.y): CTA x of object y runs fwd_step_kernel's CTA x.
+// Forward sweep step k of the objects 0 .. gridDim.y, gridDim.z right-hand sides each (the descriptors of one object
+// consecutive): CTA x of right-hand side z of object y runs fwd_step_kernel's CTA x.
 template <class Obj>
 __global__ void __launch_bounds__(256) fwd_step_grouped_kernel(const Obj* __restrict__ objs, const int64_t k0) {
-  const Obj& o = objs[blockIdx.y];
+  const Obj& o = objs[blockIdx.y * gridDim.z + blockIdx.z];
   if ((int64_t)blockIdx.x >= 1 + (o.n_pad - k0 - 128 + 63) / 64) return;
   fwd_step_at(o.a, o.n_pad, k0, o.n_pad, o.u, o.z, blockIdx.x);
 }
@@ -727,10 +743,11 @@ __global__ void __launch_bounds__(128) pred_build_grouped_kernel(const PredObj* 
   cov_build_at<DIM>(a, r, (chunk * 128 + threadIdx.x) * 2);
 }
 
-// Backward sweep launch s of the objects objs[0 .. gridDim.y): object y runs bwd_step_kernel's CTA x of its block
-// n_pad / 128 - 1 - s.
-__global__ void __launch_bounds__(256) bwd_step_grouped_kernel(const PredObj* __restrict__ objs, const int64_t s) {
-  const PredObj& o = objs[blockIdx.y];
+// Backward sweep launch s of the objects 0 .. gridDim.y, gridDim.z right-hand sides each (as fwd_step_grouped_kernel):
+// right-hand side z of object y runs bwd_step_kernel's CTA x of its block n_pad / 128 - 1 - s.
+template <class Obj>
+__global__ void __launch_bounds__(256) bwd_step_grouped_kernel(const Obj* __restrict__ objs, const int64_t s) {
+  const Obj& o = objs[blockIdx.y * gridDim.z + blockIdx.z];
   const int64_t k = o.n_pad / 128 - 1 - s;
   if ((int64_t)blockIdx.x > k) return;
   bwd_step_at(o.a, o.n_pad, k * 128, o.z, o.alpha, blockIdx.x);
@@ -784,6 +801,87 @@ __global__ void __launch_bounds__(256) pred_finish_grouped_kernel(const PredObj*
     o.mean[e] = nan("");
     if (o.var) o.var[e] = nan("");
   }
+}
+
+// One object of a grouped leave-one-out (large_loo_grouped).  `cov` comes from the host, as cgp_cov_matrix_dev and
+// cgp_large_loo_dev build it.
+struct LooObj {
+  Cov cov;
+  const double* x; const double* y; const double* m; const double* yerr;   // m, yerr may be null
+  double* a;                 // n_pad x n_pad covariance -> blocked factor
+  double* r;                 // residual y - m, consumed by the forward sweep
+  double* ones;              // ones vector, consumed by the forward sweep (recentred mode; null otherwise)
+  double* alpha;             // K^-1 r
+  double* kinv1;             // K^-1 1 (recentred mode; null otherwise)
+  double* negd;              // -diag(K^-1)
+  double* rsum;              // sum r
+  double* pred; double* pvar; double* pull; double* resid;   // the object's n outputs (each may be null)
+  int64_t n, n_pad;
+  int64_t io;                // position in `order`: info
+  int64_t cta_a, cta_epi;    // first CTA of the object in the build and in the epilogue launch
+};
+// One right-hand side of the sweeps: u -> z = L^-1 u (forward), z -> alpha = L^-T z (backward).
+struct SolveObj { double* a; double* u; double* z; double* alpha; int64_t n_pad; };
+// One object's pass of the diag(K^-1) solve: `rows` identity rows of width w staged at v (leading dimension ld), their
+// negated squared norms to negd.
+struct DiagObj { double* v; int64_t ld, w, rows; double* negd; int64_t cta; };
+
+// A = K(x, x) + noise and r = y - m of every object of a wave, as pred_build_grouped_kernel builds them, and the ones
+// vector of ones_kernel in the recentred mode.
+template <int DIM>
+__global__ void __launch_bounds__(128) loo_build_grouped_kernel(const LooObj* __restrict__ objs, const int n_obj) {
+  const int64_t t = blockIdx.x;
+  const LooObj& o = owner(objs, n_obj, t, &LooObj::cta_a);
+  const int64_t per_row = (o.n_pad + 255) / 256;
+  const int64_t local = t - o.cta_a, r = local / per_row, chunk = local - r * per_row;
+  if (chunk == 0 && threadIdx.x == 0) {
+    o.r[r] = r < o.n ? o.y[r] - (o.m ? o.m[r] : 0.0) : 0.0;        // residual_kernel
+    if (o.ones) o.ones[r] = r < o.n ? 1.0 : 0.0;                   // ones_kernel
+  }
+  CovArgs a;
+  a.dim = DIM; a.cov = o.cov; a.autocov = 1;
+  a.xc = o.x; a.n = o.n; a.xr = o.x; a.m = o.n; a.yerr = o.yerr;
+  a.out = o.a; a.ld = o.n_pad; a.rows_pad = o.n_pad; a.cols_pad = o.n_pad;
+  cov_build_at<DIM>(a, r, (chunk * 128 + threadIdx.x) * 2);
+}
+
+// sum r of object blockIdx.x (sum_kernel, 1024 threads).
+__global__ void __launch_bounds__(1024) sum_grouped_kernel(const LooObj* __restrict__ objs) {
+  const LooObj& o = objs[blockIdx.x];
+  const double s = block_sum(o.r, o.n);
+  if (threadIdx.x == 0) *o.rsum = s;
+}
+
+// The identity rows of object blockIdx.y of a diag(K^-1) pass (identity_rows_kernel).
+__global__ void __launch_bounds__(256) identity_rows_grouped_kernel(const DiagObj* __restrict__ objs) {
+  const DiagObj& o = objs[blockIdx.y];
+  identity_rows_at(o.v, o.ld, o.rows, o.w, (int64_t)blockIdx.x * blockDim.x + threadIdx.x, (int64_t)gridDim.x * blockDim.x);
+}
+
+// -|row|^2 of the rows of a diag(K^-1) pass (row_norm_var_kernel with amp* = 0): ceil(rows / 8) CTAs per object.
+__global__ void __launch_bounds__(256) diag_norm_grouped_kernel(const DiagObj* __restrict__ objs, const int n_obj) {
+  const int64_t t = blockIdx.x;
+  const DiagObj& o = owner(objs, n_obj, t, &DiagObj::cta);
+  row_norm_var_at(o.v, o.ld, o.w, o.rows, 0.0, o.negd, t - o.cta);
+}
+
+// loo_epilogue_kernel for every object of a wave: object i owns max(1, ceil(n / 256)) CTAs from cta_epi on; its first
+// CTA writes info (first_bad_pivot).
+__global__ void __launch_bounds__(256) loo_finish_grouped_kernel(const LooObj* __restrict__ objs, const int n_obj,
+                                                                 const int* __restrict__ infob, const int64_t* __restrict__ koff,
+                                                                 int* __restrict__ info) {
+  const int64_t t = blockIdx.x;
+  const LooObj& o = owner(objs, n_obj, t, &LooObj::cta_epi);
+  __shared__ int bad_s;
+  if (threadIdx.x == 0) {
+    const int bad = first_bad_pivot(infob, koff, (int)(&o - objs), (int)(o.n_pad / 128));
+    bad_s = bad;
+    if (t == o.cta_epi) info[o.io] = bad;
+  }
+  __syncthreads();
+  const int64_t i = (t - o.cta_epi) * blockDim.x + threadIdx.x;
+  if (i < o.n)
+    loo_epilogue_at(o.cov, o.n, o.y, o.m, o.yerr, o.alpha, o.negd, o.kinv1, o.rsum, bad_s, o.pred, o.pvar, o.pull, o.resid, i);
 }
 
 }  // namespace
@@ -1257,7 +1355,7 @@ int64_t large_ll_ws_doubles(int64_t n) {
 // launch of every wave is recorded on the host first; the arguments (object descriptors, GEMM problems, block offsets)
 // are packed into one byte table that crosses to the device in one copy into stream-ordered scratch.
 namespace {
-enum { L_DIAG, L_GEMM, L_COV, L_FWD, L_FIN, L_PACK, L_BWD, L_MEAN, L_HB, L_VAR };
+enum { L_DIAG, L_GEMM, L_COV, L_FWD, L_FIN, L_PACK, L_BWD, L_MEAN, L_HB, L_VAR, L_ID, L_NORM, L_SUM };
 struct Launch { int kind; int64_t grid, count, k0; size_t t0, t1, t2; double* ldb; int* infob; };
 
 // One object of a wave: position j in `order`, object id b, n points, n_pad = 128 nblk (at least one block).
@@ -1454,6 +1552,50 @@ struct GroupSchedule {
     }
     return e;
   }
+  // negd[i] = -diag(K^-1) for the objects of a factored wave, as large_diag_inv computes it: passes of chunk_rows identity
+  // rows staged at v[i] (chunk_rows x n_pad); in pass r0 every object with n_pad > r0 (a prefix) takes part with
+  // min(chunk_rows, n_pad - r0) rows.  Per pass one identity-rows launch, per pair of block columns from r0 / 128 on the
+  // four GEMMs of large_diag_inv (shapes, row clipping, alpha / beta) as grouped launches over the objects with those
+  // blocks, then one row-norm launch.
+  int diag_inv(const WaveTables& t, const std::vector<double*>& v, const std::vector<double*>& negd, int64_t chunk_rows) {
+    int e = 0;
+    for (int64_t r0 = 0; r0 < t.ld[0] && !e; r0 += chunk_rows) {
+      const int kb0 = (int)(r0 / 128);
+      std::vector<DiagObj> d;
+      int64_t cta = 0, blocks = 0;
+      for (int i = 0; i < (int)t.ld.size() && t.ld[i] > r0; ++i) {
+        const int64_t np = t.ld[i], c = std::min(chunk_rows, np - r0), w = np - r0;
+        d.push_back({v[i] + r0, np, w, c, negd[i] + r0, cta});
+        cta += (c + 7) / 8;
+        blocks = std::max(blocks, (c * (w / 2) + 255) / 256);
+      }
+      const int P = (int)d.size();
+      const size_t td = put(d.data(), P * sizeof(DiagObj));
+      launches.push_back({L_ID, std::min<int64_t>(blocks, 148 * 16), P, 0, td, 0, 0, nullptr, nullptr});
+      auto rows = [&](int i, int k) { return std::min<int64_t>((int64_t)(k - kb0 + 1) * 128, d[i].rows); };
+      auto lk = [&](int i, int k) { return t.a[i] + (int64_t)k * 128 * t.ld[i] + (int64_t)k * 128; };
+      for (int k = kb0; k < t.nblk[0] && !e; k += 2) {
+        const int64_t j0 = (int64_t)(k - kb0) * 128;    // block column k inside the pass
+        for (int i = 0; i < P && t.nblk[i] > k; ++i)   // V_k T_kk^T
+          gemm(d[i].v + j0, d[i].ld, lk(i, k), t.ld[i], d[i].v + j0, d[i].ld, rows(i, k), 128, 128, 1.0, 0.0, 0);
+        if ((e = flush())) break;
+        for (int i = 0; i < P && t.nblk[i] > k + 1; ++i)   // V_{k+1} -= V_k L_{k+1,k}^T
+          gemm(d[i].v + j0, d[i].ld, lk(i, k) + 128 * t.ld[i], t.ld[i], d[i].v + j0 + 128, d[i].ld, rows(i, k), 128, 128, -1.0, 1.0, 0);
+        if ((e = flush())) break;
+        for (int i = 0; i < P && t.nblk[i] > k + 1; ++i)   // V_{k+1} T_{k+1,k+1}^T
+          gemm(d[i].v + j0 + 128, d[i].ld, lk(i, k) + 128 * t.ld[i] + 128, t.ld[i], d[i].v + j0 + 128, d[i].ld, rows(i, k + 1), 128,
+               128, 1.0, 0.0, 0);
+        if ((e = flush())) break;
+        for (int i = 0; i < P && t.nblk[i] > k + 2; ++i)   // V[:, k+2:] -= V[:, k:k+2] L[k+2:, k:k+2]^T, K = 256
+          gemm(d[i].v + j0, d[i].ld, lk(i, k) + 256 * t.ld[i], t.ld[i], d[i].v + j0 + 256, d[i].ld, rows(i, k + 1),
+               t.ld[i] - (int64_t)(k + 2) * 128, 256, -1.0, 1.0, 0);
+        e = flush();
+      }
+      if (cta > 2147483647LL) return (int)cudaErrorInvalidValue;
+      launches.push_back({L_NORM, cta, P, 0, td, 0, 0, nullptr, nullptr});
+    }
+    return e;
+  }
   // Copies the table to the device and runs the recorded launches in order: the diagonal blocks and the GEMMs here,
   // every other kind through other(launch, device table).
   template <class F>
@@ -1486,6 +1628,13 @@ struct GroupSchedule {
         case L_GEMM:
           gemm_nt_grouped_kernel<<<(unsigned)l.grid, GEMM_THREADS, GEMM_SMEM, st>>>(
               reinterpret_cast<const GemmArgs*>(td + l.t0), reinterpret_cast<const int*>(td + l.t1), (int)l.count);
+          break;
+        case L_ID:
+          identity_rows_grouped_kernel<<<dim3((unsigned)l.grid, (unsigned)l.count), 256, 0, st>>>(
+              reinterpret_cast<const DiagObj*>(td + l.t0));
+          break;
+        case L_NORM:
+          diag_norm_grouped_kernel<<<(unsigned)l.grid, 256, 0, st>>>(reinterpret_cast<const DiagObj*>(td + l.t0), (int)l.count);
           break;
         default:
           other(l, td);
@@ -1722,7 +1871,7 @@ int large_predict_grouped(int dim, const int64_t* off, const double* x, const do
         fwd_step_grouped_kernel<PredObj><<<dim3((unsigned)l.grid, (unsigned)l.count), 256, 0, st>>>(objs, l.k0);
         break;
       case L_BWD:
-        bwd_step_grouped_kernel<<<dim3((unsigned)l.grid, (unsigned)l.count), 256, 0, st>>>(objs, l.k0);
+        bwd_step_grouped_kernel<PredObj><<<dim3((unsigned)l.grid, (unsigned)l.count), 256, 0, st>>>(objs, l.k0);
         break;
       case L_MEAN:
         if (dim == 1) stream_mean_grouped_kernel<1><<<(unsigned)l.grid, 256, 2 * 1024 * sizeof(double), st>>>(objs, (int)l.count);
@@ -1738,6 +1887,97 @@ int large_predict_grouped(int dim, const int64_t* off, const double* x, const do
       case L_FIN:
         pred_finish_grouped_kernel<<<dim3((unsigned)l.grid, (unsigned)l.count), 256, 0, st>>>(
             objs, l.infob, reinterpret_cast<const int64_t*>(td + l.t1), info);
+        break;
+    }
+  });
+}
+
+int64_t large_loo_ws_doubles(int64_t n, int64_t chunk_rows) {
+  const int64_t np = n <= 0 ? 128 : (n + 127) / 128 * 128;
+  // factor, the first diag(K^-1) pass, r / z / alpha, 1 / z_1 / K^-1 1, -d, sum r and one double that keeps the next
+  // object 16-byte aligned
+  return np * np + std::min(np, chunk_rows) * np + 7 * np + 2;
+}
+
+// Leave-one-out pulls of the objects order[0 .. n_active) (object ids; NULL: 0 .. n_active), object order[j] with covs[j],
+// outputs at pred / pvar / pull / resid + off[b] (each may be null), by every step of cgp_cov_matrix_dev + cgp_potrf_dev +
+// cgp_large_loo_dev run for all objects of a wave at once: A, r (and the ones vector) in one launch; sum r in one launch
+// (recentred mode); the factorisation (GroupSchedule::factor); one forward- and one backward-sweep launch per block for
+// both right-hand sides; -diag(K^-1) (GroupSchedule::diag_inv); one epilogue launch that writes info[j] and NaN outputs
+// where info != 0.  Waves: plan_waves, each object's part of the workspace large_loo_ws_doubles(n_b, chunk_rows).  The
+// caller checks that every object fits.
+int large_loo_grouped(int dim, const int64_t* off, const double* x, const double* y, const double* m, const double* yerr,
+                      const Cov* covs, int recenter, const int* order, int64_t n_active, int* info, double* pred, double* pvar,
+                      double* pull, double* resid, int64_t chunk_rows, double* work, int64_t work_doubles, cudaStream_t st) {
+  const Waves waves = plan_waves(order, n_active, off, work_doubles,
+                                 [&](const WaveItem& it) { return large_loo_ws_doubles(it.n, chunk_rows); });
+  GroupSchedule s;
+  s.block_csr(waves);
+  BlockScratch blk(st);
+  if (int ce = blk.alloc(waves)) return ce;
+  const int nrhs = recenter ? 2 : 1;
+
+  for (const auto& w : waves) {
+    const int W = (int)w.size(), nb_max = w[0].nblk;
+    std::vector<LooObj> objs(W);
+    std::vector<SolveObj> rhs;
+    std::vector<double*> a(W), v(W), negd(W);
+    int64_t cur = 0, cta = 0, cta_epi = 0;
+    for (int i = 0; i < W; ++i) {
+      const WaveItem& it = w[i];
+      const int64_t np = it.n_pad, o0 = off[it.b];
+      LooObj& o = objs[i];
+      o.cov = covs[it.j];
+      o.x = x + dim * o0; o.y = y + o0; o.m = m ? m + o0 : nullptr; o.yerr = yerr ? yerr + o0 : nullptr;
+      o.a = work + cur; v[i] = o.a + np * np;
+      double* vec = v[i] + std::min(np, chunk_rows) * np;
+      o.r = vec; o.alpha = vec + 2 * np;
+      o.ones = recenter ? vec + 3 * np : nullptr; o.kinv1 = recenter ? vec + 5 * np : nullptr;
+      o.negd = negd[i] = vec + 6 * np; o.rsum = vec + 7 * np;
+      o.pred = pred ? pred + o0 : nullptr; o.pvar = pvar ? pvar + o0 : nullptr;
+      o.pull = pull ? pull + o0 : nullptr; o.resid = resid ? resid + o0 : nullptr;
+      o.n = it.n; o.n_pad = np; o.io = it.j; o.cta_a = cta; o.cta_epi = cta_epi;
+      rhs.push_back({o.a, o.r, vec + np, o.alpha, np});
+      if (recenter) rhs.push_back({o.a, o.ones, vec + 4 * np, o.kinv1, np});
+      cur += large_loo_ws_doubles(it.n, chunk_rows);
+      cta += np * ((np + 255) / 256); cta_epi += std::max<int64_t>((it.n + 255) / 256, 1);
+      a[i] = o.a;
+    }
+    if (cta > 2147483647LL || cta_epi > 2147483647LL) return (int)cudaErrorInvalidValue;
+    const size_t t_objs = s.put(objs.data(), W * sizeof(LooObj));
+    const size_t t_rhs = s.put(rhs.data(), rhs.size() * sizeof(SolveObj));
+    const WaveTables t = s.tables(w, std::move(a));
+    s.launches.push_back({L_COV, cta, W, 0, t_objs, 0, 0, nullptr, nullptr});
+    if (recenter) s.launches.push_back({L_SUM, W, W, 0, t_objs, 0, 0, nullptr, nullptr});   // before the sweep consumes r
+    if (int e = s.factor(work, t, blk.ldb(), blk.infob(t))) return e;
+    for (int k = 0; k < nb_max; ++k)                 // large_potrs forward, both right-hand sides
+      s.launches.push_back({L_FWD, 1 + (t.ld[0] - (int64_t)k * 128 - 128 + 63) / 64, t.count(k), (int64_t)k * 128, t_rhs, 0, 0,
+                            nullptr, nullptr});
+    for (int q = 0; q < nb_max; ++q)                 // large_potrs backward: block nblk - 1 - q of each
+      s.launches.push_back({L_BWD, nb_max - q, t.count(q), q, t_rhs, 0, 0, nullptr, nullptr});
+    if (int e = s.diag_inv(t, v, negd, chunk_rows)) return e;
+    s.launches.push_back({L_FIN, cta_epi, W, 0, t_objs, t.t_koff, 0, blk.ldb(), blk.infob(t)});
+  }
+  return s.run(work, st, [&](const Launch& l, const char* td) {
+    const LooObj* objs = reinterpret_cast<const LooObj*>(td + l.t0);
+    const SolveObj* rhs = reinterpret_cast<const SolveObj*>(td + l.t0);
+    switch (l.kind) {
+      case L_COV:
+        if (dim == 1) loo_build_grouped_kernel<1><<<(unsigned)l.grid, 128, 0, st>>>(objs, (int)l.count);
+        else loo_build_grouped_kernel<2><<<(unsigned)l.grid, 128, 0, st>>>(objs, (int)l.count);
+        break;
+      case L_SUM:
+        sum_grouped_kernel<<<(unsigned)l.grid, 1024, 0, st>>>(objs);
+        break;
+      case L_FWD:
+        fwd_step_grouped_kernel<SolveObj><<<dim3((unsigned)l.grid, (unsigned)l.count, nrhs), 256, 0, st>>>(rhs, l.k0);
+        break;
+      case L_BWD:
+        bwd_step_grouped_kernel<SolveObj><<<dim3((unsigned)l.grid, (unsigned)l.count, nrhs), 256, 0, st>>>(rhs, l.k0);
+        break;
+      case L_FIN:
+        loo_finish_grouped_kernel<<<(unsigned)l.grid, 256, 0, st>>>(objs, (int)l.count, l.infob,
+                                                                    reinterpret_cast<const int64_t*>(td + l.t1), info);
         break;
     }
   });

@@ -136,21 +136,29 @@ class LargeObject:
         return kinv[:self.n, :self.n].cpu().numpy()
 
 
+def loo_chunk_rows(n_pad, chunk_rows=None):
+    """Identity rows per pass of the diag(K^-1) solve for objects of at most n_pad (padded) points: chunk_rows rounded
+    down to a multiple of 128 (default: all rows while a pass stays under 4 GB, i.e. up to about 23 000 points), at
+    most n_pad."""
+    if chunk_rows is None:
+        chunk_rows = max(128, (4 << 30) // (8 * n_pad))
+    return min(n_pad, int(chunk_rows) // 128 * 128 or 128)
+
+
 class LargeLoo:
     """Closed-form leave-one-out pulls of objects too large for the shared-memory path, one object per launch
     sequence: covariance build -> blocked Cholesky -> cgp_large_loo_dev, written straight into slices of device
     outputs.  The factor buffer and the diag(K^-1) workspace are allocated once, for the largest object (max_n
-    points), and reused; nothing here synchronises.
-    chunk_rows: identity rows per pass of the diag(K^-1) solve (default: all rows while the workspace stays under
-    4 GB, i.e. up to about 23 000 points)."""
+    points), and reused; nothing here synchronises.  This is the per-object reference of loo_grouped; build_pull
+    uses it for a call with exactly one large object, where large_potrf's look-ahead makes it the faster route, and
+    loo_grouped for several.
+    chunk_rows: identity rows per pass of the diag(K^-1) solve (loo_chunk_rows)."""
 
     def __init__(self, max_n, dim, flags=0, chunk_rows=None):
         self.dev = _dev()
         self.dim, self.flags = int(dim), int(flags)
         n_pad = pad128(max_n)
-        if chunk_rows is None:
-            chunk_rows = max(128, (4 << 30) // (8 * n_pad))
-        self.chunk = min(n_pad, int(chunk_rows) // 128 * 128 or 128)
+        self.chunk = loo_chunk_rows(n_pad, chunk_rows)
         self.a = torch.empty(n_pad * n_pad, dtype=torch.float64, device=self.dev)
         self.vwork = torch.empty(self.chunk * n_pad, dtype=torch.float64, device=self.dev)
 
@@ -381,3 +389,42 @@ def predictions(x, off, y, y0, y_err, grid, goff, new_y0, hyp, nugget, dim, flag
             var[c0:c1] = vd[:c1 - c0].cpu().numpy()
         info[b0:b1] = infod.cpu().numpy()
     return mean, var, moff, info
+
+
+def loo_ws_doubles(n, chunk_rows):
+    """Device workspace (doubles) of objects of n points in loo_grouped with chunk_rows identity rows per diag(K^-1)
+    pass, elementwise (cgp_large_loo_ws_doubles): n_pad^2 + min(n_pad, chunk_rows) n_pad + 7 n_pad + 2."""
+    n_pad = np.maximum((np.asarray(n, dtype=np.int64) + 127) // 128, 1) * 128
+    return n_pad * n_pad + np.minimum(n_pad, np.int64(chunk_rows)) * n_pad + 7 * n_pad + 2
+
+
+def loo_grouped(batch, objects, hyp, nugget, mode, outs, flags=0, chunk_rows=None, work_doubles=None):
+    """LargeLoo.run of the objects `objects` of a DeviceBatch (its x, y, y0 as the mean, y_err) in one grouped call
+    (cgp_large_loo_objhyp_dev), each output bit for bit LargeLoo's at the same chunk_rows.  hyp: (n_hyp,) shared, or
+    one row per object of `objects`; nugget: scalar or one per object.  outs: (pred, pred_var, pull, resid, info)
+    device tensors in the batch's layout, as DeviceBatch.loo_dev returns them; the objects' points and their info
+    entries are written in place.  chunk_rows: as LargeLoo's for the largest object (loo_chunk_rows).  work_doubles:
+    device workspace (default: the objects' needs summed up to 2 GB, at least the largest one's).  Does not
+    synchronise."""
+    L = _lib.lib()
+    ids = np.asarray(objects, dtype=np.int64)
+    k = len(ids)
+    if not k:
+        return
+    nh = 2 if batch.dim == 1 else 4
+    rows = np.ascontiguousarray(np.broadcast_to(np.asarray(hyp, dtype=np.float64).reshape(-1, nh), (k, nh)))
+    nug_rows = np.ascontiguousarray(np.broadcast_to(np.asarray(nugget, dtype=np.float64).reshape(-1), (k,)))
+    n = batch.off_host[ids + 1] - batch.off_host[ids]
+    chunk = loo_chunk_rows(pad128(int(n.max())), chunk_rows)
+    if work_doubles is None:
+        need = loo_ws_doubles(n, chunk)
+        work_doubles = max(min(int(need.sum()), (2 << 30) // 8), int(need.max()))
+    work = torch.empty(int(work_doubles), dtype=torch.float64, device=batch.device)
+    info = torch.empty(k, dtype=torch.int32, device=batch.device)
+    order = np.ascontiguousarray(ids, dtype=np.int32)
+    with torch.cuda.device(batch.device):
+        _lib.check(L.cgp_large_loo_objhyp_dev(
+            batch.n_obj, _lib.hptr(batch.off_host), batch.dim, _p(batch.x), _p(batch.y), _p(batch.y0), _p(batch.y_err),
+            _lib.hptr(rows), _lib.hptr(nug_rows), 0.0, 0.0, int(flags), int(mode), _lib.hptr(order), k, _p(info),
+            *[_p(o) for o in outs[:4]], chunk, _p(work), int(work_doubles), batch._stream()), "cgp_large_loo_objhyp_dev")
+        outs[4][torch.from_numpy(ids).to(batch.device)] = info

@@ -3,7 +3,8 @@
 The reference refits the GP N times per object on N-1 points (pull.py:66-90, O(N^4));
 here one factorisation per object gives every leave-one-out prediction and variance in
 closed form from K^-1 (SURVEY.md section 8 row a8), all objects in one launch.  The objects batch.SizeSplit calls
-large are factorised in HBM one at a time (dense.LargeLoo) in the same call, with no size limit.
+large are factorised in HBM in the same call, with no size limit: several of them in one grouped call
+(dense.loo_grouped), a single one through dense.LargeLoo.
 """
 import numpy as np
 
@@ -94,14 +95,21 @@ class build_pull:
             batch = DeviceBatch(x_flat, y_flat, off, y0=template, y_err=ye_flat, dim=dim, max_n=split.small_max_n)
             hyp, nug = self.hyperparameters, self.nugget
             outs = batch.loo_dev(hyp, nug, mode=mode, flags=self.flags, ranges=split.runs)
-            if len(split.large):
+            if len(split.large) == 1:
+                # one large object alone: LargeLoo keeps large_potrf's look-ahead side stream, which the grouped
+                # factorisation does not use (DESIGN §9: 187 against 212 ms at N = 20 000)
                 from .dense import LargeLoo
-                loo = LargeLoo(int(split.sizes[split.large].max()), dim, flags=self.flags)
-                for i in split.large:
-                    p0, p1 = int(off[i]), int(off[i + 1])
-                    x, y, m, e = (None if t is None else t[p0:p1] for t in (batch.x, batch.y, batch.y0, batch.y_err))
-                    loo.run(x, y, m, e, np.asarray(hyp)[i] if np.ndim(hyp) == 2 else hyp,
-                            np.asarray(nug)[i] if np.ndim(nug) == 1 else nug, mode, outs[4][i:i + 1], [o[p0:p1] for o in outs[:4]])
+                i = int(split.large[0])
+                p0, p1 = int(off[i]), int(off[i + 1])
+                x, y, m, e = (None if t is None else t[p0:p1] for t in (batch.x, batch.y, batch.y0, batch.y_err))
+                LargeLoo(p1 - p0, dim, flags=self.flags).run(x, y, m, e, np.asarray(hyp)[i] if np.ndim(hyp) == 2 else hyp,
+                                                             np.asarray(nug)[i] if np.ndim(nug) == 1 else nug, mode,
+                                                             outs[4][i:i + 1], [o[p0:p1] for o in outs[:4]])
+            elif len(split.large):
+                from .dense import loo_grouped
+                large = split.large
+                loo_grouped(batch, large, np.asarray(hyp)[large] if np.ndim(hyp) == 2 else hyp,
+                            np.asarray(nug)[large] if np.ndim(nug) == 1 else nug, mode, outs, flags=self.flags)
             pred, pvar, pull, resid = outs[:4]
             info = batch._down(outs[4])            # every object's status, checked once after everything is launched
             bad = np.nonzero(info)[0]

@@ -306,6 +306,25 @@ int cgp_large_predict_objhyp_dev(int64_t n_obj, const int64_t* off_host, int dim
                                  const int* order_host, int64_t n_active, const int64_t* moff_host, double* mean,
                                  double* var, int* info, int64_t chunk_rows, double* work, int64_t work_doubles,
                                  void* stream);
+/* Leave-one-out pulls of objects of any size (0..65408 points), computed for all active objects of a wave at once by the
+ * blocked HBM path, each output bit for bit what cgp_cov_matrix_dev + cgp_potrf_dev + cgp_large_loo_dev (with the same
+ * hyperparameters, floor, flags, mode and chunk_rows) compute for it alone (dense.LargeLoo.run).  Objects, order_host,
+ * hyp_rows_host and nugget_rows_host as in cgp_large_covariance_dev; y, m (may be NULL) and y_err (may be NULL): device
+ * arrays of the batch; mode: CGP_LOO_PLAIN or CGP_LOO_RECENTER.  Object order_host[j]'s outputs go to pred / pred_var /
+ * pull / resid + off_host[b] (device, the batch's own layout; each may be NULL); points of objects not listed are not
+ * touched.  info (k, device): the first failing pivot; the object's outputs are NaN where info != 0.  diag(K^-1) is
+ * solved chunk_rows (a positive multiple of 128) identity rows at a time; the bits depend on chunk_rows as those of
+ * cgp_large_loo_dev do.  work: caller-owned device workspace of work_doubles doubles (16-byte aligned); an object of
+ * n points needs cgp_large_loo_ws_doubles(n, chunk_rows) of it, whatever the mode; consecutive objects are packed into
+ * waves that fit.  Does not synchronise.  Returns 0, or < 0 with nothing launched (-2 for a workspace below the largest
+ * active object's need). */
+int64_t cgp_large_loo_ws_doubles(int64_t n, int64_t chunk_rows);
+int cgp_large_loo_objhyp_dev(int64_t n_obj, const int64_t* off_host, int dim, const double* x, const double* y,
+                             const double* m, const double* y_err, const double* hyp_rows_host,
+                             const double* nugget_rows_host, double nugget, double floor, unsigned flags, int mode,
+                             const int* order_host, int64_t n_active, int* info, double* pred, double* pred_var,
+                             double* pull, double* resid, int64_t chunk_rows, double* work, int64_t work_doubles,
+                             void* stream);
 
 /* ---- matrices for the attribute surface (kernel_matrix, inv_kernel_matrix:
  *      Gaussian_process.py:256-267, 319-325).  moff[n_obj+1]: CSR into the outputs in
