@@ -42,6 +42,8 @@ SIGNATURES = {
     "cgp_large_ll_ws_doubles": (_i64, [_i64]),
     "cgp_large_ll_objhyp_dev": (_int, [_i64, _ptr, _int] + [_ptr] * 4 + [_ptr, _ptr, _dbl, _dbl, _u32, _ptr, _i64, _ptr, _ptr,
                                                                        _ptr, _i64, _ptr]),
+    "cgp_large_ll_rows_dev": (_int, [_i64, _ptr, _int] + [_ptr] * 4 + [_ptr, _ptr, _dbl, _dbl, _u32, _ptr, _i64, _ptr, _ptr,
+                                                                     _ptr, _i64, _ptr]),
     "cgp_streamer_create": (_int, [_i64, _int, _i64, _int, _int, C.POINTER(_ptr)]),
     "cgp_streamer_destroy": (None, [_ptr]),
     "cgp_streamer_set_mean_spline": (_int, [_ptr, _ptr, _ptr, _int]),

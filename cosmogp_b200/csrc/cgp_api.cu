@@ -302,9 +302,32 @@ int cgp_large_ll_objhyp_dev(int64_t n_obj, const int64_t* off_host, int dim,
                         [](int64_t, int64_t, int64_t n, int64_t& w) { w = large_ll_ws_doubles(n); return 0; });
   if (rc) return rc;
   keep_pool_memory();
-  int e = large_ll_grouped(dim, off_host, x, y, y0, y_err, hyp_obj, nugget_obj, nugget, floor, flags, order_host, k, ll_obj, info,
-                           work, work_doubles, (cudaStream_t)stream);
+  int e = large_ll_grouped(dim, off_host, x, y, y0, y_err, nullptr, hyp_obj, nugget_obj, nugget, floor, flags, order_host, k,
+                           ll_obj, info, work, work_doubles, (cudaStream_t)stream);
   return e ? cuda_fail(e, "cgp_large_ll_objhyp_dev") : 0;
+}
+
+int cgp_large_ll_rows_dev(int64_t n_obj, const int64_t* off_host, int dim,
+                          const double* x, const double* y, const double* y0, const double* y_err,
+                          const double* hyp_rows_host, const double* nugget_rows_host, double nugget, double floor,
+                          unsigned flags, const int* order_host, int64_t n_active, double* ll_obj, int* info,
+                          double* work, int64_t work_doubles, void* stream) {
+  const char* name = "cgp_large_ll_rows_dev";
+  if (n_obj < 0 || n_active < 0) return fail(CGP_ERR_ARG, "%s: negative object count", name);
+  const int64_t k = order_host ? n_active : n_obj;
+  if (k == 0) return 0;
+  if (!off_host || !x || !y || !hyp_rows_host || !ll_obj || !info || !work) return fail(CGP_ERR_ARG, "%s: NULL argument", name);
+  if (dim != 1 && dim != 2) return fail(CGP_ERR_ARG, "dim must be 1 or 2, got %d", dim);
+  if ((uintptr_t)work & 15) return fail(CGP_ERR_ARG, "%s: work must be 16-byte aligned", name);
+  int rc = check_active(name, n_obj, off_host, order_host, k, 65535, work_doubles,
+                        [](int64_t, int64_t, int64_t n, int64_t& w) { w = large_ll_ws_doubles(n); return 0; });
+  if (rc) return rc;
+  std::vector<Cov> covs, covs_g;                     // covs: as cgp_cov_matrix_dev builds them for LargeObject.factor
+  host_covs(dim, hyp_rows_host, nugget_rows_host, nugget, floor, flags, k, covs, covs_g);
+  keep_pool_memory();
+  int e = large_ll_grouped(dim, off_host, x, y, y0, y_err, covs.data(), nullptr, nullptr, nugget, floor, flags, order_host, k,
+                           ll_obj, info, work, work_doubles, (cudaStream_t)stream);
+  return e ? cuda_fail(e, name) : 0;
 }
 
 int64_t cgp_large_cov_ws_doubles(int64_t n, int64_t m) { return n < 0 || m < 0 ? 0 : large_cov_ws_doubles(n, m); }

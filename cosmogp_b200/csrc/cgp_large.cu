@@ -556,6 +556,7 @@ struct GroupObj {
   int64_t n, n_pad;
   int64_t io;                // position in `order`: compact hyperparameters, nugget, ll and info
   int64_t cta0;              // first CTA of the object in the covariance launch
+  Cov cov;                   // host-built covariance function, read by the covariance build in host mode only
 };
 struct GroupHyp {
   const double* hyp_obj; const double* nugget_obj; double nugget, floor; unsigned flags;
@@ -589,8 +590,9 @@ __device__ __forceinline__ Cov group_cov(const GroupHyp& h, int64_t io) {
 }
 
 // Covariance of every object of a wave (the layout of cov_build_kernel) and its residual.  Object i owns
-// n_pad * ceil(n_pad / 256) CTAs from objs[i].cta0 on: one row, 256 columns each.
-template <int DIM>
+// n_pad * ceil(n_pad / 256) CTAs from objs[i].cta0 on: one row, 256 columns each.  HOST_COV: the covariance function is
+// the object's host-built `cov` (as cgp_cov_matrix_dev's make_cov builds it), otherwise group_cov on the device.
+template <int DIM, bool HOST_COV>
 __global__ void __launch_bounds__(128) cov_build_grouped_kernel(const GroupObj* __restrict__ objs, const int n_obj,
                                                                 const GroupHyp h) {
   const int64_t t = blockIdx.x;
@@ -598,7 +600,8 @@ __global__ void __launch_bounds__(128) cov_build_grouped_kernel(const GroupObj* 
   const int64_t per_row = (o.n_pad + 255) / 256;
   const int64_t local = t - o.cta0, r = local / per_row, chunk = local - r * per_row;
   CovArgs a;
-  a.dim = DIM; a.cov = group_cov<DIM>(h, o.io); a.autocov = 1;
+  a.dim = DIM; a.autocov = 1;
+  if constexpr (HOST_COV) a.cov = o.cov; else a.cov = group_cov<DIM>(h, o.io);
   a.xc = o.x; a.n = o.n; a.xr = o.x; a.m = o.n; a.yerr = o.yerr;
   a.out = o.a; a.ld = o.n_pad; a.rows_pad = o.n_pad; a.cols_pad = o.n_pad;
   cov_build_at<DIM>(a, r, (chunk * 128 + threadIdx.x) * 2);
@@ -1651,12 +1654,14 @@ struct GroupSchedule {
 // Log-likelihoods of the objects order[0 .. n_active) (object ids; NULL: 0 .. n_active), object order[j] with the
 // hyperparameters of row j, by the blocked factorisation of large_potrf run for all objects of a wave at once (waves:
 // plan_waves, each object's part of the workspace large_ll_ws_doubles).  Per wave: one covariance launch; the
-// factorisation (GroupSchedule::factor); one forward-sweep launch per block; one epilogue.  The caller checks that
-// every object fits.
+// factorisation (GroupSchedule::factor); one forward-sweep launch per block; one epilogue.  The covariance function of
+// object order[j] is covs[j] when covs is given (built on the host, with the floor: then every step is that of
+// cgp_cov_matrix_dev + cgp_potrf_dev + cgp_large_solve_dev, and so is every bit), otherwise cov_from_hyp of
+// hyp_obj / nugget_obj on the device.  The caller checks that every object fits.
 int large_ll_grouped(int dim, const int64_t* off, const double* x, const double* y, const double* y0, const double* yerr,
-                     const double* hyp_obj, const double* nugget_obj, double nugget, double floor, unsigned flags,
-                     const int* order, int64_t n_active, double* ll, int* info, double* work, int64_t work_doubles,
-                     cudaStream_t st) {
+                     const Cov* covs, const double* hyp_obj, const double* nugget_obj, double nugget, double floor,
+                     unsigned flags, const int* order, int64_t n_active, double* ll, int* info, double* work,
+                     int64_t work_doubles, cudaStream_t st) {
   const Waves waves = plan_waves(order, n_active, off, work_doubles, [](const WaveItem& it) { return large_ll_ws_doubles(it.n); });
   GroupSchedule s;
   s.block_csr(waves);
@@ -1673,6 +1678,7 @@ int large_ll_grouped(int dim, const int64_t* off, const double* x, const double*
       g.x = x + dim * o0; g.y = y + o0; g.y0 = y0 ? y0 + o0 : nullptr; g.yerr = yerr ? yerr + o0 : nullptr;
       g.a = work + cur; g.u = g.a + np * np; g.z = g.u + np;
       g.n = it.n; g.n_pad = np; g.io = it.j; g.cta0 = cta;
+      if (covs) g.cov = covs[it.j];
       cur += np * np + 2 * np; cta += np * ((np + 255) / 256);
       a[i] = g.a;
     }
@@ -1694,8 +1700,13 @@ int large_ll_grouped(int dim, const int64_t* off, const double* x, const double*
     const GroupObj* objs = reinterpret_cast<const GroupObj*>(td + l.t0);
     switch (l.kind) {
       case L_COV:
-        if (dim == 1) cov_build_grouped_kernel<1><<<(unsigned)l.grid, 128, 0, st>>>(objs, (int)l.count, h);
-        else cov_build_grouped_kernel<2><<<(unsigned)l.grid, 128, 0, st>>>(objs, (int)l.count, h);
+        if (covs) {
+          if (dim == 1) cov_build_grouped_kernel<1, true><<<(unsigned)l.grid, 128, 0, st>>>(objs, (int)l.count, h);
+          else cov_build_grouped_kernel<2, true><<<(unsigned)l.grid, 128, 0, st>>>(objs, (int)l.count, h);
+        } else {
+          if (dim == 1) cov_build_grouped_kernel<1, false><<<(unsigned)l.grid, 128, 0, st>>>(objs, (int)l.count, h);
+          else cov_build_grouped_kernel<2, false><<<(unsigned)l.grid, 128, 0, st>>>(objs, (int)l.count, h);
+        }
         break;
       case L_FWD:
         fwd_step_grouped_kernel<GroupObj><<<dim3((unsigned)l.grid, (unsigned)l.count), 256, 0, st>>>(objs, l.k0);

@@ -391,6 +391,52 @@ def predictions(x, off, y, y0, y_err, grid, goff, new_y0, hyp, nugget, dim, flag
     return mean, var, moff, info
 
 
+LL_WS_BYTES = 2 << 30        # workspace of log_likelihoods (ll_workspace): objects beyond it run in further waves
+
+
+def ll_ws_doubles(n):
+    """Device workspace (doubles) of objects of n points in log_likelihoods, elementwise (cgp_large_ll_ws_doubles):
+    n_pad^2 + 2 n_pad + 2 n_pad / 128 with n_pad a multiple of 128 (at least 128)."""
+    n_pad = np.maximum((np.asarray(n, dtype=np.int64) + 127) // 128, 1) * 128
+    return n_pad * n_pad + 2 * n_pad + 2 * (n_pad // 128)
+
+
+def ll_workspace(n, device):
+    """The device workspace of log_likelihoods for objects of n points: their needs summed up to LL_WS_BYTES, at
+    least the largest one's.  Allocate it once and pass it to every evaluation."""
+    need = ll_ws_doubles(np.asarray(n, dtype=np.int64).reshape(-1))
+    big = int(need.max()) if len(need) else 2
+    return torch.empty(max(min(int(need.sum()), LL_WS_BYTES // 8), big), dtype=torch.float64, device=device)
+
+
+def log_likelihoods(batch, objects, hyp, nugget, flags=0, work=None):
+    """LargeObject(x_b, y_b, y_err_b, y0_b, flags=flags).factor(hyp, nugget) of the objects `objects` (default all) of
+    a DeviceBatch in one grouped call (cgp_large_ll_rows_dev), each ll and info bit for bit that loop's, whatever the
+    objects around it.  hyp: (n_hyp,) shared, or one row per object of `objects`; nugget: scalar or one per object.
+    work: a device workspace from ll_workspace, reused across calls (default: one allocated here).  One native call
+    and one synchronisation.  Returns host (ll, info), info the first failing pivot and ll NaN where it is not 0."""
+    L = _lib.lib()
+    ids = np.arange(batch.n_obj, dtype=np.int64) if objects is None else np.asarray(objects, dtype=np.int64)
+    k = len(ids)
+    if not k:
+        return np.zeros(0), np.zeros(0, dtype=np.int32)
+    nh = 2 if batch.dim == 1 else 4
+    rows = np.ascontiguousarray(np.broadcast_to(np.asarray(hyp, dtype=np.float64).reshape(-1, nh), (k, nh)))
+    nug_rows = np.ascontiguousarray(np.broadcast_to(np.asarray(nugget, dtype=np.float64).reshape(-1), (k,)))
+    if work is None:
+        work = ll_workspace(batch.off_host[ids + 1] - batch.off_host[ids], batch.device)
+    out = torch.empty(k + (k + 1) // 2, dtype=torch.float64, device=batch.device)   # ll, then info as int32
+    info = out[k:].view(torch.int32)
+    order = np.ascontiguousarray(ids, dtype=np.int32)
+    with torch.cuda.device(batch.device):
+        _lib.check(L.cgp_large_ll_rows_dev(
+            batch.n_obj, _lib.hptr(batch.off_host), batch.dim, _p(batch.x), _p(batch.y), _p(batch.y0), _p(batch.y_err),
+            _lib.hptr(rows), _lib.hptr(nug_rows), 0.0, 0.0, int(flags), _lib.hptr(order), k, _p(out), _p(info),
+            _p(work), int(work.numel()), batch._stream()), "cgp_large_ll_rows_dev")
+    host = out.cpu().numpy()
+    return host[:k].copy(), host[k:].view(np.int32)[:k].copy()
+
+
 def loo_ws_doubles(n, chunk_rows):
     """Device workspace (doubles) of objects of n points in loo_grouped with chunk_rows identity rows per diag(K^-1)
     pass, elementwise (cgp_large_loo_ws_doubles): n_pad^2 + min(n_pad, chunk_rows) n_pad + 7 n_pad + 2."""

@@ -3,8 +3,8 @@ gaussian_process_nobject (cosmogp/Gaussian_process.py:78-393): same constructor
 arguments, methods, attributes and error behaviour; numpy in, numpy out.  The
 per-object Python loops of the reference (:207, :264, :304, :349) are replaced by
 single batched launches on a device-resident copy of the data.  Which objects are too large for those launches is
-decided in one place, batch.SizeSplit; they go through the blocked HBM factorisation: one at a time for likelihoods
-under shared hyperparameters (dense.LargeObject, every object of the batch then), all at once for the likelihood
+decided in one place, batch.SizeSplit; they go through the blocked HBM factorisation, all of them at once: for
+likelihoods under shared hyperparameters (dense.log_likelihoods, every object of the batch then), for the likelihood
 evaluations of per-object fits (cgp_large_ll_objhyp_dev) and for predictions (dense.predictions: the large objects of a
 per-object prediction, or every object of a batch with a large one under shared hyperparameters).
 
@@ -204,8 +204,8 @@ class Gaussian_process:
     @property
     def _any_large(self):
         """With shared hyperparameters, a batch with any large object (batch.SizeSplit) goes through the HBM-resident
-        blocked factorisation: likelihoods one object at a time (`_large_objects`), predictions all objects in grouped
-        calls (dense.predictions).  Sharded objects decide from the sizes of
+        blocked factorisation, all objects in grouped calls: likelihoods (`_blocked_log_likelihoods`) and predictions
+        (dense.predictions).  Sharded objects decide from the sizes of
         ALL objects, so that every rank takes the same branch (and the same collectives)."""
         return len((self._all_split if self._dist else self._split).large) > 0
 
@@ -219,16 +219,21 @@ class Gaussian_process:
         o0, o1 = int(self._off[i]), int(self._off[i + 1])
         return tuple(None if a is None else a[o0:o1] for a in (self._x_flat, self._y_flat, self._ye_flat, self._y0_flat))
 
-    def _large_object(self, i):
-        """dense.LargeObject of object i; its n_pad^2 factor lives as long as the object"""
-        from .dense import LargeObject
-        return LargeObject(*self._object_slices(i), dim=self._dim, flags=self.flags)
-
-    def _large_objects(self):
-        """one LargeObject per object, kept: fits with shared hyperparameters evaluate them hundreds of times"""
-        if getattr(self, "_large", None) is None:
-            self._large = [self._large_object(i) for i in range(self.N_sn)]
-        return self._large
+    def _blocked_log_likelihoods(self, hyperparameter, nugget):
+        """(ll, info) of every object by the grouped blocked factorisation (dense.log_likelihoods), each ll bit for bit
+        dense.LargeObject.factor's; info 1 where the covariance is not positive definite.  The batch (with devices=...,
+        one of the facade's arrays on the current GPU) and a workspace bounded by dense.LL_WS_BYTES are made on the first
+        call and kept: fits evaluate hundreds of times."""
+        from . import dense
+        if not self.N_sn:
+            return np.zeros(0), np.zeros(0, dtype=np.int32)
+        if getattr(self, "_blocked", None) is None:
+            batch = self.batch if self._devices is None else DeviceBatch(
+                self._x_flat, self._y_flat, self._off, y0=self._y0_flat, y_err=self._ye_flat, dim=self._dim)
+            self._blocked = (batch, dense.ll_workspace(self._split.sizes, batch.device))
+        batch, work = self._blocked
+        ll, info = dense.log_likelihoods(batch, None, hyperparameter, nugget, self.flags, work)
+        return ll, (info != 0).astype(np.int32)
 
     @staticmethod
     def _raise_if_bad(info):
@@ -248,12 +253,7 @@ class Gaussian_process:
             Nugget = self.nugget
             hyperparameter = Hyperparameter
         if self._any_large:
-            per_object, info = np.zeros(self.N_sn), np.zeros(self.N_sn, dtype=np.int32)
-            for i, o in enumerate(self._large_objects()):
-                try:
-                    per_object[i] = o.factor(hyperparameter, Nugget)
-                except np.linalg.LinAlgError:
-                    info[i] = 1
+            per_object, info = self._blocked_log_likelihoods(hyperparameter, Nugget)
             total = None
         else:
             # the sum over objects is reduced on the device: 16 bytes come back per evaluation, the per-object

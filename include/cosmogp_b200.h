@@ -154,6 +154,19 @@ int cgp_large_ll_objhyp_dev(int64_t n_obj, const int64_t* off_host, int dim,
                             const int* order_host, int64_t n_active, double* ll_obj, int* info,
                             double* work, int64_t work_doubles, void* stream);
 
+/* cgp_large_ll_objhyp_dev with the hyperparameters of the active objects as HOST rows: hyp_rows_host (k x nh) and
+ * nugget_rows_host (k, may be NULL -> `nugget`), row j for order_host[j] (shared hyperparameters: one row repeated).
+ * The covariance function of each object is built on the host, as cgp_cov_matrix_dev builds it, so that ll_obj[j] and
+ * info[j] are bit for bit those of cgp_cov_matrix_dev + cgp_potrf_dev + cgp_large_solve_dev on that object alone
+ * (dense.LargeObject.factor), whatever the other objects of the call, their order or the wave it lands in.  An object
+ * without points gives -0.0.  Everything else (objects, order, outputs, workspace, checks) as cgp_large_ll_objhyp_dev;
+ * does not synchronise. */
+int cgp_large_ll_rows_dev(int64_t n_obj, const int64_t* off_host, int dim,
+                          const double* x, const double* y, const double* y0, const double* y_err,
+                          const double* hyp_rows_host, const double* nugget_rows_host, double nugget, double floor,
+                          unsigned flags, const int* order_host, int64_t n_active, double* ll_obj, int* info,
+                          double* work, int64_t work_doubles, void* stream);
+
 /* The whole per-object fit on the device: scipy.optimize.fmin's Nelder-Mead (what
  * Gaussian_process.py:246-247 calls) as one state machine per object, the objective of all pending
  * trial points evaluated by one batched likelihood launch per step; the host only enqueues launches.
