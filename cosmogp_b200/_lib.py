@@ -40,8 +40,6 @@ SIGNATURES = {
     "cgp_ll_batched_host": (_int, _BATCH + [_ptr] * 4 + _HYP + [_ptr, _ptr, C.POINTER(_dbl)]),
     "cgp_ll_objhyp_dev": (_int, _BATCH_DEV + [_ptr] * 4 + [_ptr, _ptr, _dbl, _dbl, _u32, _ptr, _i64, _ptr, _ptr, _ptr]),
     "cgp_large_ll_ws_doubles": (_i64, [_i64]),
-    "cgp_large_ll_objhyp_dev": (_int, [_i64, _ptr, _int] + [_ptr] * 4 + [_ptr, _ptr, _dbl, _dbl, _u32, _ptr, _i64, _ptr, _ptr,
-                                                                       _ptr, _i64, _ptr]),
     "cgp_large_ll_rows_dev": (_int, [_i64, _ptr, _int] + [_ptr] * 4 + [_ptr, _ptr, _dbl, _dbl, _u32, _ptr, _i64, _ptr, _ptr,
                                                                      _ptr, _i64, _ptr]),
     "cgp_streamer_create": (_int, [_i64, _int, _i64, _int, _int, C.POINTER(_ptr)]),

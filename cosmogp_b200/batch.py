@@ -11,7 +11,7 @@ import functools
 import numpy as np
 import torch
 
-from . import _lib
+from . import _lib, dense
 
 
 def _as_list_of_arrays(seq, dim):
@@ -258,7 +258,8 @@ class DeviceBatch:
         Compact I/O: only the k active rows cross PCIe, through persistent pinned / device buffers.
         Objects of up to 224 points go through the shared-memory kernel (cgp_ll_objhyp_dev, with the largest small
         size as max_n: the kernel a batch of the small objects alone gets), larger ones through the grouped blocked
-        factorisation (cgp_large_ll_objhyp_dev) in a workspace allocated once per batch.  One synchronisation."""
+        factorisation (dense.log_likelihoods_dev, from the host rows: each bit for bit dense.LargeObject.factor) in a
+        workspace allocated once per batch.  One synchronisation."""
         k, nh = len(idx), (2 if self.dim == 1 else 4)
         if k == 0:
             return np.zeros(0), np.zeros(0, dtype=np.int32)
@@ -276,41 +277,35 @@ class DeviceBatch:
             c["large"] = ~split.small
             c["small_max_n"] = split.small_max_n if len(split.large) else self.max_n
             if len(split.large):
-                need = np.array([_lib.lib().cgp_large_ll_ws_doubles(int(n)) for n in split.sizes[split.large]], dtype=np.int64)
-                c["work"] = torch.empty(int(max(need.max(), min(need.sum(), (4 << 30) // 8))), dtype=torch.float64,
-                                        device=self.device)
+                need = dense.ll_ws_doubles(split.sizes[split.large])
+                c["work"] = torch.empty(dense.capped_ws_doubles(need, 4 << 30), dtype=torch.float64, device=self.device)
         idx = np.asarray(idx, dtype=np.int64)
         big = c["large"][idx]
         perm = np.concatenate([np.nonzero(~big)[0], np.nonzero(big)[0]]) if big.any() else None
         ks = k - int(big.sum())
         rows = np.asarray(hyp_rows, dtype=np.float64).reshape(k, nh)
-        c["hyp_h"].numpy()[:k] = rows if perm is None else rows[perm]
-        c["ord_h"].numpy()[:k] = idx if perm is None else idx[perm]
-        c["hyp_d"][:k].copy_(c["hyp_h"][:k], non_blocking=True)
-        c["ord_d"][:k].copy_(c["ord_h"][:k], non_blocking=True)
-        nd = None
+        hyp_h, ord_h, nug_h = c["hyp_h"].numpy()[:k], c["ord_h"].numpy()[:k], c["nug_h"].numpy()[:k]
+        hyp_h[:] = rows if perm is None else rows[perm]
+        ord_h[:] = idx if perm is None else idx[perm]
         if nugget_rows is not None:
             nug = np.asarray(nugget_rows, dtype=np.float64)
-            c["nug_h"].numpy()[:k] = nug if perm is None else nug[perm]
-            c["nug_d"][:k].copy_(c["nug_h"][:k], non_blocking=True)
-            nd = c["nug_d"]
+            nug_h[:] = nug if perm is None else nug[perm]
         with torch.cuda.device(self.device):
             if ks:
+                c["hyp_d"][:ks].copy_(c["hyp_h"][:ks], non_blocking=True)
+                c["ord_d"][:ks].copy_(c["ord_h"][:ks], non_blocking=True)
+                nd = None
+                if nugget_rows is not None:
+                    c["nug_d"][:ks].copy_(c["nug_h"][:ks], non_blocking=True)
+                    nd = c["nug_d"]
                 rc = _lib.lib().cgp_ll_objhyp_dev(self.n_obj, self._p(self.off), c["small_max_n"], self.dim, self._p(self.x),
                                                   self._p(self.y), self._p(self.y0), self._p(self.y_err), self._p(c["hyp_d"]),
                                                   self._p(nd), float(nugget), float(floor), int(flags), self._p(c["ord_d"]), ks,
                                                   self._p(c["ll_d"]), self._p(c["info_d"]), self._stream())
                 _lib.check(rc, "cgp_ll_objhyp_dev")
             if ks < k:
-                order = c["ord_h"].numpy()[ks:k]                # host copy of the schedule
-                rc = _lib.lib().cgp_large_ll_objhyp_dev(self.n_obj, _lib.hptr(self.off_host), self.dim, self._p(self.x),
-                                                        self._p(self.y), self._p(self.y0), self._p(self.y_err),
-                                                        self._p(c["hyp_d"]) + 8 * nh * ks,
-                                                        None if nd is None else self._p(nd) + 8 * ks, float(nugget),
-                                                        float(floor), int(flags), order.ctypes.data, k - ks,
-                                                        self._p(c["ll_d"]) + 8 * ks, self._p(c["info_d"]) + 4 * ks,
-                                                        self._p(c["work"]), int(c["work"].numel()), self._stream())
-                _lib.check(rc, "cgp_large_ll_objhyp_dev")
+                dense.log_likelihoods_dev(self, ord_h[ks:], hyp_h[ks:], nugget if nugget_rows is None else nug_h[ks:],
+                                          c["ll_d"][ks:k], c["info_d"][ks:k], c["work"], floor, flags)
         c["ll_h"][:k].copy_(c["ll_d"][:k], non_blocking=True)
         c["info_h"][:k].copy_(c["info_d"][:k], non_blocking=True)
         torch.cuda.current_stream(self.device).synchronize()

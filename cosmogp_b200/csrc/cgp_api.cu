@@ -177,6 +177,36 @@ static void host_covs(int dim, const double* hyp_rows, const double* nugget_rows
   }
 }
 
+static int no_checks() { return 0; }
+
+// The steps every grouped large-object entry shares, in this order: the object counts; pre(), the entry's checks that
+// hold with no active object; the return for no active object; the NULL arguments (`args`: the entry's own pointers are
+// set); dim; the alignment of work; post(), the entry's remaining argument checks; check_active with max_pts and the
+// entry's per-object check; the host Covs of the active objects (host_covs); then launch(k, covs, covs_g), whose CUDA
+// error is reported under `name`.
+template <class Pre, class Post, class Check, class Launch>
+static int grouped_entry(const char* name, int64_t n_obj, const int64_t* off, int dim, const int* order, int64_t n_active,
+                         bool args, const double* hyp_rows, const double* nugget_rows, double nugget, double floor,
+                         unsigned flags, const double* work, int64_t work_doubles, int64_t max_pts, Pre&& pre, Post&& post,
+                         Check&& check, Launch&& launch) {
+  if (n_obj < 0 || n_active < 0) return fail(CGP_ERR_ARG, "%s: negative object count", name);
+  if (int rc = pre()) return rc;
+  const int64_t k = order ? n_active : n_obj;
+  if (k == 0) return 0;
+  if (!args || !off || !hyp_rows || !work) return fail(CGP_ERR_ARG, "%s: NULL argument", name);
+  if (dim != 1 && dim != 2) return fail(CGP_ERR_ARG, "dim must be 1 or 2, got %d", dim);
+  if ((uintptr_t)work & 15) return fail(CGP_ERR_ARG, "%s: work must be 16-byte aligned", name);
+  if (int rc = post()) return rc;
+  if (int rc = check_active(name, n_obj, off, order, k, max_pts, work_doubles, check)) return rc;
+  std::vector<Cov> covs, covs_g;
+  host_covs(dim, hyp_rows, nugget_rows, nugget, floor, flags, k, covs, covs_g);
+  keep_pool_memory();
+  const int e = launch(k, covs.data(), covs_g.data());
+  return e ? cuda_fail(e, name) : 0;
+}
+// padded sizes stay within the 65535 rows cgp_cov_matrix_dev builds an auto-covariance for
+static const int64_t LARGE_MAX_PTS = 65535 / 128 * 128;
+
 }  // namespace cgp
 
 using namespace cgp;
@@ -286,48 +316,19 @@ int cgp_ll_objhyp_dev(int64_t n_obj, const int64_t* off, int max_n, int dim,
 
 int64_t cgp_large_ll_ws_doubles(int64_t n) { return n < 0 ? 0 : large_ll_ws_doubles(n); }
 
-int cgp_large_ll_objhyp_dev(int64_t n_obj, const int64_t* off_host, int dim,
-                            const double* x, const double* y, const double* y0, const double* y_err,
-                            const double* hyp_obj, const double* nugget_obj, double nugget, double floor, unsigned flags,
-                            const int* order_host, int64_t n_active, double* ll_obj, int* info,
-                            double* work, int64_t work_doubles, void* stream) {
-  if (n_obj < 0 || n_active < 0) return fail(CGP_ERR_ARG, "cgp_large_ll_objhyp_dev: negative object count");
-  const int64_t k = order_host ? n_active : n_obj;
-  if (k == 0) return 0;
-  if (!off_host || !x || !y || !hyp_obj || !ll_obj || !info || !work)
-    return fail(CGP_ERR_ARG, "cgp_large_ll_objhyp_dev: NULL argument");
-  if (dim != 1 && dim != 2) return fail(CGP_ERR_ARG, "dim must be 1 or 2, got %d", dim);
-  if ((uintptr_t)work & 15) return fail(CGP_ERR_ARG, "cgp_large_ll_objhyp_dev: work must be 16-byte aligned");
-  int rc = check_active("cgp_large_ll_objhyp_dev", n_obj, off_host, order_host, k, 65535, work_doubles,
-                        [](int64_t, int64_t, int64_t n, int64_t& w) { w = large_ll_ws_doubles(n); return 0; });
-  if (rc) return rc;
-  keep_pool_memory();
-  int e = large_ll_grouped(dim, off_host, x, y, y0, y_err, nullptr, hyp_obj, nugget_obj, nugget, floor, flags, order_host, k,
-                           ll_obj, info, work, work_doubles, (cudaStream_t)stream);
-  return e ? cuda_fail(e, "cgp_large_ll_objhyp_dev") : 0;
-}
-
 int cgp_large_ll_rows_dev(int64_t n_obj, const int64_t* off_host, int dim,
                           const double* x, const double* y, const double* y0, const double* y_err,
                           const double* hyp_rows_host, const double* nugget_rows_host, double nugget, double floor,
                           unsigned flags, const int* order_host, int64_t n_active, double* ll_obj, int* info,
                           double* work, int64_t work_doubles, void* stream) {
-  const char* name = "cgp_large_ll_rows_dev";
-  if (n_obj < 0 || n_active < 0) return fail(CGP_ERR_ARG, "%s: negative object count", name);
-  const int64_t k = order_host ? n_active : n_obj;
-  if (k == 0) return 0;
-  if (!off_host || !x || !y || !hyp_rows_host || !ll_obj || !info || !work) return fail(CGP_ERR_ARG, "%s: NULL argument", name);
-  if (dim != 1 && dim != 2) return fail(CGP_ERR_ARG, "dim must be 1 or 2, got %d", dim);
-  if ((uintptr_t)work & 15) return fail(CGP_ERR_ARG, "%s: work must be 16-byte aligned", name);
-  int rc = check_active(name, n_obj, off_host, order_host, k, 65535, work_doubles,
-                        [](int64_t, int64_t, int64_t n, int64_t& w) { w = large_ll_ws_doubles(n); return 0; });
-  if (rc) return rc;
-  std::vector<Cov> covs, covs_g;                     // covs: as cgp_cov_matrix_dev builds them for LargeObject.factor
-  host_covs(dim, hyp_rows_host, nugget_rows_host, nugget, floor, flags, k, covs, covs_g);
-  keep_pool_memory();
-  int e = large_ll_grouped(dim, off_host, x, y, y0, y_err, covs.data(), nullptr, nullptr, nugget, floor, flags, order_host, k,
-                           ll_obj, info, work, work_doubles, (cudaStream_t)stream);
-  return e ? cuda_fail(e, name) : 0;
+  return grouped_entry(
+      "cgp_large_ll_rows_dev", n_obj, off_host, dim, order_host, n_active, x && y && ll_obj && info, hyp_rows_host,
+      nugget_rows_host, nugget, floor, flags, work, work_doubles, 65535, no_checks, no_checks,
+      [](int64_t, int64_t, int64_t n, int64_t& w) { w = large_ll_ws_doubles(n); return 0; },
+      [&](int64_t k, const Cov* covs, const Cov*) {   // covs: as cgp_cov_matrix_dev builds them for LargeObject.factor
+        return large_ll_grouped(dim, off_host, x, y, y0, y_err, covs, order_host, k, ll_obj, info, work, work_doubles,
+                                (cudaStream_t)stream);
+      });
 }
 
 int64_t cgp_large_cov_ws_doubles(int64_t n, int64_t m) { return n < 0 || m < 0 ? 0 : large_cov_ws_doubles(n, m); }
@@ -338,33 +339,27 @@ int cgp_large_covariance_dev(int64_t n_obj, const int64_t* off_host, int dim, co
                              const int* order_host, int64_t n_active, double* cov, const int64_t* coff_host, int* info,
                              double* work, int64_t work_doubles, void* stream) {
   const char* name = "cgp_large_covariance_dev";
-  if (n_obj < 0 || n_active < 0) return fail(CGP_ERR_ARG, "%s: negative object count", name);
-  const int64_t k = order_host ? n_active : n_obj;
-  if (k == 0) return 0;
-  if (!off_host || !x || !hyp_rows_host || !xnew || !cov || !coff_host || !info || !work)
-    return fail(CGP_ERR_ARG, "%s: NULL argument", name);
-  if (dim != 1 && dim != 2) return fail(CGP_ERR_ARG, "dim must be 1 or 2, got %d", dim);
-  if ((uintptr_t)work & 15) return fail(CGP_ERR_ARG, "%s: work must be 16-byte aligned", name);
-  // padded sizes stay within the 65535 rows cgp_cov_matrix_dev builds an auto-covariance for
-  const int64_t max_pts = 65535 / 128 * 128;
-  if (!goff_host && (m_shared < 0 || m_shared > max_pts))
-    return fail(CGP_ERR_SIZE, "%s: shared grid of %lld points (0..%lld)", name, (long long)m_shared, (long long)max_pts);
-  int rc = check_active(name, n_obj, off_host, order_host, k, max_pts, work_doubles, [&](int64_t j, int64_t b, int64_t n, int64_t& w) {
-    const int64_t m = goff_host ? goff_host[b + 1] - goff_host[b] : m_shared;
-    if (m < 0 || m > max_pts)
-      return fail(CGP_ERR_SIZE, "%s: grid of object %lld has %lld points (0..%lld)", name, (long long)b, (long long)m, (long long)max_pts);
-    if (coff_host[j + 1] - coff_host[j] != m * m)
-      return fail(CGP_ERR_ARG, "%s: coff[%lld + 1] - coff[%lld] is not the grid's %lld^2 entries", name, (long long)j, (long long)j, (long long)m);
-    w = large_cov_ws_doubles(n, m);
-    return 0;
-  });
-  if (rc) return rc;
-  std::vector<Cov> covs, covs_g;                     // as cgp_cov_matrix_dev builds them
-  host_covs(dim, hyp_rows_host, nugget_rows_host, nugget, floor, flags, k, covs, covs_g);
-  keep_pool_memory();
-  int e = large_cov_grouped(dim, off_host, x, y_err, covs.data(), covs_g.data(), xnew, goff_host, m_shared, order_host, k, cov, coff_host,
-                            info, work, work_doubles, (cudaStream_t)stream);
-  return e ? cuda_fail(e, name) : 0;
+  return grouped_entry(
+      name, n_obj, off_host, dim, order_host, n_active, x && xnew && cov && coff_host && info, hyp_rows_host,
+      nugget_rows_host, nugget, floor, flags, work, work_doubles, LARGE_MAX_PTS, no_checks,
+      [&] {
+        if (!goff_host && (m_shared < 0 || m_shared > LARGE_MAX_PTS))
+          return fail(CGP_ERR_SIZE, "%s: shared grid of %lld points (0..%lld)", name, (long long)m_shared, (long long)LARGE_MAX_PTS);
+        return 0;
+      },
+      [&](int64_t j, int64_t b, int64_t n, int64_t& w) {
+        const int64_t m = goff_host ? goff_host[b + 1] - goff_host[b] : m_shared;
+        if (m < 0 || m > LARGE_MAX_PTS)
+          return fail(CGP_ERR_SIZE, "%s: grid of object %lld has %lld points (0..%lld)", name, (long long)b, (long long)m, (long long)LARGE_MAX_PTS);
+        if (coff_host[j + 1] - coff_host[j] != m * m)
+          return fail(CGP_ERR_ARG, "%s: coff[%lld + 1] - coff[%lld] is not the grid's %lld^2 entries", name, (long long)j, (long long)j, (long long)m);
+        w = large_cov_ws_doubles(n, m);
+        return 0;
+      },
+      [&](int64_t k, const Cov* covs, const Cov* covs_g) {   // as cgp_cov_matrix_dev builds them
+        return large_cov_grouped(dim, off_host, x, y_err, covs, covs_g, xnew, goff_host, m_shared, order_host, k, cov,
+                                 coff_host, info, work, work_doubles, (cudaStream_t)stream);
+      });
 }
 
 int64_t cgp_large_pred_ws_doubles(int64_t n, int64_t rows) { return n < 0 || rows < 0 ? 0 : large_pred_ws_doubles(n, rows); }
@@ -377,32 +372,27 @@ int cgp_large_predict_objhyp_dev(int64_t n_obj, const int64_t* off_host, int dim
                                  double* var, int* info, int64_t chunk_rows, double* work, int64_t work_doubles,
                                  void* stream) {
   const char* name = "cgp_large_predict_objhyp_dev";
-  if (n_obj < 0 || n_active < 0) return fail(CGP_ERR_ARG, "%s: negative object count", name);
-  const int64_t k = order_host ? n_active : n_obj;
-  if (k == 0) return 0;
-  if (!off_host || !x || !y || !hyp_rows_host || !xnew || !moff_host || !mean || !info || !work)
-    return fail(CGP_ERR_ARG, "%s: NULL argument", name);
-  if (dim != 1 && dim != 2) return fail(CGP_ERR_ARG, "dim must be 1 or 2, got %d", dim);
-  if ((uintptr_t)work & 15) return fail(CGP_ERR_ARG, "%s: work must be 16-byte aligned", name);
-  if (var && (chunk_rows <= 0 || chunk_rows % 128)) return fail(CGP_ERR_ARG, "%s: chunk_rows must be a positive multiple of 128", name);
-  if (!goff_host && m_shared < 0) return fail(CGP_ERR_ARG, "%s: negative grid size", name);
-  // padded sizes stay within the 65535 rows cgp_cov_matrix_dev builds an auto-covariance for
-  const int64_t max_pts = 65535 / 128 * 128;
-  int rc = check_active(name, n_obj, off_host, order_host, k, max_pts, work_doubles, [&](int64_t j, int64_t b, int64_t n, int64_t& w) {
-    const int64_t m = goff_host ? goff_host[b + 1] - goff_host[b] : m_shared;
-    if (m < 0) return fail(CGP_ERR_ARG, "%s: grid of object %lld has %lld points", name, (long long)b, (long long)m);
-    if (moff_host[j + 1] - moff_host[j] != m)
-      return fail(CGP_ERR_ARG, "%s: moff[%lld + 1] - moff[%lld] is not the grid's %lld points", name, (long long)j, (long long)j, (long long)m);
-    w = large_pred_ws_doubles(n, var ? std::min(m, chunk_rows) : 0);
-    return 0;
-  });
-  if (rc) return rc;
-  std::vector<Cov> covs, covs_g;                     // as LargeObject's make_cov calls build them
-  host_covs(dim, hyp_rows_host, nugget_rows_host, nugget, floor, flags, k, covs, covs_g);
-  keep_pool_memory();
-  int e = large_predict_grouped(dim, off_host, x, y, y0, y_err, covs.data(), covs_g.data(), xnew, goff_host, m_shared, new_y0,
-                                order_host, k, moff_host, mean, var, info, chunk_rows, work, work_doubles, (cudaStream_t)stream);
-  return e ? cuda_fail(e, name) : 0;
+  return grouped_entry(
+      name, n_obj, off_host, dim, order_host, n_active, x && y && xnew && moff_host && mean && info, hyp_rows_host,
+      nugget_rows_host, nugget, floor, flags, work, work_doubles, LARGE_MAX_PTS, no_checks,
+      [&] {
+        if (var && (chunk_rows <= 0 || chunk_rows % 128)) return fail(CGP_ERR_ARG, "%s: chunk_rows must be a positive multiple of 128", name);
+        if (!goff_host && m_shared < 0) return fail(CGP_ERR_ARG, "%s: negative grid size", name);
+        return 0;
+      },
+      [&](int64_t j, int64_t b, int64_t n, int64_t& w) {
+        const int64_t m = goff_host ? goff_host[b + 1] - goff_host[b] : m_shared;
+        if (m < 0) return fail(CGP_ERR_ARG, "%s: grid of object %lld has %lld points", name, (long long)b, (long long)m);
+        if (moff_host[j + 1] - moff_host[j] != m)
+          return fail(CGP_ERR_ARG, "%s: moff[%lld + 1] - moff[%lld] is not the grid's %lld points", name, (long long)j, (long long)j, (long long)m);
+        w = large_pred_ws_doubles(n, var ? std::min(m, chunk_rows) : 0);
+        return 0;
+      },
+      [&](int64_t k, const Cov* covs, const Cov* covs_g) {   // as LargeObject's make_cov calls build them
+        return large_predict_grouped(dim, off_host, x, y, y0, y_err, covs, covs_g, xnew, goff_host, m_shared, new_y0,
+                                     order_host, k, moff_host, mean, var, info, chunk_rows, work, work_doubles,
+                                     (cudaStream_t)stream);
+      });
 }
 
 int64_t cgp_large_loo_ws_doubles(int64_t n, int64_t chunk_rows) {
@@ -416,27 +406,20 @@ int cgp_large_loo_objhyp_dev(int64_t n_obj, const int64_t* off_host, int dim, co
                              double* pull, double* resid, int64_t chunk_rows, double* work, int64_t work_doubles,
                              void* stream) {
   const char* name = "cgp_large_loo_objhyp_dev";
-  if (n_obj < 0 || n_active < 0) return fail(CGP_ERR_ARG, "%s: negative object count", name);
-  if (mode != CGP_LOO_PLAIN && mode != CGP_LOO_RECENTER) return fail(CGP_ERR_ARG, "%s: bad mode %d", name, mode);
-  if (chunk_rows <= 0 || chunk_rows % 128) return fail(CGP_ERR_ARG, "%s: chunk_rows must be a positive multiple of 128", name);
-  const int64_t k = order_host ? n_active : n_obj;
-  if (k == 0) return 0;
-  if (!off_host || !x || !y || !hyp_rows_host || !info || !work) return fail(CGP_ERR_ARG, "%s: NULL argument", name);
-  if (dim != 1 && dim != 2) return fail(CGP_ERR_ARG, "dim must be 1 or 2, got %d", dim);
-  if ((uintptr_t)work & 15) return fail(CGP_ERR_ARG, "%s: work must be 16-byte aligned", name);
-  // padded sizes stay within the 65535 rows cgp_cov_matrix_dev builds an auto-covariance for
-  const int64_t max_pts = 65535 / 128 * 128;
-  int rc = check_active(name, n_obj, off_host, order_host, k, max_pts, work_doubles, [&](int64_t, int64_t, int64_t n, int64_t& w) {
-    w = large_loo_ws_doubles(n, chunk_rows);
-    return 0;
-  });
-  if (rc) return rc;
-  std::vector<Cov> covs, covs_g;                     // covs: as cgp_cov_matrix_dev and cgp_large_loo_dev build them
-  host_covs(dim, hyp_rows_host, nugget_rows_host, nugget, floor, flags, k, covs, covs_g);
-  keep_pool_memory();
-  int e = large_loo_grouped(dim, off_host, x, y, m, y_err, covs.data(), mode == CGP_LOO_RECENTER, order_host, k, info, pred,
-                            pred_var, pull, resid, chunk_rows, work, work_doubles, (cudaStream_t)stream);
-  return e ? cuda_fail(e, name) : 0;
+  return grouped_entry(
+      name, n_obj, off_host, dim, order_host, n_active, x && y && info, hyp_rows_host, nugget_rows_host, nugget, floor,
+      flags, work, work_doubles, LARGE_MAX_PTS,
+      [&] {
+        if (mode != CGP_LOO_PLAIN && mode != CGP_LOO_RECENTER) return fail(CGP_ERR_ARG, "%s: bad mode %d", name, mode);
+        if (chunk_rows <= 0 || chunk_rows % 128) return fail(CGP_ERR_ARG, "%s: chunk_rows must be a positive multiple of 128", name);
+        return 0;
+      },
+      no_checks,
+      [&](int64_t, int64_t, int64_t n, int64_t& w) { w = large_loo_ws_doubles(n, chunk_rows); return 0; },
+      [&](int64_t k, const Cov* covs, const Cov*) {   // covs: as cgp_cov_matrix_dev and cgp_large_loo_dev build them
+        return large_loo_grouped(dim, off_host, x, y, m, y_err, covs, mode == CGP_LOO_RECENTER, order_host, k, info, pred,
+                                 pred_var, pull, resid, chunk_rows, work, work_doubles, (cudaStream_t)stream);
+      });
 }
 
 int cgp_fit_objects_dev(int64_t n_obj, const int64_t* off, int max_n, int dim,

@@ -155,12 +155,10 @@ int large_diag_inv(const double* a, int64_t n_pad, int64_t ld, double* v, int64_
 int large_loo(const double* a, int64_t n, int64_t n_pad, int64_t ld, const Cov& cov, const double* y, const double* m,
               const double* yerr, int recenter, const int* info, double* vwork, int64_t chunk_rows,
               double* pred, double* pvar, double* pull, double* resid, cudaStream_t st);
-// grouped likelihood of large objects, covs[j] built on the host (see cgp_large_ll_rows_dev) or, when covs is NULL, from
-// per-object hyperparameters on the device (see cgp_large_ll_objhyp_dev)
+// grouped likelihood of large objects, covs[j] (with the floor) built on the host (see cgp_large_ll_rows_dev)
 int64_t large_ll_ws_doubles(int64_t n);
 int large_ll_grouped(int dim, const int64_t* off, const double* x, const double* y, const double* y0, const double* yerr,
-                     const Cov* covs, const double* hyp_obj, const double* nugget_obj, double nugget, double floor,
-                     unsigned flags, const int* order, int64_t n_active, double* ll, int* info, double* work,
+                     const Cov* covs, const int* order, int64_t n_active, double* ll, int* info, double* work,
                      int64_t work_doubles, cudaStream_t st);
 // grouped predictive covariance matrices of large objects, covs[j] (data covariance, with the floor) and covs_g[j] (H and
 // K**, without it) built on the host (see cgp_large_covariance_dev)

@@ -545,19 +545,28 @@ __global__ void __launch_bounds__(256) loo_epilogue_kernel(const Cov cov, int64_
 }
 
 // ---------------------------------------------------------------------------------------
-// Grouped likelihood of many large objects, each with its own hyperparameters (large_ll_grouped).  Every kernel
-// below runs the body of its single-object counterpart on one object at a time, so an object's arithmetic does not
-// depend on the other objects of its launch.
-struct GroupObj {
+// Grouped pipelines of large objects (large_ll_grouped, large_predict_grouped, large_loo_grouped, large_cov_grouped).
+// Every kernel below runs the body of its single-object counterpart on one object at a time, so an object's arithmetic
+// does not depend on the other objects of its launch.
+
+// What build_grouped_kernel reads of an object of a grouped likelihood, prediction or leave-one-out: its covariance
+// function, built on the host with the floor (as cgp_cov_matrix_dev's make_cov builds it), its data (y0: the mean
+// subtracted from y, may be null; yerr may be null) and where A, the residual and the ones vector go.
+struct BuildObj {
+  Cov cov;
   const double* x; const double* y; const double* y0; const double* yerr;
   double* a;                 // n_pad x n_pad covariance -> blocked factor (leading dimension n_pad)
-  double* u;                 // residual y - y0 (n_pad, zero padded), consumed by the forward sweep
-  double* z;                 // z = L^-1 (y - y0)
+  double* r;                 // residual y - y0 (n_pad, zero padded), consumed by the forward sweep
+  double* ones;              // ones vector, consumed by the forward sweep (leave-one-out recentred mode; null otherwise)
   int64_t n, n_pad;
-  int64_t io;                // position in `order`: compact hyperparameters, nugget, ll and info
-  int64_t cta0;              // first CTA of the object in the covariance launch
-  Cov cov;                   // host-built covariance function, read by the covariance build in host mode only
+  int64_t cta;               // first CTA of the object in the build launch
 };
+// One object of a grouped likelihood (large_ll_grouped).
+struct GroupObj : BuildObj {
+  double* z;                 // z = L^-1 (y - y0)
+  int64_t io;                // position in `order`: ll and info
+};
+// Per-object hyperparameter rows in device memory, from which cov_gram_kernel<OBJHYP> builds each object's Cov.
 struct GroupHyp {
   const double* hyp_obj; const double* nugget_obj; double nugget, floor; unsigned flags;
 };
@@ -589,23 +598,24 @@ __device__ __forceinline__ Cov group_cov(const GroupHyp& h, int64_t io) {
   return cov_from_hyp(DIM, h.hyp_obj + io * (DIM == 1 ? 2 : 4), h.nugget_obj ? h.nugget_obj[io] : h.nugget, h.floor, h.flags);
 }
 
-// Covariance of every object of a wave (the layout of cov_build_kernel) and its residual.  Object i owns
-// n_pad * ceil(n_pad / 256) CTAs from objs[i].cta0 on: one row, 256 columns each.  HOST_COV: the covariance function is
-// the object's host-built `cov` (as cgp_cov_matrix_dev's make_cov builds it), otherwise group_cov on the device.
-template <int DIM, bool HOST_COV>
-__global__ void __launch_bounds__(128) cov_build_grouped_kernel(const GroupObj* __restrict__ objs, const int n_obj,
-                                                                const GroupHyp h) {
+// A = K(x, x) + noise (the layout of cov_build_kernel), the residual (residual_kernel) and, where `ones` is set, the
+// ones vector (ones_kernel) of every object of a wave.  Object i owns n_pad * ceil(n_pad / 256) CTAs from objs[i].cta
+// on: one row, 256 columns each.  O: the pipeline's descriptor, which sets the stride of objs.
+template <int DIM, class O>
+__global__ void __launch_bounds__(128) build_grouped_kernel(const O* __restrict__ objs, const int n_obj) {
   const int64_t t = blockIdx.x;
-  const GroupObj& o = owner(objs, n_obj, t, &GroupObj::cta0);
+  const BuildObj& o = owner<O>(objs, n_obj, t, &O::cta);
   const int64_t per_row = (o.n_pad + 255) / 256;
-  const int64_t local = t - o.cta0, r = local / per_row, chunk = local - r * per_row;
+  const int64_t local = t - o.cta, r = local / per_row, chunk = local - r * per_row;
+  if (chunk == 0 && threadIdx.x == 0) {
+    o.r[r] = r < o.n ? o.y[r] - (o.y0 ? o.y0[r] : 0.0) : 0.0;      // residual_kernel
+    if (o.ones) o.ones[r] = r < o.n ? 1.0 : 0.0;                   // ones_kernel
+  }
   CovArgs a;
-  a.dim = DIM; a.autocov = 1;
-  if constexpr (HOST_COV) a.cov = o.cov; else a.cov = group_cov<DIM>(h, o.io);
+  a.dim = DIM; a.cov = o.cov; a.autocov = 1;
   a.xc = o.x; a.n = o.n; a.xr = o.x; a.m = o.n; a.yerr = o.yerr;
   a.out = o.a; a.ld = o.n_pad; a.rows_pad = o.n_pad; a.cols_pad = o.n_pad;
   cov_build_at<DIM>(a, r, (chunk * 128 + threadIdx.x) * 2);
-  if (chunk == 0 && threadIdx.x == 0) o.u[r] = r < o.n ? o.y[r] - (o.y0 ? o.y0[r] : 0.0) : 0.0;   // residual_kernel
 }
 
 // Forward sweep step k of the objects 0 .. gridDim.y, gridDim.z right-hand sides each (the descriptors of one object
@@ -614,7 +624,7 @@ template <class Obj>
 __global__ void __launch_bounds__(256) fwd_step_grouped_kernel(const Obj* __restrict__ objs, const int64_t k0) {
   const Obj& o = objs[blockIdx.y * gridDim.z + blockIdx.z];
   if ((int64_t)blockIdx.x >= 1 + (o.n_pad - k0 - 128 + 63) / 64) return;
-  fwd_step_at(o.a, o.n_pad, k0, o.n_pad, o.u, o.z, blockIdx.x);
+  fwd_step_at(o.a, o.n_pad, k0, o.n_pad, o.r, o.z, blockIdx.x);
 }
 
 // One CTA per object: quad = |z|^2 (dot_sq_kernel), log det and info summed over the blocks in the order of
@@ -705,21 +715,17 @@ __global__ void __launch_bounds__(256) cov_pack_grouped_kernel(const CovObj* __r
   }
 }
 
-// One object of a grouped prediction (large_predict_grouped).  `cov` (with the floor, for A) and `cov_g` (without it, for
-// the mean, H and the variance) come from the host, as the make_cov calls of LargeObject.factor / cgp_large_predict_dev
-// build them.
-struct PredObj {
-  Cov cov, cov_g;
-  const double* x; const double* y; const double* y0; const double* yerr;
+// One object of a grouped prediction (large_predict_grouped).  `cov_g` (without the floor, for the mean, H and the
+// variance) comes from the host, as the make_cov calls of LargeObject.factor / cgp_large_predict_dev build it.
+struct PredObj : BuildObj {
+  Cov cov_g;
   const double* g; const double* new_y0;   // grid (m points) and the mean function on it (may be null)
-  double* a;                 // n_pad x n_pad covariance -> blocked factor
-  double* u;                 // residual, consumed by the forward sweep
   double* z;                 // L^-1 (y - y0), consumed by the backward sweep
   double* alpha;             // K^-1 (y - y0)
   double* mean; double* var; // the object's m outputs
-  int64_t n, n_pad, m;
+  int64_t m;
   int64_t io;                // position in `order`: info
-  int64_t cta_a, cta_mean;   // first CTA of the object in the build and in the mean launch
+  int64_t cta_mean;          // first CTA of the object in the mean launch
 };
 // One object's rows [r0, r0 + rows) of one variance pass.
 struct PassObj {
@@ -730,21 +736,6 @@ struct PassObj {
   int64_t n, n_pad, rows, rows_pad;
   int64_t cta_h, cta_var;    // first CTA of the object in the H build and in the variance launch
 };
-
-// A = K(x, x) + noise and u = y - y0 of every object of a wave, as cov_build_grouped_kernel builds them.
-template <int DIM>
-__global__ void __launch_bounds__(128) pred_build_grouped_kernel(const PredObj* __restrict__ objs, const int n_obj) {
-  const int64_t t = blockIdx.x;
-  const PredObj& o = owner(objs, n_obj, t, &PredObj::cta_a);
-  const int64_t per_row = (o.n_pad + 255) / 256;
-  const int64_t local = t - o.cta_a, r = local / per_row, chunk = local - r * per_row;
-  if (chunk == 0 && threadIdx.x == 0) o.u[r] = r < o.n ? o.y[r] - (o.y0 ? o.y0[r] : 0.0) : 0.0;   // residual_kernel
-  CovArgs a;
-  a.dim = DIM; a.cov = o.cov; a.autocov = 1;
-  a.xc = o.x; a.n = o.n; a.xr = o.x; a.m = o.n; a.yerr = o.yerr;
-  a.out = o.a; a.ld = o.n_pad; a.rows_pad = o.n_pad; a.cols_pad = o.n_pad;
-  cov_build_at<DIM>(a, r, (chunk * 128 + threadIdx.x) * 2);
-}
 
 // Backward sweep launch s of the objects 0 .. gridDim.y, gridDim.z right-hand sides each (as fwd_step_grouped_kernel):
 // right-hand side z of object y runs bwd_step_kernel's CTA x of its block n_pad / 128 - 1 - s.
@@ -806,47 +797,21 @@ __global__ void __launch_bounds__(256) pred_finish_grouped_kernel(const PredObj*
   }
 }
 
-// One object of a grouped leave-one-out (large_loo_grouped).  `cov` comes from the host, as cgp_cov_matrix_dev and
-// cgp_large_loo_dev build it.
-struct LooObj {
-  Cov cov;
-  const double* x; const double* y; const double* m; const double* yerr;   // m, yerr may be null
-  double* a;                 // n_pad x n_pad covariance -> blocked factor
-  double* r;                 // residual y - m, consumed by the forward sweep
-  double* ones;              // ones vector, consumed by the forward sweep (recentred mode; null otherwise)
+// One object of a grouped leave-one-out (large_loo_grouped); y0 is the mean m, as cgp_large_loo_dev takes it.
+struct LooObj : BuildObj {
   double* alpha;             // K^-1 r
   double* kinv1;             // K^-1 1 (recentred mode; null otherwise)
   double* negd;              // -diag(K^-1)
   double* rsum;              // sum r
   double* pred; double* pvar; double* pull; double* resid;   // the object's n outputs (each may be null)
-  int64_t n, n_pad;
   int64_t io;                // position in `order`: info
-  int64_t cta_a, cta_epi;    // first CTA of the object in the build and in the epilogue launch
+  int64_t cta_epi;           // first CTA of the object in the epilogue launch
 };
-// One right-hand side of the sweeps: u -> z = L^-1 u (forward), z -> alpha = L^-T z (backward).
-struct SolveObj { double* a; double* u; double* z; double* alpha; int64_t n_pad; };
+// One right-hand side of the sweeps: r -> z = L^-1 r (forward), z -> alpha = L^-T z (backward).
+struct SolveObj { double* a; double* r; double* z; double* alpha; int64_t n_pad; };
 // One object's pass of the diag(K^-1) solve: `rows` identity rows of width w staged at v (leading dimension ld), their
 // negated squared norms to negd.
 struct DiagObj { double* v; int64_t ld, w, rows; double* negd; int64_t cta; };
-
-// A = K(x, x) + noise and r = y - m of every object of a wave, as pred_build_grouped_kernel builds them, and the ones
-// vector of ones_kernel in the recentred mode.
-template <int DIM>
-__global__ void __launch_bounds__(128) loo_build_grouped_kernel(const LooObj* __restrict__ objs, const int n_obj) {
-  const int64_t t = blockIdx.x;
-  const LooObj& o = owner(objs, n_obj, t, &LooObj::cta_a);
-  const int64_t per_row = (o.n_pad + 255) / 256;
-  const int64_t local = t - o.cta_a, r = local / per_row, chunk = local - r * per_row;
-  if (chunk == 0 && threadIdx.x == 0) {
-    o.r[r] = r < o.n ? o.y[r] - (o.m ? o.m[r] : 0.0) : 0.0;        // residual_kernel
-    if (o.ones) o.ones[r] = r < o.n ? 1.0 : 0.0;                   // ones_kernel
-  }
-  CovArgs a;
-  a.dim = DIM; a.cov = o.cov; a.autocov = 1;
-  a.xc = o.x; a.n = o.n; a.xr = o.x; a.m = o.n; a.yerr = o.yerr;
-  a.out = o.a; a.ld = o.n_pad; a.rows_pad = o.n_pad; a.cols_pad = o.n_pad;
-  cov_build_at<DIM>(a, r, (chunk * 128 + threadIdx.x) * 2);
-}
 
 // sum r of object blockIdx.x (sum_kernel, 1024 threads).
 __global__ void __launch_bounds__(1024) sum_grouped_kernel(const LooObj* __restrict__ objs) {
@@ -884,7 +849,7 @@ __global__ void __launch_bounds__(256) loo_finish_grouped_kernel(const LooObj* _
   __syncthreads();
   const int64_t i = (t - o.cta_epi) * blockDim.x + threadIdx.x;
   if (i < o.n)
-    loo_epilogue_at(o.cov, o.n, o.y, o.m, o.yerr, o.alpha, o.negd, o.kinv1, o.rsum, bad_s, o.pred, o.pvar, o.pull, o.resid, i);
+    loo_epilogue_at(o.cov, o.n, o.y, o.y0, o.yerr, o.alpha, o.negd, o.kinv1, o.rsum, bad_s, o.pred, o.pvar, o.pull, o.resid, i);
 }
 
 }  // namespace
@@ -1186,7 +1151,7 @@ int large_ll_total(const double* ll, const int* info, int64_t n, double* out2, c
 // (cosmogp/Gaussian_process.py:356-361).  One CTA per 64 x 64 block: V_i^T and V_j^T staged in shared memory
 // (k-major, so that a thread's four rows are 32 contiguous bytes), 4 x 4 outputs per thread, K(g_i, g_j) generated
 // on the fly.  8 bytes written per ~64 FMAs + one exp: bound by the HBM write of the M x M matrices.
-// OBJHYP: object b's CTAs build their own Cov from h (row b, as in the grouped likelihood) instead of reading `cov`.
+// OBJHYP: object b's CTAs build their own Cov from h (group_cov of row b) instead of reading `cov`.
 template <int DIM, bool OBJHYP>
 __global__ void __launch_bounds__(256) cov_gram_kernel(Cov cov, const double* __restrict__ grid, const int64_t* __restrict__ goff,
                                                        int64_t m_shared, const double* __restrict__ v, int ldv,
@@ -1652,15 +1617,12 @@ struct GroupSchedule {
 }  // namespace
 
 // Log-likelihoods of the objects order[0 .. n_active) (object ids; NULL: 0 .. n_active), object order[j] with the
-// hyperparameters of row j, by the blocked factorisation of large_potrf run for all objects of a wave at once (waves:
-// plan_waves, each object's part of the workspace large_ll_ws_doubles).  Per wave: one covariance launch; the
-// factorisation (GroupSchedule::factor); one forward-sweep launch per block; one epilogue.  The covariance function of
-// object order[j] is covs[j] when covs is given (built on the host, with the floor: then every step is that of
-// cgp_cov_matrix_dev + cgp_potrf_dev + cgp_large_solve_dev, and so is every bit), otherwise cov_from_hyp of
-// hyp_obj / nugget_obj on the device.  The caller checks that every object fits.
+// covariance function covs[j] (built on the host, with the floor), by every step of cgp_cov_matrix_dev + cgp_potrf_dev +
+// cgp_large_solve_dev run for all objects of a wave at once: one covariance launch; the factorisation
+// (GroupSchedule::factor); one forward-sweep launch per block; one epilogue.  Waves: plan_waves, each object's part of
+// the workspace large_ll_ws_doubles.  The caller checks that every object fits.
 int large_ll_grouped(int dim, const int64_t* off, const double* x, const double* y, const double* y0, const double* yerr,
-                     const Cov* covs, const double* hyp_obj, const double* nugget_obj, double nugget, double floor,
-                     unsigned flags, const int* order, int64_t n_active, double* ll, int* info, double* work,
+                     const Cov* covs, const int* order, int64_t n_active, double* ll, int* info, double* work,
                      int64_t work_doubles, cudaStream_t st) {
   const Waves waves = plan_waves(order, n_active, off, work_doubles, [](const WaveItem& it) { return large_ll_ws_doubles(it.n); });
   GroupSchedule s;
@@ -1675,10 +1637,10 @@ int large_ll_grouped(int dim, const int64_t* off, const double* x, const double*
       const WaveItem& it = w[i];
       const int64_t o0 = off[it.b], np = it.n_pad;
       GroupObj& g = objs[i];
+      g.cov = covs[it.j];
       g.x = x + dim * o0; g.y = y + o0; g.y0 = y0 ? y0 + o0 : nullptr; g.yerr = yerr ? yerr + o0 : nullptr;
-      g.a = work + cur; g.u = g.a + np * np; g.z = g.u + np;
-      g.n = it.n; g.n_pad = np; g.io = it.j; g.cta0 = cta;
-      if (covs) g.cov = covs[it.j];
+      g.a = work + cur; g.r = g.a + np * np; g.ones = nullptr; g.z = g.r + np;
+      g.n = it.n; g.n_pad = np; g.io = it.j; g.cta = cta;
       cur += np * np + 2 * np; cta += np * ((np + 255) / 256);
       a[i] = g.a;
     }
@@ -1694,19 +1656,12 @@ int large_ll_grouped(int dim, const int64_t* off, const double* x, const double*
                             nullptr, nullptr});
     s.launches.push_back({L_FIN, W, W, 0, t_objs, t.t_koff, 0, ldb, infob});
   }
-
-  GroupHyp h; h.hyp_obj = hyp_obj; h.nugget_obj = nugget_obj; h.nugget = nugget; h.floor = floor; h.flags = flags;
   return s.run(work, st, [&](const Launch& l, const char* td) {
     const GroupObj* objs = reinterpret_cast<const GroupObj*>(td + l.t0);
     switch (l.kind) {
       case L_COV:
-        if (covs) {
-          if (dim == 1) cov_build_grouped_kernel<1, true><<<(unsigned)l.grid, 128, 0, st>>>(objs, (int)l.count, h);
-          else cov_build_grouped_kernel<2, true><<<(unsigned)l.grid, 128, 0, st>>>(objs, (int)l.count, h);
-        } else {
-          if (dim == 1) cov_build_grouped_kernel<1, false><<<(unsigned)l.grid, 128, 0, st>>>(objs, (int)l.count, h);
-          else cov_build_grouped_kernel<2, false><<<(unsigned)l.grid, 128, 0, st>>>(objs, (int)l.count, h);
-        }
+        if (dim == 1) build_grouped_kernel<1><<<(unsigned)l.grid, 128, 0, st>>>(objs, (int)l.count);
+        else build_grouped_kernel<2><<<(unsigned)l.grid, 128, 0, st>>>(objs, (int)l.count);
         break;
       case L_FWD:
         fwd_step_grouped_kernel<GroupObj><<<dim3((unsigned)l.grid, (unsigned)l.count), 256, 0, st>>>(objs, l.k0);
@@ -1827,9 +1782,9 @@ int large_predict_grouped(int dim, const int64_t* off, const double* x, const do
       o.cov = covs[it.j]; o.cov_g = covs_g[it.j];
       o.x = x + dim * o0; o.y = y + o0; o.y0 = y0 ? y0 + o0 : nullptr; o.yerr = yerr ? yerr + o0 : nullptr;
       o.g = goff ? xnew + dim * goff[it.b] : xnew; o.new_y0 = new_y0 ? new_y0 + moff[it.j] : nullptr;
-      o.a = work + cur; o.u = o.a + np * np; o.z = o.u + np; o.alpha = o.z + np; v[i] = o.alpha + np;
+      o.a = work + cur; o.r = o.a + np * np; o.ones = nullptr; o.z = o.r + np; o.alpha = o.z + np; v[i] = o.alpha + np;
       o.mean = mean + moff[it.j]; o.var = var ? var + moff[it.j] : nullptr;
-      o.n = it.n; o.n_pad = np; o.m = grid_size(it.b); o.io = it.j; o.cta_a = cta; o.cta_mean = cta_mean;
+      o.n = it.n; o.n_pad = np; o.m = grid_size(it.b); o.io = it.j; o.cta = cta; o.cta_mean = cta_mean;
       cur += large_pred_ws_doubles(it.n, pass_rows(it.b));
       cta += np * ((np + 255) / 256); cta_mean += (o.m + 255) / 256;
       m_max = std::max(m_max, o.m);
@@ -1875,8 +1830,8 @@ int large_predict_grouped(int dim, const int64_t* off, const double* x, const do
     const PassObj* pass = reinterpret_cast<const PassObj*>(td + l.t0);
     switch (l.kind) {
       case L_COV:
-        if (dim == 1) pred_build_grouped_kernel<1><<<(unsigned)l.grid, 128, 0, st>>>(objs, (int)l.count);
-        else pred_build_grouped_kernel<2><<<(unsigned)l.grid, 128, 0, st>>>(objs, (int)l.count);
+        if (dim == 1) build_grouped_kernel<1><<<(unsigned)l.grid, 128, 0, st>>>(objs, (int)l.count);
+        else build_grouped_kernel<2><<<(unsigned)l.grid, 128, 0, st>>>(objs, (int)l.count);
         break;
       case L_FWD:
         fwd_step_grouped_kernel<PredObj><<<dim3((unsigned)l.grid, (unsigned)l.count), 256, 0, st>>>(objs, l.k0);
@@ -1939,7 +1894,7 @@ int large_loo_grouped(int dim, const int64_t* off, const double* x, const double
       const int64_t np = it.n_pad, o0 = off[it.b];
       LooObj& o = objs[i];
       o.cov = covs[it.j];
-      o.x = x + dim * o0; o.y = y + o0; o.m = m ? m + o0 : nullptr; o.yerr = yerr ? yerr + o0 : nullptr;
+      o.x = x + dim * o0; o.y = y + o0; o.y0 = m ? m + o0 : nullptr; o.yerr = yerr ? yerr + o0 : nullptr;
       o.a = work + cur; v[i] = o.a + np * np;
       double* vec = v[i] + std::min(np, chunk_rows) * np;
       o.r = vec; o.alpha = vec + 2 * np;
@@ -1947,7 +1902,7 @@ int large_loo_grouped(int dim, const int64_t* off, const double* x, const double
       o.negd = negd[i] = vec + 6 * np; o.rsum = vec + 7 * np;
       o.pred = pred ? pred + o0 : nullptr; o.pvar = pvar ? pvar + o0 : nullptr;
       o.pull = pull ? pull + o0 : nullptr; o.resid = resid ? resid + o0 : nullptr;
-      o.n = it.n; o.n_pad = np; o.io = it.j; o.cta_a = cta; o.cta_epi = cta_epi;
+      o.n = it.n; o.n_pad = np; o.io = it.j; o.cta = cta; o.cta_epi = cta_epi;
       rhs.push_back({o.a, o.r, vec + np, o.alpha, np});
       if (recenter) rhs.push_back({o.a, o.ones, vec + 4 * np, o.kinv1, np});
       cur += large_loo_ws_doubles(it.n, chunk_rows);
@@ -1974,8 +1929,8 @@ int large_loo_grouped(int dim, const int64_t* off, const double* x, const double
     const SolveObj* rhs = reinterpret_cast<const SolveObj*>(td + l.t0);
     switch (l.kind) {
       case L_COV:
-        if (dim == 1) loo_build_grouped_kernel<1><<<(unsigned)l.grid, 128, 0, st>>>(objs, (int)l.count);
-        else loo_build_grouped_kernel<2><<<(unsigned)l.grid, 128, 0, st>>>(objs, (int)l.count);
+        if (dim == 1) build_grouped_kernel<1><<<(unsigned)l.grid, 128, 0, st>>>(objs, (int)l.count);
+        else build_grouped_kernel<2><<<(unsigned)l.grid, 128, 0, st>>>(objs, (int)l.count);
         break;
       case L_SUM:
         sum_grouped_kernel<<<(unsigned)l.grid, 1024, 0, st>>>(objs);

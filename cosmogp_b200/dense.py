@@ -269,15 +269,29 @@ def _gather(flat, off, ids):
     return flat[idx], new_off
 
 
-def _request(off, objects, grid, goff, hyp, nugget, dim):
-    """The objects of a grouped call: (off as int64, their ids (objects, default all), their (k, n_hyp) hyperparameter
-    rows and k nugget rows (hyp, nugget: shared, or one per object of `objects`), their grid sizes)."""
-    off = np.asarray(off, dtype=np.int64)
-    ids = np.arange(len(off) - 1, dtype=np.int64) if objects is None else np.asarray(objects, dtype=np.int64)
-    k = len(ids)
+def _rows(hyp, nugget, k, dim):
+    """The (k, n_hyp) hyperparameter rows and k nugget rows of a grouped call, C-contiguous host arrays: hyp (n_hyp,)
+    shared or one row per object; nugget scalar or one per object."""
     nh = 2 if dim == 1 else 4
     rows = np.ascontiguousarray(np.broadcast_to(np.asarray(hyp, dtype=np.float64).reshape(-1, nh), (k, nh)))
     nug_rows = np.ascontiguousarray(np.broadcast_to(np.asarray(nugget, dtype=np.float64).reshape(-1), (k,)))
+    return rows, nug_rows
+
+
+def capped_ws_doubles(need, cap_bytes):
+    """Workspace (doubles) of a grouped call whose objects need `need` doubles each: their needs summed up to cap_bytes,
+    at least the largest need (objects beyond the cap run in further waves)."""
+    need = np.asarray(need, dtype=np.int64).reshape(-1)
+    return max(min(int(need.sum()), cap_bytes // 8), int(need.max()) if len(need) else 2)
+
+
+def _request(off, objects, grid, goff, hyp, nugget, dim):
+    """The objects of a grouped call: (off as int64, their ids (objects, default all), their hyperparameter and nugget
+    rows (_rows), their grid sizes)."""
+    off = np.asarray(off, dtype=np.int64)
+    ids = np.arange(len(off) - 1, dtype=np.int64) if objects is None else np.asarray(objects, dtype=np.int64)
+    k = len(ids)
+    rows, nug_rows = _rows(hyp, nugget, k, dim)
     m = np.diff(np.asarray(goff, dtype=np.int64))[ids] if goff is not None else np.full(k, len(grid), dtype=np.int64)
     return off, ids, rows, nug_rows, m
 
@@ -402,37 +416,39 @@ def ll_ws_doubles(n):
 
 
 def ll_workspace(n, device):
-    """The device workspace of log_likelihoods for objects of n points: their needs summed up to LL_WS_BYTES, at
-    least the largest one's.  Allocate it once and pass it to every evaluation."""
-    need = ll_ws_doubles(np.asarray(n, dtype=np.int64).reshape(-1))
-    big = int(need.max()) if len(need) else 2
-    return torch.empty(max(min(int(need.sum()), LL_WS_BYTES // 8), big), dtype=torch.float64, device=device)
+    """The device workspace of log_likelihoods for objects of n points: capped_ws_doubles of their needs with cap
+    LL_WS_BYTES.  Allocate it once and pass it to every evaluation."""
+    return torch.empty(capped_ws_doubles(ll_ws_doubles(n), LL_WS_BYTES), dtype=torch.float64, device=device)
+
+
+def log_likelihoods_dev(batch, ids, hyp, nugget, ll, info, work, floor=0.0, flags=0):
+    """Enqueue log_likelihoods' grouped call (cgp_large_ll_rows_dev) for the objects `ids` (k > 0) of a DeviceBatch:
+    ll (k float64) and info (k int32), device tensors, receive the results.  hyp, nugget as in log_likelihoods; work: a
+    device workspace from ll_workspace or larger.  Does not synchronise."""
+    k = len(ids)
+    rows, nug_rows = _rows(hyp, nugget, k, batch.dim)
+    order = np.ascontiguousarray(ids, dtype=np.int32)
+    with torch.cuda.device(batch.device):
+        _lib.check(_lib.lib().cgp_large_ll_rows_dev(
+            batch.n_obj, _lib.hptr(batch.off_host), batch.dim, _p(batch.x), _p(batch.y), _p(batch.y0), _p(batch.y_err),
+            _lib.hptr(rows), _lib.hptr(nug_rows), 0.0, float(floor), int(flags), _lib.hptr(order), k, _p(ll), _p(info),
+            _p(work), int(work.numel()), batch._stream()), "cgp_large_ll_rows_dev")
 
 
 def log_likelihoods(batch, objects, hyp, nugget, flags=0, work=None):
     """LargeObject(x_b, y_b, y_err_b, y0_b, flags=flags).factor(hyp, nugget) of the objects `objects` (default all) of
-    a DeviceBatch in one grouped call (cgp_large_ll_rows_dev), each ll and info bit for bit that loop's, whatever the
+    a DeviceBatch in one grouped call (log_likelihoods_dev), each ll and info bit for bit that loop's, whatever the
     objects around it.  hyp: (n_hyp,) shared, or one row per object of `objects`; nugget: scalar or one per object.
     work: a device workspace from ll_workspace, reused across calls (default: one allocated here).  One native call
     and one synchronisation.  Returns host (ll, info), info the first failing pivot and ll NaN where it is not 0."""
-    L = _lib.lib()
     ids = np.arange(batch.n_obj, dtype=np.int64) if objects is None else np.asarray(objects, dtype=np.int64)
     k = len(ids)
     if not k:
         return np.zeros(0), np.zeros(0, dtype=np.int32)
-    nh = 2 if batch.dim == 1 else 4
-    rows = np.ascontiguousarray(np.broadcast_to(np.asarray(hyp, dtype=np.float64).reshape(-1, nh), (k, nh)))
-    nug_rows = np.ascontiguousarray(np.broadcast_to(np.asarray(nugget, dtype=np.float64).reshape(-1), (k,)))
     if work is None:
         work = ll_workspace(batch.off_host[ids + 1] - batch.off_host[ids], batch.device)
     out = torch.empty(k + (k + 1) // 2, dtype=torch.float64, device=batch.device)   # ll, then info as int32
-    info = out[k:].view(torch.int32)
-    order = np.ascontiguousarray(ids, dtype=np.int32)
-    with torch.cuda.device(batch.device):
-        _lib.check(L.cgp_large_ll_rows_dev(
-            batch.n_obj, _lib.hptr(batch.off_host), batch.dim, _p(batch.x), _p(batch.y), _p(batch.y0), _p(batch.y_err),
-            _lib.hptr(rows), _lib.hptr(nug_rows), 0.0, 0.0, int(flags), _lib.hptr(order), k, _p(out), _p(info),
-            _p(work), int(work.numel()), batch._stream()), "cgp_large_ll_rows_dev")
+    log_likelihoods_dev(batch, ids, hyp, nugget, out[:k], out[k:].view(torch.int32), work, flags=flags)
     host = out.cpu().numpy()
     return host[:k].copy(), host[k:].view(np.int32)[:k].copy()
 
@@ -450,21 +466,17 @@ def loo_grouped(batch, objects, hyp, nugget, mode, outs, flags=0, chunk_rows=Non
     one row per object of `objects`; nugget: scalar or one per object.  outs: (pred, pred_var, pull, resid, info)
     device tensors in the batch's layout, as DeviceBatch.loo_dev returns them; the objects' points and their info
     entries are written in place.  chunk_rows: as LargeLoo's for the largest object (loo_chunk_rows).  work_doubles:
-    device workspace (default: the objects' needs summed up to 2 GB, at least the largest one's).  Does not
-    synchronise."""
+    device workspace (default: capped_ws_doubles of the objects' needs with a cap of 2 GB).  Does not synchronise."""
     L = _lib.lib()
     ids = np.asarray(objects, dtype=np.int64)
     k = len(ids)
     if not k:
         return
-    nh = 2 if batch.dim == 1 else 4
-    rows = np.ascontiguousarray(np.broadcast_to(np.asarray(hyp, dtype=np.float64).reshape(-1, nh), (k, nh)))
-    nug_rows = np.ascontiguousarray(np.broadcast_to(np.asarray(nugget, dtype=np.float64).reshape(-1), (k,)))
+    rows, nug_rows = _rows(hyp, nugget, k, batch.dim)
     n = batch.off_host[ids + 1] - batch.off_host[ids]
     chunk = loo_chunk_rows(pad128(int(n.max())), chunk_rows)
     if work_doubles is None:
-        need = loo_ws_doubles(n, chunk)
-        work_doubles = max(min(int(need.sum()), (2 << 30) // 8), int(need.max()))
+        work_doubles = capped_ws_doubles(loo_ws_doubles(n, chunk), 2 << 30)
     work = torch.empty(int(work_doubles), dtype=torch.float64, device=batch.device)
     info = torch.empty(k, dtype=torch.int32, device=batch.device)
     order = np.ascontiguousarray(ids, dtype=np.int32)

@@ -5,8 +5,9 @@ per-object Python loops of the reference (:207, :264, :304, :349) are replaced b
 single batched launches on a device-resident copy of the data.  Which objects are too large for those launches is
 decided in one place, batch.SizeSplit; they go through the blocked HBM factorisation, all of them at once: for
 likelihoods under shared hyperparameters (dense.log_likelihoods, every object of the batch then), for the likelihood
-evaluations of per-object fits (cgp_large_ll_objhyp_dev) and for predictions (dense.predictions: the large objects of a
-per-object prediction, or every object of a batch with a large one under shared hyperparameters).
+evaluations of per-object fits (dense.log_likelihoods_dev, from DeviceBatch.ll_objhyp) and for predictions
+(dense.predictions: the large objects of a per-object prediction, or every object of a batch with a large one under
+shared hyperparameters).  Each of these results is bit for bit that of the object alone on the blocked path.
 
 Differences (SURVEY.md section 9.1):
   * `svd_method`: every object is factorised by the device Cholesky kernels whatever the flag says (for a
@@ -349,8 +350,9 @@ class Gaussian_process:
         simplices live on the device too (cgp_fit_objects_dev, no host round trips); 'host': the numpy
         statement of the same rules (cosmogp_b200.fit), kept as the cross-check -- both give identical results.
         Objects above 224 points are fitted too: every evaluation factors all of them at once by the grouped blocked
-        factorisation (cgp_large_ll_objhyp_dev), driven by the numpy statement in both modes; with optimizer='device'
-        the objects of up to 224 points still run cgp_fit_objects_dev, on a batch of their own.
+        factorisation (dense.log_likelihoods_dev, each likelihood bit for bit dense.LargeObject.factor's), driven by the
+        numpy statement in both modes; with optimizer='device' the objects of up to 224 points still run
+        cgp_fit_objects_dev, on a batch of their own.
         Sets `hyperparameters_per_object` (N_sn, n_hyp), `nugget_per_object` (N_sn,) and
         `log_likelihood_per_object`; an object whose covariance is not positive definite at a trial
         point gets +inf there (the reference would abort with LinAlgError)."""

@@ -136,31 +136,23 @@ int cgp_ll_objhyp_dev(int64_t n_obj, const int64_t* off, int max_n, int dim,
                       const double* hyp_obj, const double* nugget_obj, double nugget, double floor, unsigned flags,
                       const int* order, int64_t n_active, double* ll_obj, int* info, void* stream);
 
-/* cgp_ll_objhyp_dev for objects of ANY size (up to 65535 points) through the blocked HBM factorisation of
- * cgp_potrf_dev, all active objects of a wave sharing each launch: per-object fits of objects above 224 points.
+/* Log-likelihoods of objects of ANY size (up to 65535 points) through the blocked HBM factorisation of cgp_potrf_dev,
+ * all active objects of a wave sharing each launch, each object with its own hyperparameter row: per-object fits of
+ * objects above 224 points, and joint fits of batches that hold one.
  * off_host: the CSR offsets (HOST copy); x, y, y0 (may be NULL), y_err (may be NULL): device arrays of the batch.
- * order_host (HOST, may be NULL = objects 0 .. n_obj-1) lists the n_active object ids to evaluate; hyp_obj (k x nh),
- * nugget_obj (k, may be NULL -> `nugget`), ll_obj and info (k each) are device arrays indexed by position in the list.
+ * order_host (HOST, may be NULL = objects 0 .. n_obj-1) lists the n_active object ids to evaluate; hyp_rows_host
+ * (k x nh, nh = 2 or 4) and nugget_rows_host (k, may be NULL -> `nugget`) are HOST rows, row j for order_host[j]
+ * (shared hyperparameters: one row repeated); ll_obj and info (k each) are device arrays indexed by position in the
+ * list.  The covariance function of each object is built on the host, as cgp_cov_matrix_dev builds it, so that
+ * ll_obj[j] and info[j] are bit for bit those of cgp_cov_matrix_dev + cgp_potrf_dev + cgp_large_solve_dev on that
+ * object alone (dense.LargeObject.factor), whatever the other objects of the call, their order or the wave it lands
+ * in: ll_obj = -0.5 ((|z|^2 + log det K) + n log 2 pi), NaN where info != 0 (the first failing pivot, as cgp_potrf_dev
+ * reports it); an object without points gives -0.0.
  * work: caller-owned device workspace of work_doubles doubles (16-byte aligned); an object of n points needs
  * cgp_large_ll_ws_doubles(n) of it.  Consecutive objects are packed into waves that fit; a workspace of at least
- * the sum over the active objects runs them as one wave.  ll_obj = -0.5 ((|z|^2 + log det K) + n log 2 pi), NaN where
- * info != 0 (the first failing pivot, as cgp_potrf_dev reports it).  An object's result does not depend on the other
- * objects of the call, their order or the wave it lands in.  Does not synchronise.  Returns 0, or < 0 with nothing
+ * the sum over the active objects runs them as one wave.  Does not synchronise.  Returns 0, or < 0 with nothing
  * launched (-2 for a workspace below the largest active object's need). */
 int64_t cgp_large_ll_ws_doubles(int64_t n);
-int cgp_large_ll_objhyp_dev(int64_t n_obj, const int64_t* off_host, int dim,
-                            const double* x, const double* y, const double* y0, const double* y_err,
-                            const double* hyp_obj, const double* nugget_obj, double nugget, double floor, unsigned flags,
-                            const int* order_host, int64_t n_active, double* ll_obj, int* info,
-                            double* work, int64_t work_doubles, void* stream);
-
-/* cgp_large_ll_objhyp_dev with the hyperparameters of the active objects as HOST rows: hyp_rows_host (k x nh) and
- * nugget_rows_host (k, may be NULL -> `nugget`), row j for order_host[j] (shared hyperparameters: one row repeated).
- * The covariance function of each object is built on the host, as cgp_cov_matrix_dev builds it, so that ll_obj[j] and
- * info[j] are bit for bit those of cgp_cov_matrix_dev + cgp_potrf_dev + cgp_large_solve_dev on that object alone
- * (dense.LargeObject.factor), whatever the other objects of the call, their order or the wave it lands in.  An object
- * without points gives -0.0.  Everything else (objects, order, outputs, workspace, checks) as cgp_large_ll_objhyp_dev;
- * does not synchronise. */
 int cgp_large_ll_rows_dev(int64_t n_obj, const int64_t* off_host, int dim,
                           const double* x, const double* y, const double* y0, const double* y_err,
                           const double* hyp_rows_host, const double* nugget_rows_host, double nugget, double floor,

@@ -1,5 +1,5 @@
 """Per-object fits of large objects on one GPU: one likelihood evaluation of K objects of N points through the grouped
-entry point (cgp_large_ll_objhyp_dev) against a loop of dense.LargeObject.factor, K in {1, 8, 64}, N in {300, 1000,
+entry point (cgp_large_ll_rows_dev, as DeviceBatch.ll_objhyp calls it) against a loop of dense.LargeObject.factor, K in {1, 8, 64}, N in {300, 1000,
 2000}, 1D and 2D; a whole per-object fit of 64 2D objects of 2000 points, with the time the loop would take for the
 same evaluation count; a torch.profiler kernel breakdown of one grouped evaluation at K = 64, N = 1000.
 Writes profiles/bench_large_fits_r01.json.
@@ -54,7 +54,7 @@ def grouped_call(k, n, dim, rng):
     xs, ys, ye = objects(rng, k, n, dim)
     xf, off = pack_csr(xs, dim)
     b = DeviceBatch(xf, pack_csr(ys)[0], off, y_err=pack_csr(ye)[0], dim=dim)
-    hyp = torch.tensor(np.tile(hyp_of(dim), (k, 1)), dtype=torch.float64, device=b.device)
+    hyp = np.ascontiguousarray(np.tile(hyp_of(dim), (k, 1)), dtype=np.float64)
     need = k * int(_lib.lib().cgp_large_ll_ws_doubles(n))
     work = torch.empty(need, dtype=torch.float64, device=b.device)
     ll = torch.empty(k, dtype=torch.float64, device=b.device); info = torch.empty(k, dtype=torch.int32, device=b.device)
@@ -63,10 +63,10 @@ def grouped_call(k, n, dim, rng):
     L = _lib.lib()
 
     def run():
-        _lib.check(L.cgp_large_ll_objhyp_dev(k, _lib.hptr(b.off_host), dim, b.x.data_ptr(), b.y.data_ptr(), None,
-                                             b.y_err.data_ptr(), hyp.data_ptr(), None, 0.0, 0.0, 0, order.ctypes.data, k,
-                                             ll.data_ptr(), info.data_ptr(), work.data_ptr(), need, st),
-                   "cgp_large_ll_objhyp_dev")
+        _lib.check(L.cgp_large_ll_rows_dev(k, _lib.hptr(b.off_host), dim, b.x.data_ptr(), b.y.data_ptr(), None,
+                                           b.y_err.data_ptr(), _lib.hptr(hyp), None, 0.0, 0.0, 0, order.ctypes.data, k,
+                                           ll.data_ptr(), info.data_ptr(), work.data_ptr(), need, st),
+                   "cgp_large_ll_rows_dev")
     los = [dense.LargeObject(xs[i], ys[i], ye[i], dim=dim) for i in range(k)]
 
     def loop():

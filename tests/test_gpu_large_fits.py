@@ -1,7 +1,9 @@
 """Per-object fits and predictions of objects above CGP_SMALL_MAX_N points: the grouped likelihood entry point
-cgp_large_ll_objhyp_dev (every object of a wave factored by the same launches, each with its own hyperparameters)
+cgp_large_ll_rows_dev (every object of a wave factored by the same launches, each with its own hyperparameter row)
 against the single-object path and the oracle, its group invariance, and the facade over batches that mix such
 objects with small ones."""
+from fractions import Fraction
+
 import numpy as np
 import pytest
 from scipy.optimize import fmin
@@ -42,7 +44,7 @@ def _ws(n):
 
 
 class Group:
-    """A batch on the device and direct calls of cgp_large_ll_objhyp_dev on it."""
+    """A batch on the device and direct calls of cgp_large_ll_rows_dev on it."""
 
     def __init__(self, xs, ys, dim, y_err=None, y0=None):
         import torch
@@ -63,16 +65,16 @@ class Group:
         if work_doubles is None:
             work_doubles = sum(_ws(self.b.off_host[i + 1] - self.b.off_host[i]) for i in order) or 2
         work = t.empty(int(work_doubles), dtype=t.float64, device=dev)
-        hd = t.from_numpy(np.ascontiguousarray(hyp_rows, dtype=np.float64).reshape(max(k, 1), -1)).to(dev)
-        nd = None if nug_rows is None else t.from_numpy(np.ascontiguousarray(nug_rows, dtype=np.float64)).to(dev)
+        hr = np.ascontiguousarray(hyp_rows, dtype=np.float64).reshape(max(k, 1), -1)
+        nr = None if nug_rows is None else np.ascontiguousarray(nug_rows, dtype=np.float64)
         ll = t.full((max(k, 1),), -1.0, dtype=t.float64, device=dev)
         info = t.full((max(k, 1),), -7, dtype=t.int32, device=dev)
         p = lambda v: None if v is None else v.data_ptr()
         n0 = _lib.lib().cgp_launch_count()
-        rc = _lib.lib().cgp_large_ll_objhyp_dev(self.b.n_obj, _lib.hptr(self.b.off_host), self.dim, p(self.b.x), p(self.b.y),
-                                                p(self.b.y0), p(self.b.y_err), p(hd), p(nd), float(nugget), 0.0, 0, order.ctypes.data, k,
-                                                p(ll), p(info), p(work), int(work_doubles),
-                                                t.cuda.current_stream(dev).cuda_stream)
+        rc = _lib.lib().cgp_large_ll_rows_dev(self.b.n_obj, _lib.hptr(self.b.off_host), self.dim, p(self.b.x), p(self.b.y),
+                                              p(self.b.y0), p(self.b.y_err), _lib.hptr(hr), _lib.hptr(nr), float(nugget), 0.0, 0,
+                                              order.ctypes.data, k, p(ll), p(info), p(work), int(work_doubles),
+                                              t.cuda.current_stream(dev).cuda_stream)
         self.launches = _lib.lib().cgp_launch_count() - n0
         t.cuda.synchronize()
         return rc, ll.cpu().numpy()[:k], info.cpu().numpy()[:k]
@@ -81,19 +83,29 @@ class Group:
 SIZES = (225, 255, 256, 257, 383, 384, 385, 1000, 2000)
 
 
+def _fused_det_differs(row):
+    """Whether lx^2 ly^2 - lxy^2 of a 2D row rounds differently when the first product is fused into the subtraction
+    (one rounding, as a device compiler may contract it) than with every operation rounded (the host's cov_from_hyp)."""
+    lx2, ly2, lxy2 = row[1] * row[1], row[2] * row[2], row[3] * row[3]
+    return float(Fraction(lx2) * Fraction(ly2) - Fraction(lxy2)) != lx2 * ly2 - lxy2
+
+
 @pytest.mark.parametrize("dim", [1, 2])
 @pytest.mark.parametrize("extras", [False, True])
-def test_entry_matches_single_object_path(cg, dim, extras):
-    """Every size of SIZES in one grouped call against dense.LargeObject.factor (1e-12) and the oracle (1e-9); with
-    extras: y0, y_err and per-object nuggets and hyperparameters; without: a shared nugget keeps cond(K) near 1e3."""
+def test_rows_entry_matches_single_object_path(cg, dim, extras):
+    """Every size of SIZES in one grouped call against dense.LargeObject.factor (bit for bit) and the oracle (1e-9);
+    with extras: y0, y_err and per-object nuggets and hyperparameters, in 2D with rows whose metric determinant rounds
+    differently when contracted into one FMA; without: a shared nugget keeps cond(K) near 1e3."""
     from cosmogp_b200.dense import LargeObject
     rng = np.random.default_rng(7 + dim + 10 * extras)
     objs = [_object(rng, n, dim) for n in SIZES]
     xs, ys = [o[0] for o in objs], [o[1] for o in objs]
     ye = [o[2] for o in objs] if extras else None
     y0 = [0.1 * np.cos(np.arange(len(y))) for y in ys] if extras else None
-    base = np.array(_hyp(dim))
+    base = np.array([1.1, 4.3, 3.7, 0.9] if dim == 2 and extras else _hyp(dim))
     hyp = np.array([base * (1.0 + 0.05 * i) for i in range(len(SIZES))]) if extras else np.tile(base, (len(SIZES), 1))
+    if dim == 2 and extras:
+        assert any(_fused_det_differs(h) for h in hyp)
     nug = 0.02 + 0.01 * np.arange(len(SIZES)) if extras else None
     g = Group(xs, ys, dim, y_err=ye, y0=y0)
     rc, ll, info = g.run(hyp, np.arange(len(SIZES)), nug, nugget=0.2)
@@ -101,13 +113,13 @@ def test_entry_matches_single_object_path(cg, dim, extras):
     for i, n in enumerate(SIZES):
         nu = 0.2 if nug is None else nug[i]
         lo = LargeObject(xs[i], ys[i], None if ye is None else ye[i], None if y0 is None else y0[i], dim=dim)
-        assert_close(ll[i], lo.factor(hyp[i], nu), 1e-12, 0.0, "n=%d vs LargeObject" % n)
+        np.testing.assert_array_equal(ll[i], lo.factor(hyp[i], nu), "n=%d vs LargeObject" % n)
         ref = O.log_likelihood(ys[i], xs[i], hyp[i], nu, None if ye is None else ye[i], None if y0 is None else y0[i],
                                kind="1d" if dim == 1 else "2d")
         assert_close(ll[i], ref, 1e-9, 0.0, "n=%d vs oracle" % n)
 
 
-def test_group_invariance_bitwise(cg):
+def test_rows_entry_group_invariance_bitwise(cg):
     """An object's ll is bit-identical alone, in a group of other sizes, in reversed order and across waves."""
     rng = np.random.default_rng(11)
     sizes = [1000, 300, 1000, 257, 1000, 385, 100, 2000]
@@ -135,7 +147,7 @@ def test_group_invariance_bitwise(cg):
     assert g.launches > one_wave_launches.launches            # more waves, more launch sequences
 
 
-def test_failures_stay_local(cg):
+def test_rows_entry_failures_stay_local(cg):
     """A non-positive-definite object in the middle gets info != 0 and NaN; its neighbours keep their bits.  A workspace
     below the largest object's need is refused before anything is launched; no active object returns 0."""
     from cosmogp_b200 import _lib

@@ -42,7 +42,9 @@ def test_gather_csr():
 
 def test_entry_size_limits_refused_before_any_launch():
     """Objects and grids are limited to 65408 points (padded to 128, at most the 65535 rows an auto-covariance build
-    takes); larger ones, and a too small workspace, are refused by the host checks, before any device work."""
+    takes); larger ones, and a too small workspace, are refused by the host checks, before any device work.  The shared
+    grid is checked after the alignment of the workspace and before the objects, and not at all without an active
+    object."""
     from cosmogp_b200 import build, _lib
     build.build()
     L = _lib.lib()
@@ -50,15 +52,18 @@ def test_entry_size_limits_refused_before_any_launch():
     hyp, nug = np.array([1.0, 2.0]), np.array([0.05])
     info = fake
 
-    def call(n, m_shared=None, goff=None, m=0, work_doubles=1 << 40):
+    def call(n, m_shared=None, goff=None, m=0, work_doubles=1 << 40, k=1, work=fake):
         off = np.array([0, n], dtype=np.int64)
         coff = np.array([0, m * m], dtype=np.int64)
-        return L.cgp_large_covariance_dev(1, _lib.hptr(off), 1, fake, None, _lib.hptr(hyp), _lib.hptr(nug), 0.0, 0.0, 0,
+        return L.cgp_large_covariance_dev(k, _lib.hptr(off), 1, fake, None, _lib.hptr(hyp), _lib.hptr(nug), 0.0, 0.0, 0,
                                           fake, _lib.hptr(goff), 0 if m_shared is None else m_shared, None, 1, fake,
-                                          _lib.hptr(coff), info, fake, work_doubles, None)
+                                          _lib.hptr(coff), info, work, work_doubles, None)
 
     assert call(65409) == -2 and "65408" in _lib.last_error()
     assert call(10, m_shared=65409, m=65409) == -2 and "65408" in _lib.last_error()
     assert call(10, goff=np.array([0, 65409], dtype=np.int64), m=65409) == -2 and "65408" in _lib.last_error()
     assert call(65408, m_shared=65408, m=65408, work_doubles=1) == -2 and "workspace" in _lib.last_error()
     assert call(10, m_shared=7, m=6) == -1 and "coff" in _lib.last_error()
+    assert call(10, m_shared=65409, m=65409, work=fake + 8) == -1 and "aligned" in _lib.last_error()
+    assert call(65409, m_shared=65409, m=65409) == -2 and "shared grid" in _lib.last_error()
+    assert call(10, m_shared=65409, m=65409, k=0) == 0

@@ -53,5 +53,7 @@ def test_entry_checks_before_any_launch():
     assert call(300, order=[1]) == -1 and "object id" in _lib.last_error()
     assert call(300, work=fake + 8) == -1 and "aligned" in _lib.last_error()
     assert call(300, hyp_rows=None) == -1 and "NULL" in _lib.last_error()
+    assert call(65536, dim=3, work=fake + 8) == -1 and "dim" in _lib.last_error()
+    assert call(65536, hyp_rows=None, dim=3) == -1 and "NULL" in _lib.last_error()
     assert call(300, order=[], k=0) == 0
     assert L.cgp_launch_count() == n0

@@ -20,7 +20,8 @@ def test_loo_ws_doubles_matches_the_library():
 
 def test_entry_checks_before_any_launch():
     """A bad mode, a chunk_rows that is not a positive multiple of 128, an oversized object and a short workspace are
-    refused by the host checks, before any device work; no active object launches nothing."""
+    refused by the host checks, before any device work; no active object launches nothing, but a bad mode or chunk_rows
+    is refused even then, after a negative object count."""
     from cosmogp_b200 import build, _lib
     build.build()
     L = _lib.lib()
@@ -43,4 +44,7 @@ def test_entry_checks_before_any_launch():
     assert call(300, work_doubles=need - 1) == -2 and "workspace" in _lib.last_error()
     assert L.cgp_large_loo_ws_doubles(300, 0) == 0 and L.cgp_large_loo_ws_doubles(-1, 128) == 0
     assert call(300, n_active=0) == 0
+    assert call(300, mode=2, n_active=0) == -1 and "mode" in _lib.last_error()
+    assert call(300, chunk_rows=100, n_active=0) == -1 and "chunk_rows" in _lib.last_error()
+    assert call(300, mode=2, n_active=-1) == -1 and "negative" in _lib.last_error()
     assert L.cgp_launch_count() == n0
